@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline metric of BASELINE.json: complex Msamples/s of the fused RX chain, whole box, + HBM roofline.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path (slb_rx_process_device, RX-SSB-f32 chain) over one batch of synthetic I/Q.
   N = 1: BASELINE configs[1], 1024 independent 48 kHz channels x 10 s (480 000 frames) = 1.97 GB in + 1.97 GB out per step.
@@ -11,6 +11,8 @@ A step = one pass of the hot path (slb_rx_process_device, RX-SSB-f32 chain) over
 Both are far larger than the 126 MB L2. `value` has inputs resident in HBM; `e2e` is the same batch through the host-buffer
 C-ABI call (slb_rx_process_host: pinned host memory -> H2D -> kernel -> D2H, sliced and overlapped) with the plain pinned
 cudaMemcpyAsync duplex ceiling of the same bytes measured beside it on every rank at once (`e2e.pcie_ceiling_gbs`).
+--dump-outputs DIR writes, after the timed steps, what the last of them returned (see dump_outputs), so that two builds can be
+compared output for output: the inputs and the number of calls are fixed by the arguments.
 """
 import argparse
 import json
@@ -110,6 +112,27 @@ def synth_on_gpu(torch, channels, frames, device, first_channel):
         iq += 0.01 * torch.randn(iq.shape, device=device, generator=g)
         out[c0:c1] = torch.clamp(torch.round(iq * 32768.0), -32768, 32767).to(torch.int16)
     return out
+
+
+DUMP_BYTES = 60 * 10**6        # .npy payload of one --dump-outputs run, all ranks together (under 64 MB with the headers)
+
+
+def dump_outputs(out_dir, y, rank, world):
+    """Writes a fixed sample of y (int16 [channels][frames][2], this rank's output of the last timed step) as float32
+    [n][frames][2] to out_dir/rx_out.npy (rx_out_rank<r>.npy when several ranks run): the n channels are drawn without
+    replacement by numpy's default_rng(0) from this rank's channel range and kept in ascending order, so row i is global
+    channel rank * channels_per_gpu + ch[i]; n is the most whole channels that fit this rank's share of DUMP_BYTES (at least
+    one, cut to the frames that fit)."""
+    import numpy as np
+    import torch
+    C, T, _ = y.shape
+    budget = DUMP_BYTES // world
+    n = max(1, min(C, budget // (T * 2 * 4)))
+    frames = min(T, budget // (n * 2 * 4))
+    ch = np.sort(np.random.default_rng(0).choice(C, n, replace=False))
+    sample = y[torch.from_numpy(ch).to(y.device), :frames].float().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rx_out.npy" if world == 1 else "rx_out_rank%d.npy" % rank), sample)
 
 
 def cpu_reference_run(threads, budget_s):
@@ -275,6 +298,8 @@ def run_ours(args):
     torch.cuda.profiler.stop()
     clocks = sampler.stop()
     launches = d.kernel_launches() - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, y, rank, world)
     step_ms = [evs[i].elapsed_time(evs[i + 1]) for i in range(args.steps)]
     if os.environ.get("BENCH_DEBUG"):
         print("step_ms", [round(v, 3) for v in step_ms], file=sys.stderr)
@@ -433,7 +458,12 @@ def main():
     ap.add_argument("--no-traffic", action="store_true", help="skip the ncu pass that measures the kernel's DRAM traffic")
     ap.add_argument("--traffic-probe", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--seconds", type=int, default=SECONDS, help="signal seconds per channel per step (profiling runs only; the headline uses the default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's output to DIR/rx_out.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the GPU path's output (--impl ours)")
     if args.traffic_probe:
         traffic_probe(args)
     elif args.impl == "reference":

@@ -66,8 +66,23 @@ def golden_fft_fixed(ref):
     print("cfft_fixed.npz", os.path.getsize(os.path.join(HERE, "cfft_fixed.npz")), "bytes")
 
 
+def golden_pinning():
+    """pinning.npz: what the oracle returns on the fixed inputs of the tests that compare the port with the reference
+    (test_oracle_pinning.py, test_golden.py::test_am_chain_port_vs_ref), recorded by running those tests; the ref_or_recorded
+    fixture replays it where the reference build is absent. Recorded from the reference build when it exists, else from the
+    port (the file's `source` says which), whose agreement with the reference is what those same tests check."""
+    import pytest
+    tests = os.path.dirname(HERE)
+    os.environ["SLB_RECORD_PINNING"] = os.path.join(HERE, "pinning.npz")
+    rc = pytest.main(["-q", "-p", "no:cacheprovider", os.path.join(tests, "test_oracle_pinning.py"),
+                      os.path.join(tests, "test_golden.py") + "::test_am_chain_port_vs_ref"])
+    print("pinning.npz", os.path.getsize(os.path.join(HERE, "pinning.npz")), "bytes, pytest rc", int(rc))
+
+
 def main():
     oracle_lib.build_oracles()
+    if len(sys.argv) > 1 and sys.argv[1] == "pinning":
+        return golden_pinning()
     ref = oracle_lib.Oracle("ref")
     if len(sys.argv) > 1 and sys.argv[1] == "fft_fixed":
         return golden_fft_fixed(ref)

@@ -358,6 +358,57 @@ class Oracle:
         return out.reshape(bins, hops, 2), audio.reshape(bins, hops), gain.reshape(bins, -1), st
 
 
+def _digest(name, args):
+    """Stable digest of one oracle call: routine name and every argument (arrays by dtype, shape and bytes)."""
+    import hashlib
+    h = hashlib.sha256(name.encode())
+
+    def put(a):
+        if isinstance(a, dict):
+            for k in sorted(a):
+                h.update(str(k).encode()); put(a[k])
+        elif isinstance(a, (np.ndarray, np.generic)):
+            a = np.ascontiguousarray(a); h.update(("%s%s" % (a.dtype.str, a.shape)).encode()); h.update(a.tobytes())
+        else:
+            h.update(repr(a).encode())
+    for a in args:
+        put(a)
+    return h.hexdigest()
+
+
+class Recorded:
+    """An oracle replayed from stored outputs (tests/golden/pinning.npz, make_golden.py pinning): the i-th call a test makes
+    returns what the recorded oracle returned for that test's i-th call, and fails when the arguments differ from the ones
+    recorded. With `live` set it records instead: it calls `live` and stores the results in `store`."""
+
+    def __init__(self, store, test_name, live=None):
+        self.store, self.test, self.live, self.n = store, test_name, live, 0
+        self.kind = "recorded from %s" % (live.kind if live is not None else str(store["source"]))
+
+    def __getattr__(self, name):
+        if name.startswith("_"):
+            raise AttributeError(name)
+
+        def call(*args):
+            key = "%s|%d" % (self.test, self.n); self.n += 1
+            dig = _digest(name, args)
+            if self.live is not None:
+                res = getattr(self.live, name)(*args)
+                parts = res if isinstance(res, tuple) else (res,)
+                self.store[key + "|call"] = np.array("%s %s %d" % (name, dig, len(parts) if isinstance(res, tuple) else -1))
+                for j, p in enumerate(parts):
+                    if isinstance(p, (np.ndarray, np.generic, int, float)):
+                        self.store["%s|%d" % (key, j)] = np.asarray(p)
+                return res
+            if key + "|call" not in self.store:
+                raise AssertionError("no recorded call %s (%s): re-record with tests/golden/make_golden.py pinning" % (key, name))
+            rname, rdig, n = str(self.store[key + "|call"]).split()
+            assert (rname, rdig) == (name, dig), ("inputs differ from the recorded call", key, name, rname)
+            parts = [self.store["%s|%d" % (key, j)][()] if "%s|%d" % (key, j) in self.store else None for j in range(max(int(n), 1))]
+            return tuple(parts) if int(n) >= 0 else parts[0]
+        return call
+
+
 class RefRing:
     """The UNMODIFIED reference dsp_if.c built for one sample rate (oracle/_ref/libdspif_<fs>.so)."""
 

@@ -220,8 +220,9 @@ def test_q15_chain_blocking_independence(port):
     assert np.array_equal(np.concatenate(parts), whole)
 
 
-def test_am_chain_port_vs_ref(port, ref):
+def test_am_chain_port_vs_ref(port, ref_or_recorded):
     """RX chain with the envelope detector (mode AM): the restatement against the reference build on the same input."""
+    ref = ref_or_recorded
     g = np.load(os.path.join(GOLD, "rx_ssb_f32.npz"))
     prm = rx_params(g, "usb"); prm["envelope"] = 1
     x = g["rx_usb_in"]

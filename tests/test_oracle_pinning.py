@@ -1,10 +1,16 @@
 """Pin the plain-C restatement (oracle/port) against the reference itself run here (oracle/_ref = the vendored
 CMSIS-DSP V1.5.3 sources compiled for x86, SURVEY.md §8c). The reference ships no golden vectors (SURVEY.md §4), so
-execution of its own code is the pin. Integer routines must agree bit for bit; float routines to a stated tolerance."""
+execution of its own code is the pin. Integer routines must agree bit for bit; float routines to a stated tolerance.
+Where the reference build is absent, `ref` replays the outputs recorded on these same inputs (tests/golden/pinning.npz)."""
 import numpy as np
 import pytest
 
 BLOCK = 48
+
+
+@pytest.fixture
+def ref(ref_or_recorded):
+    return ref_or_recorded
 
 
 def q15(rng, n, amp=32767):
