@@ -49,6 +49,9 @@ extern "C" {
 
 #define SLB_CHAIN_RX_SSB_Q15  4    /* all-integer phasing SSB demodulator: fir_q15 Hilbert pair -> add/sub -> q15 AGC (bit-exact) */
 
+#define SLB_CHAIN_TX_F32      5    /* all-mode transmit: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_TX_SSB_F32; AM (carrier +
+                                      envelope) and FM (integer-phase NCO) from the same band-limited mic (DESIGN.md §3.4) */
+
 #define SLB_MAX_STAGES 4
 #define SLB_MAX_MASKS  8
 
@@ -81,6 +84,16 @@ typedef struct
   uint32_t alc_block;                    /* ALC detector block [arm_cmplx_mag_f32 + arm_max_f32] = firmware block; this build: 48 */
   float    alc_target, alc_decay, alc_floor, alc_gmax;
 } slb_tx_f32_params;
+
+/* Modulator constants of SLB_CHAIN_TX_F32 (DESIGN.md §3.4). The ALC of slb_tx_f32_params measures max |Re z| per block for AM
+ * and FM and holds it at am_depth (AM) or at 2 fm_deviation_hz / fs half-turns per sample (FM); alc_target is the SSB target. */
+typedef struct
+{
+  float am_carrier;                      /* AM: I = am_carrier (1 + g Re z), Q = 0 [arm_offset_f32, arm_scale_f32]; (0, 1) */
+  float am_depth;                        /* AM: peak modulation depth the ALC holds, (0, 1]: the envelope stays in carrier (1 +- depth) */
+  float fm_deviation_hz;                 /* FM: peak deviation the ALC holds, (0, fs / 4] */
+  float fm_level;                        /* FM: I + jQ = fm_level e^(j phi) [arm_cos_f32, arm_sin_f32, arm_scale_f32]; (0, 1) */
+} slb_tx_mod_params;
 
 /* CHAN-64-f32 chain parameters (DESIGN.md §3; BASELINE config 4). The context's `channels` are WIDEBAND streams; each
  * yields `bins` narrowband channels at fs/bins. Oracle stage for each field in brackets. */
@@ -133,6 +146,10 @@ int slb_get_rx_f32_params (const slb_ctx *ctx, slb_rx_f32_params *p);
 int slb_default_tx_f32_params (uint32_t fs, slb_tx_f32_params *out);
 int slb_set_tx_f32_params (slb_ctx *ctx, const slb_tx_f32_params *p);
 int slb_get_tx_f32_params (const slb_ctx *ctx, slb_tx_f32_params *p);
+/* AM / FM modulator constants (SLB_CHAIN_TX_F32 contexts only; defaults: carrier 0.5, depth 0.8, deviation 2500 Hz, level 0.5) */
+int slb_default_tx_mod_params (uint32_t fs, slb_tx_mod_params *out);
+int slb_set_tx_mod_params (slb_ctx *ctx, const slb_tx_mod_params *p);
+int slb_get_tx_mod_params (const slb_ctx *ctx, slb_tx_mod_params *p);
 int slb_default_rx_q15_params (uint32_t fs, slb_rx_q15_params *out);
 int slb_set_rx_q15_params (slb_ctx *ctx, const slb_rx_q15_params *p);
 int slb_get_rx_q15_params (const slb_ctx *ctx, slb_rx_q15_params *p);
@@ -189,7 +206,7 @@ int slb_ring_get_iq (slb_ctx *ctx, int which, int16_t *i, int16_t *q);
  * *_host: host pointers; stages through pinned memory with chunked H2D / kernel / D2H overlap, synchronous. */
 int slb_rx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream);
 int slb_rx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames);
-/* TX direction (context created with SLB_CHAIN_TX_SSB_F32): in = mic frames (L = R as the codec delivers them in TX,
+/* TX direction (context created with SLB_CHAIN_TX_SSB_F32 or SLB_CHAIN_TX_F32): in = mic frames (L = R as the codec delivers them in TX,
  * Core/Src/codec_if.c:304-306; L is used), out = modulated I/Q frames. Same shapes and rules as the RX calls. With this
  * chain SLB_DSP_In_Buff_Write runs the modulator at the 1 ms cadence exactly as it runs the demodulator for RX. */
 int slb_tx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream);
@@ -208,6 +225,9 @@ int slb_chan_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, ui
  * are written by the next slb_rx_process_device call(s) when non-NULL (device pointers). TX chain: d_audio receives
  * the pre-ALC complex baseband [channels][frames][2] f32. */
 int slb_rx_set_debug_taps (slb_ctx *ctx, float *d_audio, float *d_gain);
+/* SLB_CHAIN_TX_F32: the FM phase accumulator phi[n] (uint32, units of 2^-32 turn) after each sample, [channels][frames], device
+ * pointer, written by the next slb_tx_process_device call(s) for FM channels when non-NULL (other channels' rows are left alone) */
+int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase);
 /* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48] */
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain);
 
@@ -357,7 +377,7 @@ int slb_sync (slb_ctx *ctx);
 
 /* ---- single-channel drop-in with the firmware's own names and signatures (Core/Inc/dsp_if.h:42-51).
  * They drive one process-global 1-channel context on device 0 (env SELENITE_B200_DEVICE, SELENITE_B200_FS,
- * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|rx_ssb_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
+ * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
  * they return void; failures are reported through slb_dropin_status(). ---- */
 void DSP_Init (void);
 void DSP_Set_RX (void);

@@ -24,6 +24,10 @@ class TxF32Params(C.Structure):
                 ("alc_target", C.c_float), ("alc_decay", C.c_float), ("alc_floor", C.c_float), ("alc_gmax", C.c_float)]
 
 
+class TxModParams(C.Structure):
+    _fields_ = [("am_carrier", C.c_float), ("am_depth", C.c_float), ("fm_deviation_hz", C.c_float), ("fm_level", C.c_float)]
+
+
 class RxQ15Params(C.Structure):
     _fields_ = [("ntaps", C.c_uint32), ("agc_block", C.c_uint32), ("agc_window", C.c_uint32),
                 ("taps_i", C.c_int16 * 64), ("taps_q", C.c_int16 * 64), ("rel", C.c_int16 * 32),

@@ -33,6 +33,7 @@ struct slb_ctx
   // chain configuration
   slb_rx_f32_params rx{};
   slb_tx_f32_params tx{};
+  slb_tx_mod_params tx_mod{};          // SLB_CHAIN_TX_F32: AM / FM modulator constants
   BiquadScanTables tables{};
   std::vector<float> masks_host;       // [SLB_MAX_MASKS][2*fft_len], unscaled, as set
   std::vector<uint8_t> slot_host;      // [C]
@@ -55,7 +56,7 @@ struct slb_ctx
   int16_t *d_ovl[2] = { nullptr, nullptr }; int ovl_parity = 0;
   float *d_state = nullptr; unsigned *d_flag = nullptr;
   unsigned flag_base = 0;
-  float *dbg_audio = nullptr, *dbg_gain = nullptr;
+  float *dbg_audio = nullptr, *dbg_gain = nullptr; uint32_t *dbg_phase = nullptr;
 
   // device: firmware rings (de-interleaved planes) + per-call block staging
   RingPtrs ring_in, ring_out;
@@ -91,7 +92,9 @@ struct slb_ctx
     }                                                                                              \
   } while (0)
 
-static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || chain == SLB_CHAIN_TX_SSB_F32; }
+// the two transmit chains share everything but the modes they accept (check_mode): kernels, state, ring handling
+static inline bool is_tx_chain (uint32_t chain) { return chain == SLB_CHAIN_TX_SSB_F32 || chain == SLB_CHAIN_TX_F32; }
+static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || is_tx_chain (chain); }
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
 
@@ -143,7 +146,7 @@ static int upload_chain_constants (slb_ctx *ctx)
   // caller-supplied one may not) and the AM slot (two outputs per sample) stay on the FFT kernel
   {
     std::vector<uint8_t> planes ((size_t) SLB_MAX_MASKS * kTcPlaneBytes, 0);
-    if (ctx->cfg.chain == SLB_CHAIN_TX_SSB_F32)
+    if (is_tx_chain (ctx->cfg.chain))
     {
       std::vector<uint8_t> txp ((size_t) SLB_MAX_MASKS * kTcTxPlaneBytes, 0);
       for (int m = 0; m < SLB_MAX_MASKS; m++)
@@ -168,7 +171,7 @@ static int upload_chain_constants (slb_ctx *ctx)
       CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kFmMaskSlot * kTcAmPlaneBytes, amp.data (), amp.size (), cudaMemcpyHostToDevice, ctx->stream));
       CK (ctx, cudaStreamSynchronize (ctx->stream));
     }
-    if (ctx->cfg.chain != SLB_CHAIN_TX_SSB_F32)
+    if (!is_tx_chain (ctx->cfg.chain))
     for (int m = 0; m < SLB_MAX_MASKS; m++)
       if (m < kAmMaskSlot) ctx->tc_ok[m] = N == 512 && tc_build_planes (ctx->masks_host.data () + (size_t) m * 2 * N, ctx->rx.biquad, planes.data () + (size_t) m * kTcPlaneBytes, &ctx->tc_s0[m], &ctx->tc_sz[m]);
     CK (ctx, cudaMemcpyAsync (ctx->d_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice, ctx->stream));
@@ -206,6 +209,7 @@ uint64_t slb_kernel_launches (const slb_ctx *ctx) { return ctx ? ctx->launches :
 
 int slb_default_rx_f32_params (uint32_t fs, slb_rx_f32_params *out) { return design_default_rx_f32 (fs, out); }
 int slb_default_tx_f32_params (uint32_t fs, slb_tx_f32_params *out) { return design_default_tx_f32 (fs, out); }
+int slb_default_tx_mod_params (uint32_t fs, slb_tx_mod_params *out) { return design_default_tx_mod (fs, out); }
 int slb_default_mask (uint32_t fs, uint32_t fft_len, uint8_t mode, float *mask_out) { return design_default_mask (fs, fft_len, mode, mask_out); }
 
 int slb_create (const slb_config *cfg, slb_ctx **out)
@@ -229,6 +233,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   // decay with fs in design_default_*): 1 ms at 48 kHz, half a firmware block at 96 kHz, a quarter at 192 kHz
   design_default_rx_f32 (cfg->fs, &ctx->rx);
   design_default_tx_f32 (cfg->fs, &ctx->tx);
+  design_default_tx_mod (cfg->fs, &ctx->tx_mod);
   const uint32_t C = cfg->channels, N = ctx->rx.fft_len, hop = ctx->rx.hop, ovl = N - hop, R = ctx->geo.ring_frames;
 
   ctx->masks_host.assign ((size_t) SLB_MAX_MASKS * 2 * N, 0.0f);
@@ -245,6 +250,8 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   CKC (cudaMalloc (&ctx->d_am_planes, (size_t) SLB_MAX_MASKS * kTcAmPlaneBytes));
   CKC (cudaMalloc (&ctx->d_slot, C));
   CKC (cudaMalloc (&ctx->d_twiddle, kTwiddleFloats * sizeof (float)));
+  CKC (cudaMalloc (&ctx->d_sin513, 513 * sizeof (float)));   // arm_sin_f32's table: the side-tone and the FM NCO
+  CKC (cudaMemcpy (ctx->d_sin513, host_sin_table (), 513 * sizeof (float), cudaMemcpyHostToDevice));
   for (int p = 0; p < 2; p++) CKC (cudaMalloc (&ctx->d_ovl[p], (size_t) C * ovl * 4));
   CKC (cudaMalloc (&ctx->d_state, (size_t) C * 8 * sizeof (float)));
   CKC (cudaMalloc (&ctx->d_flag, (size_t) C * sizeof (unsigned)));
@@ -328,6 +335,20 @@ int slb_set_tx_f32_params (slb_ctx *ctx, const slb_tx_f32_params *p)
 }
 int slb_get_tx_f32_params (const slb_ctx *ctx, slb_tx_f32_params *p) { if (!ctx || !p) return SLB_ERR_ARG; *p = ctx->tx; return SLB_OK; }
 
+int slb_set_tx_mod_params (slb_ctx *ctx, const slb_tx_mod_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (ctx->cfg.chain != SLB_CHAIN_TX_F32) return fail (ctx, SLB_ERR_STATE, "AM / FM modulator constants belong to SLB_CHAIN_TX_F32 contexts");
+  // carrier and level below full scale, depth at most 100 % (no overmodulation), deviation at most fs / 4 (|increment| <= a quarter turn:
+  // the q31 increment cannot saturate)
+  if (!(p->am_carrier > 0.f && p->am_carrier < 1.f) || !(p->am_depth > 0.f && p->am_depth <= 1.f) || !(p->fm_level > 0.f && p->fm_level < 1.f)
+      || !(p->fm_deviation_hz > 0.f && p->fm_deviation_hz <= 0.25f * (float) ctx->cfg.fs))
+    return fail (ctx, SLB_ERR_ARG, "modulator constants out of range (0 < carrier, level < 1; 0 < depth <= 1; 0 < deviation <= fs / 4)");
+  ctx->tx_mod = *p;
+  return SLB_OK;
+}
+int slb_get_tx_mod_params (const slb_ctx *ctx, slb_tx_mod_params *p) { if (!ctx || !p) return SLB_ERR_ARG; *p = ctx->tx_mod; return SLB_OK; }
+
 int slb_set_mask (slb_ctx *ctx, uint8_t mode, const float *mask)
 {
   if (!ctx || !mask) return SLB_ERR_ARG;
@@ -403,6 +424,13 @@ int slb_rx_set_debug_taps (slb_ctx *ctx, float *d_audio, float *d_gain)
   if (ctx->chan) chan64_set_debug (ctx->chan, d_audio, d_gain);
   return SLB_OK;
 }
+int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase)
+{
+  if (!ctx) return SLB_ERR_ARG;
+  if (ctx->cfg.chain != SLB_CHAIN_TX_F32) return fail (ctx, SLB_ERR_STATE, "the FM phase tap belongs to SLB_CHAIN_TX_F32 contexts");
+  ctx->dbg_phase = d_phase;
+  return SLB_OK;
+}
 
 // ------------------------------------------------------------------------------------------------------------------
 // Firmware API, batched
@@ -452,10 +480,9 @@ int SLB_DSP_Set_Sidetone (slb_ctx *ctx, uint32_t freq_hz, float level)
   const uint32_t C = ctx->cfg.channels, fs = ctx->cfg.fs;
   if (!ctx->d_tone)
   {
-    CK (ctx, cudaMalloc (&ctx->d_tone, (size_t) fs * 2)); CK (ctx, cudaMalloc (&ctx->d_sin513, 513 * sizeof (float)));
+    CK (ctx, cudaMalloc (&ctx->d_tone, (size_t) fs * 2));
     CK (ctx, cudaMalloc (&ctx->d_key, C)); CK (ctx, cudaMalloc (&ctx->d_tone_cnt, (size_t) C * 4));
     CK (ctx, cudaMemset (ctx->d_key, 0, C)); CK (ctx, cudaMemset (ctx->d_tone_cnt, 0, (size_t) C * 4));
-    CK (ctx, cudaMemcpy (ctx->d_sin513, host_sin_table (), 513 * sizeof (float), cudaMemcpyHostToDevice));
   }
   ctx->tone_hz = freq_hz; ctx->tone_level = level;
   CK (ctx, launch_tone_table (ctx->d_tone, fs, level, ctx->d_sin513, ctx->stream));
@@ -482,10 +509,10 @@ int SLB_DSP_Key (slb_ctx *ctx, const uint8_t *key_down)
 static int check_mode (slb_ctx *ctx, uint8_t mode)
 {
   if (mode_to_mask_slot (mode) < 0) return fail (ctx, SLB_ERR_UNSUPPORTED, "not an FT-817 mode byte (LSB, USB, CW, CW-R, AM, FM, DIG, PKT are served; rxtx_if.h:33-43)");
-  if (mode == SLB_MODE_AM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 chain (envelope detector) and the channelizer only");
-  if (mode == SLB_MODE_FM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 chain (limiter-discriminator) only");
+  if (mode == SLB_MODE_AM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 chain (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only");
+  if (mode == SLB_MODE_FM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 chain (limiter-discriminator) and the TX-f32 chain (FM modulator) only");
   if (mode == SLB_MODE_FM && ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 && !ctx->tc_ok[kFmMaskSlot])
     return fail (ctx, SLB_ERR_UNSUPPORTED, "the FM slot has no tensor-core planes (fft_len must be 512 and the FM mask a 129-tap FIR)");
   return SLB_OK;
@@ -536,7 +563,7 @@ int SLB_DSP_Set_Mode (slb_ctx *ctx, uint8_t mode)     // dsp_if.c:367-370 is the
 
 // The FFT kernel over the contiguous channel range [ch0, ch0 + nch)
 static int run_rx_fft_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
-                              float *dbg_audio, float *dbg_gain, cudaStream_t stream)
+                              float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase = nullptr)
 {
   const uint32_t ovl = ctx->rx.fft_len - ctx->rx.hop;
   RxF32Launch L{};
@@ -545,7 +572,15 @@ static int run_rx_fft_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out,
   L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
   L.masks = ctx->d_masks; L.mask_slot = ctx->d_slot + ch0; L.twiddle = ctx->d_twiddle;
   L.flag_base = ctx->flag_base; L.channels = nch; L.frames = frames;
-  L.tx = ctx->cfg.chain == SLB_CHAIN_TX_SSB_F32;
+  L.tx = is_tx_chain (ctx->cfg.chain);
+  L.tx_mod = ctx->cfg.chain == SLB_CHAIN_TX_F32;
+  if (L.tx_mod)
+  {
+    const slb_tx_mod_params &m = ctx->tx_mod;
+    L.am_depth = m.am_depth; L.am_carrier = m.am_carrier; L.fm_level = m.fm_level;
+    L.fm_target = 2.0f * m.fm_deviation_hz / (float) ctx->cfg.fs;                 // half-turns per sample (oracle: the same float expression)
+    L.phase_dbg = dbg_phase; L.sin513 = ctx->d_sin513;
+  }
   if (L.tx) { L.agc_target = ctx->tx.alc_target; L.agc_decay = ctx->tx.alc_decay; L.agc_floor = ctx->tx.alc_floor; L.agc_gmax = ctx->tx.alc_gmax; }
   else { L.agc_target = ctx->rx.agc_target; L.agc_decay = ctx->rx.agc_decay; L.agc_floor = ctx->rx.agc_floor; L.agc_gmax = ctx->rx.agc_gmax; }
   L.tables = &ctx->tables;
@@ -567,9 +602,9 @@ static bool tc_path_enabled ()
 // channel groups reproduce the whole bit for bit. AM channels, caller-supplied masks that are no FIR, and TX stay on
 // the FFT kernel (contiguous runs).
 static int run_rx_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
-                          float *dbg_audio, float *dbg_gain, cudaStream_t stream)
+                          float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase = nullptr)
 {
-  const bool is_tx = ctx->cfg.chain == SLB_CHAIN_TX_SSB_F32;
+  const bool is_tx = is_tx_chain (ctx->cfg.chain);
   if (ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && !is_tx)
     return run_rx_fft_kernel (ctx, d_in, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream);
   // slb_set_rx_path (SLB_RX_PATH_FFT) / SELENITE_B200_RX_PATH=fft keep every channel on the FFT kernel — except FM, whose
@@ -682,7 +717,8 @@ static int run_rx_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uin
     if (on_tc[i]) { i++; continue; }
     uint32_t e = i; while (e < nch && !on_tc[e]) e++;
     const int rc = run_rx_fft_kernel (ctx, d_in + (size_t) i * frames * 2, d_out + (size_t) i * frames * 2, ch0 + i, e - i, frames,
-                                      dbg_audio ? dbg_audio + (size_t) i * frames * (is_tx ? 2 : 1) : nullptr, dbg_gain ? dbg_gain + (size_t) i * (frames / kAgcBlock) : nullptr, stream);
+                                      dbg_audio ? dbg_audio + (size_t) i * frames * (is_tx ? 2 : 1) : nullptr, dbg_gain ? dbg_gain + (size_t) i * (frames / kAgcBlock) : nullptr, stream,
+                                      dbg_phase ? dbg_phase + (size_t) i * frames : nullptr);
     if (rc) return rc;
     i = e;
   }
@@ -1302,7 +1338,7 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
 {
   if (!ctx || !d_in || !d_out || frames == 0) return SLB_ERR_ARG;
   if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
-  if (want_tx != (ctx->cfg.chain == SLB_CHAIN_TX_SSB_F32)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
+  if (want_tx != is_tx_chain (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   if (ctx->cfg.chain == SLB_CHAIN_PASS)
   {
@@ -1318,7 +1354,7 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
     return SLB_OK;
   }
   if (frames % ctx->rx.hop != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the hop (384)");
-  int rc = run_rx_kernel (ctx, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->dbg_audio, ctx->dbg_gain, (cudaStream_t) stream);
+  int rc = run_rx_kernel (ctx, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->dbg_audio, ctx->dbg_gain, (cudaStream_t) stream, ctx->dbg_phase);
   if (rc) return rc;
   rx_advance (ctx, frames);
   return SLB_OK;
@@ -1412,7 +1448,7 @@ static int process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint
 {
   if (!ctx || !h_in || !h_out || frames == 0) return SLB_ERR_ARG;
   if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
-  if (want_tx != (ctx->cfg.chain == SLB_CHAIN_TX_SSB_F32)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
+  if (want_tx != is_tx_chain (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   const bool chain = is_ssb_chain (ctx->cfg.chain);
   if (chain && frames % ctx->rx.hop != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the hop (384)");
@@ -1640,6 +1676,7 @@ slb_ctx *dropin ()
     cfg.fs = fs ? (uint32_t) std::atoi (fs) : 48000u;
     cfg.device = dev ? std::atoi (dev) : 0;
     cfg.chain = (ch && std::strcmp (ch, "rx_ssb_f32") == 0) ? SLB_CHAIN_RX_SSB_F32 : (ch && std::strcmp (ch, "tx_ssb_f32") == 0) ? SLB_CHAIN_TX_SSB_F32
+              : (ch && std::strcmp (ch, "tx_f32") == 0) ? SLB_CHAIN_TX_F32
               : (ch && std::strcmp (ch, "rx_ssb_q15") == 0) ? SLB_CHAIN_RX_SSB_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
     g_dropin_status = slb_create (&cfg, &g_dropin);
     if (g_dropin_status != SLB_OK) std::fprintf (stderr, "selenite-b200: drop-in context failed: %s\n", slb_last_error (nullptr));

@@ -51,6 +51,15 @@ int design_default_tx_f32 (uint32_t fs, slb_tx_f32_params *p)
   return SLB_OK;
 }
 
+// TX AM / FM (SLB_CHAIN_TX_F32): the carrier at -6 dBFS leaves 80 % peak modulation room below full scale (0.5 * 1.8 = 0.9); 2.5 kHz peak
+// deviation is narrow-band FM on a 6 kHz audio band (Carson: 2 (2.5 + 3) = 11 kHz); the FM level matches the SSB ALC target.
+int design_default_tx_mod (uint32_t fs, slb_tx_mod_params *p)
+{
+  if (!p || (fs != 48000u && fs != 96000u && fs != 192000u)) return SLB_ERR_ARG;
+  p->am_carrier = 0.5f; p->am_depth = 0.8f; p->fm_deviation_hz = 2500.0f; p->fm_level = 0.5f;
+  return SLB_OK;
+}
+
 int mode_to_mask_slot (uint8_t mode)
 {
   switch (mode)

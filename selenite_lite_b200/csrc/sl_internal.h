@@ -41,6 +41,7 @@ struct RingPtrs
 // ---------------------------------------------------------------------------------------------------------
 int design_default_rx_f32 (uint32_t fs, slb_rx_f32_params *out);
 int design_default_tx_f32 (uint32_t fs, slb_tx_f32_params *out);
+int design_default_tx_mod (uint32_t fs, slb_tx_mod_params *out);
 int design_default_mask (uint32_t fs, uint32_t fft_len, uint8_t mode, float *mask_out);
 int mode_to_mask_slot (uint8_t mode);   // -1 for a byte that is no FT-817 mode
 constexpr int kAmMaskSlot = 6;          // channels on this slot use the envelope detector (arm_cmplx_mag_f32) instead of Re
@@ -111,6 +112,13 @@ struct RxF32Launch
   float agc_target, agc_decay, agc_floor, agc_gmax;
   const BiquadScanTables *tables;          // host pointer, copied into the kernel parameter block
   bool tx;                                 // TX-SSB-f32: mic (L) in, I/Q out through the ALC; audio_dbg is then [C][T][2]
+  // TX-f32 (all modes): channels on the AM / FM slots run the modulators of DESIGN.md §3.4 instead of the SSB ALC; the FM phase
+  // accumulator is carried in state[c][5] (uint32 bits)
+  bool tx_mod;
+  float am_depth, am_carrier;              // AM: ALC target, carrier level
+  float fm_target, fm_level;               // FM: ALC target 2 deviation / fs (half-turns per sample), output level
+  uint32_t *phase_dbg;                     // optional [C][T]: phi[n] of FM channels
+  const float *sin513;                     // device, arm_sin_f32's 513-entry table (host_sin_table)
 };
 int launch_rx_ssb_f32 (const RxF32Launch &L, int sm_count, void *stream);
 uint32_t rx_ssb_f32_launches_per_call ();

@@ -64,7 +64,7 @@ constexpr int kRawBufs = SL_RX_RAWBUFS;          // raw staging: filled by bulk 
 
 // dynamic shared memory layout (bytes). RX keeps three audio tiles in flight so that the FFT warps and the recurrence
 // warp only meet when one side is a whole tile late; the TX tile is twice as large (complex) and stays double-buffered.
-template <bool kTx> struct Smem
+template <bool kTx, bool kMod = false> struct Smem
 {
   static constexpr int kAudioBufs = kTx ? 2 : SL_RX_AUDIOBUFS;
   static constexpr int kAudioWords = kBlocksPerTile * (kTx ? kTxBlkStride : kBlkStride);
@@ -73,7 +73,8 @@ template <bool kTx> struct Smem
   static constexpr size_t raw = audio + (size_t) kAudioBufs * kAudioWords * 4;
   static constexpr size_t tw = raw + (size_t) kRawBufs * kRawWords * 4;
   static constexpr size_t bars = tw + 6 * 32 * 16;
-  static constexpr size_t bytes = bars + (2 * kRawBufs + 2 * kAudioBufs) * 8;
+  static constexpr size_t sin = bars + (2 * kRawBufs + 2 * kAudioBufs) * 8;
+  static constexpr size_t bytes = sin + (kMod ? 516 * 4 : 0);   // TX all-mode: arm_sin_f32's 513-entry table
 };
 
 // shared-memory index of FFT point i inside a plane. The LSU data pipe is the busiest unit of this kernel (ncu:
@@ -137,6 +138,9 @@ struct KParams
   uint32_t channels, frames, tiles_per_channel, items_per_channel;
   float agc_target, agc_decay, agc_floor, agc_gmax;
   BiquadScanTables tab;
+  float am_depth, am_carrier15, fm_target, fm_level15;   // TX all-mode (x15: the final x32768 of arm_float_to_q15 folded in)
+  uint32_t *phase_dbg;
+  const float *sin513;
 };
 
 __device__ __forceinline__ unsigned ld_acquire (const unsigned *p)
@@ -181,6 +185,38 @@ __device__ __forceinline__ uint32_t pack_iq (float i_times_32768, float q_times_
   asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(a) : "f"(i_times_32768));
   asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(b) : "f"(q_times_32768));
   return (uint32_t) (uint16_t) a | ((uint32_t) (uint16_t) b << 16);              // interleaved I,Q as on the I2S bus (main.c:333-341)
+}
+
+// arm_float_to_q31.c (V1.5.3, ARM_MATH_ROUNDING not defined): clip_q63_to_q31 ((q63_t) (x * 2147483648.0f)). The product is exact
+// (power of two); F2I.S32.TRUNC.SAT truncates toward zero and saturates like the cast + clip for every finite x
+__device__ __forceinline__ int32_t f2q31 (float x)
+{
+  int32_t v;
+  asm ("cvt.rzi.sat.s32.f32 %0, %1;" : "=r"(v) : "f"(x * 2147483648.0f));
+  return v;
+}
+// arm_sin_f32.c:72-119 / arm_cos_f32.c, op for op (sl_stages.cu OpSinCosF32): table lookup + linear interpolation
+__device__ __forceinline__ float arm_sincos (float v, const float *tab, bool is_cos)
+{
+  float in; int n;
+  if (!is_cos)
+  {
+    if (v < 0.0f && v >= -1.9e-7f) return v;
+    in = __fmul_rn (v, 0.159154943092f); n = (int) in; if (v < 0.0f) n--;
+  }
+  else { in = __fadd_rn (__fmul_rn (v, 0.159154943092f), 0.25f); n = (int) in; if (in < 0.0f) n--; }
+  in = __fsub_rn (in, (float) n);
+  const float findex = __fmul_rn (512.0f, in);
+  const unsigned idx = ((unsigned) (uint16_t) (int) findex) & 0x1ffu;
+  const float fract = __fsub_rn (findex, (float) idx);
+  return __fadd_rn (__fmul_rn (__fsub_rn (1.0f, fract), tab[idx]), __fmul_rn (fract, tab[idx + 1]));
+}
+// FM NCO of one sample (oracle tx_fm_nco): arm_q31_to_float ((int32) phi) -> arm_scale_f32 (pi) -> arm_cos_f32 / arm_sin_f32 ->
+// arm_scale_f32 (level) -> arm_float_to_q15. The 1/2^31 of arm_q31_to_float and the x32768 are powers of two, folded into the constants.
+__device__ __forceinline__ uint32_t fm_nco (uint32_t phi, const float *tab, float level15)
+{
+  const float x = __fmul_rn (__int2float_rn ((int) phi), 3.14159265f / 2147483648.0f);
+  return pack_iq (__fmul_rn (arm_sincos (x, tab, true), level15), __fmul_rn (arm_sincos (x, tab, false), level15));
 }
 
 // ---- bulk asynchronous copy (TMA engine, SASS UBLKCP) + mbarrier: raw tiles are staged global -> shared without
@@ -371,7 +407,9 @@ __device__ __forceinline__ void fft512x2 (u64 *xr, u64 *xi, float *sre, const fl
 // kTx = true : TX-SSB-f32 (mic audio = L of the L = R frames in, complex I/Q out through the ALC): same overlap-save
 //              filter with the mode's one-sided mask acting as band-pass + Hilbert pair, no biquad; the post warp measures
 //              |I + jQ| per firmware block (arm_cmplx_mag_f32 + arm_max_f32) and applies the same gain law.
-template <bool kTx>
+// kMod (TX only, SLB_CHAIN_TX_F32): channels on the AM and FM slots are modulated as DESIGN.md §3.4 describes; the other slots run the
+//              TX-SSB code unchanged.
+template <bool kTx, bool kMod = false>
 #ifdef SL_RX_MAXNREG
 __global__ void __maxnreg__ (SL_RX_MAXNREG) ssb_f32_kernel
 #else
@@ -379,7 +417,7 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
 #endif
  (const __grid_constant__ KParams P)
 {
-  typedef Smem<kTx> S;
+  typedef Smem<kTx, kMod> S;
   constexpr int kAB = S::kAudioBufs;
   extern __shared__ __align__ (128) unsigned char smem[];
   float *sScratch = reinterpret_cast<float *> (smem + S::scratch);
@@ -399,6 +437,9 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
   const int hw_warp = tid >> 5, rec_warp = (blockIdx.x + blockIdx.x / 148u) % (kFftWarps + 1);
   const int warp = (hw_warp == rec_warp) ? kFftWarps : (hw_warp < rec_warp ? hw_warp : hw_warp - 1);
   for (int i = tid; i < 6 * 32; i += kThreads) sTw[i] = P.twiddle[i];
+  float *sSin = reinterpret_cast<float *> (smem + S::sin);
+  if constexpr (kMod)
+    for (int i = tid; i < 513; i += kThreads) sSin[i] = P.sin513[i];
   if (tid == 0)
   {
 #pragma unroll
@@ -550,23 +591,40 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
     // ===================================== TX post warp: ALC =====================================
     // Lane l owns firmware block l of the tile (48 complex samples = 192 output bytes). Pass 1 finds the block peak of
     // |I + jQ|, the envelope walk is the AGC's, pass 2 re-reads the tile, scales, packs and stores.
+    // kMod, AM / FM channels: the peak is max |Re z| (arm_abs_f32 + arm_max_f32) and pass 2 runs the modulator of the channel's slot.
     const float decay = P.agc_decay;
     float env = 0.f;
+    uint32_t phase = 0;                                                            // FM phase accumulator (kMod), carried like env
     TileIter it; it.start (P);
     for (; it.valid (); it.next (P), tile_seq++)
     {
       const uint32_t c = it.c, t0 = it.t0 ();
       const int nblk = it.hops (P) * (kHop / kAgcBlock);
       const float4 *blk = reinterpret_cast<const float4 *> (sAudio + abuf * S::kAudioWords + lane * kTxBlkStride);
+      // 0: SSB-style, 1: AM, 2: FM (uniform across the warp: one channel per tile)
+      int mod = 0;
+      if constexpr (kMod) { const int slot = P.mask_slot[c]; mod = slot == kAmMaskSlot ? 1 : slot == kFmMaskSlot ? 2 : 0; }
       mbar_wait (aFull + abuf, ause & 1);                                          // I/Q tile is complete
       // arm_cmplx_mag_f32.c:72 : sqrt(re*re + im*im), each product rounded (no contraction in the oracle build);
       // arm_max_f32 over the block. sqrt is monotonic and correctly rounded, so max(sqrt) = sqrt(max).
       float m2 = 0.f;
-#pragma unroll
-      for (int k = 0; k < kAgcBlock / 2; k++)
+      if (mod == 0)
       {
-        const float4 v = blk[k];
-        m2 = fmaxf (m2, fmaxf (__fadd_rn (__fmul_rn (v.x, v.x), __fmul_rn (v.y, v.y)), __fadd_rn (__fmul_rn (v.z, v.z), __fmul_rn (v.w, v.w))));
+#pragma unroll
+        for (int k = 0; k < kAgcBlock / 2; k++)
+        {
+          const float4 v = blk[k];
+          m2 = fmaxf (m2, fmaxf (__fadd_rn (__fmul_rn (v.x, v.x), __fmul_rn (v.y, v.y)), __fadd_rn (__fmul_rn (v.z, v.z), __fmul_rn (v.w, v.w))));
+        }
+      }
+      else
+      {
+#pragma unroll
+        for (int k = 0; k < kAgcBlock / 2; k++)
+        {
+          const float4 v = blk[k];
+          m2 = fmaxf (m2, fmaxf (fabsf (v.x), fabsf (v.z)));
+        }
       }
       if (it.first_of_item ())
       {
@@ -579,10 +637,34 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
         }
         __syncwarp ();
         env = __ldcg (P.state + (size_t) c * 8 + 4);
+        if constexpr (kMod) phase = __ldcg (reinterpret_cast<const unsigned *> (P.state) + (size_t) c * 8 + 5);
       }
-      const float e = env_scan (__fsqrt_rn (m2), env, decay, lane);
+      const float e = env_scan (mod == 0 ? __fsqrt_rn (m2) : m2, env, decay, lane);
       env = __shfl_sync (0xffffffffu, e, nblk - 1);
-      const float g = fminf (__fdiv_rn (P.agc_target, fmaxf (e, P.agc_floor)), P.agc_gmax);
+      const float target = mod == 0 ? P.agc_target : mod == 1 ? P.am_depth : P.fm_target;
+      const float g = fminf (__fdiv_rn (target, fmaxf (e, P.agc_floor)), P.agc_gmax);
+      uint32_t phi = 0;                                                            // FM: phase before the lane's first sample
+      if (kMod && mod == 2)
+      {
+        // phi[n] = phi[n-1] + inc[n] mod 2^32 is an integer prefix sum, so it is associative: each lane sums its block's increments,
+        // a warp exclusive scan over the blocks plus the carried phase gives every block's start phase, bit for bit the sequential walk
+        uint32_t sum = 0;
+#pragma unroll
+        for (int k = 0; k < kAgcBlock / 2; k++)
+        {
+          const float4 v = blk[k];
+          sum += (uint32_t) f2q31 (__fmul_rn (v.x, g)) + (uint32_t) f2q31 (__fmul_rn (v.z, g));
+        }
+        uint32_t incl = sum;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1)
+        {
+          const uint32_t o = __shfl_up_sync (0xffffffffu, incl, d);
+          if (lane >= d) incl += o;
+        }
+        phi = phase + incl - sum;
+        phase += __shfl_sync (0xffffffffu, incl, nblk - 1);
+      }
       if (lane < nblk)
       {
         if (P.audio_dbg)
@@ -592,13 +674,47 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
           for (int k = 0; k < kAgcBlock / 2; k++) adbg[k] = blk[k];
         }
         if (P.gain_dbg) P.gain_dbg[(size_t) c * (P.frames / kAgcBlock) + t0 / kAgcBlock + lane] = g;
-        const float g15 = g * 32768.0f;                                           // arm_scale_f32 then arm_float_to_q15: exact fold
         uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0 + lane * kAgcBlock);
-#pragma unroll
-        for (int k = 0; k < kAgcBlock / 4; k++)
+        if (mod == 0)
         {
-          const float4 u = blk[2 * k], v = blk[2 * k + 1];
-          st_na (dst + k, make_uint4 (pack_iq (u.x * g15, u.y * g15), pack_iq (u.z * g15, u.w * g15), pack_iq (v.x * g15, v.y * g15), pack_iq (v.z * g15, v.w * g15)));
+          const float g15 = g * 32768.0f;                                         // arm_scale_f32 then arm_float_to_q15: exact fold
+#pragma unroll
+          for (int k = 0; k < kAgcBlock / 4; k++)
+          {
+            const float4 u = blk[2 * k], v = blk[2 * k + 1];
+            st_na (dst + k, make_uint4 (pack_iq (u.x * g15, u.y * g15), pack_iq (u.z * g15, u.w * g15), pack_iq (v.x * g15, v.y * g15), pack_iq (v.z * g15, v.w * g15)));
+          }
+        }
+        else if (kMod && mod == 1)
+        {
+          // AM: arm_scale_f32 (g) -> arm_offset_f32 (1) -> arm_scale_f32 (carrier) -> arm_float_to_q15 as I, Q = 0; each op rounded in
+          // the oracle's order (only the x32768 is folded, into the carrier)
+          const float c15 = P.am_carrier15;
+#pragma unroll
+          for (int k = 0; k < kAgcBlock / 4; k++)
+          {
+            const float4 u = blk[2 * k], v = blk[2 * k + 1];
+            st_na (dst + k, make_uint4 (pack_iq (__fmul_rn (__fadd_rn (__fmul_rn (u.x, g), 1.0f), c15), 0.f), pack_iq (__fmul_rn (__fadd_rn (__fmul_rn (u.z, g), 1.0f), c15), 0.f),
+                                        pack_iq (__fmul_rn (__fadd_rn (__fmul_rn (v.x, g), 1.0f), c15), 0.f), pack_iq (__fmul_rn (__fadd_rn (__fmul_rn (v.z, g), 1.0f), c15), 0.f)));
+          }
+        }
+        else if (kMod)
+        {
+          // FM: arm_scale_f32 (g) -> arm_float_to_q31 = the phase increment; the accumulator walks the block from its start phase
+          const float l15 = P.fm_level15;
+          uint4 *pdbg = P.phase_dbg ? reinterpret_cast<uint4 *> (P.phase_dbg + (size_t) c * P.frames + t0 + lane * kAgcBlock) : nullptr;
+#pragma unroll 2
+          for (int k = 0; k < kAgcBlock / 4; k++)
+          {
+            const float4 u = blk[2 * k], v = blk[2 * k + 1];
+            const uint32_t p0 = phi + (uint32_t) f2q31 (__fmul_rn (u.x, g));
+            const uint32_t p1 = p0 + (uint32_t) f2q31 (__fmul_rn (u.z, g));
+            const uint32_t p2 = p1 + (uint32_t) f2q31 (__fmul_rn (v.x, g));
+            const uint32_t p3 = p2 + (uint32_t) f2q31 (__fmul_rn (v.z, g));
+            phi = p3;
+            if (pdbg) pdbg[k] = make_uint4 (p0, p1, p2, p3);
+            st_na (dst + k, make_uint4 (fm_nco (p0, sSin, l15), fm_nco (p1, sSin, l15), fm_nco (p2, sSin, l15), fm_nco (p3, sSin, l15)));
+          }
         }
       }
       __syncwarp ();
@@ -607,6 +723,7 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
       if (it.last_of_item () && lane == 0)
       {
         __stcg (P.state + (size_t) c * 8 + 4, env);
+        if constexpr (kMod) __stcg (reinterpret_cast<unsigned *> (P.state) + (size_t) c * 8 + 5, phase);
         __threadfence ();
         st_release (P.flag + c, P.flag_base + it.seg () + 1u);
       }
@@ -816,12 +933,15 @@ int launch_rx_ssb_f32 (const RxF32Launch &L, int sm_count, void *stream_)
   P.tiles_per_channel = (L.frames + kTile - 1) / kTile;
   P.items_per_channel = (P.tiles_per_channel + kTilesPerItem - 1) / kTilesPerItem;
   P.agc_target = L.agc_target; P.agc_decay = L.agc_decay; P.agc_floor = L.agc_floor; P.agc_gmax = L.agc_gmax;
+  P.am_depth = L.am_depth; P.am_carrier15 = L.am_carrier * 32768.0f; P.fm_target = L.fm_target; P.fm_level15 = L.fm_level * 32768.0f;
+  P.phase_dbg = L.phase_dbg; P.sin513 = L.sin513;
   P.tab = *L.tables;
 
   // the bulk copies need 16-byte aligned sources: frames % 384 == 0 keeps every channel row and every tile start aligned
   if ((reinterpret_cast<uintptr_t> (L.in) | reinterpret_cast<uintptr_t> (L.ovl_in)) & 15u) return (int) cudaErrorMisalignedAddress;
-  const size_t smem = L.tx ? Smem<true>::bytes : Smem<false>::bytes;
-  const void *fn = L.tx ? (const void *) ssb_f32_kernel<true> : (const void *) ssb_f32_kernel<false>;
+  if (L.tx_mod && (!L.tx || !L.sin513)) return (int) cudaErrorInvalidValue;
+  const size_t smem = L.tx_mod ? Smem<true, true>::bytes : L.tx ? Smem<true>::bytes : Smem<false>::bytes;
+  const void *fn = L.tx_mod ? (const void *) ssb_f32_kernel<true, true> : L.tx ? (const void *) ssb_f32_kernel<true> : (const void *) ssb_f32_kernel<false>;
   cudaError_t e = cudaFuncSetAttribute (fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
   if (e != cudaSuccess) return (int) e;
   int per_sm = 0;
@@ -844,7 +964,8 @@ int launch_rx_ssb_f32 (const RxF32Launch &L, int sm_count, void *stream_)
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeCooperative; at[0].val.cooperative = 1;
   lc.attrs = at; lc.numAttrs = 1;
-  e = L.tx ? cudaLaunchKernelEx (&lc, ssb_f32_kernel<true>, P) : cudaLaunchKernelEx (&lc, ssb_f32_kernel<false>, P);
+  e = L.tx_mod ? cudaLaunchKernelEx (&lc, ssb_f32_kernel<true, true>, P)
+      : L.tx ? cudaLaunchKernelEx (&lc, ssb_f32_kernel<true>, P) : cudaLaunchKernelEx (&lc, ssb_f32_kernel<false>, P);
   return (int) (e != cudaSuccess ? e : cudaGetLastError ());
 }
 

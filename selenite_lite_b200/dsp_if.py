@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _lib
 
-CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15 = 0, 1, 2, 3, 4
+CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32 = 0, 1, 2, 3, 4, 5
 MODE_LSB, MODE_USB, MODE_CW, MODE_CWR, MODE_AM, MODE_FM, MODE_DIG, MODE_PKT = 0x00, 0x01, 0x02, 0x03, 0x04, 0x08, 0x0A, 0x0C
 RX_PATH_AUTO, RX_PATH_FFT = 0, 1
 
@@ -38,6 +38,21 @@ def default_tx_f32_params(fs=48000):
 def tx_params_to_dict(p, mask):
     return dict(fft_len=p.fft_len, hop=p.hop, alc_block=p.alc_block, alc_target=p.alc_target, alc_decay=p.alc_decay,
                 alc_floor=p.alc_floor, alc_gmax=p.alc_gmax, mask=mask)
+
+
+def default_tx_mod_params(fs=48000):
+    p = _lib.TxModParams()
+    rc = _lib.load().slb_default_tx_mod_params(fs, C.byref(p))
+    if rc:
+        raise SeleniteError("slb_default_tx_mod_params -> %d" % rc)
+    return p
+
+
+def tx_mod_params_to_dict(tx, mod, mask, fs, mode):
+    """The AM / FM transmit chain as plain data (the oracle's tx_mod_f32 parameters): `tx` the ALC, `mod` the modulator constants."""
+    return dict(fft_len=tx.fft_len, hop=tx.hop, alc_block=tx.alc_block, fs=fs, alc_decay=tx.alc_decay, alc_floor=tx.alc_floor,
+                alc_gmax=tx.alc_gmax, mask=mask, modulator=1 if mode == MODE_AM else 2, am_carrier=mod.am_carrier,
+                am_depth=mod.am_depth, fm_deviation_hz=mod.fm_deviation_hz, fm_level=mod.fm_level)
 
 
 def default_chan_params(fs=192000):
@@ -300,6 +315,20 @@ class DspIf:
 
     def set_tx_params(self, p): self._ck(self.lib.slb_set_tx_f32_params(self.h, C.byref(p)), "set_tx_f32_params")
 
+    def tx_mod_params(self):
+        """AM / FM modulator constants of a CHAIN_TX_F32 context."""
+        p = _lib.TxModParams()
+        self._ck(self.lib.slb_get_tx_mod_params(self.h, C.byref(p)), "get_tx_mod_params")
+        return p
+
+    def set_tx_mod_params(self, p): self._ck(self.lib.slb_set_tx_mod_params(self.h, C.byref(p)), "set_tx_mod_params")
+
+    def set_phase_tap(self, phase=None):
+        """CHAIN_TX_F32: phase = torch CUDA int32/uint32 [channels][frames] receiving the FM phase accumulator (2^-32 turn) after each
+        sample of FM channels on the next tx_process calls (None switches the tap off)."""
+        self._keep_phase = phase
+        self._ck(self.lib.slb_tx_set_phase_tap(self.h, phase.data_ptr() if phase is not None else None), "tx_set_phase_tap")
+
     def chan_params(self):
         p = _lib.ChanParams()
         self._ck(self.lib.slb_get_chan_params(self.h, C.byref(p)), "get_chan_params")
@@ -325,7 +354,9 @@ class DspIf:
             return q15_params_to_dict(self.rx_q15_params(), lsb=mode in (MODE_LSB, MODE_CWR))
         if self.chain == CHAIN_CHAN64_F32:
             return chan_params_to_dict(self.chan_params())
-        if self.chain == CHAIN_TX_SSB_F32:
+        if self.chain == CHAIN_TX_F32 and mode in (MODE_AM, MODE_FM):
+            return tx_mod_params_to_dict(self.tx_params(), self.tx_mod_params(), self.mask(mode), self.fs, mode)
+        if self.chain in (CHAIN_TX_SSB_F32, CHAIN_TX_F32):
             return tx_params_to_dict(self.tx_params(), self.mask(mode))
         prm = params_to_dict(self.rx_params(), self.mask(mode))
         prm["envelope"] = 1 if mode == MODE_AM else 2 if mode == MODE_FM else 0   # the oracle chain's detector: Re, |z| (AM), limiter-discriminator (FM)
@@ -350,7 +381,7 @@ class DspIf:
         return out
 
     def tx_process(self, x, out=None, stream=None):
-        """TX direction (context created with CHAIN_TX_SSB_F32): mic frames (L = R) in, modulated I/Q frames out."""
+        """TX direction (context created with CHAIN_TX_SSB_F32 or CHAIN_TX_F32): mic frames (L = R) in, modulated I/Q frames out."""
         return self.rx_process(x, out, stream, _dir="tx")
 
     def chan_process(self, x, out=None, stream=None):
