@@ -231,6 +231,21 @@ int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase);
 /* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48] */
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain);
 
+/* ---- per-channel tuning within the I/Q band (DESIGN.md §3.5): SLB_CHAIN_RX_SSB_F32, SLB_CHAIN_TX_SSB_F32, SLB_CHAIN_TX_F32 ----
+ * A channel with offset f != 0 has its int16 I/Q mixed by a table NCO: in front of the RX chain (the chain then demodulates what sits
+ * at +f Hz of the channel's input) and behind the TX chain (the signal leaves at +f Hz), so one offset pairs a TX and an RX context.
+ * The NCO increment is inc = llround (f 2^32 / fs) (2^-32 turn per sample, computed in double); the realized offset is inc fs / 2^32,
+ * and an offset is refused (SLB_ERR_ARG) unless |inc| <= 2^31 - 1, i.e. |f| < fs / 2. A rotated component that exceeds full scale
+ * (|z| > 1) saturates. The phase is carried per channel in the context's state (a retune keeps it: phase-continuous), is zeroed by a
+ * direction switch and SLB_DSP_Init, and is part of the checkpoint; the offsets are configuration that a direction switch keeps and
+ * that the caller sets again on a context restored with slb_state_load, like chain parameters and masks. Calls and pushes issued
+ * before a setter returns use the old offsets, those issued after it the new ones. A channel with offset 0 is passed unchanged and costs
+ * nothing; its phase is kept (not advanced) until it is tuned again.
+ * Other chains refuse with SLB_ERR_UNSUPPORTED. */
+int slb_set_tune (slb_ctx *ctx, const double *offset_hz);                              /* host [channels] in Hz; NULL = all 0 */
+int slb_set_tune_channel (slb_ctx *ctx, uint32_t ch, double offset_hz);
+int slb_get_tune_channel (const slb_ctx *ctx, uint32_t ch, int32_t *inc, double *realized_hz);   /* either output may be NULL */
+
 /* ---- carried state = the checkpoint (SURVEY.md §5): overlap tail, biquad d1/d2, AGC envelope, ring ---- */
 int slb_state_size (const slb_ctx *ctx, size_t *bytes);
 int slb_state_save (slb_ctx *ctx, void *host_buf, size_t bytes);

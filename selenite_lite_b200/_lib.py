@@ -49,7 +49,8 @@ class ChanParams(C.Structure):
 # binding cannot drift from the ABI
 _P = C.c_void_p
 _SCALARS = {"int": C.c_int, "int8_t": C.c_int8, "uint8_t": C.c_uint8, "int16_t": C.c_int16, "uint16_t": C.c_uint16,
-            "int32_t": C.c_int32, "uint32_t": C.c_uint32, "uint64_t": C.c_uint64, "size_t": C.c_size_t, "float": C.c_float}
+            "int32_t": C.c_int32, "uint32_t": C.c_uint32, "uint64_t": C.c_uint64, "size_t": C.c_size_t, "float": C.c_float,
+            "double": C.c_double}
 HEADER = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "include", "selenite_b200.h")
 
 

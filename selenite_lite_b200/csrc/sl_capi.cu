@@ -53,6 +53,12 @@ struct slb_ctx
   struct TcLists { uint32_t *d = nullptr; size_t cap = 0; uint32_t groups = 0, groups_ssb = 0, n_chan = 0, n_pairs = 0; uint64_t version = ~0ull; std::vector<uint8_t> on_tc; };
   std::map<uint64_t, TcLists> tc_lists; uint64_t mode_version = 0;
   bool force_fft = false;              // slb_set_rx_path (SLB_RX_PATH_FFT)
+  // per-channel tuning (slb_set_tune, DESIGN.md §3.5): NCO increments (2^-32 turn per sample), empty until a non-zero offset is set;
+  // the list {row, inc} of a channel range (tuned rows, then the untuned ones with inc = 0) is cached per range like tc_lists and
+  // rebuilt when an offset changes (tune_version)
+  std::vector<int32_t> tune_inc; uint32_t n_tuned = 0;
+  struct TuneList { uint32_t *d = nullptr; size_t cap = 0; uint32_t n = 0, n_all = 0; uint64_t version = ~0ull; };
+  std::map<uint64_t, TuneList> tune_lists; uint64_t tune_version = 0;
   int16_t *d_ovl[2] = { nullptr, nullptr }; int ovl_parity = 0;
   float *d_state = nullptr; unsigned *d_flag = nullptr;
   unsigned flag_base = 0;
@@ -284,6 +290,7 @@ void slb_destroy (slb_ctx *ctx)
   rxq15_destroy (ctx->q15);
   cudaFree (ctx->d_masks); cudaFree (ctx->d_slot); cudaFree (ctx->d_twiddle); cudaFree (ctx->d_planes); cudaFree (ctx->d_tx_planes); cudaFree (ctx->d_am_planes);
   for (auto &kv : ctx->tc_lists) cudaFree (kv.second.d);
+  for (auto &kv : ctx->tune_lists) cudaFree (kv.second.d);
   for (int p = 0; p < 2; p++) { cudaFree (ctx->d_ovl[p]); cudaFree (ctx->d_proc[p]); }
   cudaFree (ctx->d_state); cudaFree (ctx->d_flag);
   cudaFree (ctx->d_acc_off);
@@ -429,6 +436,63 @@ int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase)
   if (!ctx) return SLB_ERR_ARG;
   if (ctx->cfg.chain != SLB_CHAIN_TX_F32) return fail (ctx, SLB_ERR_STATE, "the FM phase tap belongs to SLB_CHAIN_TX_F32 contexts");
   ctx->dbg_phase = d_phase;
+  return SLB_OK;
+}
+
+// ---- per-channel tuning (DESIGN.md §3.5) ----
+static int check_tune_chain (slb_ctx *ctx)
+{
+  if (!is_ssb_chain (ctx->cfg.chain))
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "tuning is served by the RX-SSB-f32, TX-SSB-f32 and TX-f32 chains only");
+  return SLB_OK;
+}
+// inc = llround (hz 2^32 / fs) in double; the offset is refused unless |inc| <= 2^31 - 1 (strictly inside +-fs/2)
+static bool tune_increment (const slb_ctx *ctx, double hz, int32_t *inc)
+{
+  const double v = hz * 4294967296.0 / (double) ctx->cfg.fs;
+  if (!(std::fabs (v) < 2147483647.5)) return false;   // (also refuses NaN and infinities)
+  *inc = (int32_t) std::llround (v);
+  return true;
+}
+static void tune_store (slb_ctx *ctx, uint32_t ch0, const int32_t *inc, uint32_t n)
+{
+  bool any = false;
+  for (uint32_t i = 0; i < n; i++) any = any || inc[i] != 0;
+  if (!any && ctx->tune_inc.empty ()) return;                         // never tuned: nothing to keep
+  if (ctx->tune_inc.empty ()) ctx->tune_inc.assign (ctx->cfg.channels, 0);
+  std::copy (inc, inc + n, ctx->tune_inc.begin () + ch0);
+  ctx->n_tuned = (uint32_t) std::count_if (ctx->tune_inc.begin (), ctx->tune_inc.end (), [] (int32_t v) { return v != 0; });
+  ctx->tune_version++;   // run_rx_kernel rebuilds its lists, after the device has finished every call that reads the old ones
+}
+int slb_set_tune (slb_ctx *ctx, const double *offset_hz)
+{
+  if (!ctx) return SLB_ERR_ARG;
+  { const int rc = check_tune_chain (ctx); if (rc) return rc; }
+  const uint32_t C = ctx->cfg.channels;
+  std::vector<int32_t> inc (C, 0);
+  if (offset_hz)
+    for (uint32_t c = 0; c < C; c++)
+      if (!tune_increment (ctx, offset_hz[c], &inc[c])) return fail (ctx, SLB_ERR_ARG, "tuning offset out of range (|offset| < fs / 2)");
+  tune_store (ctx, 0, inc.data (), C);
+  return SLB_OK;
+}
+int slb_set_tune_channel (slb_ctx *ctx, uint32_t ch, double offset_hz)
+{
+  if (!ctx) return SLB_ERR_ARG;
+  { const int rc = check_tune_chain (ctx); if (rc) return rc; }
+  if (ch >= ctx->cfg.channels) return fail (ctx, SLB_ERR_ARG, "channel out of range");
+  int32_t inc = 0;
+  if (!tune_increment (ctx, offset_hz, &inc)) return fail (ctx, SLB_ERR_ARG, "tuning offset out of range (|offset| < fs / 2)");
+  tune_store (ctx, ch, &inc, 1);
+  return SLB_OK;
+}
+int slb_get_tune_channel (const slb_ctx *ctx, uint32_t ch, int32_t *inc, double *realized_hz)
+{
+  if (!ctx || ch >= ctx->cfg.channels) return SLB_ERR_ARG;
+  if (!is_ssb_chain (ctx->cfg.chain)) return SLB_ERR_UNSUPPORTED;
+  const int32_t v = ctx->tune_inc.empty () ? 0 : ctx->tune_inc[ch];
+  if (inc) *inc = v;
+  if (realized_hz) *realized_hz = (double) v * (double) ctx->cfg.fs / 4294967296.0;
   return SLB_OK;
 }
 
@@ -596,13 +660,72 @@ static bool tc_path_enabled ()
   return on;
 }
 
+// The channels of [ch0, ch0 + nch) as a device list {row, inc}, the n tuned ones first (cached per range), nullptr when none is tuned
+static int tune_list (slb_ctx *ctx, uint32_t ch0, uint32_t nch, const slb_ctx::TuneList **out)
+{
+  *out = nullptr;
+  if (ctx->n_tuned == 0) return SLB_OK;
+  slb_ctx::TuneList &tl = ctx->tune_lists[((uint64_t) ch0 << 32) | nch];
+  if (tl.version != ctx->tune_version)
+  {
+    std::vector<uint32_t> pack;
+    for (int tuned = 1; tuned >= 0; tuned--)
+      for (uint32_t i = 0; i < nch; i++)
+        if ((ctx->tune_inc[ch0 + i] != 0) == (tuned != 0)) { pack.push_back (i); pack.push_back ((uint32_t) ctx->tune_inc[ch0 + i]); }
+    uint32_t n = 0;
+    while (n < nch && pack[2 * n + 1] != 0) n++;
+    if (n != 0)
+    {
+      // a mixer of an earlier call may still be reading the old list (any stream): offsets change rarely, so wait
+      CK (ctx, cudaDeviceSynchronize ());
+      if (pack.size () > tl.cap) { CK (ctx, cudaFree (tl.d)); tl.d = nullptr; CK (ctx, cudaMalloc (&tl.d, pack.size () * 4)); tl.cap = pack.size (); }
+      CK (ctx, cudaMemcpy (tl.d, pack.data (), pack.size () * 4, cudaMemcpyHostToDevice));
+      CK (ctx, cudaDeviceSynchronize ());   // (a pageable copy may still be in flight when cudaMemcpy returns; the mixer may run on a non-blocking stream)
+    }
+    tl.n = n; tl.n_all = nch; tl.version = ctx->tune_version;
+  }
+  if (tl.n) *out = &tl;
+  return SLB_OK;
+}
+
 // One pass of the SSB chain over channels [ch0, ch0 + nch); d_in / d_out / debug taps point at channel ch0.
 // RX: every channel whose mask is a 129-tap FIR goes to the tensor-core kernel — in groups of up to 8 channels of one
 // mask slot; which kernel serves a channel depends on its mode only, never on how the batch is cut, so shards and
 // channel groups reproduce the whole bit for bit. AM channels, caller-supplied masks that are no FIR, and TX stay on
 // the FFT kernel (contiguous runs).
+// Tuned channels (slb_set_tune) are mixed in front of an RX chain and behind a TX chain, on `stream`. in_owned: d_in is the library's
+// own buffer, consumed by this pass only, so RX mixes it in place (tuned rows only); a caller's input (slb_rx_process_device) is
+// staged through scratch: the same launch mixes the tuned rows into it and copies the others.
+static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
+                         float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase);
 static int run_rx_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
-                          float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase = nullptr)
+                          float *dbg_audio, float *dbg_gain, cudaStream_t stream, bool in_owned, uint32_t *dbg_phase = nullptr)
+{
+  const slb_ctx::TuneList *tu = nullptr;
+  { const int rc = tune_list (ctx, ch0, nch, &tu); if (rc) return rc; }
+  if (!tu) return run_rx_chain (ctx, d_in, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream, dbg_phase);
+  const bool is_tx = is_tx_chain (ctx->cfg.chain);
+  float *state = ctx->d_state + (size_t) ch0 * 8;
+  if (!is_tx)
+  {
+    int16_t *mixed = const_cast<int16_t *> (d_in);
+    if (!in_owned)
+    {
+      mixed = static_cast<int16_t *> (ctx_scratch_on (ctx, (size_t) nch * frames * 4, stream));
+      if (!mixed) return SLB_ERR_CUDA;
+    }
+    CK (ctx, launch_tune (d_in, mixed, tu->d, in_owned ? tu->n : tu->n_all, tu->n, state, frames, false, ctx->d_sin513, stream));
+    ctx->launches += 2;
+    return run_rx_chain (ctx, mixed, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream, dbg_phase);
+  }
+  const int rc = run_rx_chain (ctx, d_in, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream, dbg_phase);
+  if (rc) return rc;
+  CK (ctx, launch_tune (d_out, d_out, tu->d, tu->n, tu->n, state, frames, true, ctx->d_sin513, stream));
+  ctx->launches += 2;
+  return SLB_OK;
+}
+static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
+                         float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase)
 {
   const bool is_tx = is_tx_chain (ctx->cfg.chain);
   if (ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && !is_tx)
@@ -842,10 +965,11 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
       if (!runs.empty ())
       {
         if (ctx->tc_lists.size () > 64) { for (auto &kv : ctx->tc_lists) cudaFree (kv.second.d); ctx->tc_lists.clear (); }   // (lists are cached per channel range)
+        if (ctx->tune_lists.size () > 64) { CK (ctx, cudaDeviceSynchronize ()); for (auto &kv : ctx->tune_lists) cudaFree (kv.second.d); ctx->tune_lists.clear (); }
         const uint32_t ovl = ctx->rx.fft_len - hop;
         for (auto &r : runs)
         {
-          rc = run_rx_kernel (ctx, ctx->d_acc + (size_t) r.first * hop * 2, ctx->d_proc[0] + (size_t) r.first * hop * 2, r.first, r.second, hop, nullptr, nullptr, ctx->stream);
+          rc = run_rx_kernel (ctx, ctx->d_acc + (size_t) r.first * hop * 2, ctx->d_proc[0] + (size_t) r.first * hop * 2, r.first, r.second, hop, nullptr, nullptr, ctx->stream, true);
           if (rc) return rc;
         }
         // the other channels sit this launch out: their raw tail and hand-over counter move on unchanged
@@ -905,7 +1029,7 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
     // 3. a full super-block runs through the fused chain
     if (ctx->acc_fill == hop)
     {
-      int rc = run_rx_kernel (ctx, ctx->d_acc, ctx->d_proc[ctx->proc_cur ^ 1], 0, C, hop, nullptr, nullptr, ctx->stream);
+      int rc = run_rx_kernel (ctx, ctx->d_acc, ctx->d_proc[ctx->proc_cur ^ 1], 0, C, hop, nullptr, nullptr, ctx->stream, true);
       if (rc) return rc;
       rx_advance (ctx, hop);
       ctx->proc_cur ^= 1; ctx->acc_fill = 0;
@@ -1040,7 +1164,7 @@ int slb_feeder_run (slb_ctx *ctx, const slb_feeder_io *io, uint32_t ticks)
     {
       // the ring is fed from the PREVIOUS processed super-block (the chain's 384 frames of latency, as behind the per-call
       // API): the first 8 ticks come from the carried super-block, the last super-block of this run becomes the carry
-      int rc = run_rx_kernel (ctx, d_raw, d_prc, 0, C, (uint32_t) frames, nullptr, nullptr, st);
+      int rc = run_rx_kernel (ctx, d_raw, d_prc, 0, C, (uint32_t) frames, nullptr, nullptr, st, true);
       if (rc) return rc;
       rx_advance (ctx, (uint32_t) frames);
       src_a = ctx->d_proc[ctx->proc_cur]; stride_a = hop; ticks_a = per_hop; src_b = d_prc;
@@ -1187,7 +1311,7 @@ int slb_live_push (slb_live *lv, const int16_t *adc, const int16_t *usb_out)
     }
     else if (f32)
     {
-      int rc = run_rx_kernel (ctx, sl.d_adc, sl.d_prc, 0, C, (uint32_t) lv->frames, nullptr, nullptr, st);
+      int rc = run_rx_kernel (ctx, sl.d_adc, sl.d_prc, 0, C, (uint32_t) lv->frames, nullptr, nullptr, st, true);
       if (rc) return rc;
       rx_advance (ctx, (uint32_t) lv->frames);
       src_a = ctx->d_proc[ctx->proc_cur]; stride_a = hop; ticks_a = per_hop; src_b = sl.d_prc;
@@ -1354,7 +1478,7 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
     return SLB_OK;
   }
   if (frames % ctx->rx.hop != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the hop (384)");
-  int rc = run_rx_kernel (ctx, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->dbg_audio, ctx->dbg_gain, (cudaStream_t) stream, ctx->dbg_phase);
+  int rc = run_rx_kernel (ctx, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->dbg_audio, ctx->dbg_gain, (cudaStream_t) stream, false, ctx->dbg_phase);
   if (rc) return rc;
   rx_advance (ctx, frames);
   return SLB_OK;
@@ -1430,7 +1554,7 @@ static int process_host_sliced (slb_ctx *ctx, const int16_t *h_in, int16_t *h_ou
       }
       else
       {
-        const int rc = run_rx_kernel (ctx, ctx->d_bulk_in[slot], ctx->d_bulk_out[slot], c0, nc, n, nullptr, nullptr, s_k); if (rc) return rc;
+        const int rc = run_rx_kernel (ctx, ctx->d_bulk_in[slot], ctx->d_bulk_out[slot], c0, nc, n, nullptr, nullptr, s_k, true); if (rc) return rc;
       }
       CK (ctx, cudaEventRecord (ctx->slice_ev[slot][1], s_k));
       CK (ctx, cudaStreamWaitEvent (s_out, ctx->slice_ev[slot][1], 0));

@@ -102,7 +102,8 @@ struct RxF32Launch
   const int16_t *in; int16_t *out;         // [C][T][2]
   float *audio_dbg; float *gain_dbg;       // optional taps
   const int16_t *ovl_in; int16_t *ovl_out; // [C][ovl][2] carried raw-input tail (ping-pong between calls)
-  float *state;                            // [C][8] {d1_0,d2_0,d1_1,d2_1,env,-,-,-}
+  float *state;                            // [C][8] {d1_0,d2_0,d1_1,d2_1,env,-,-,tune phase}: RX-FM also uses words 5-6, TX-FM word 5;
+                                           // word 7 (uint32 bits) is the tuner's NCO phase (sl_tune.cu), written by no chain kernel
   unsigned *flag;                          // [C] tiles completed, monotonically increasing across calls
   const float *masks;                      // [SLB_MAX_MASKS][2*fft_len] in the kernel's packed layout (rx_ssb_f32_pack_mask)
   const uint8_t *mask_slot;                // [C]
@@ -121,6 +122,14 @@ struct RxF32Launch
   const float *sin513;                     // device, arm_sin_f32's 513-entry table (host_sin_table)
 };
 int launch_rx_ssb_f32 (const RxF32Launch &L, int sm_count, void *stream);
+
+// per-channel tuning (sl_tune.cu): rows d_list[e][0] of [C][frames][2] q15 I/Q (relative to d_in / d_out / state) are rotated by the
+// NCO of increment d_list[e][1] (2^-32 turn per sample) starting at the phase in word 7 of the row's state record, which then advances
+// by frames * inc. The first n_tuned entries are the tuned rows; entries after them have inc = 0 and are copied (an out-of-place pass
+// must fill every row). up = true moves the signal up by the increment (TX), false moves what sits at +increment down to 0 (RX).
+// d_in may be d_out; frames % 4 == 0, rows 16-byte aligned. Two launches (mix, then advance).
+int launch_tune (const int16_t *d_in, int16_t *d_out, const uint32_t *d_list, uint32_t n_list, uint32_t n_tuned, float *state, uint32_t frames,
+                 bool up, const float *sin513, void *stream);
 uint32_t rx_ssb_f32_launches_per_call ();
 uint32_t rx_ssb_f32_tiles (uint32_t frames);   // how far a call of `frames` advances the per-channel hand-over flag
 void rx_ssb_f32_pack_twiddles (float *out /* kTwiddleFloats */);

@@ -33,6 +33,7 @@ namespace sl {
 
 namespace {
 #include "sl_stress.cuh"
+#include "sl_nco.cuh"
 
 constexpr int kN = 512;                          // FFT length
 constexpr int kHop = 384;                        // new frames per FFT frame
@@ -179,14 +180,6 @@ __device__ __forceinline__ uint32_t pack_lr (float x_times_32768)
   return __byte_perm ((uint32_t) (uint16_t) v, 0u, 0x1010);   // stereo endpoint, L = R
 }
 
-__device__ __forceinline__ uint32_t pack_iq (float i_times_32768, float q_times_32768)
-{
-  short a, b;
-  asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(a) : "f"(i_times_32768));
-  asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(b) : "f"(q_times_32768));
-  return (uint32_t) (uint16_t) a | ((uint32_t) (uint16_t) b << 16);              // interleaved I,Q as on the I2S bus (main.c:333-341)
-}
-
 // arm_float_to_q31.c (V1.5.3, ARM_MATH_ROUNDING not defined): clip_q63_to_q31 ((q63_t) (x * 2147483648.0f)). The product is exact
 // (power of two); F2I.S32.TRUNC.SAT truncates toward zero and saturates like the cast + clip for every finite x
 __device__ __forceinline__ int32_t f2q31 (float x)
@@ -195,27 +188,11 @@ __device__ __forceinline__ int32_t f2q31 (float x)
   asm ("cvt.rzi.sat.s32.f32 %0, %1;" : "=r"(v) : "f"(x * 2147483648.0f));
   return v;
 }
-// arm_sin_f32.c:72-119 / arm_cos_f32.c, op for op (sl_stages.cu OpSinCosF32): table lookup + linear interpolation
-__device__ __forceinline__ float arm_sincos (float v, const float *tab, bool is_cos)
-{
-  float in; int n;
-  if (!is_cos)
-  {
-    if (v < 0.0f && v >= -1.9e-7f) return v;
-    in = __fmul_rn (v, 0.159154943092f); n = (int) in; if (v < 0.0f) n--;
-  }
-  else { in = __fadd_rn (__fmul_rn (v, 0.159154943092f), 0.25f); n = (int) in; if (in < 0.0f) n--; }
-  in = __fsub_rn (in, (float) n);
-  const float findex = __fmul_rn (512.0f, in);
-  const unsigned idx = ((unsigned) (uint16_t) (int) findex) & 0x1ffu;
-  const float fract = __fsub_rn (findex, (float) idx);
-  return __fadd_rn (__fmul_rn (__fsub_rn (1.0f, fract), tab[idx]), __fmul_rn (fract, tab[idx + 1]));
-}
 // FM NCO of one sample (oracle tx_fm_nco): arm_q31_to_float ((int32) phi) -> arm_scale_f32 (pi) -> arm_cos_f32 / arm_sin_f32 ->
 // arm_scale_f32 (level) -> arm_float_to_q15. The 1/2^31 of arm_q31_to_float and the x32768 are powers of two, folded into the constants.
 __device__ __forceinline__ uint32_t fm_nco (uint32_t phi, const float *tab, float level15)
 {
-  const float x = __fmul_rn (__int2float_rn ((int) phi), 3.14159265f / 2147483648.0f);
+  const float x = nco_arg (phi);
   return pack_iq (__fmul_rn (arm_sincos (x, tab, true), level15), __fmul_rn (arm_sincos (x, tab, false), level15));
 }
 

@@ -11,7 +11,7 @@
 // x = 256 xh + xl (signed high byte, unsigned low byte), map entries quantised to 24 bits as three balanced base-256
 // digits, all six digit products by tcgen05.mma kind::i8 into four int32 TMEM accumulators by weight (2^24, 2^16, 2^8, 1).
 // No product is dropped: the only deviation from infinite precision is the 2^-24 quantisation of the map, of the order
-// of one float32 epsilon of the INPUT level like the oracle's own FFT noise (tolerances: DESIGN.md §3.5).
+// of one float32 epsilon of the INPUT level like the oracle's own FFT noise (tolerances: DESIGN.md §3.6).
 //
 //   MMA shape: M = 128 rows = 8 channels (the 8 rows of a core matrix) x 16 consecutive firmware blocks (row groups),
 //   N = 208 (high data byte: 52 outputs of a block = 48 audio + 4 end-state, x 4 map digits) or 160 (low data byte: the top 3 digits + 4 rows), K = 32 bytes = 16 frames (I, Q bytes) per

@@ -84,15 +84,8 @@ struct KParams
 };
 
 #include "sl_tc_common.cuh"
+#include "sl_nco.cuh"
 
-__device__ __forceinline__ uint32_t pack_iq (float i_times_32768, float q_times_32768)
-{
-  // arm_float_to_q15.c:147 per component: truncation toward zero, then saturation; interleaved I,Q as on the I2S bus (main.c:333-341)
-  short a, b;
-  asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(a) : "f"(i_times_32768));
-  asm ("cvt.rzi.sat.s16.f32 %0, %1;" : "=h"(b) : "f"(q_times_32768));
-  return (uint32_t) (uint16_t) a | ((uint32_t) (uint16_t) b << 16);
-}
 // bytes 1 (hi) or 0 (lo) of four consecutive frames' L halves
 __device__ __forceinline__ uint32_t hi4 (uint4 v) { return __byte_perm (__byte_perm (v.x, v.y, 0x0051), __byte_perm (v.z, v.w, 0x0051), 0x5410); }
 __device__ __forceinline__ uint32_t lo4 (uint4 v) { return __byte_perm (__byte_perm (v.x, v.y, 0x0040), __byte_perm (v.z, v.w, 0x0040), 0x5410); }

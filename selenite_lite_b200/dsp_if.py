@@ -329,6 +329,24 @@ class DspIf:
         self._keep_phase = phase
         self._ck(self.lib.slb_tx_set_phase_tap(self.h, phase.data_ptr() if phase is not None else None), "tx_set_phase_tap")
 
+    # ---- per-channel tuning (CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_TX_F32) ----
+    def set_tune(self, hz):
+        """Offset of every channel within its I/Q band, in Hz: a scalar (all channels), an array [channels], or None (all 0).
+        RX demodulates what sits at +hz of the input; TX puts the signal at +hz."""
+        if hz is None:
+            self._ck(self.lib.slb_set_tune(self.h, None), "set_tune"); return
+        a = np.ascontiguousarray(np.broadcast_to(np.asarray(hz, np.float64), (self.channels,)))
+        self._ck(self.lib.slb_set_tune(self.h, a.ctypes.data), "set_tune")
+
+    def set_tune_channel(self, ch, hz):
+        self._ck(self.lib.slb_set_tune_channel(self.h, int(ch), float(hz)), "set_tune_channel")
+
+    def tune(self, ch):
+        """(inc, realized_hz) of channel ch: the NCO increment in 2^-32 turn per sample and the offset it realizes."""
+        inc = C.c_int32(); hz = C.c_double()
+        self._ck(self.lib.slb_get_tune_channel(self.h, int(ch), C.byref(inc), C.byref(hz)), "get_tune_channel")
+        return inc.value, hz.value
+
     def chan_params(self):
         p = _lib.ChanParams()
         self._ck(self.lib.slb_get_chan_params(self.h, C.byref(p)), "get_chan_params")

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Device-resident throughput of the chains that are not the headline bench line (TX-SSB-f32 = config 3,
-CHAN-64-f32 = config 4, RX at other widths, TX AM / FM). Prints one JSON line per chain after a line naming the card, its power
+CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, tuned channels). Prints one JSON line per chain after a line naming the card, its power
 limit and the HBM copy rate measured in the same run (hbm_frac_measured divides by that). Profiling aid, not the bench contract."""
 import argparse
 import json
@@ -102,6 +102,39 @@ def main():
             x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
             d = slb.DspIf(C, chain=slb.CHAIN_RX_SSB_F32); d.DSP_Set_Mode(slb.MODE_FM); y = torch.empty_like(x)
             ms = timeit(lambda: d.rx_process(x, y), args.steps); n = C * T; name = "rx fm (complex-detector tensor-core kernel, %d channels x %d s)" % (C, args.seconds)
+        elif which in ("rx_tuned", "rx_half_tuned", "tx_usb", "tx_usb_tuned"):
+            # per-channel tuning (DESIGN.md §3.5): every / every other channel offset by 7.3 kHz; TX-F32 in USB untuned and tuned
+            C, T = args.rx_channels, 48000 * args.seconds // 384 * 384
+            tx = which.startswith("tx")
+            x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
+            d = slb.DspIf(C, chain=slb.CHAIN_TX_F32 if tx else slb.CHAIN_RX_SSB_F32); y = torch.empty_like(x)
+            if which != "tx_usb":
+                hz = torch.full((C,), 7300.0, dtype=torch.float64)
+                if which == "rx_half_tuned":
+                    hz[1::2] = 0.0
+                d.set_tune(hz.numpy())
+            ms = timeit(lambda: (d.tx_process if tx else d.rx_process)(x, y), args.steps); n = C * T
+            name = "%s (%d channels x %d s)" % ({"rx_tuned": "rx_ssb_f32 USB, all channels tuned", "rx_half_tuned": "rx_ssb_f32 USB, half the channels tuned",
+                                                 "tx_usb": "tx_f32 USB untuned", "tx_usb_tuned": "tx_f32 USB, all channels tuned"}[which], C, args.seconds)
+        elif which == "tune_kernel":
+            # the mixer's own time, from a torch.profiler run of its own: an RX call with every channel tuned (8 B per tuned sample)
+            C, T = args.rx_channels, 48000 * args.seconds // 384 * 384
+            x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
+            d = slb.DspIf(C, chain=slb.CHAIN_RX_SSB_F32); y = torch.empty_like(x); d.set_tune([7300.0] * C)
+            d.rx_process(x, y); torch.cuda.synchronize()
+            from torch.profiler import ProfilerActivity, profile
+            with profile(activities=[ProfilerActivity.CUDA]) as prof:
+                for _ in range(args.steps):
+                    d.rx_process(x, y)
+                torch.cuda.synchronize()
+            us = [e.device_time_total for e in prof.key_averages() if "tune_mix_kernel" in e.key]
+            us_adv = [e.device_time_total for e in prof.key_averages() if "tune_advance_kernel" in e.key]
+            ms = sum(us) / 1e3 / args.steps; n = C * T
+            gbps = n * 8 / (ms * 1e-3) / 1e9
+            print(json.dumps({"kernel": "tune_mix_kernel (RX, %d channels x %d s, all tuned)" % (C, args.seconds), "ms_per_call": ms,
+                              "advance_ms_per_call": sum(us_adv) / 1e3 / args.steps, "GBps_at_8B_per_sample": gbps, "frac_of_measured_copy": gbps / roof}))
+            del d
+            continue
         else:
             C, T = args.rx_channels, 48000 * args.seconds // 384 * 384
             x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
