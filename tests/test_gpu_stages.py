@@ -122,6 +122,39 @@ def test_fir_family_bit_exact_with_carried_state(ctx, best_oracle, rng, name, dt
         assert np.array_equal(got[ch], exp), (name, ch)
 
 
+def run_fir_calls(ctx, name, c, x, lengths, tdt):
+    """One FIR call per entry of `lengths`, over consecutive pieces of x [C][sum(lengths)], the history carried between calls."""
+    hist = torch.zeros((C, len(c) - 1), dtype=tdt, device="cuda")
+    outs, a = [], 0
+    for n in lengths:
+        d = torch.zeros((C, n), dtype=tdt, device="cuda")
+        ctx.st(name, c, len(c), hist, dev(x[:, a:a + n]), d, n)
+        outs.append(d.cpu().numpy()); a += n
+    return np.concatenate(outs, 1), hist.cpu().numpy()
+
+
+@pytest.mark.parametrize("name", ["fir_f32", "fir_q31"])
+def test_fir_grid_stride_and_short_calls_with_carried_state(ctx, best_oracle, rng, name):
+    """fir_common caps the grid at 1024 x 256 threads: only a call of more than 262 144 outputs per channel runs the grid-stride
+    loop of fir_kernel (two calls of 300 000 here). A call shorter than the history (n < ntaps - 1) leaves a new history that is
+    partly the old one; the call after it shows whether that history was right."""
+    if name == "fir_f32":
+        dt, tdt, c = np.float32, torch.float32, f32(rng, 129, amp=0.1)
+        x = f32(rng, C, 600000)
+    else:
+        dt, tdt, c = np.int32, torch.int32, rng.integers(-2**28, 2**28, 64).astype(np.int32)
+        x = rng.integers(-2**31, 2**31 - 1, (C, 600000)).astype(np.int32)
+    ntaps = len(c)
+    short = 96 if ntaps == 129 else 48                        # a whole number of oracle blocks, shorter than the history
+    for lengths in ((300000, 300000), (480, short, 480)):
+        xs = x[:, :sum(lengths)]
+        got, hist = run_fir_calls(ctx, name, c, xs, lengths, tdt)
+        for ch in range(C):
+            exp, _ = getattr(best_oracle, name)(c, np.zeros(ntaps + B, dt), xs[ch], B)
+            assert np.array_equal(got[ch], exp), (name, lengths, ch, int(np.argmax(got[ch] != exp)))
+            assert np.array_equal(hist[ch], xs[ch, -(ntaps - 1):]), (name, lengths, "history", ch)
+
+
 def test_stage_calls_on_two_streams_do_not_share_staged_coefficients(ctx, best_oracle, rng):
     """The stage library stages a call's coefficients in the context's scratch buffer and consumes them on the caller's stream.
     Calls of one context on DIFFERENT streams are ordered through that buffer (ctx_scratch_on), so a second filter's
@@ -220,7 +253,9 @@ def test_cfft_fixed_golden_vectors(ctx):
         for ifft in (0, 1):
             d = dev(x)
             ctx.st("cfft_" + kind, d, N, 1, ifft)
-            assert np.array_equal(d.cpu().numpy()[C - 1, 0], g["%s_%d_%s_%d" % (kind, N, tag, ifft)]), (key, ifft)
+            got = d.cpu().numpy()
+            for ch in range(C):
+                assert np.array_equal(got[ch, 0], g["%s_%d_%s_%d" % (kind, N, tag, ifft)]), (key, ifft, ch)
 
 
 @pytest.mark.parametrize("ntaps", [8, 32, 64])
@@ -245,6 +280,74 @@ def test_lms_norm_f32_bit_exact_with_carried_state(ctx, best_oracle, rng, ntaps)
         assert np.array_equal(cf[ch], ec) and np.array_equal(stt[ch, :ntaps - 1], es[:ntaps - 1]) and np.array_equal(stt[ch, ntaps - 1:], ex), ch
     if ntaps >= 32:
         assert np.std(got_e[:, -2000:]) < 0.5 * np.std(d[:, -2000:])
+
+
+@pytest.mark.parametrize("ntaps", [96, 128])
+def test_lms_norm_f32_large_taps_partial_warp(best_oracle, rng, ntaps):
+    """Above 84 taps the kernel's dynamic shared memory exceeds 48 KB (the opt-in attribute path), and 70 channels make three
+    warps of channels, the last one partial (6 of 32 lanes): every channel bit for bit, over two calls of ragged length."""
+    Cl = 70
+    lctx = slb.DspIf(Cl, chain=slb.CHAIN_PASS)
+    n1, n2 = 48 * 6 + 17, 48 * 4
+    t = np.arange(n1 + n2)
+    d = np.stack([(0.3 * np.sin(2 * np.pi * (500.0 + 37.0 * ch) * t / 48000.0) + 0.05 * rng.standard_normal(t.size)) for ch in range(Cl)]).astype(np.float32)
+    x = np.concatenate([np.zeros((Cl, 3), np.float32), d[:, :-3]], 1)
+    coeffs = torch.zeros((Cl, ntaps), dtype=torch.float32, device="cuda"); state = torch.zeros((Cl, ntaps + 1), dtype=torch.float32, device="cuda")
+    outs, errs = [], []
+    for a, b in ((0, n1), (n1, n1 + n2)):
+        o = torch.zeros((Cl, b - a), dtype=torch.float32, device="cuda"); e = torch.zeros_like(o)
+        lctx.st("lms_norm_f32", coeffs, ntaps, 0.05, state, dev(x[:, a:b]), dev(d[:, a:b]), o, e, b - a)
+        outs.append(o.cpu().numpy()); errs.append(e.cpu().numpy())
+    got_o, got_e = np.concatenate(outs, 1), np.concatenate(errs, 1)
+    cf, stt = coeffs.cpu().numpy(), state.cpu().numpy()
+    for ch in range(Cl):
+        eo, ee, ec, es, ex = best_oracle.lms_norm_f32(np.zeros(ntaps, np.float32), 0.05, np.zeros(ntaps + 1, np.float32), np.zeros(2, np.float32), x[ch], d[ch], 1)
+        assert np.array_equal(got_o[ch], eo) and np.array_equal(got_e[ch], ee), (ntaps, ch)
+        assert np.array_equal(cf[ch], ec) and np.array_equal(stt[ch, :ntaps - 1], es[:ntaps - 1]) and np.array_equal(stt[ch, ntaps - 1:], ex), (ntaps, ch)
+
+
+def test_biquads_at_the_stage_limit_and_q15_postshifts(ctx, best_oracle, rng):
+    """SLB_MAX_STAGES = 4 stages for every biquad form (the existing test runs 2), and biquad_df1_q15 with postshift 0 and 2 beside
+    the 1 tested elsewhere; state carried across two calls."""
+    ns = slb._lib.MAX_STAGES
+    cf = np.tile(np.array(slb.default_rx_f32_params(48000).biquad[:10], np.float32), 2)
+    x = f32(rng, C, 2 * N, amp=0.3)
+    for name, per_stage in (("biquad_df2T_f32", 2), ("biquad_df1_f32", 4)):
+        st = torch.zeros((C, per_stage * ns), dtype=torch.float32, device="cuda"); outs = []
+        for part in (x[:, :N], x[:, N:]):
+            d = torch.zeros((C, N), dtype=torch.float32, device="cuda")
+            ctx.st(name, cf, ns, st, dev(part), d, N); outs.append(d.cpu().numpy())
+        got = np.concatenate(outs, 1)
+        for ch in range(C):
+            exp, est = getattr(best_oracle, name)(cf, ns, np.zeros(per_stage * ns, np.float32), x[ch], B)
+            assert np.array_equal(got[ch], exp) and np.array_equal(st[ch].cpu().numpy(), est), (name, ch)
+    xs = f32(rng, C, 2 * N, amp=0.3)
+    st = torch.zeros((C, 4 * ns), dtype=torch.float32, device="cuda"); d = torch.zeros((C, 2 * N), dtype=torch.float32, device="cuda")
+    ctx.st("biquad_stereo_df2T_f32", cf, ns, st, dev(xs), d, N)
+    for ch in range(C):
+        exp, est = best_oracle.biquad_stereo_df2T_f32(cf, ns, np.zeros(4 * ns, np.float32), xs[ch], B)
+        assert np.array_equal(d[ch].cpu().numpy(), exp) and np.array_equal(st[ch].cpu().numpy(), est), ("stereo", ch)
+    c15 = np.tile(np.array([8000, 0, -16000, 8000, 15000, -7000, 4000, 0, 8000, 4000, 9000, -3000], np.int16), 2)
+    xq = q15(rng, C, 2 * N, amp=20000)
+    for ps in (0, 2):
+        st = torch.zeros((C, 4 * ns), dtype=torch.int16, device="cuda"); outs = []
+        for part in (xq[:, :N], xq[:, N:]):
+            d = torch.zeros((C, N), dtype=torch.int16, device="cuda")
+            ctx.st("biquad_df1_q15", c15, ns, ps, st, dev(part), d, N); outs.append(d.cpu().numpy())
+        got = np.concatenate(outs, 1)
+        for ch in range(C):
+            exp, est = best_oracle.biquad_df1_q15(c15, ns, ps, np.zeros(4 * ns, np.int16), xq[ch], B)
+            assert np.array_equal(got[ch], exp) and np.array_equal(st[ch].cpu().numpy(), est), ("df1_q15", ps, ch)
+    c31 = np.tile((np.array([0.25, -0.5, 0.25, 0.45, -0.2, 0.12, 0.24, 0.12, 0.27, -0.09]) * 2**31).astype(np.int64).astype(np.int32), 2)
+    x31 = rng.integers(-2**30, 2**30, (C, 2 * N)).astype(np.int32)
+    st = torch.zeros((C, 4 * ns), dtype=torch.int32, device="cuda"); outs = []
+    for part in (x31[:, :N], x31[:, N:]):
+        d = torch.zeros((C, N), dtype=torch.int32, device="cuda")
+        ctx.st("biquad_df1_q31", c31, ns, 1, st, dev(part), d, N); outs.append(d.cpu().numpy())
+    got = np.concatenate(outs, 1)
+    for ch in range(C):
+        exp, est = best_oracle.biquad_df1_q31(c31, ns, 1, np.zeros(4 * ns, np.int32), x31[ch], B)
+        assert np.array_equal(got[ch], exp) and np.array_equal(st[ch].cpu().numpy(), est), ("df1_q31", ch)
 
 
 def test_biquads_bit_exact_with_carried_state(ctx, best_oracle, rng):
