@@ -52,6 +52,9 @@ extern "C" {
 #define SLB_CHAIN_TX_F32      5    /* all-mode transmit: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_TX_SSB_F32; AM (carrier +
                                       envelope) and FM (integer-phase NCO) from the same band-limited mic (DESIGN.md §3.4) */
 
+#define SLB_CHAIN_TX_SSB_Q15  6    /* all-integer phasing SSB modulator: mic (L of L=R) -> the fir_q15 Hilbert pair of RX-SSB-q15 -> rail
+                                      order by sideband -> q15 ALC -> I/Q pack (bit-exact, DESIGN.md §3.7) */
+
 #define SLB_MAX_STAGES 4
 #define SLB_MAX_MASKS  8
 
@@ -109,9 +112,13 @@ typedef struct
   float    proto[SLB_CHAN_BINS * SLB_CHAN_TAPS];   /* prototype low-pass h[n]; branch r uses e_r[p] = h[bins*p + bins-1-r] */
 } slb_chan_params;
 
-/* RX-SSB-q15 chain parameters (DESIGN.md §3): every stage is an integer CMSIS-DSP routine, results are bit-exact.
- * Oracle stage for each field in brackets. The sideband follows the channel's mode (SLB_DSP_Set_Mode: LSB / CW-R
- * subtract the quadrature rail, every other SSB-style mode adds it). */
+/* Parameters of the integer chains, RX-SSB-q15 and TX-SSB-q15 (DESIGN.md §3, §3.7): the Hilbert pair and the gain law both directions
+ * share. Every stage is an integer CMSIS-DSP routine, results are bit-exact. Oracle stage for each field in brackets. The sideband
+ * follows the channel's mode (SLB_DSP_Set_Mode): RX: LSB / CW-R subtract the quadrature rail, every other SSB-style mode adds it;
+ * TX: LSB / CW-R emit (I, Q) = (fi, fq), the others (fq, fi). On a TX context the agc_* fields are the ALC (its peak is the larger
+ * of max |I| and max |Q| per block), and the chain runs on the tcgen05 kernel only: bq_stages != 0, a tap >= 32640 (one that does not
+ * split into two signed bytes) or agc_window > 17 is refused with SLB_ERR_UNSUPPORTED and the parameters stay as they were.
+ * Defaults: 48 kHz only. */
 #define SLB_Q15_TAPS 64
 #define SLB_Q15_WIN  32
 typedef struct
@@ -206,9 +213,10 @@ int slb_ring_get_iq (slb_ctx *ctx, int which, int16_t *i, int16_t *q);
  * *_host: host pointers; stages through pinned memory with chunked H2D / kernel / D2H overlap, synchronous. */
 int slb_rx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream);
 int slb_rx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames);
-/* TX direction (context created with SLB_CHAIN_TX_SSB_F32 or SLB_CHAIN_TX_F32): in = mic frames (L = R as the codec delivers them in TX,
- * Core/Src/codec_if.c:304-306; L is used), out = modulated I/Q frames. Same shapes and rules as the RX calls. With this
- * chain SLB_DSP_In_Buff_Write runs the modulator at the 1 ms cadence exactly as it runs the demodulator for RX. */
+/* TX direction (context created with SLB_CHAIN_TX_SSB_F32, SLB_CHAIN_TX_F32 or SLB_CHAIN_TX_SSB_Q15): in = mic frames (L = R as the
+ * codec delivers them in TX, Core/Src/codec_if.c:304-306; L is used), out = modulated I/Q frames. Same shapes and rules as the RX calls
+ * (SLB_CHAIN_TX_SSB_Q15: frames % 48 == 0, as RX-SSB-q15). With these chains SLB_DSP_In_Buff_Write runs the modulator at the 1 ms cadence
+ * exactly as it runs the demodulator for RX (SLB_CHAIN_TX_SSB_Q15: in the call that delivers the block, no added latency). */
 int slb_tx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream);
 int slb_tx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames);
 /* Channelizer (context created with SLB_CHAIN_CHAN64_F32): in = wideband I/Q [streams][frames][2] int16, out =
@@ -228,7 +236,8 @@ int slb_rx_set_debug_taps (slb_ctx *ctx, float *d_audio, float *d_gain);
 /* SLB_CHAIN_TX_F32: the FM phase accumulator phi[n] (uint32, units of 2^-32 turn) after each sample, [channels][frames], device
  * pointer, written by the next slb_tx_process_device call(s) for FM channels when non-NULL (other channels' rows are left alone) */
 int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase);
-/* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48] */
+/* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48].
+ * TX-SSB-q15: d_audio receives the pre-ALC (I, Q) int16[channels][frames][2] (after the rail order), d_gain the same gain words. */
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain);
 
 /* ---- per-channel tuning within the I/Q band (DESIGN.md §3.5): SLB_CHAIN_RX_SSB_F32, SLB_CHAIN_TX_SSB_F32, SLB_CHAIN_TX_F32 ----
@@ -376,6 +385,9 @@ int slb_design_tc_tx_block (const float *mask_re_im, const int16_t *window, doub
 /* and for the integer chain (sl_rx_q15_tc.cu): window = int16[112][2] I/Q frames from 64 before the block, out = the 48 arm_fir_q15
  * results of rail I, then of rail Q; SLB_ERR_UNSUPPORTED when a tap does not split into two signed bytes (|tap| >= 32640) */
 int slb_design_q15_tc_block (const int16_t taps_i[64], const int16_t taps_q[64], const int16_t *window, int32_t out96[96]);
+/* the TX planes of the same kernel (TX-SSB-q15): window = int16[112][2] L=R mic frames from 64 before the block, out = the 48 arm_fir_q15
+ * results of L with taps_i (rail fi), then with taps_q (rail fq), before the rail order; R meets zero weight */
+int slb_design_q15_tc_tx_block (const int16_t taps_i[64], const int16_t taps_q[64], const int16_t *window /* [112][2] L=R */, int32_t out96[96]);
 int slb_design_mask (uint32_t fs, uint8_t mode, float *mask_re_im);
 /* tables of the tensor-core kernel's time-parallel biquad for blocks of 48 samples: Mp[4][16] = A^(48 k), M192[16], Cresp[48][4] */
 int slb_biquad_tc_tables (const float coef10[10], float *Mp64, float *M192, float *Cresp192);
@@ -392,7 +404,7 @@ int slb_sync (slb_ctx *ctx);
 
 /* ---- single-channel drop-in with the firmware's own names and signatures (Core/Inc/dsp_if.h:42-51).
  * They drive one process-global 1-channel context on device 0 (env SELENITE_B200_DEVICE, SELENITE_B200_FS,
- * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
+ * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15|tx_ssb_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
  * they return void; failures are reported through slb_dropin_status(). ---- */
 void DSP_Init (void);
 void DSP_Set_RX (void);

@@ -40,7 +40,7 @@ struct slb_ctx
   std::vector<uint8_t> mode_host;      // [C]
   bool tx_mode = false;
   Chan64State *chan = nullptr;         // SLB_CHAIN_CHAN64_F32 only
-  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15 only
+  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15 and SLB_CHAIN_TX_SSB_Q15 only
 
   // device: chain constants + carried state
   float *d_masks = nullptr; uint8_t *d_slot = nullptr; float *d_twiddle = nullptr;
@@ -98,9 +98,12 @@ struct slb_ctx
     }                                                                                              \
   } while (0)
 
-// the two transmit chains share everything but the modes they accept (check_mode): kernels, state, ring handling
-static inline bool is_tx_chain (uint32_t chain) { return chain == SLB_CHAIN_TX_SSB_F32 || chain == SLB_CHAIN_TX_F32; }
-static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || is_tx_chain (chain); }
+// the two f32 transmit chains share everything but the modes they accept (check_mode): kernels, state, ring handling
+static inline bool is_f32_tx_chain (uint32_t chain) { return chain == SLB_CHAIN_TX_SSB_F32 || chain == SLB_CHAIN_TX_F32; }
+static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || is_f32_tx_chain (chain); }
+// the direction a context was created for: slb_tx_process_* serve these chains, slb_rx_process_* the others
+static inline bool is_tx_direction (uint32_t chain) { return is_f32_tx_chain (chain) || chain == SLB_CHAIN_TX_SSB_Q15; }
+static inline bool is_q15_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15; }
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
 
@@ -152,7 +155,7 @@ static int upload_chain_constants (slb_ctx *ctx)
   // caller-supplied one may not) and the AM slot (two outputs per sample) stay on the FFT kernel
   {
     std::vector<uint8_t> planes ((size_t) SLB_MAX_MASKS * kTcPlaneBytes, 0);
-    if (is_tx_chain (ctx->cfg.chain))
+    if (is_f32_tx_chain (ctx->cfg.chain))
     {
       std::vector<uint8_t> txp ((size_t) SLB_MAX_MASKS * kTcTxPlaneBytes, 0);
       for (int m = 0; m < SLB_MAX_MASKS; m++)
@@ -177,7 +180,7 @@ static int upload_chain_constants (slb_ctx *ctx)
       CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kFmMaskSlot * kTcAmPlaneBytes, amp.data (), amp.size (), cudaMemcpyHostToDevice, ctx->stream));
       CK (ctx, cudaStreamSynchronize (ctx->stream));
     }
-    if (!is_tx_chain (ctx->cfg.chain))
+    if (!is_f32_tx_chain (ctx->cfg.chain))
     for (int m = 0; m < SLB_MAX_MASKS; m++)
       if (m < kAmMaskSlot) ctx->tc_ok[m] = N == 512 && tc_build_planes (ctx->masks_host.data () + (size_t) m * 2 * N, ctx->rx.biquad, planes.data () + (size_t) m * kTcPlaneBytes, &ctx->tc_s0[m], &ctx->tc_sz[m]);
     CK (ctx, cudaMemcpyAsync (ctx->d_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice, ctx->stream));
@@ -224,7 +227,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   *out = nullptr;
   if (cfg->channels == 0) return fail (nullptr, SLB_ERR_ARG, "channels must be > 0");
   if (cfg->fs != 48000u && cfg->fs != 96000u && cfg->fs != 192000u) return fail (nullptr, SLB_ERR_ARG, "fs must be 48000, 96000 or 192000");
-  if (cfg->chain != SLB_CHAIN_PASS && !is_ssb_chain (cfg->chain) && cfg->chain != SLB_CHAIN_CHAN64_F32 && cfg->chain != SLB_CHAIN_RX_SSB_Q15) return fail (nullptr, SLB_ERR_ARG, "unknown chain");
+  if (cfg->chain != SLB_CHAIN_PASS && !is_ssb_chain (cfg->chain) && cfg->chain != SLB_CHAIN_CHAN64_F32 && !is_q15_chain (cfg->chain)) return fail (nullptr, SLB_ERR_ARG, "unknown chain");
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount (&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -275,7 +278,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   int rc = upload_chain_constants (ctx);
   if (rc == SLB_OK) rc = reset_state (ctx);
   if (rc == SLB_OK && cfg->chain == SLB_CHAIN_CHAN64_F32) rc = chan64_create (ctx, C, cfg->fs, &ctx->chan);
-  if (rc == SLB_OK && cfg->chain == SLB_CHAIN_RX_SSB_Q15) rc = rxq15_create (ctx, C, cfg->fs, &ctx->q15);
+  if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, cfg->chain == SLB_CHAIN_TX_SSB_Q15, &ctx->q15);
   if (rc != SLB_OK) { g_create_error = ctx->err; slb_destroy (ctx); return rc; }
   *out = ctx;
   return SLB_OK;
@@ -395,7 +398,7 @@ int slb_default_rx_q15_params (uint32_t fs, slb_rx_q15_params *out) { return des
 int slb_set_rx_q15_params (slb_ctx *ctx, const slb_rx_q15_params *p)
 {
   if (!ctx || !p) return SLB_ERR_ARG;
-  if (!ctx->q15) return fail (ctx, SLB_ERR_STATE, "not an RX-SSB-q15 context");
+  if (!ctx->q15) return fail (ctx, SLB_ERR_STATE, "not an RX-SSB-q15 or TX-SSB-q15 context");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   CK (ctx, cudaStreamSynchronize (ctx->stream));
   return rxq15_set_params (ctx, ctx->q15, p);
@@ -574,9 +577,11 @@ static int check_mode (slb_ctx *ctx, uint8_t mode)
 {
   if (mode_to_mask_slot (mode) < 0) return fail (ctx, SLB_ERR_UNSUPPORTED, "not an FT-817 mode byte (LSB, USB, CW, CW-R, AM, FM, DIG, PKT are served; rxtx_if.h:33-43)");
   if (mode == SLB_MODE_AM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 chain (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only");
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 chain (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only; "
+                                           "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
   if (mode == SLB_MODE_FM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 chain (limiter-discriminator) and the TX-f32 chain (FM modulator) only");
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 chain (limiter-discriminator) and the TX-f32 chain (FM modulator) only; "
+                                           "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
   if (mode == SLB_MODE_FM && ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 && !ctx->tc_ok[kFmMaskSlot])
     return fail (ctx, SLB_ERR_UNSUPPORTED, "the FM slot has no tensor-core planes (fft_len must be 512 and the FM mask a 129-tap FIR)");
   return SLB_OK;
@@ -636,7 +641,7 @@ static int run_rx_fft_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out,
   L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
   L.masks = ctx->d_masks; L.mask_slot = ctx->d_slot + ch0; L.twiddle = ctx->d_twiddle;
   L.flag_base = ctx->flag_base; L.channels = nch; L.frames = frames;
-  L.tx = is_tx_chain (ctx->cfg.chain);
+  L.tx = is_f32_tx_chain (ctx->cfg.chain);
   L.tx_mod = ctx->cfg.chain == SLB_CHAIN_TX_F32;
   if (L.tx_mod)
   {
@@ -704,7 +709,7 @@ static int run_rx_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uin
   const slb_ctx::TuneList *tu = nullptr;
   { const int rc = tune_list (ctx, ch0, nch, &tu); if (rc) return rc; }
   if (!tu) return run_rx_chain (ctx, d_in, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream, dbg_phase);
-  const bool is_tx = is_tx_chain (ctx->cfg.chain);
+  const bool is_tx = is_f32_tx_chain (ctx->cfg.chain);
   float *state = ctx->d_state + (size_t) ch0 * 8;
   if (!is_tx)
   {
@@ -727,7 +732,7 @@ static int run_rx_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uin
 static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
                          float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase)
 {
-  const bool is_tx = is_tx_chain (ctx->cfg.chain);
+  const bool is_tx = is_f32_tx_chain (ctx->cfg.chain);
   if (ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && !is_tx)
     return run_rx_fft_kernel (ctx, d_in, d_out, ch0, nch, frames, dbg_audio, dbg_gain, stream);
   // slb_set_rx_path (SLB_RX_PATH_FFT) / SELENITE_B200_RX_PATH=fft keep every channel on the FFT kernel — except FM, whose
@@ -933,9 +938,9 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
     auto is_on = [&] (uint32_t c) { return !active || active[c] != 0; };
     if (which == 0 && ctx->q15)
     {
-      // the integer chain demodulates a block in the call that delivers it (dsp_if.c:286-289): the channels that fired run through the
+      // the integer chains demodulate (or modulate) a block in the call that delivers it (dsp_if.c:286-289): the channels that fired run through the
       // kernel (one launch per run of neighbours), the others carry their state over unchanged
-      if (frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "with the RX-SSB-q15 chain the block must be a whole number of 48-frame firmware blocks");
+      if (frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "with a q15 chain the block must be a whole number of 48-frame firmware blocks");
       for (auto &r : channel_runs (C, is_on))
       {
         rc = rxq15_launch (ctx, ctx->q15, ctx->d_blk + (size_t) r.first * frames * 2, ctx->d_proc[0] + (size_t) r.first * frames * 2, r.first, r.second, frames, ctx->sm_count, ctx->stream, false);
@@ -993,9 +998,9 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
   }
   if (which == 0 && ctx->q15)
   {
-    // the integer chain works at the firmware's own block size: the block is demodulated and enters the ring in the same
+    // the integer chains work at the firmware's own block size: the block is demodulated (or modulated) and enters the ring in the same
     // call, where the firmware would have called it (dsp_if.c:286-289), with no added latency
-    if (frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "with the RX-SSB-q15 chain the block must be a whole number of 48-frame firmware blocks");
+    if (frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "with a q15 chain the block must be a whole number of 48-frame firmware blocks");
     int rc = ensure_blk (ctx, frames); if (rc) return rc;
     CK (ctx, cudaMemcpyAsync (ctx->d_blk, pbuf, (size_t) C * frames * 4, cudaMemcpyHostToDevice, ctx->stream));
     rc = rxq15_launch (ctx, ctx->q15, ctx->d_blk, ctx->d_proc[0], 0, C, frames, ctx->sm_count, ctx->stream, false);
@@ -1438,7 +1443,15 @@ int slb_design_q15_tc_block (const int16_t taps_i[64], const int16_t taps_q[64],
 {
   if (!taps_i || !taps_q || !window || !out96) return SLB_ERR_ARG;
   std::vector<uint8_t> planes (kTcQ15PlaneBytes);
-  if (!q15_tc_build_planes (taps_i, taps_q, planes.data ())) return SLB_ERR_UNSUPPORTED;
+  if (!q15_tc_build_planes (taps_i, taps_q, planes.data (), false)) return SLB_ERR_UNSUPPORTED;
+  q15_tc_apply_planes (planes.data (), window, out96);
+  return SLB_OK;
+}
+int slb_design_q15_tc_tx_block (const int16_t taps_i[64], const int16_t taps_q[64], const int16_t *window, int32_t out96[96])
+{
+  if (!taps_i || !taps_q || !window || !out96) return SLB_ERR_ARG;
+  std::vector<uint8_t> planes (kTcQ15PlaneBytes);
+  if (!q15_tc_build_planes (taps_i, taps_q, planes.data (), true)) return SLB_ERR_UNSUPPORTED;
   q15_tc_apply_planes (planes.data (), window, out96);
   return SLB_OK;
 }
@@ -1462,7 +1475,7 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
 {
   if (!ctx || !d_in || !d_out || frames == 0) return SLB_ERR_ARG;
   if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
-  if (want_tx != is_tx_chain (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
+  if (want_tx != is_tx_direction (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   if (ctx->cfg.chain == SLB_CHAIN_PASS)
   {
@@ -1572,7 +1585,7 @@ static int process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint
 {
   if (!ctx || !h_in || !h_out || frames == 0) return SLB_ERR_ARG;
   if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
-  if (want_tx != is_tx_chain (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
+  if (want_tx != is_tx_direction (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   const bool chain = is_ssb_chain (ctx->cfg.chain);
   if (chain && frames % ctx->rx.hop != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the hop (384)");
@@ -1801,7 +1814,8 @@ slb_ctx *dropin ()
     cfg.device = dev ? std::atoi (dev) : 0;
     cfg.chain = (ch && std::strcmp (ch, "rx_ssb_f32") == 0) ? SLB_CHAIN_RX_SSB_F32 : (ch && std::strcmp (ch, "tx_ssb_f32") == 0) ? SLB_CHAIN_TX_SSB_F32
               : (ch && std::strcmp (ch, "tx_f32") == 0) ? SLB_CHAIN_TX_F32
-              : (ch && std::strcmp (ch, "rx_ssb_q15") == 0) ? SLB_CHAIN_RX_SSB_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
+              : (ch && std::strcmp (ch, "rx_ssb_q15") == 0) ? SLB_CHAIN_RX_SSB_Q15
+              : (ch && std::strcmp (ch, "tx_ssb_q15") == 0) ? SLB_CHAIN_TX_SSB_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
     g_dropin_status = slb_create (&cfg, &g_dropin);
     if (g_dropin_status != SLB_OK) std::fprintf (stderr, "selenite-b200: drop-in context failed: %s\n", slb_last_error (nullptr));
   }

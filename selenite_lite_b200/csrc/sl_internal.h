@@ -213,10 +213,10 @@ int chan64_launch (slb_ctx *ctx, Chan64State *st, const int16_t *d_in, int16_t *
                    int sm_count, void *stream, bool with_debug);
 void chan64_advance (Chan64State *st);
 
-// ---- RX-SSB-q15 (sl_rx_ssb_q15.cu): state object owned by the context ----
+// ---- RX-SSB-q15 and TX-SSB-q15 (sl_rx_ssb_q15.cu): state object owned by the context ----
 struct RxQ15State;
 int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p);
-int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, RxQ15State **out);
+int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, RxQ15State **out);   // tx: TX-SSB-q15 (the same state)
 void rxq15_destroy (RxQ15State *st);
 int rxq15_reset (slb_ctx *ctx, RxQ15State *st);
 int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p);
@@ -248,9 +248,9 @@ struct RxAmTcLaunch
 };
 int launch_rx_am_tc (const RxAmTcLaunch &L, int sm_count, void *stream);
 
-// ---- RX-SSB-q15 on the tensor cores (sl_rx_q15_tc.cu): same chain, same state, bit-identical results ----
+// ---- RX-SSB-q15 on the tensor cores (sl_rx_q15_tc.cu): same chain, same state, bit-identical results; TX-SSB-q15 (tx) runs only here ----
 constexpr size_t kTcQ15PlaneBytes = 7 * 24 * 256;
-bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes /* kTcQ15PlaneBytes */);
+bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes /* kTcQ15PlaneBytes */, bool tx);
 void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96);
 struct RxQ15TcLaunch
 {
@@ -259,6 +259,7 @@ struct RxQ15TcLaunch
   const uint8_t *planes, *lsb; int16_t *audio_dbg; uint32_t *gain_dbg;
   const int16_t *rel;                      // host, [SLB_Q15_WIN]
   uint32_t channels, frames, window; int32_t target, floor_; uint32_t gmax;
+  bool tx;                                 // TX-SSB-q15: mic frames in, I/Q frames out, audio_dbg = pre-ALC I/Q [C][T][2]
 };
 int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream);
 

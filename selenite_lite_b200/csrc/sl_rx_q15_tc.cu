@@ -13,6 +13,10 @@
 // rows are zero at the other rail's byte positions) into 2 x 192 accumulator columns, one accumulator buffer. The epilogue is
 // all integer: thread (block q, channel j) rebuilds the 48 FIR outputs of both rails, mixes, takes the block peak; block
 // peaks of the last four supertiles live in shared memory, which is all the finite AGC window (<= 17 blocks) needs.
+//
+// TX-SSB-q15 (kTx, DESIGN.md §3.7) is the same kernel: the input frames are the mic (L = R), both rails' taps sit at the L byte
+// positions of the planes (R gets zero weight, so R is ignored), and the epilogue keeps (I, Q) = (fi, fq) or (fq, fi) by sideband
+// instead of mixing, takes the block peak over |I| and |Q|, scales both rails with one gain word and stores I/Q frames.
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdlib>
@@ -91,8 +95,10 @@ __device__ __forceinline__ int sat16 (int v) { short r; asm ("cvt.sat.s16.s32 %0
 __device__ __forceinline__ int sat16 (int v) { return max (-32768, min (32767, v)); }
 #endif
 
+template <bool kTx>
 __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_constant__ KParams P)
 {
+  static_assert (!(kTx && SL_Q15TC_SPLIT), "the split-epilogue A/B variant serves RX only");
   extern __shared__ __align__ (1024) unsigned char smem[];
   unsigned char *sA = smem + Smem::a, *sB = smem + Smem::b, *sRaw = smem + Smem::raw, *sHist = smem + Smem::hist;
   int *sPk = reinterpret_cast<int *> (smem + Smem::pk), *sPkC = reinterpret_cast<int *> (smem + Smem::pkc);
@@ -407,7 +413,8 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         const int nblk = (int) (nfr / kBlk);
         mbar_wait (t_full + (kk & 1), (kk >> 1) & 1);
         tc_fence_after ();
-        // ---- accumulators -> the two FIR outputs (arm_fir_q15.c:642 + __SSAT), mix (arm_add_q15 / arm_sub_q15), |.| (arm_abs_q15)
+        // ---- accumulators -> the two FIR outputs (arm_fir_q15.c:642 + __SSAT), mix (arm_add_q15 / arm_sub_q15), |.| (arm_abs_q15);
+        //      TX: the rail order, |.| of both rails
         int aud[kBlk];
         int pk = 0;
         const uint32_t taddr = tmem + ((uint32_t) (32 * w) << 16);
@@ -426,9 +433,19 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
           for (int n = 0; n < 8; n++)
           {
             const int fq = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
-            const int v = sat16 (sub ? fi[n] - fq : fi[n] + fq);
-            aud[8 * i + n] = v;
-            pk = max (pk, min (abs (v), 32767));
+            if constexpr (kTx)
+            {
+              // the rail order is the sideband: LSB / CW-R (I, Q) = (fi, fq), the others (fq, fi); the pair stays packed (I | Q << 16)
+              const int vi = sub ? fi[n] : fq, vq = sub ? fq : fi[n];
+              aud[8 * i + n] = (int) __byte_perm ((uint32_t) vi, (uint32_t) vq, 0x5410);
+              pk = max (pk, max (min (abs (vi), 32767), min (abs (vq), 32767)));
+            }
+            else
+            {
+              const int v = sat16 (sub ? fi[n] - fq : fi[n] + fq);
+              aud[8 * i + n] = v;
+              pk = max (pk, min (abs (v), 32767));
+            }
           }
         }
         tc_fence_before ();
@@ -464,22 +481,47 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         {
           const size_t blk = (size_t) k * kQ + q, t0 = blk * kBlk;
           if (P.gain_dbg) P.gain_dbg[(size_t) c * P.blocks + blk] = gq;
-          if (P.audio_dbg)
+          if constexpr (kTx)
           {
-            uint4 *ad = reinterpret_cast<uint4 *> (P.audio_dbg + (size_t) c * P.frames + t0);
+            if (P.audio_dbg)
+            {
+              // pre-ALC (I, Q) frames, int16 [C][T][2]
+              uint4 *ad = reinterpret_cast<uint4 *> (P.audio_dbg + 2 * ((size_t) c * P.frames + t0));
+#pragma unroll
+              for (int n = 0; n < kBlk; n += 4) ad[n / 4] = make_uint4 ((uint32_t) aud[n], (uint32_t) aud[n + 1], (uint32_t) aud[n + 2], (uint32_t) aud[n + 3]);
+            }
+            uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0);
+            // arm_scale_q15 on each rail with the same gain word: I from the low half, Q (arithmetic shift) from the high half. Its __SSAT
+            // is left out because it cannot fire here: the envelope is never below the block's peak over both rails and q rounds down,
+            // so |y| <= target for |v| <= 32767, and v = -32768 (peak 32767) meets q <= 32768 and gives y >= -32768 (DESIGN.md §3.7).
+            // Bit-identical to the saturating form; 316 vs 254 Gsamples/s at 1024 channels (the per-sample store arithmetic bounds TX).
+#define SL_Q15_TXOUT(n) __byte_perm ((uint32_t) ((((int) (int16_t) aud[n]) * m) >> (15 - sh)), (uint32_t) (((aud[n] >> 16) * m) >> (15 - sh)), 0x5410)
 #pragma unroll
             for (int n = 0; n < kBlk; n += 8)
-              ad[n / 8] = make_uint4 ((uint32_t) (uint16_t) aud[n] | ((uint32_t) (uint16_t) aud[n + 1] << 16), (uint32_t) (uint16_t) aud[n + 2] | ((uint32_t) (uint16_t) aud[n + 3] << 16),
-                                      (uint32_t) (uint16_t) aud[n + 4] | ((uint32_t) (uint16_t) aud[n + 5] << 16), (uint32_t) (uint16_t) aud[n + 6] | ((uint32_t) (uint16_t) aud[n + 7] << 16));
+              asm volatile ("st.global.L1::no_allocate.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst + n / 4),
+                            "r"(SL_Q15_TXOUT (n)), "r"(SL_Q15_TXOUT (n + 1)), "r"(SL_Q15_TXOUT (n + 2)), "r"(SL_Q15_TXOUT (n + 3)),
+                            "r"(SL_Q15_TXOUT (n + 4)), "r"(SL_Q15_TXOUT (n + 5)), "r"(SL_Q15_TXOUT (n + 6)), "r"(SL_Q15_TXOUT (n + 7)) : "memory");
+#undef SL_Q15_TXOUT
           }
-          uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0);
+          else
+          {
+            if (P.audio_dbg)
+            {
+              uint4 *ad = reinterpret_cast<uint4 *> (P.audio_dbg + (size_t) c * P.frames + t0);
+#pragma unroll
+              for (int n = 0; n < kBlk; n += 8)
+                ad[n / 8] = make_uint4 ((uint32_t) (uint16_t) aud[n] | ((uint32_t) (uint16_t) aud[n + 1] << 16), (uint32_t) (uint16_t) aud[n + 2] | ((uint32_t) (uint16_t) aud[n + 3] << 16),
+                                        (uint32_t) (uint16_t) aud[n + 4] | ((uint32_t) (uint16_t) aud[n + 5] << 16), (uint32_t) (uint16_t) aud[n + 6] | ((uint32_t) (uint16_t) aud[n + 7] << 16));
+            }
+            uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0);
 #define SL_Q15_OUT(n) __byte_perm ((uint32_t) sat16 ((aud[n] * m) >> (15 - sh)), 0u, 0x1010)
 #pragma unroll
-          for (int n = 0; n < kBlk; n += 8)
-            asm volatile ("st.global.L1::no_allocate.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst + n / 4),
-                          "r"(SL_Q15_OUT (n)), "r"(SL_Q15_OUT (n + 1)), "r"(SL_Q15_OUT (n + 2)), "r"(SL_Q15_OUT (n + 3)),
-                          "r"(SL_Q15_OUT (n + 4)), "r"(SL_Q15_OUT (n + 5)), "r"(SL_Q15_OUT (n + 6)), "r"(SL_Q15_OUT (n + 7)) : "memory");
+            for (int n = 0; n < kBlk; n += 8)
+              asm volatile ("st.global.L1::no_allocate.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst + n / 4),
+                            "r"(SL_Q15_OUT (n)), "r"(SL_Q15_OUT (n + 1)), "r"(SL_Q15_OUT (n + 2)), "r"(SL_Q15_OUT (n + 3)),
+                            "r"(SL_Q15_OUT (n + 4)), "r"(SL_Q15_OUT (n + 5)), "r"(SL_Q15_OUT (n + 6)), "r"(SL_Q15_OUT (n + 7)) : "memory");
 #undef SL_Q15_OUT
+          }
         }
         if (k + 1 == supers && jvalid)
         {
@@ -526,8 +568,9 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
 
 // taps -> B operand: rows [rail I: hh (48) | hl (48) | rail Q: hh | hl], K byte m = 32 ks + kk = frame m / 2 of the 112-frame
 // window (64 before the block), rail m & 1; output n of the block meets tap d = 64 + n - frame. false when a tap does not
-// split into two signed bytes (|tap| >= 32640).
-bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes)
+// split into two signed bytes (|tap| >= 32640). tx: both rails filter the mic, so both place their taps at the L bytes (m = 2 frame)
+// and the R bytes get zero weight.
+bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes, bool tx)
 {
   std::memset (planes, 0, kTcQ15PlaneBytes);
   for (int rail = 0; rail < 2; rail++)
@@ -539,7 +582,7 @@ bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t 
         const int h = rail ? taps_q[d] : taps_i[d];
         const int hl = ((h + 128) & 255) - 128, hh = (h - hl) >> 8;
         if (hh < -128 || hh > 127) return false;
-        const int m = 2 * f + rail, ks = m / 32, kk = m % 32;
+        const int m = 2 * f + (tx ? 0 : rail), ks = m / 32, kk = m % 32;
         const int rows[2] = { rail * 96 + n, rail * 96 + 48 + n };
         const int dg[2] = { hh, hl };
         for (int g = 0; g < 2; g++)
@@ -549,7 +592,8 @@ bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t 
 }
 
 // host-side evaluation of the planes on one raw window (design check, tests/test_tc_math.py): the integer contraction the
-// kernel runs and its reconstruction of arm_fir_q15's result; out[0..47] = rail I, out[48..95] = rail Q
+// kernel runs and its reconstruction of arm_fir_q15's result; out[0..47] = rail I, out[48..95] = rail Q. The same for TX planes:
+// the contraction runs over all 224 bytes of the window as the kernel's does, and the R bytes meet zero weight there
 void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96)
 {
   for (int rail = 0; rail < 2; rail++)
@@ -580,12 +624,13 @@ int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream)
   P.gsz = (uint32_t) std::min<uint64_t> (kJ, std::max<uint64_t> (1, ((uint64_t) L.channels + (uint64_t) sm_count - 1) / (uint64_t) sm_count));
   P.n_groups = (L.channels + P.gsz - 1) / P.gsz;
   P.window = L.window; P.target = L.target; P.floor_ = L.floor_; P.gmax = L.gmax;
-  cudaError_t e = cudaFuncSetAttribute (rx_q15_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) Smem::bytes);
+  auto kernel = L.tx ? rx_q15_tc_kernel<true> : rx_q15_tc_kernel<false>;
+  cudaError_t e = cudaFuncSetAttribute (kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) Smem::bytes);
   if (e != cudaSuccess) return (int) e;
   uint32_t grid = (uint32_t) sm_count;
   if (grid > P.n_groups) grid = P.n_groups;
   if (const char *gs = std::getenv ("SELENITE_B200_TC_GRID")) { const long v = std::atol (gs); if (v > 0 && (uint32_t) v <= grid) grid = (uint32_t) v; }
-  rx_q15_tc_kernel<<<grid, kThreads, Smem::bytes, (cudaStream_t) stream>>> (P);
+  kernel<<<grid, kThreads, Smem::bytes, (cudaStream_t) stream>>> (P);
   return (int) cudaGetLastError ();
 }
 

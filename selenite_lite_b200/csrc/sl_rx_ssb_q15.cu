@@ -325,6 +325,7 @@ __global__ void __launch_bounds__ (kThreads, 4) rx_ssb_q15_kernel (const __grid_
 struct RxQ15State
 {
   uint32_t channels = 0;
+  bool tx = false;                      // TX-SSB-q15: the tcgen05 kernel's kTx form, with TX planes (no mma.sync form, no biquad)
   slb_rx_q15_params prm{};
   uint32_t *d_tail[2] = { nullptr, nullptr }; int16_t *d_peaks[2] = { nullptr, nullptr }; int parity = 0;
   uint32_t *d_afrag = nullptr; uint8_t *d_lsb = nullptr;
@@ -407,11 +408,11 @@ static void pack_afrag (const int16_t *taps, uint32_t ntaps, uint32_t *hi /* [10
   }
 }
 
-int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, RxQ15State **out)
+int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, RxQ15State **out)
 {
-  if (fs != 48000u) return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "the RX-SSB-q15 kernel is built for 48 kHz (48-frame firmware blocks)");
+  if (fs != 48000u) return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "the q15 kernels are built for 48 kHz (48-frame firmware blocks)");
   RxQ15State *st = new RxQ15State ();
-  st->channels = channels;
+  st->channels = channels; st->tx = tx;
   bool ok = true;
   for (int p = 0; p < 2; p++)
   {
@@ -457,6 +458,12 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
   if (p->agc_window < 1 || p->agc_window > (uint32_t) kWin || p->agc_floor < 1 || p->agc_target < 1 || p->agc_gmax_q15 < 1 || p->agc_gmax_q15 > (255u << 15))
     return ctx_fail (ctx, SLB_ERR_ARG, "AGC constants out of range");
   if (p->bq_stages > (uint32_t) SLB_MAX_STAGES || p->bq_postshift < 0 || p->bq_postshift > 14) return ctx_fail (ctx, SLB_ERR_ARG, "optional biquad: 0..4 stages, postshift 0..14");
+  // the tcgen05 kernel serves the chain when every tap splits into two signed bytes and the AGC window fits the peaks it keeps
+  std::vector<uint8_t> planes (kTcQ15PlaneBytes);
+  const bool tc_ok = q15_tc_build_planes (p->taps_i, p->taps_q, planes.data (), st->tx) && p->agc_window <= 17;
+  // TX-SSB-q15 has the tcgen05 kernel only, and no audio filter: refused before anything changes
+  if (st->tx && (p->bq_stages != 0 || !tc_ok))
+    return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "TX-SSB-q15 runs on the tcgen05 kernel only: bq_stages = 0, every tap < 32640, agc_window <= 17");
   if (p->bq_stages != st->prm.bq_stages || std::memcmp (p->bq_coeffs, st->prm.bq_coeffs, sizeof p->bq_coeffs) != 0)
     if (cudaMemset (st->d_bq, 0, (size_t) st->channels * 16 * 2) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state reset failed");   // a new filter starts from rest
   if (cudaMemcpy (st->d_rel, p->rel, kWin * 2, cudaMemcpyHostToDevice) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "release table upload failed");
@@ -464,12 +471,8 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
   pack_afrag (p->taps_i, p->ntaps, frag.data (), frag.data () + 320);
   pack_afrag (p->taps_q, p->ntaps, frag.data () + 640, frag.data () + 960);
   if (cudaMemcpy (st->d_afrag, frag.data (), frag.size () * 4, cudaMemcpyHostToDevice) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "tap upload failed");
-  {
-    // the tcgen05 kernel serves the chain when every tap splits into two signed bytes and the AGC window fits the peaks it keeps
-    std::vector<uint8_t> planes (kTcQ15PlaneBytes);
-    st->tc_ok = q15_tc_build_planes (p->taps_i, p->taps_q, planes.data ()) && p->agc_window <= 17;
-    if (st->tc_ok && cudaMemcpy (st->d_tc_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "tap upload failed");
-  }
+  st->tc_ok = tc_ok;
+  if (st->tc_ok && cudaMemcpy (st->d_tc_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "tap upload failed");
   st->prm = *p;
   return SLB_OK;
 }
@@ -521,7 +524,7 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
     ctx_count_launch (ctx, 2);
     return SLB_OK;
   };
-  if (st->tc_ok && !legacy_only)
+  if (st->tx || (st->tc_ok && !legacy_only))                                     // (TX: the only kernel; set_params guarantees tc_ok)
   {
     RxQ15TcLaunch L{};
     L.in = d_in; L.out = d_out;
@@ -531,6 +534,7 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
     L.audio_dbg = aud_tap; L.gain_dbg = gain_tap;
     L.rel = st->prm.rel; L.channels = nch; L.frames = frames; L.window = st->prm.agc_window;
     L.target = st->prm.agc_target; L.floor_ = st->prm.agc_floor; L.gmax = st->prm.agc_gmax_q15;
+    L.tx = st->tx;
     const int e = launch_rx_q15_tc (L, sm_count, stream);
     if (e != 0) return ctx_fail (ctx, SLB_ERR_CUDA, cudaGetErrorString ((cudaError_t) e));
     ctx_count_launch (ctx);

@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _lib
 
-CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32 = 0, 1, 2, 3, 4, 5
+CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15 = 0, 1, 2, 3, 4, 5, 6
 MODE_LSB, MODE_USB, MODE_CW, MODE_CWR, MODE_AM, MODE_FM, MODE_DIG, MODE_PKT = 0x00, 0x01, 0x02, 0x03, 0x04, 0x08, 0x0A, 0x0C
 RX_PATH_AUTO, RX_PATH_FFT = 0, 1
 
@@ -362,13 +362,14 @@ class DspIf:
     def set_rx_q15_params(self, p): self._ck(self.lib.slb_set_rx_q15_params(self.h, C.byref(p)), "set_rx_q15_params")
 
     def set_q15_debug_taps(self, audio=None, gain=None):
-        """audio: torch CUDA int16 [channels][frames]; gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block)."""
+        """audio: torch CUDA int16 [channels][frames] (RX-SSB-q15: pre-AGC audio) or [channels][frames][2] (TX-SSB-q15: pre-ALC I/Q);
+        gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block)."""
         self._keep_taps = (audio, gain)
         self._ck(self.lib.slb_rx_q15_set_debug_taps(self.h, audio.data_ptr() if audio is not None else None,
                                                     gain.data_ptr() if gain is not None else None), "rx_q15_set_debug_taps")
 
     def oracle_params(self, mode=MODE_USB):
-        if self.chain == CHAIN_RX_SSB_Q15:
+        if self.chain in (CHAIN_RX_SSB_Q15, CHAIN_TX_SSB_Q15):
             return q15_params_to_dict(self.rx_q15_params(), lsb=mode in (MODE_LSB, MODE_CWR))
         if self.chain == CHAIN_CHAN64_F32:
             return chan_params_to_dict(self.chan_params())
@@ -399,7 +400,8 @@ class DspIf:
         return out
 
     def tx_process(self, x, out=None, stream=None):
-        """TX direction (context created with CHAIN_TX_SSB_F32 or CHAIN_TX_F32): mic frames (L = R) in, modulated I/Q frames out."""
+        """TX direction (context created with CHAIN_TX_SSB_F32, CHAIN_TX_F32 or CHAIN_TX_SSB_Q15): mic frames (L = R) in, modulated I/Q
+        frames out."""
         return self.rx_process(x, out, stream, _dir="tx")
 
     def chan_process(self, x, out=None, stream=None):

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Device-resident throughput of the chains that are not the headline bench line (TX-SSB-f32 = config 3,
-CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, tuned channels). Prints one JSON line per chain after a line naming the card, its power
+CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, TX-SSB-q15, tuned channels). Prints one JSON line per chain after a line naming the card, its power
 limit and the HBM copy rate measured in the same run (hbm_frac_measured divides by that). Profiling aid, not the bench contract."""
 import argparse
 import json
@@ -86,6 +86,11 @@ def main():
             x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
             d = slb.DspIf(C, chain=slb.CHAIN_RX_SSB_Q15); y = torch.empty_like(x)
             ms = timeit(lambda: d.rx_process(x, y), args.steps); n = C * T; name = "rx_ssb_q15 (%d channels x %d s)" % (C, args.seconds)
+        elif which == "txq15":
+            C, T = args.rx_channels, 48000 * args.seconds
+            m = torch.randint(-8000, 8000, (C, T, 1), dtype=torch.int16, device=dev, generator=g).expand(C, T, 2).contiguous()
+            d = slb.DspIf(C, chain=slb.CHAIN_TX_SSB_Q15); y = torch.empty_like(m)
+            ms = timeit(lambda: d.tx_process(m, y), args.steps); n = C * T; name = "tx_ssb_q15 (%d mic channels x %d s)" % (C, args.seconds)
         elif which == "pass":
             C, T = args.rx_channels, 48000 * args.seconds // 384 * 384
             x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
