@@ -48,16 +48,18 @@ struct slb_ctx
   uint8_t *d_planes = nullptr; bool tc_ok[SLB_MAX_MASKS] = {}; float tc_s0[SLB_MAX_MASKS] = {}; float tc_sz[SLB_MAX_MASKS] = {}; TcBiquadTables tc_tables{};
   uint8_t *d_tx_planes = nullptr; float tx_unit[SLB_MAX_MASKS] = {};
   uint8_t *d_am_planes = nullptr; float am_unit[SLB_MAX_MASKS] = {};   // RX contexts: the AM slot's two-rail planes (sl_rx_am_tc.cu)   // TX-SSB-f32 contexts: tc_ok[] then refers to these planes
+  // a device uint32_t list of one channel range: grow-only buffer, stamped with the version of the host state it was built from
+  struct DevList { uint32_t *d = nullptr; size_t cap = 0; uint64_t version = ~0ull; };
   // channel lists of the tensor-core launches, cached per channel range (the bulk paths cut the batch the same way every
   // call) and rebuilt when a mode or a mask changes (mode_version)
-  struct TcLists { uint32_t *d = nullptr; size_t cap = 0; uint32_t groups = 0, groups_ssb = 0, n_chan = 0, n_pairs = 0; uint64_t version = ~0ull; std::vector<uint8_t> on_tc; };
+  struct TcLists : DevList { uint32_t groups = 0, groups_ssb = 0, n_chan = 0, n_pairs = 0; std::vector<uint8_t> on_tc; };
   std::map<uint64_t, TcLists> tc_lists; uint64_t mode_version = 0;
   bool force_fft = false;              // slb_set_rx_path (SLB_RX_PATH_FFT)
   // per-channel tuning (slb_set_tune, DESIGN.md §3.5): NCO increments (2^-32 turn per sample), empty until a non-zero offset is set;
   // the list {row, inc} of a channel range (tuned rows, then the untuned ones with inc = 0) is cached per range like tc_lists and
   // rebuilt when an offset changes (tune_version)
   std::vector<int32_t> tune_inc; uint32_t n_tuned = 0;
-  struct TuneList { uint32_t *d = nullptr; size_t cap = 0; uint32_t n = 0, n_all = 0; uint64_t version = ~0ull; };
+  struct TuneList : DevList { uint32_t n = 0, n_all = 0; };
   std::map<uint64_t, TuneList> tune_lists; uint64_t tune_version = 0;
   int16_t *d_ovl[2] = { nullptr, nullptr }; int ovl_parity = 0;
   float *d_state = nullptr; unsigned *d_flag = nullptr;
@@ -85,7 +87,7 @@ struct slb_ctx
 
   // host bulk path
   int16_t *d_bulk_in[kBulkSlots] = {}; int16_t *d_bulk_out[kBulkSlots] = {}; size_t bulk_bytes = 0;
-  cudaStream_t bulk_stream[kBulkSlots] = {}; cudaEvent_t bulk_done[kBulkSlots] = {};
+  cudaStream_t bulk_stream[kBulkSlots] = {};
   cudaEvent_t slice_ev[kBulkSlots][3] = {};   // time-sliced SSB host path: H2D landed / kernel done / D2H done, per staging slot
 };
 
@@ -106,6 +108,40 @@ static inline bool is_tx_direction (uint32_t chain) { return is_f32_tx_chain (ch
 static inline bool is_q15_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15; }
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
+
+// A kernel of an earlier call may still be reading a cached channel list (any stream): lists change rarely, so the device is idle
+// before a list is replaced, and again after the copy (a pageable copy may still be in flight when cudaMemcpy returns; the kernels
+// that read the list run on non-blocking streams).
+static int upload_list (slb_ctx *ctx, slb_ctx::DevList &l, const std::vector<uint32_t> &pack)
+{
+  CK (ctx, cudaDeviceSynchronize ());
+  if (pack.size () > l.cap) { CK (ctx, cudaFree (l.d)); l.d = nullptr; CK (ctx, cudaMalloc (&l.d, pack.size () * 4)); l.cap = pack.size (); }
+  CK (ctx, cudaMemcpy (l.d, pack.data (), pack.size () * 4, cudaMemcpyHostToDevice));
+  CK (ctx, cudaDeviceSynchronize ());
+  return SLB_OK;
+}
+// frees a list cache once it holds more than `keep` channel ranges
+template <class Lists> static int drop_lists (slb_ctx *ctx, Lists &lists, size_t keep)
+{
+  if (lists.size () <= keep) return SLB_OK;
+  CK (ctx, cudaDeviceSynchronize ());
+  for (auto &kv : lists) cudaFree (kv.second.d);
+  lists.clear ();
+  return SLB_OK;
+}
+
+// What every chain launch carries from one call to the next, from channel ch0 on (the launch structs share these field names):
+// the raw-input tail (ping-pong by ovl_parity), the per-channel state record and hand-over flag
+template <class Launch> static void set_carry (Launch &L, const slb_ctx *ctx, uint32_t ch0)
+{
+  const size_t ovl = ctx->rx.fft_len - ctx->rx.hop;
+  L.ovl_in = ctx->d_ovl[ctx->ovl_parity] + ch0 * ovl * 2; L.ovl_out = ctx->d_ovl[ctx->ovl_parity ^ 1] + ch0 * ovl * 2;
+  L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
+}
+template <class Launch> static void set_rx_agc (Launch &L, const slb_rx_f32_params &p)
+{
+  L.agc_target = p.agc_target; L.agc_decay = p.agc_decay; L.agc_floor = p.agc_floor; L.agc_gmax = p.agc_gmax;
+}
 
 namespace sl {
 int ctx_device (const slb_ctx *ctx) { return ctx->cfg.device; }
@@ -151,38 +187,35 @@ static int upload_chain_constants (slb_ctx *ctx)
     rx_ssb_f32_pack_mask (ctx->masks_host.data () + (size_t) m * 2 * N, inv, scaled.data () + (size_t) m * 2 * N);
   CK (ctx, cudaMemcpyAsync (ctx->d_masks, scaled.data (), scaled.size () * sizeof (float), cudaMemcpyHostToDevice, ctx->stream));
   CK (ctx, cudaMemcpyAsync (ctx->d_slot, ctx->slot_host.data (), ctx->slot_host.size (), cudaMemcpyHostToDevice, ctx->stream));
-  // the same masks as 24-bit FIR taps in tensor-core layout; a mask whose impulse response does not fit 129 taps (a
-  // caller-supplied one may not) and the AM slot (two outputs per sample) stay on the FFT kernel
+  // the same masks as 24-bit FIR taps in tensor-core layout, one plane set for the context's direction; a mask whose impulse
+  // response does not fit 129 taps (a caller-supplied one may not) and the AM slot (two outputs per sample) stay on the FFT kernel.
+  // The host buffers live until the stream synchronise at the end.
+  const float *mask = ctx->masks_host.data ();
+  std::vector<uint8_t> planes, amp;
+  if (is_f32_tx_chain (ctx->cfg.chain))
   {
-    std::vector<uint8_t> planes ((size_t) SLB_MAX_MASKS * kTcPlaneBytes, 0);
-    if (is_f32_tx_chain (ctx->cfg.chain))
-    {
-      std::vector<uint8_t> txp ((size_t) SLB_MAX_MASKS * kTcTxPlaneBytes, 0);
-      for (int m = 0; m < SLB_MAX_MASKS; m++)
-        ctx->tc_ok[m] = N == 512 && m < kAmMaskSlot && tc_build_tx_planes (ctx->masks_host.data () + (size_t) m * 2 * N, txp.data () + (size_t) m * kTcTxPlaneBytes, &ctx->tx_unit[m]);
-      CK (ctx, cudaMemcpyAsync (ctx->d_tx_planes, txp.data (), txp.size (), cudaMemcpyHostToDevice, ctx->stream));
-      CK (ctx, cudaStreamSynchronize (ctx->stream));
-    }
-    else
-    {
-      // the AM slot: both rails of the filter on the tensor cores, envelope and biquad in the epilogue (sl_rx_am_tc.cu)
-      std::vector<uint8_t> amp (kTcAmPlaneBytes, 0);
-      // Measured slower than the FFT kernel (135.7 vs 144.8 Gsamples/s at 1024 channels: 46 MMAs per supertile, one accumulator
-      // buffer, and the biquad recurrence back on the CUDA cores), so AM channels take it only on request: SELENITE_B200_AM_PATH=tc
-      const char *am_env = std::getenv ("SELENITE_B200_AM_PATH");
-      ctx->tc_ok[kAmMaskSlot] = am_env && std::strcmp (am_env, "tc") == 0 && N == 512 && tc_build_am_planes (ctx->masks_host.data () + (size_t) kAmMaskSlot * 2 * N, amp.data (), &ctx->am_unit[kAmMaskSlot]);
-      CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kAmMaskSlot * kTcAmPlaneBytes, amp.data (), amp.size (), cudaMemcpyHostToDevice, ctx->stream));
-      CK (ctx, cudaStreamSynchronize (ctx->stream));
-      // the FM slot: the same two-rail planes; the limiter-discriminator exists on the complex-detector tensor-core kernel only
-      // (sl_rx_am_tc.cu), so an FM mask must be a 129-tap FIR (slb_set_mask refuses others)
-      std::fill (amp.begin (), amp.end (), (uint8_t) 0);
-      ctx->tc_ok[kFmMaskSlot] = N == 512 && tc_build_am_planes (ctx->masks_host.data () + (size_t) kFmMaskSlot * 2 * N, amp.data (), &ctx->am_unit[kFmMaskSlot]);
-      CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kFmMaskSlot * kTcAmPlaneBytes, amp.data (), amp.size (), cudaMemcpyHostToDevice, ctx->stream));
-      CK (ctx, cudaStreamSynchronize (ctx->stream));
-    }
-    if (!is_f32_tx_chain (ctx->cfg.chain))
+    planes.assign ((size_t) SLB_MAX_MASKS * kTcTxPlaneBytes, 0);
     for (int m = 0; m < SLB_MAX_MASKS; m++)
-      if (m < kAmMaskSlot) ctx->tc_ok[m] = N == 512 && tc_build_planes (ctx->masks_host.data () + (size_t) m * 2 * N, ctx->rx.biquad, planes.data () + (size_t) m * kTcPlaneBytes, &ctx->tc_s0[m], &ctx->tc_sz[m]);
+      ctx->tc_ok[m] = N == 512 && m < kAmMaskSlot && tc_build_tx_planes (mask + (size_t) m * 2 * N, planes.data () + (size_t) m * kTcTxPlaneBytes, &ctx->tx_unit[m]);
+    CK (ctx, cudaMemcpyAsync (ctx->d_tx_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice, ctx->stream));
+  }
+  else
+  {
+    amp.assign (2 * kTcAmPlaneBytes, 0);
+    uint8_t *am = amp.data (), *fm = amp.data () + kTcAmPlaneBytes;
+    // the AM slot: both rails of the filter on the tensor cores, envelope and biquad in the epilogue (sl_rx_am_tc.cu).
+    // Measured slower than the FFT kernel (135.7 vs 144.8 Gsamples/s at 1024 channels: 46 MMAs per supertile, one accumulator
+    // buffer, and the biquad recurrence back on the CUDA cores), so AM channels take it only on request: SELENITE_B200_AM_PATH=tc
+    const char *am_env = std::getenv ("SELENITE_B200_AM_PATH");
+    ctx->tc_ok[kAmMaskSlot] = am_env && std::strcmp (am_env, "tc") == 0 && N == 512 && tc_build_am_planes (mask + (size_t) kAmMaskSlot * 2 * N, am, &ctx->am_unit[kAmMaskSlot]);
+    CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kAmMaskSlot * kTcAmPlaneBytes, am, kTcAmPlaneBytes, cudaMemcpyHostToDevice, ctx->stream));
+    // the FM slot: the same two-rail planes; the limiter-discriminator exists on the complex-detector tensor-core kernel only
+    // (sl_rx_am_tc.cu), so an FM mask must be a 129-tap FIR (slb_set_mask refuses others)
+    ctx->tc_ok[kFmMaskSlot] = N == 512 && tc_build_am_planes (mask + (size_t) kFmMaskSlot * 2 * N, fm, &ctx->am_unit[kFmMaskSlot]);
+    CK (ctx, cudaMemcpyAsync (ctx->d_am_planes + (size_t) kFmMaskSlot * kTcAmPlaneBytes, fm, kTcAmPlaneBytes, cudaMemcpyHostToDevice, ctx->stream));
+    planes.assign ((size_t) SLB_MAX_MASKS * kTcPlaneBytes, 0);
+    for (int m = 0; m < kAmMaskSlot; m++)
+      ctx->tc_ok[m] = N == 512 && tc_build_planes (mask + (size_t) m * 2 * N, ctx->rx.biquad, planes.data () + (size_t) m * kTcPlaneBytes, &ctx->tc_s0[m], &ctx->tc_sz[m]);
     CK (ctx, cudaMemcpyAsync (ctx->d_planes, planes.data (), planes.size (), cudaMemcpyHostToDevice, ctx->stream));
   }
   CK (ctx, cudaStreamSynchronize (ctx->stream));
@@ -191,17 +224,26 @@ static int upload_chain_constants (slb_ctx *ctx)
   return SLB_OK;
 }
 
-static int reset_state (slb_ctx *ctx)
+// Zero the samples of both rings and everything the chain carries from one call to the next: filter history, biquad and AGC / ALC
+// state, hand-over flags, the pending super-blocks. The ring pointers and the per-channel fill levels (acc_fill_pc) are left alone.
+static int clear_chain_state (slb_ctx *ctx)
 {
   const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, ovl = ctx->rx.fft_len - ctx->rx.hop, hop = ctx->rx.hop;
+  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) CK (ctx, cudaMemsetAsync (ctx->d_ring[w][k], 0, (size_t) C * R * 2, ctx->stream));
   for (int p = 0; p < 2; p++) CK (ctx, cudaMemsetAsync (ctx->d_ovl[p], 0, (size_t) C * ovl * 4, ctx->stream));
   CK (ctx, cudaMemsetAsync (ctx->d_state, 0, (size_t) C * 8 * sizeof (float), ctx->stream));
   CK (ctx, cudaMemsetAsync (ctx->d_flag, 0, (size_t) C * sizeof (unsigned), ctx->stream));
-  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) CK (ctx, cudaMemsetAsync (ctx->d_ring[w][k], 0, (size_t) C * R * 2, ctx->stream));
   CK (ctx, cudaMemsetAsync (ctx->d_acc, 0, (size_t) C * hop * 4, ctx->stream));
   for (int p = 0; p < 2; p++) CK (ctx, cudaMemsetAsync (ctx->d_proc[p], 0, (size_t) C * hop * 4, ctx->stream));
   CK (ctx, cudaStreamSynchronize (ctx->stream));
   ctx->flag_base = 0; ctx->ovl_parity = 0; ctx->acc_fill = 0; ctx->proc_cur = 0;
+  return SLB_OK;
+}
+
+static int reset_state (slb_ctx *ctx)
+{
+  { const int rc = clear_chain_state (ctx); if (rc) return rc; }
+  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames;
   ctx->ring_in.reset (R); ctx->ring_out.reset (R);
   ctx->ring_pc = false;
   if (ctx->d_key) { CK (ctx, cudaMemset (ctx->d_key, 0, C)); CK (ctx, cudaMemset (ctx->d_tone_cnt, 0, (size_t) C * 4)); ctx->any_key = false; }
@@ -292,8 +334,7 @@ void slb_destroy (slb_ctx *ctx)
   chan64_destroy (ctx->chan);
   rxq15_destroy (ctx->q15);
   cudaFree (ctx->d_masks); cudaFree (ctx->d_slot); cudaFree (ctx->d_twiddle); cudaFree (ctx->d_planes); cudaFree (ctx->d_tx_planes); cudaFree (ctx->d_am_planes);
-  for (auto &kv : ctx->tc_lists) cudaFree (kv.second.d);
-  for (auto &kv : ctx->tune_lists) cudaFree (kv.second.d);
+  drop_lists (ctx, ctx->tc_lists, 0); drop_lists (ctx, ctx->tune_lists, 0);
   for (int p = 0; p < 2; p++) { cudaFree (ctx->d_ovl[p]); cudaFree (ctx->d_proc[p]); }
   cudaFree (ctx->d_state); cudaFree (ctx->d_flag);
   cudaFree (ctx->d_acc_off);
@@ -305,7 +346,6 @@ void slb_destroy (slb_ctx *ctx)
   {
     cudaFree (ctx->d_bulk_in[s]); cudaFree (ctx->d_bulk_out[s]);
     if (ctx->bulk_stream[s]) cudaStreamDestroy (ctx->bulk_stream[s]);
-    if (ctx->bulk_done[s]) cudaEventDestroy (ctx->bulk_done[s]);
     for (int e = 0; e < 3; e++) if (ctx->slice_ev[s][e]) cudaEventDestroy (ctx->slice_ev[s][e]);
   }
   if (ctx->stream) cudaStreamDestroy (ctx->stream);
@@ -521,15 +561,7 @@ static int switch_direction (slb_ctx *ctx, bool tx)
   ctx->tx_mode = tx;
   if (ctx->chan) return SLB_OK;                                                            // the channelizer has no firmware rings
   CK (ctx, cudaSetDevice (ctx->cfg.device));
-  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, ovl = ctx->rx.fft_len - ctx->rx.hop, hop = ctx->rx.hop;
-  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) CK (ctx, cudaMemsetAsync (ctx->d_ring[w][k], 0, (size_t) C * R * 2, ctx->stream));
-  for (int p = 0; p < 2; p++) CK (ctx, cudaMemsetAsync (ctx->d_ovl[p], 0, (size_t) C * ovl * 4, ctx->stream));
-  CK (ctx, cudaMemsetAsync (ctx->d_state, 0, (size_t) C * 8 * sizeof (float), ctx->stream));
-  CK (ctx, cudaMemsetAsync (ctx->d_flag, 0, (size_t) C * sizeof (unsigned), ctx->stream));
-  CK (ctx, cudaMemsetAsync (ctx->d_acc, 0, (size_t) C * hop * 4, ctx->stream));
-  for (int p = 0; p < 2; p++) CK (ctx, cudaMemsetAsync (ctx->d_proc[p], 0, (size_t) C * hop * 4, ctx->stream));
-  CK (ctx, cudaStreamSynchronize (ctx->stream));
-  ctx->flag_base = 0; ctx->ovl_parity = 0; ctx->acc_fill = 0; ctx->proc_cur = 0;
+  { const int rc = clear_chain_state (ctx); if (rc) return rc; }
   if (ctx->q15) return rxq15_reset (ctx, ctx->q15);
   return SLB_OK;
 }
@@ -634,11 +666,9 @@ int SLB_DSP_Set_Mode (slb_ctx *ctx, uint8_t mode)     // dsp_if.c:367-370 is the
 static int run_rx_fft_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
                               float *dbg_audio, float *dbg_gain, cudaStream_t stream, uint32_t *dbg_phase = nullptr)
 {
-  const uint32_t ovl = ctx->rx.fft_len - ctx->rx.hop;
   RxF32Launch L{};
   L.in = d_in; L.out = d_out; L.audio_dbg = dbg_audio; L.gain_dbg = dbg_gain;
-  L.ovl_in = ctx->d_ovl[ctx->ovl_parity] + (size_t) ch0 * ovl * 2; L.ovl_out = ctx->d_ovl[ctx->ovl_parity ^ 1] + (size_t) ch0 * ovl * 2;
-  L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
+  set_carry (L, ctx, ch0);
   L.masks = ctx->d_masks; L.mask_slot = ctx->d_slot + ch0; L.twiddle = ctx->d_twiddle;
   L.flag_base = ctx->flag_base; L.channels = nch; L.frames = frames;
   L.tx = is_f32_tx_chain (ctx->cfg.chain);
@@ -651,7 +681,7 @@ static int run_rx_fft_kernel (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out,
     L.phase_dbg = dbg_phase; L.sin513 = ctx->d_sin513;
   }
   if (L.tx) { L.agc_target = ctx->tx.alc_target; L.agc_decay = ctx->tx.alc_decay; L.agc_floor = ctx->tx.alc_floor; L.agc_gmax = ctx->tx.alc_gmax; }
-  else { L.agc_target = ctx->rx.agc_target; L.agc_decay = ctx->rx.agc_decay; L.agc_floor = ctx->rx.agc_floor; L.agc_gmax = ctx->rx.agc_gmax; }
+  else set_rx_agc (L, ctx->rx);
   L.tables = &ctx->tables;
   CK (ctx, launch_rx_ssb_f32 (L, ctx->sm_count, stream));
   ctx->launches += rx_ssb_f32_launches_per_call ();
@@ -679,14 +709,7 @@ static int tune_list (slb_ctx *ctx, uint32_t ch0, uint32_t nch, const slb_ctx::T
         if ((ctx->tune_inc[ch0 + i] != 0) == (tuned != 0)) { pack.push_back (i); pack.push_back ((uint32_t) ctx->tune_inc[ch0 + i]); }
     uint32_t n = 0;
     while (n < nch && pack[2 * n + 1] != 0) n++;
-    if (n != 0)
-    {
-      // a mixer of an earlier call may still be reading the old list (any stream): offsets change rarely, so wait
-      CK (ctx, cudaDeviceSynchronize ());
-      if (pack.size () > tl.cap) { CK (ctx, cudaFree (tl.d)); tl.d = nullptr; CK (ctx, cudaMalloc (&tl.d, pack.size () * 4)); tl.cap = pack.size (); }
-      CK (ctx, cudaMemcpy (tl.d, pack.data (), pack.size () * 4, cudaMemcpyHostToDevice));
-      CK (ctx, cudaDeviceSynchronize ());   // (a pageable copy may still be in flight when cudaMemcpy returns; the mixer may run on a non-blocking stream)
-    }
+    if (n != 0) { const int rc = upload_list (ctx, tl, pack); if (rc) return rc; }
     tl.n = n; tl.n_all = nch; tl.version = ctx->tune_version;
   }
   if (tl.n) *out = &tl;
@@ -780,25 +803,21 @@ static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint
       std::memcpy (pack.data (), gstart.data (), G * 4); std::memcpy (pack.data () + G, ginfo.data (), G * 4);
       std::memcpy (pack.data () + 2 * (size_t) G, chan.data (), chan.size () * 4);
       if (!pairs.empty ()) std::memcpy (pack.data () + 2 * (size_t) G + chan.size (), pairs.data (), pairs.size () * 4);
-      // a kernel of an earlier call may still be reading the old lists (any stream): modes change rarely, so wait
-      CK (ctx, cudaDeviceSynchronize ());
-      if (pack.size () > tl.cap) { CK (ctx, cudaFree (tl.d)); tl.d = nullptr; CK (ctx, cudaMalloc (&tl.d, pack.size () * 4)); tl.cap = pack.size (); }
-      CK (ctx, cudaMemcpy (tl.d, pack.data (), pack.size () * 4, cudaMemcpyHostToDevice));
+      const int rc = upload_list (ctx, tl, pack); if (rc) return rc;
     }
     tl.groups = G; tl.version = ctx->mode_version;
   }
   const std::vector<uint8_t> &on_tc = tl.on_tc;
+  const unsigned flag_final = ctx->flag_base + rx_ssb_f32_tiles (frames);
   if (tl.groups != 0 && is_tx)
   {
     const uint32_t G = tl.groups;
-    const uint32_t ovl = ctx->rx.fft_len - ctx->rx.hop;
     TxTcLaunch L{};
     L.in = d_in; L.out = d_out; L.iq_dbg = dbg_audio; L.gain_dbg = dbg_gain;
-    L.ovl_in = ctx->d_ovl[ctx->ovl_parity] + (size_t) ch0 * ovl * 2; L.ovl_out = ctx->d_ovl[ctx->ovl_parity ^ 1] + (size_t) ch0 * ovl * 2;
-    L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
+    set_carry (L, ctx, ch0);
     L.gstart = tl.d; L.ginfo = tl.d + G; L.chan = tl.d + 2 * (size_t) G;
     L.planes = ctx->d_tx_planes; L.unit = ctx->tx_unit;
-    L.flag_final = ctx->flag_base + rx_ssb_f32_tiles (frames);
+    L.flag_final = flag_final;
     L.n_groups = G; L.frames = frames;
     L.alc_target = ctx->tx.alc_target; L.alc_decay = ctx->tx.alc_decay; L.alc_floor = ctx->tx.alc_floor; L.alc_gmax = ctx->tx.alc_gmax;
     CK (ctx, launch_tx_ssb_tc (L, ctx->sm_count, stream));
@@ -807,19 +826,17 @@ static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint
   else if (tl.groups != 0)
   {
     const uint32_t G = tl.groups, Gs = tl.groups_ssb;
-    const uint32_t ovl = ctx->rx.fft_len - ctx->rx.hop;
     if (Gs != 0)
     {
       RxTcLaunch L{};
       L.in = d_in; L.out = d_out; L.audio_dbg = dbg_audio; L.gain_dbg = dbg_gain;
-      L.ovl_in = ctx->d_ovl[ctx->ovl_parity] + (size_t) ch0 * ovl * 2; L.ovl_out = ctx->d_ovl[ctx->ovl_parity ^ 1] + (size_t) ch0 * ovl * 2;
-      L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
+      set_carry (L, ctx, ch0);
       L.gstart = tl.d; L.ginfo = tl.d + G; L.chan = tl.d + 2 * (size_t) G;
       L.pairs = tl.d + 2 * (size_t) G + tl.n_chan; L.n_pairs = tl.n_pairs;
       L.planes = ctx->d_planes; L.s0 = ctx->tc_s0; L.sz = ctx->tc_sz;
-      L.flag_final = ctx->flag_base + rx_ssb_f32_tiles (frames);
+      L.flag_final = flag_final;
       L.n_groups = Gs; L.frames = frames;
-      L.agc_target = ctx->rx.agc_target; L.agc_decay = ctx->rx.agc_decay; L.agc_floor = ctx->rx.agc_floor; L.agc_gmax = ctx->rx.agc_gmax;
+      set_rx_agc (L, ctx->rx);
       L.tables = &ctx->tc_tables;
       CK (ctx, launch_rx_ssb_tc (L, ctx->sm_count, stream));
       ctx->launches++;
@@ -828,13 +845,12 @@ static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint
     {
       RxAmTcLaunch L{};
       L.in = d_in; L.out = d_out; L.audio_dbg = dbg_audio; L.gain_dbg = dbg_gain;
-      L.ovl_in = ctx->d_ovl[ctx->ovl_parity] + (size_t) ch0 * ovl * 2; L.ovl_out = ctx->d_ovl[ctx->ovl_parity ^ 1] + (size_t) ch0 * ovl * 2;
-      L.state = ctx->d_state + (size_t) ch0 * 8; L.flag = ctx->d_flag + ch0;
+      set_carry (L, ctx, ch0);
       L.gstart = tl.d + Gs; L.ginfo = tl.d + G + Gs; L.chan = tl.d + 2 * (size_t) G;
       L.planes = ctx->d_am_planes; L.unit = ctx->am_unit;
-      L.flag_final = ctx->flag_base + rx_ssb_f32_tiles (frames);
+      L.flag_final = flag_final;
       L.n_groups = G - Gs; L.frames = frames;
-      L.agc_target = ctx->rx.agc_target; L.agc_decay = ctx->rx.agc_decay; L.agc_floor = ctx->rx.agc_floor; L.agc_gmax = ctx->rx.agc_gmax;
+      set_rx_agc (L, ctx->rx);
       L.tables = &ctx->tc_tables;
       CK (ctx, launch_rx_am_tc (L, ctx->sm_count, stream));
       ctx->launches++;
@@ -969,8 +985,9 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
       const auto runs = channel_runs (C, ready);
       if (!runs.empty ())
       {
-        if (ctx->tc_lists.size () > 64) { for (auto &kv : ctx->tc_lists) cudaFree (kv.second.d); ctx->tc_lists.clear (); }   // (lists are cached per channel range)
-        if (ctx->tune_lists.size () > 64) { CK (ctx, cudaDeviceSynchronize ()); for (auto &kv : ctx->tune_lists) cudaFree (kv.second.d); ctx->tune_lists.clear (); }
+        // (lists are cached per channel range, and the runs of ready channels change from call to call)
+        rc = drop_lists (ctx, ctx->tc_lists, 64); if (rc) return rc;
+        rc = drop_lists (ctx, ctx->tune_lists, 64); if (rc) return rc;
         const uint32_t ovl = ctx->rx.fft_len - hop;
         for (auto &r : runs)
         {
@@ -1051,6 +1068,7 @@ static int ring_read_common (slb_ctx *ctx, int which, void *pbuf, uint32_t frame
   if (!pbuf || frames == 0) return fail (ctx, SLB_ERR_ARG, "empty read");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   int rc = ensure_blk (ctx, frames); if (rc) return rc;
+  const uint32_t *d_first = nullptr;     // per-channel cadence: the pointer records, which mark the channels skipped this call
   if (per_channel || ctx->ring_pc)
   {
     if (which == 0 && !ctx->ring_pc && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->acc_fill != 0)
@@ -1061,40 +1079,50 @@ static int ring_read_common (slb_ctx *ctx, int which, void *pbuf, uint32_t frame
     CK (ctx, launch_ring_plan (ctx->d_rptr[which], d_act, C, R, false, which != 0, frames, ctx->stream));
     CK (ctx, launch_ring_read_pc (ctx->d_blk, ctx->d_ring[which][0], ctx->d_ring[which][1], C, R, ctx->d_rptr[which], frames, ctx->stream));
     ctx->launches += 2;
-    if (which == 1 && ctx->any_key && ctx->tone_hz)                                                      // "mix CW tone to speaker signal here" (dsp_if.c:218)
-    { CK (ctx, launch_sidetone_mix (ctx->d_blk, C, frames, ctx->d_key, ctx->d_tone_cnt, ctx->d_rptr[1], ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, ctx->stream)); ctx->launches++; }
-    CK (ctx, cudaMemcpyAsync (pbuf, ctx->d_blk, (size_t) C * frames * 4, cudaMemcpyDeviceToHost, ctx->stream));
-    CK (ctx, cudaStreamSynchronize (ctx->stream));
-    return SLB_OK;
+    d_first = ctx->d_rptr[which];
   }
-  RingPtrs &rp = which ? ctx->ring_out : ctx->ring_in;
-  const uint32_t rd0 = rp.plan_read (which != 0, frames);
-  CK (ctx, launch_ring_read (ctx->d_blk, ctx->d_ring[which][0], ctx->d_ring[which][1], C, R, rd0, frames, ctx->stream));
-  ctx->launches++;
+  else
+  {
+    RingPtrs &rp = which ? ctx->ring_out : ctx->ring_in;
+    const uint32_t rd0 = rp.plan_read (which != 0, frames);
+    CK (ctx, launch_ring_read (ctx->d_blk, ctx->d_ring[which][0], ctx->d_ring[which][1], C, R, rd0, frames, ctx->stream));
+    ctx->launches++;
+  }
   if (which == 1 && ctx->any_key && ctx->tone_hz)                                                        // "mix CW tone to speaker signal here" (dsp_if.c:218)
-  { CK (ctx, launch_sidetone_mix (ctx->d_blk, C, frames, ctx->d_key, ctx->d_tone_cnt, nullptr, ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, ctx->stream)); ctx->launches++; }
+  { CK (ctx, launch_sidetone_mix (ctx->d_blk, C, frames, ctx->d_key, ctx->d_tone_cnt, d_first, ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, ctx->stream)); ctx->launches++; }
   CK (ctx, cudaMemcpyAsync (pbuf, ctx->d_blk, (size_t) C * frames * 4, cudaMemcpyDeviceToHost, ctx->stream));
   CK (ctx, cudaStreamSynchronize (ctx->stream));
   return SLB_OK;
 }
 
-int SLB_DSP_In_Buff_Write (slb_ctx *ctx, const uint16_t *pbuf, uint16_t size)      // size in half-words
-{ if (!ctx) return SLB_ERR_ARG; if (size < 2 || (size & 1)) return fail (ctx, SLB_ERR_ARG, "size must be an even number of half-words >= 2"); return ring_write_common (ctx, 0, pbuf, size / 2u); }
-int SLB_DSP_In_Buff_Read (slb_ctx *ctx, uint8_t *pbuf, uint32_t size)              // size in bytes
-{ if (!ctx) return SLB_ERR_ARG; if (size < 4 || (size & 3)) return fail (ctx, SLB_ERR_ARG, "size must be a multiple of 4 bytes"); return ring_read_common (ctx, 0, pbuf, size / 4u); }
-int SLB_DSP_Out_Buff_Write (slb_ctx *ctx, const uint8_t *pbuf, uint32_t size)      // size in bytes
-{ if (!ctx) return SLB_ERR_ARG; if (size < 4 || (size & 3)) return fail (ctx, SLB_ERR_ARG, "size must be a multiple of 4 bytes"); return ring_write_common (ctx, 1, pbuf, size / 4u); }
-int SLB_DSP_Out_Buff_Read (slb_ctx *ctx, uint16_t *pbuf, uint16_t size)            // size in half-words
-{ if (!ctx) return SLB_ERR_ARG; if (size < 2 || (size & 1)) return fail (ctx, SLB_ERR_ARG, "size must be an even number of half-words >= 2"); return ring_read_common (ctx, 1, pbuf, size / 2u); }
+// the block size of a buffer call, in half-words (I2S side) or in bytes (USB side): whole frames of two 16-bit words either way
+static int check_halfwords (slb_ctx *ctx, uint32_t size)
+{
+  if (!ctx) return SLB_ERR_ARG;
+  return (size < 2 || (size & 1)) ? fail (ctx, SLB_ERR_ARG, "size must be an even number of half-words >= 2") : SLB_OK;
+}
+static int check_bytes (slb_ctx *ctx, uint32_t size)
+{
+  if (!ctx) return SLB_ERR_ARG;
+  return (size < 4 || (size & 3)) ? fail (ctx, SLB_ERR_ARG, "size must be a multiple of 4 bytes") : SLB_OK;
+}
+int SLB_DSP_In_Buff_Write (slb_ctx *ctx, const uint16_t *pbuf, uint16_t size)
+{ const int rc = check_halfwords (ctx, size); return rc ? rc : ring_write_common (ctx, 0, pbuf, size / 2u); }
+int SLB_DSP_In_Buff_Read (slb_ctx *ctx, uint8_t *pbuf, uint32_t size)
+{ const int rc = check_bytes (ctx, size); return rc ? rc : ring_read_common (ctx, 0, pbuf, size / 4u); }
+int SLB_DSP_Out_Buff_Write (slb_ctx *ctx, const uint8_t *pbuf, uint32_t size)
+{ const int rc = check_bytes (ctx, size); return rc ? rc : ring_write_common (ctx, 1, pbuf, size / 4u); }
+int SLB_DSP_Out_Buff_Read (slb_ctx *ctx, uint16_t *pbuf, uint16_t size)
+{ const int rc = check_halfwords (ctx, size); return rc ? rc : ring_read_common (ctx, 1, pbuf, size / 2u); }
 
 int SLB_DSP_In_Buff_Write_Ch (slb_ctx *ctx, const uint16_t *pbuf, uint16_t size, const uint8_t *active)
-{ if (!ctx) return SLB_ERR_ARG; if (size < 2 || (size & 1)) return fail (ctx, SLB_ERR_ARG, "size must be an even number of half-words >= 2"); return ring_write_common (ctx, 0, pbuf, size / 2u, active, true); }
+{ const int rc = check_halfwords (ctx, size); return rc ? rc : ring_write_common (ctx, 0, pbuf, size / 2u, active, true); }
 int SLB_DSP_In_Buff_Read_Ch (slb_ctx *ctx, uint8_t *pbuf, uint32_t size, const uint8_t *active)
-{ if (!ctx) return SLB_ERR_ARG; if (size < 4 || (size & 3)) return fail (ctx, SLB_ERR_ARG, "size must be a multiple of 4 bytes"); return ring_read_common (ctx, 0, pbuf, size / 4u, active, true); }
+{ const int rc = check_bytes (ctx, size); return rc ? rc : ring_read_common (ctx, 0, pbuf, size / 4u, active, true); }
 int SLB_DSP_Out_Buff_Write_Ch (slb_ctx *ctx, const uint8_t *pbuf, uint32_t size, const uint8_t *active)
-{ if (!ctx) return SLB_ERR_ARG; if (size < 4 || (size & 3)) return fail (ctx, SLB_ERR_ARG, "size must be a multiple of 4 bytes"); return ring_write_common (ctx, 1, pbuf, size / 4u, active, true); }
+{ const int rc = check_bytes (ctx, size); return rc ? rc : ring_write_common (ctx, 1, pbuf, size / 4u, active, true); }
 int SLB_DSP_Out_Buff_Read_Ch (slb_ctx *ctx, uint16_t *pbuf, uint16_t size, const uint8_t *active)
-{ if (!ctx) return SLB_ERR_ARG; if (size < 2 || (size & 1)) return fail (ctx, SLB_ERR_ARG, "size must be an even number of half-words >= 2"); return ring_read_common (ctx, 1, pbuf, size / 2u, active, true); }
+{ const int rc = check_halfwords (ctx, size); return rc ? rc : ring_read_common (ctx, 1, pbuf, size / 2u, active, true); }
 int slb_ring_get_ptrs_channel (slb_ctx *ctx, int which, uint32_t channel, uint32_t out[3])
 {
   if (!ctx || !out || which < 0 || which > 1 || channel >= ctx->cfg.channels) return SLB_ERR_ARG;
@@ -1120,18 +1148,74 @@ int SLB_AUDIO_AudioCmd (slb_ctx *ctx, uint8_t *pbuf, uint32_t size, uint8_t cmd)
 // ------------------------------------------------------------------------------------------------------------------
 // Host stream feeder
 // ------------------------------------------------------------------------------------------------------------------
+// Both feeders (stream and live) replay the one shared cadence of a context that has firmware rings; a chain behind the RX ring
+// takes whole super-blocks
+static int check_feeder (slb_ctx *ctx, bool with_rx, uint32_t ticks)
+{
+  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
+  if (ctx->ring_pc) return fail (ctx, SLB_ERR_STATE, "the feeder replays one shared cadence; per-channel cadence is on");
+  if (with_rx && is_ssb_chain (ctx->cfg.chain) && (ticks % (ctx->rx.hop / ctx->geo.block_frames) != 0 || ctx->acc_fill != 0))
+    return fail (ctx, SLB_ERR_ARG, "with an FFT chain the feeder moves whole 384-frame super-blocks (ticks % 8 == 0)");
+  return SLB_OK;
+}
+// {write index, read index} of every tick, the firmware's arithmetic in call order: the TX ring is read, then written, per tick;
+// the RX ring is written, then read
+static void plan_ticks (RingPtrs &rp, bool is_out, uint32_t *plan, uint32_t ticks, uint32_t B)
+{
+  for (uint32_t t = 0; t < ticks; t++)
+    if (is_out) { plan[2 * t + 1] = rp.plan_read (true, B); plan[2 * t] = rp.plan_write (true, B); }
+    else { plan[2 * t] = rp.plan_write (false, B); plan[2 * t + 1] = rp.plan_read (false, B); }
+}
+// TX ring: the USB stream in, the DAC stream out, with the side-tone of all `ticks` reads at once (keys constant over the run)
+static int replay_tx (slb_ctx *ctx, const int16_t *d_usb_out, int16_t *d_dac, const uint32_t *d_plan, uint32_t ticks, cudaStream_t st)
+{
+  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, B = ctx->geo.block_frames, frames = ticks * B;
+  CK (ctx, launch_ring_replay (false, nullptr, 0, 0, d_usb_out, frames, d_dac, ctx->d_ring[1][0], ctx->d_ring[1][1], C, R, d_plan, ticks, B, st));
+  ctx->launches++;
+  if (ctx->any_key && ctx->tone_hz)
+  { CK (ctx, launch_sidetone_mix (d_dac, C, frames, ctx->d_key, ctx->d_tone_cnt, nullptr, ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, st)); ctx->launches++; }
+  return SLB_OK;
+}
+// RX ring: the ADC stream through the chain (d_prc: its output, d_adc may be overwritten), the USB stream out
+static int replay_rx (slb_ctx *ctx, int16_t *d_adc, int16_t *d_prc, int16_t *d_usb_in, const uint32_t *d_plan, uint32_t ticks, cudaStream_t st)
+{
+  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, B = ctx->geo.block_frames, hop = ctx->rx.hop, frames = ticks * B;
+  const bool f32 = is_ssb_chain (ctx->cfg.chain);        // RX demodulator or TX modulator: both sit where the I2S half enters
+  const int16_t *src_a = nullptr, *src_b = d_adc; uint32_t stride_a = 0, ticks_a = 0;
+  if (ctx->q15)
+  {
+    int rc = rxq15_launch (ctx, ctx->q15, d_adc, d_prc, 0, C, frames, ctx->sm_count, st, false);
+    if (rc) return rc;
+    rxq15_advance (ctx->q15);
+    src_b = d_prc;
+  }
+  else if (f32)
+  {
+    // the ring is fed from the PREVIOUS processed super-block (the chain's 384 frames of latency, as behind the per-call
+    // API): the first 8 ticks come from the carried super-block, the last super-block of this run becomes the carry
+    int rc = run_rx_kernel (ctx, d_adc, d_prc, 0, C, frames, nullptr, nullptr, st, true);
+    if (rc) return rc;
+    rx_advance (ctx, frames);
+    src_a = ctx->d_proc[ctx->proc_cur]; stride_a = hop; ticks_a = hop / B; src_b = d_prc;
+  }
+  CK (ctx, launch_ring_replay (true, src_a, stride_a, ticks_a, src_b, frames, d_usb_in, ctx->d_ring[0][0], ctx->d_ring[0][1], C, R, d_plan, ticks, B, st));
+  ctx->launches++;
+  if (f32)
+  {
+    CK (ctx, cudaMemcpy2DAsync (ctx->d_proc[ctx->proc_cur ^ 1], (size_t) hop * 4, reinterpret_cast<const char *> (d_prc) + (size_t) (frames - hop) * 4, (size_t) frames * 4,
+                                (size_t) hop * 4, C, cudaMemcpyDeviceToDevice, st));
+    ctx->proc_cur ^= 1;
+  }
+  return SLB_OK;
+}
+
 int slb_feeder_run (slb_ctx *ctx, const slb_feeder_io *io, uint32_t ticks)
 {
   if (!ctx || !io || ticks == 0) return SLB_ERR_ARG;
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
-  if (ctx->ring_pc) return fail (ctx, SLB_ERR_STATE, "the feeder replays one shared cadence; per-channel cadence is on");
   if ((io->adc == nullptr) != (io->usb_in == nullptr) || (io->usb_out == nullptr) != (io->dac == nullptr)) return fail (ctx, SLB_ERR_ARG, "give both buffers of a direction or neither");
-  const bool f32 = is_ssb_chain (ctx->cfg.chain);        // RX demodulator or TX modulator: both sit where the I2S half enters
-  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, B = ctx->geo.block_frames, hop = ctx->rx.hop, per_hop = hop / B;
-  if (io->adc && f32 && (ticks % per_hop != 0 || ctx->acc_fill != 0))
-    return fail (ctx, SLB_ERR_ARG, "with an FFT chain the feeder moves whole 384-frame super-blocks (ticks % 8 == 0)");
+  { const int rc = check_feeder (ctx, io->adc != nullptr, ticks); if (rc) return rc; }
   CK (ctx, cudaSetDevice (ctx->cfg.device));
-  const size_t frames = (size_t) ticks * B, bytes = (size_t) C * frames * 4;
+  const size_t frames = (size_t) ticks * ctx->geo.block_frames, bytes = (size_t) ctx->cfg.channels * frames * 4;
   // scratch: raw stream, processed stream, ring output, plan
   char *scr = static_cast<char *> (ctx_scratch_on (ctx, 3 * bytes + (size_t) ticks * 8 + 256, ctx->stream));
   if (!scr) return SLB_ERR_CUDA;
@@ -1139,49 +1223,21 @@ int slb_feeder_run (slb_ctx *ctx, const slb_feeder_io *io, uint32_t ticks)
   uint32_t *d_plan = reinterpret_cast<uint32_t *> (scr + 3 * bytes);
   std::vector<uint32_t> plan ((size_t) ticks * 2);
   cudaStream_t st = ctx->stream;
-
-  if (io->usb_out)                                                                     // ---- TX ring: read, then write, per tick
+  if (io->usb_out)
   {
-    for (uint32_t t = 0; t < ticks; t++) { plan[2 * t + 1] = ctx->ring_out.plan_read (true, B); plan[2 * t] = ctx->ring_out.plan_write (true, B); }
+    plan_ticks (ctx->ring_out, true, plan.data (), ticks, ctx->geo.block_frames);
     CK (ctx, cudaMemcpyAsync (d_plan, plan.data (), plan.size () * 4, cudaMemcpyHostToDevice, st));
     CK (ctx, cudaMemcpyAsync (d_raw, io->usb_out, bytes, cudaMemcpyHostToDevice, st));
-    CK (ctx, launch_ring_replay (false, nullptr, 0, 0, d_raw, (uint32_t) frames, d_out, ctx->d_ring[1][0], ctx->d_ring[1][1], C, R, d_plan, ticks, B, st));
-    ctx->launches++;
-    if (ctx->any_key && ctx->tone_hz)                                                  // the side-tone of all `ticks` reads at once (keys constant over the run)
-    { CK (ctx, launch_sidetone_mix (d_out, C, (uint32_t) frames, ctx->d_key, ctx->d_tone_cnt, nullptr, ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, st)); ctx->launches++; }
+    { const int rc = replay_tx (ctx, d_raw, d_out, d_plan, ticks, st); if (rc) return rc; }
     CK (ctx, cudaMemcpyAsync (io->dac, d_out, bytes, cudaMemcpyDeviceToHost, st));
     CK (ctx, cudaStreamSynchronize (st));
   }
-  if (io->adc)                                                                         // ---- RX ring: write, then read, per tick
+  if (io->adc)
   {
-    for (uint32_t t = 0; t < ticks; t++) { plan[2 * t] = ctx->ring_in.plan_write (false, B); plan[2 * t + 1] = ctx->ring_in.plan_read (false, B); }
+    plan_ticks (ctx->ring_in, false, plan.data (), ticks, ctx->geo.block_frames);
     CK (ctx, cudaMemcpyAsync (d_plan, plan.data (), plan.size () * 4, cudaMemcpyHostToDevice, st));
     CK (ctx, cudaMemcpyAsync (d_raw, io->adc, bytes, cudaMemcpyHostToDevice, st));
-    const int16_t *src_a = nullptr, *src_b = d_raw; uint32_t stride_a = 0, ticks_a = 0;
-    if (ctx->q15)
-    {
-      int rc = rxq15_launch (ctx, ctx->q15, d_raw, d_prc, 0, C, (uint32_t) frames, ctx->sm_count, st, false);
-      if (rc) return rc;
-      rxq15_advance (ctx->q15);
-      src_b = d_prc;
-    }
-    else if (f32)
-    {
-      // the ring is fed from the PREVIOUS processed super-block (the chain's 384 frames of latency, as behind the per-call
-      // API): the first 8 ticks come from the carried super-block, the last super-block of this run becomes the carry
-      int rc = run_rx_kernel (ctx, d_raw, d_prc, 0, C, (uint32_t) frames, nullptr, nullptr, st, true);
-      if (rc) return rc;
-      rx_advance (ctx, (uint32_t) frames);
-      src_a = ctx->d_proc[ctx->proc_cur]; stride_a = hop; ticks_a = per_hop; src_b = d_prc;
-    }
-    CK (ctx, launch_ring_replay (true, src_a, stride_a, ticks_a, src_b, (uint32_t) frames, d_out, ctx->d_ring[0][0], ctx->d_ring[0][1], C, R, d_plan, ticks, B, st));
-    ctx->launches++;
-    if (f32)
-    {
-      CK (ctx, cudaMemcpy2DAsync (ctx->d_proc[ctx->proc_cur ^ 1], (size_t) hop * 4, reinterpret_cast<const char *> (d_prc) + (frames - hop) * 4, frames * 4,
-                                  (size_t) hop * 4, C, cudaMemcpyDeviceToDevice, st));
-      ctx->proc_cur ^= 1;
-    }
+    { const int rc = replay_rx (ctx, d_raw, d_prc, d_out, d_plan, ticks, st); if (rc) return rc; }
     CK (ctx, cudaMemcpyAsync (io->usb_in, d_out, bytes, cudaMemcpyDeviceToHost, st));
     CK (ctx, cudaStreamSynchronize (st));
   }
@@ -1213,15 +1269,11 @@ int slb_live_open (slb_ctx *ctx, uint32_t ticks_per_chunk, uint32_t depth, int w
 {
   if (!ctx || !out || ticks_per_chunk == 0 || depth < 2 || depth > 8 || (!with_rx && !with_tx)) return SLB_ERR_ARG;
   *out = nullptr;
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
-  if (ctx->ring_pc) return fail (ctx, SLB_ERR_STATE, "the feeder replays one shared cadence; per-channel cadence is on");
-  const uint32_t B = ctx->geo.block_frames, per_hop = ctx->rx.hop / B;
-  if (with_rx && is_ssb_chain (ctx->cfg.chain) && (ticks_per_chunk % per_hop != 0 || ctx->acc_fill != 0))
-    return fail (ctx, SLB_ERR_ARG, "with an FFT chain the feeder moves whole 384-frame super-blocks (ticks % 8 == 0)");
+  { const int rc = check_feeder (ctx, with_rx != 0, ticks_per_chunk); if (rc) return rc; }
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   slb_live *lv = new slb_live ();
   lv->ctx = ctx; lv->ticks = ticks_per_chunk; lv->depth = depth; lv->rx = with_rx != 0; lv->tx = with_tx != 0;
-  lv->frames = (size_t) ticks_per_chunk * B; lv->bytes = (size_t) ctx->cfg.channels * lv->frames * 4;
+  lv->frames = (size_t) ticks_per_chunk * ctx->geo.block_frames; lv->bytes = (size_t) ctx->cfg.channels * lv->frames * 4;
   lv->slots.resize (depth);
   bool ok = cudaStreamCreateWithFlags (&lv->s_in, cudaStreamNonBlocking) == cudaSuccess && cudaStreamCreateWithFlags (&lv->s_work, cudaStreamNonBlocking) == cudaSuccess &&
             cudaStreamCreateWithFlags (&lv->s_out, cudaStreamNonBlocking) == cudaSuccess;
@@ -1274,20 +1326,19 @@ int slb_live_push (slb_live *lv, const int16_t *adc, const int16_t *usb_out)
   if (ctx->ring_pc) return fail (ctx, SLB_ERR_STATE, "the feeder replays one shared cadence; per-channel cadence is on");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   slb_live::Slot &sl = lv->slots[lv->n_pushed % lv->depth];
-  const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames, B = ctx->geo.block_frames, hop = ctx->rx.hop, per_hop = hop / B, ticks = lv->ticks;
-  const bool f32 = is_ssb_chain (ctx->cfg.chain);
+  const uint32_t ticks = lv->ticks;
   sl.pushed = std::chrono::steady_clock::now ();
   // 1. staging (pinned) and the pointer plan of every tick of the chunk — the firmware's arithmetic, on the host, in call order
   uint32_t *plan_tx = sl.h_plan, *plan_rx = sl.h_plan + (size_t) ticks * 2;
   if (lv->tx)
   {
     std::memcpy (sl.h_usb_out, usb_out, lv->bytes);
-    for (uint32_t t = 0; t < ticks; t++) { plan_tx[2 * t + 1] = ctx->ring_out.plan_read (true, B); plan_tx[2 * t] = ctx->ring_out.plan_write (true, B); }
+    plan_ticks (ctx->ring_out, true, plan_tx, ticks, ctx->geo.block_frames);
   }
   if (lv->rx)
   {
     std::memcpy (sl.h_adc, adc, lv->bytes);
-    for (uint32_t t = 0; t < ticks; t++) { plan_rx[2 * t] = ctx->ring_in.plan_write (false, B); plan_rx[2 * t + 1] = ctx->ring_in.plan_read (false, B); }
+    plan_ticks (ctx->ring_in, false, plan_rx, ticks, ctx->geo.block_frames);
   }
   // 2. copy in (stream s_in)
   CK (ctx, cudaMemcpyAsync (sl.d_plan, sl.h_plan, (size_t) ticks * 4 * sizeof (uint32_t), cudaMemcpyHostToDevice, lv->s_in));
@@ -1297,39 +1348,8 @@ int slb_live_push (slb_live *lv, const int16_t *adc, const int16_t *usb_out)
   // 3. the chunk's kernels (stream s_work: chunks in order — chain state and rings carry from one to the next)
   CK (ctx, cudaStreamWaitEvent (lv->s_work, sl.in_done, 0));
   cudaStream_t st = lv->s_work;
-  if (lv->tx)
-  {
-    CK (ctx, launch_ring_replay (false, nullptr, 0, 0, sl.d_usb_out, (uint32_t) lv->frames, sl.d_dac, ctx->d_ring[1][0], ctx->d_ring[1][1], C, R, sl.d_plan, ticks, B, st));
-    ctx->launches++;
-    if (ctx->any_key && ctx->tone_hz)
-    { CK (ctx, launch_sidetone_mix (sl.d_dac, C, (uint32_t) lv->frames, ctx->d_key, ctx->d_tone_cnt, nullptr, ctx->d_tone, ctx->tone_hz, ctx->cfg.fs, st)); ctx->launches++; }
-  }
-  if (lv->rx)
-  {
-    const int16_t *src_a = nullptr, *src_b = sl.d_adc; uint32_t stride_a = 0, ticks_a = 0;
-    if (ctx->q15)
-    {
-      int rc = rxq15_launch (ctx, ctx->q15, sl.d_adc, sl.d_prc, 0, C, (uint32_t) lv->frames, ctx->sm_count, st, false);
-      if (rc) return rc;
-      rxq15_advance (ctx->q15);
-      src_b = sl.d_prc;
-    }
-    else if (f32)
-    {
-      int rc = run_rx_kernel (ctx, sl.d_adc, sl.d_prc, 0, C, (uint32_t) lv->frames, nullptr, nullptr, st, true);
-      if (rc) return rc;
-      rx_advance (ctx, (uint32_t) lv->frames);
-      src_a = ctx->d_proc[ctx->proc_cur]; stride_a = hop; ticks_a = per_hop; src_b = sl.d_prc;
-    }
-    CK (ctx, launch_ring_replay (true, src_a, stride_a, ticks_a, src_b, (uint32_t) lv->frames, sl.d_usb_in, ctx->d_ring[0][0], ctx->d_ring[0][1], C, R, sl.d_plan + (size_t) ticks * 2, ticks, B, st));
-    ctx->launches++;
-    if (f32)
-    {
-      CK (ctx, cudaMemcpy2DAsync (ctx->d_proc[ctx->proc_cur ^ 1], (size_t) hop * 4, reinterpret_cast<const char *> (sl.d_prc) + (lv->frames - hop) * 4, lv->frames * 4,
-                                  (size_t) hop * 4, C, cudaMemcpyDeviceToDevice, st));
-      ctx->proc_cur ^= 1;
-    }
-  }
+  if (lv->tx) { const int rc = replay_tx (ctx, sl.d_usb_out, sl.d_dac, sl.d_plan, ticks, st); if (rc) return rc; }
+  if (lv->rx) { const int rc = replay_rx (ctx, sl.d_adc, sl.d_prc, sl.d_usb_in, sl.d_plan + (size_t) ticks * 2, ticks, st); if (rc) return rc; }
   CK (ctx, cudaEventRecord (sl.work_done, st));
   // 4. copy out (stream s_out)
   CK (ctx, cudaStreamWaitEvent (lv->s_out, sl.work_done, 0));
@@ -1383,20 +1403,16 @@ int slb_ring_get_iq (slb_ctx *ctx, int which, int16_t *i, int16_t *q)
   return SLB_OK;
 }
 
-uint32_t slb_ring_plan_write (uint32_t ring_frames, int is_out, uint32_t state[3], uint32_t frames)
+// one planning step of a ring whose pointers {enable, rd, wr} the caller keeps
+static uint32_t ring_plan (bool write, uint32_t ring_frames, int is_out, uint32_t state[3], uint32_t frames)
 {
   RingPtrs rp; rp.size = ring_frames; rp.enable = state[0]; rp.rd = state[1]; rp.wr = state[2];
-  const uint32_t first = rp.plan_write (is_out != 0, frames);
+  const uint32_t first = write ? rp.plan_write (is_out != 0, frames) : rp.plan_read (is_out != 0, frames);
   state[0] = rp.enable; state[1] = rp.rd; state[2] = rp.wr;
   return first;
 }
-uint32_t slb_ring_plan_read (uint32_t ring_frames, int is_out, uint32_t state[3], uint32_t frames)
-{
-  RingPtrs rp; rp.size = ring_frames; rp.enable = state[0]; rp.rd = state[1]; rp.wr = state[2];
-  const uint32_t first = rp.plan_read (is_out != 0, frames);
-  state[0] = rp.enable; state[1] = rp.rd; state[2] = rp.wr;
-  return first;
-}
+uint32_t slb_ring_plan_write (uint32_t ring_frames, int is_out, uint32_t state[3], uint32_t frames) { return ring_plan (true, ring_frames, is_out, state, frames); }
+uint32_t slb_ring_plan_read (uint32_t ring_frames, int is_out, uint32_t state[3], uint32_t frames) { return ring_plan (false, ring_frames, is_out, state, frames); }
 int slb_biquad_scan_tables (const float coef10[10], float *Mpow96, float *Cresp96)
 {
   if (!coef10 || !Mpow96 || !Cresp96) return SLB_ERR_ARG;
@@ -1500,6 +1516,52 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
 int slb_rx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream) { return process_device (ctx, d_in, d_out, frames, stream, false); }
 int slb_tx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream) { return process_device (ctx, d_in, d_out, frames, stream, true); }
 
+// Staging of the host bulk paths: kBulkSlots device buffer pairs of at least `bytes` each, and one stream per slot
+static int ensure_bulk (slb_ctx *ctx, size_t bytes)
+{
+  if (bytes <= ctx->bulk_bytes && ctx->bulk_stream[0]) return SLB_OK;
+  for (int s = 0; s < kBulkSlots; s++)
+  {
+    if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
+    if (bytes > ctx->bulk_bytes)
+    {
+      CK (ctx, cudaFree (ctx->d_bulk_in[s])); CK (ctx, cudaFree (ctx->d_bulk_out[s]));
+      ctx->d_bulk_in[s] = ctx->d_bulk_out[s] = nullptr;
+      CK (ctx, cudaMalloc (&ctx->d_bulk_in[s], bytes)); CK (ctx, cudaMalloc (&ctx->d_bulk_out[s], bytes));
+    }
+    if (!ctx->bulk_stream[s]) CK (ctx, cudaStreamCreateWithFlags (&ctx->bulk_stream[s], cudaStreamNonBlocking));
+  }
+  ctx->bulk_bytes = std::max (ctx->bulk_bytes, bytes);
+  return SLB_OK;
+}
+
+// Chains whose channels (or channelizer streams) are independent, through host buffers: the batch is cut into groups of at most
+// 48 MiB, and H2D / kernel / D2H of consecutive groups overlap, round-robin over the slot streams. launch (d_in, d_out, c0, n, stream)
+// runs the chain on the n channels from c0 staged in d_in.
+using GroupLaunch = std::function<int (const int16_t *, int16_t *, uint32_t, uint32_t, cudaStream_t)>;
+static int process_host_groups (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames, const GroupLaunch &launch)
+{
+  const uint32_t C = ctx->cfg.channels;
+  const size_t ch_bytes = (size_t) frames * 4;          // per channel, in and out alike
+  uint32_t group = (uint32_t) ((size_t) (48u << 20) / ch_bytes);
+  if (group < 1) group = 1;
+  if (group > C) group = C;
+  { const int rc = ensure_bulk (ctx, (size_t) group * ch_bytes); if (rc) return rc; }
+  CK (ctx, cudaStreamSynchronize (ctx->stream));
+  int slot = 0;
+  for (uint32_t c0 = 0; c0 < C; c0 += group, slot = (slot + 1) % kBulkSlots)
+  {
+    const uint32_t n = (C - c0 < group) ? C - c0 : group;
+    cudaStream_t st = ctx->bulk_stream[slot];
+    const size_t off = (size_t) c0 * ch_bytes, bytes = (size_t) n * ch_bytes;
+    CK (ctx, cudaMemcpyAsync (ctx->d_bulk_in[slot], reinterpret_cast<const char *> (h_in) + off, bytes, cudaMemcpyHostToDevice, st));
+    { const int rc = launch (ctx->d_bulk_in[slot], ctx->d_bulk_out[slot], c0, n, st); if (rc) return rc; }
+    CK (ctx, cudaMemcpyAsync (reinterpret_cast<char *> (h_out) + off, ctx->d_bulk_out[slot], bytes, cudaMemcpyDeviceToHost, st));
+  }
+  for (int s = 0; s < kBulkSlots; s++) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
+  return SLB_OK;
+}
+
 // SSB chains (f32 and q15) through host buffers: the batch is cut in TIME. Every slice carries all channels (strided 2-D copies
 // straight from / to the caller's [channels][frames] arrays), so each launch is as wide as the batch — the tensor-core
 // kernel wants one channel group per SM — and the slices are small (~64 MB), so the copy that cannot overlap anything (the
@@ -1524,23 +1586,7 @@ static int process_host_sliced (slb_ctx *ctx, const int16_t *h_in, int16_t *h_ou
   uint32_t slice = (uint32_t) std::min<size_t> (tile_bytes / ((size_t) block * 4), 0xFFFFFFFFu) / 1536u * 1536u;
   if (slice < 1536u) slice = 1536u;
   if (slice > frames) slice = frames;
-  const size_t need = (size_t) block * slice * 4;
-  if (need > ctx->bulk_bytes || !ctx->bulk_stream[0])
-  {
-    for (int s = 0; s < kBulkSlots; s++)
-    {
-      if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
-      if (need > ctx->bulk_bytes)
-      {
-        CK (ctx, cudaFree (ctx->d_bulk_in[s])); CK (ctx, cudaFree (ctx->d_bulk_out[s]));
-        ctx->d_bulk_in[s] = ctx->d_bulk_out[s] = nullptr;
-        CK (ctx, cudaMalloc (&ctx->d_bulk_in[s], need)); CK (ctx, cudaMalloc (&ctx->d_bulk_out[s], need));
-      }
-      if (!ctx->bulk_stream[s]) CK (ctx, cudaStreamCreateWithFlags (&ctx->bulk_stream[s], cudaStreamNonBlocking));
-      if (!ctx->bulk_done[s]) CK (ctx, cudaEventCreateWithFlags (&ctx->bulk_done[s], cudaEventDisableTiming));
-    }
-    if (need > ctx->bulk_bytes) ctx->bulk_bytes = need;
-  }
+  { const int rc = ensure_bulk (ctx, (size_t) block * slice * 4); if (rc) return rc; }
   for (int s = 0; s < kBulkSlots; s++)
     for (int e = 0; e < 3; e++)
       if (!ctx->slice_ev[s][e]) CK (ctx, cudaEventCreateWithFlags (&ctx->slice_ev[s][e], cudaEventDisableTiming));
@@ -1590,42 +1636,13 @@ static int process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint
   const bool chain = is_ssb_chain (ctx->cfg.chain);
   if (chain && frames % ctx->rx.hop != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the hop (384)");
   if (ctx->q15 && frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "frames must be a multiple of the 48-frame firmware block");
-  const uint32_t C = ctx->cfg.channels;
-  const size_t ch_bytes = (size_t) frames * 4;
   if (chain || ctx->q15) return process_host_sliced (ctx, h_in, h_out, frames);   // (the integer chain is exact, so any cut at a block boundary reproduces the uncut stream)
-  // PASS (the firmware as shipped): channels are independent, so the batch is cut into channel groups and H2D / copy kernel / D2H of
-  // consecutive groups overlap
-  uint32_t group = (uint32_t) ((size_t) (48u << 20) / ch_bytes);
-  if (group < 1) group = 1;
-  if (group > C) group = C;
-  const size_t need = (size_t) group * ch_bytes;
-  if (need > ctx->bulk_bytes)
-  {
-    for (int s = 0; s < kBulkSlots; s++)
-    {
-      if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
-      CK (ctx, cudaFree (ctx->d_bulk_in[s])); CK (ctx, cudaFree (ctx->d_bulk_out[s]));
-      ctx->d_bulk_in[s] = ctx->d_bulk_out[s] = nullptr;
-      CK (ctx, cudaMalloc (&ctx->d_bulk_in[s], need)); CK (ctx, cudaMalloc (&ctx->d_bulk_out[s], need));
-      if (!ctx->bulk_stream[s]) CK (ctx, cudaStreamCreateWithFlags (&ctx->bulk_stream[s], cudaStreamNonBlocking));
-      if (!ctx->bulk_done[s]) CK (ctx, cudaEventCreateWithFlags (&ctx->bulk_done[s], cudaEventDisableTiming));
-    }
-    ctx->bulk_bytes = need;
-  }
-  CK (ctx, cudaStreamSynchronize (ctx->stream));
-  int slot = 0;
-  for (uint32_t c0 = 0; c0 < C; c0 += group, slot = (slot + 1) % kBulkSlots)
-  {
-    const uint32_t n = (C - c0 < group) ? C - c0 : group;
-    cudaStream_t st = ctx->bulk_stream[slot];
-    const size_t bytes = (size_t) n * ch_bytes;
-    CK (ctx, cudaMemcpyAsync (ctx->d_bulk_in[slot], reinterpret_cast<const char *> (h_in) + (size_t) c0 * ch_bytes, bytes, cudaMemcpyHostToDevice, st));
-    CK (ctx, launch_copy_iq (ctx->d_bulk_in[slot], ctx->d_bulk_out[slot], (size_t) n * frames, st));
+  // PASS (the firmware as shipped)
+  return process_host_groups (ctx, h_in, h_out, frames, [&] (const int16_t *d_in, int16_t *d_out, uint32_t, uint32_t n, cudaStream_t st) -> int {
+    CK (ctx, launch_copy_iq (d_in, d_out, (size_t) n * frames, st));
     ctx->launches++;
-    CK (ctx, cudaMemcpyAsync (reinterpret_cast<char *> (h_out) + (size_t) c0 * ch_bytes, ctx->d_bulk_out[slot], bytes, cudaMemcpyDeviceToHost, st));
-  }
-  for (int s = 0; s < kBulkSlots; s++) if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
-  return SLB_OK;
+    return SLB_OK;
+  });
 }
 int slb_rx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames) { return process_host (ctx, h_in, h_out, frames, false); }
 int slb_tx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames) { return process_host (ctx, h_in, h_out, frames, true); }
@@ -1663,38 +1680,11 @@ int slb_chan_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, ui
   if (!ctx || !h_in || !h_out || frames == 0) return SLB_ERR_ARG;
   if (!ctx->chan) return fail (ctx, SLB_ERR_STATE, "not a channelizer context (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
-  const uint32_t S = ctx->cfg.channels;
-  const size_t st_bytes = (size_t) frames * 4;          // per stream, in and out alike (64 bins x frames/64 x 4 B)
-  uint32_t group = (uint32_t) ((size_t) (48u << 20) / st_bytes);
-  if (group < 1) group = 1;
-  if (group > S) group = S;
-  const size_t need = (size_t) group * st_bytes;
-  if (need > ctx->bulk_bytes)
-  {
-    for (int s = 0; s < kBulkSlots; s++)
-    {
-      if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
-      CK (ctx, cudaFree (ctx->d_bulk_in[s])); CK (ctx, cudaFree (ctx->d_bulk_out[s]));
-      ctx->d_bulk_in[s] = ctx->d_bulk_out[s] = nullptr;
-      CK (ctx, cudaMalloc (&ctx->d_bulk_in[s], need)); CK (ctx, cudaMalloc (&ctx->d_bulk_out[s], need));
-      if (!ctx->bulk_stream[s]) CK (ctx, cudaStreamCreateWithFlags (&ctx->bulk_stream[s], cudaStreamNonBlocking));
-      if (!ctx->bulk_done[s]) CK (ctx, cudaEventCreateWithFlags (&ctx->bulk_done[s], cudaEventDisableTiming));
-    }
-    ctx->bulk_bytes = need;
-  }
-  CK (ctx, cudaStreamSynchronize (ctx->stream));
-  int slot = 0;
-  for (uint32_t s0 = 0; s0 < S; s0 += group, slot = (slot + 1) % kBulkSlots)
-  {
-    const uint32_t n = (S - s0 < group) ? S - s0 : group;
-    cudaStream_t st = ctx->bulk_stream[slot];
-    const size_t bytes = (size_t) n * st_bytes;
-    CK (ctx, cudaMemcpyAsync (ctx->d_bulk_in[slot], reinterpret_cast<const char *> (h_in) + (size_t) s0 * st_bytes, bytes, cudaMemcpyHostToDevice, st));
-    int rc = chan64_launch (ctx, ctx->chan, ctx->d_bulk_in[slot], ctx->d_bulk_out[slot], s0, n, frames, ctx->sm_count, st, false);
-    if (rc) return rc;
-    CK (ctx, cudaMemcpyAsync (reinterpret_cast<char *> (h_out) + (size_t) s0 * st_bytes, ctx->d_bulk_out[slot], bytes, cudaMemcpyDeviceToHost, st));
-  }
-  for (int s = 0; s < kBulkSlots; s++) if (ctx->bulk_stream[s]) CK (ctx, cudaStreamSynchronize (ctx->bulk_stream[s]));
+  // (a stream takes as many bytes out as in: 64 bins x frames/64 x 4 B)
+  const int rc = process_host_groups (ctx, h_in, h_out, frames, [&] (const int16_t *d_in, int16_t *d_out, uint32_t s0, uint32_t n, cudaStream_t st) {
+    return chan64_launch (ctx, ctx->chan, d_in, d_out, s0, n, frames, ctx->sm_count, st, false);
+  });
+  if (rc) return rc;
   chan64_advance (ctx->chan);
   return SLB_OK;
 }
@@ -1712,10 +1702,25 @@ struct StateHeader
 };
 constexpr uint32_t kMagic = 0x534C4233u;   // 'SLB3'
 }
-static size_t state_bytes (const slb_ctx *ctx)
+// The device sections of the blob, in blob order (after the header and the mode bytes): the raw-input tail, the state records, the
+// four ring planes, the super-block being accumulated and the one processed last. The ping-pong buffers are saved from the current
+// side; a load resets ovl_parity and proc_cur to 0 first and so restores into side 0.
+struct StateSection { void *d; size_t bytes; };
+static std::vector<StateSection> state_sections (const slb_ctx *ctx)
 {
   const size_t C = ctx->cfg.channels, ovl = ctx->rx.fft_len - ctx->rx.hop, hop = ctx->rx.hop, R = ctx->geo.ring_frames;
-  return sizeof (StateHeader) + C /*modes*/ + C * ovl * 4 + C * 8 * 4 + 4 * C * R * 2 + C * hop * 4 * 2 + (ctx->chan ? chan64_state_bytes (ctx->chan) : 0) + (ctx->q15 ? rxq15_state_bytes (ctx->q15) : 0) + 2 * C * 4 * sizeof (uint32_t) /* per-channel ring pointers */;
+  std::vector<StateSection> s = { { ctx->d_ovl[ctx->ovl_parity], C * ovl * 4 }, { ctx->d_state, C * 8 * 4 } };
+  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) s.push_back ({ ctx->d_ring[w][k], C * R * 2 });
+  s.push_back ({ ctx->d_acc, C * hop * 4 });
+  s.push_back ({ ctx->d_proc[ctx->proc_cur], C * hop * 4 });
+  return s;
+}
+static size_t state_bytes (const slb_ctx *ctx)
+{
+  const size_t C = ctx->cfg.channels;
+  size_t n = sizeof (StateHeader) + C /*modes*/;
+  for (const StateSection &s : state_sections (ctx)) n += s.bytes;
+  return n + (ctx->chan ? chan64_state_bytes (ctx->chan) : 0) + (ctx->q15 ? rxq15_state_bytes (ctx->q15) : 0) + 2 * C * 4 * sizeof (uint32_t) /* per-channel ring pointers */;
 }
 int slb_state_size (const slb_ctx *ctx, size_t *bytes) { if (!ctx || !bytes) return SLB_ERR_ARG; *bytes = state_bytes (ctx); return SLB_OK; }
 
@@ -1724,7 +1729,7 @@ int slb_state_save (slb_ctx *ctx, void *buf, size_t bytes)
   if (!ctx || !buf || bytes < state_bytes (ctx)) return SLB_ERR_ARG;
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   CK (ctx, cudaStreamSynchronize (ctx->stream));
-  const size_t C = ctx->cfg.channels, ovl = ctx->rx.fft_len - ctx->rx.hop, hop = ctx->rx.hop, R = ctx->geo.ring_frames;
+  const size_t C = ctx->cfg.channels;
   char *p = static_cast<char *> (buf);
   StateHeader h{};
   h.magic = kMagic; h.channels = (uint32_t) C; h.fs = ctx->cfg.fs; h.chain = ctx->cfg.chain; h.fft_len = ctx->rx.fft_len; h.hop = ctx->rx.hop;
@@ -1734,11 +1739,7 @@ int slb_state_save (slb_ctx *ctx, void *buf, size_t bytes)
   h.ring_pc = ctx->ring_pc ? 1u : 0u;
   std::memcpy (p, &h, sizeof h); p += sizeof h;
   std::memcpy (p, ctx->mode_host.data (), C); p += C;
-  CK (ctx, cudaMemcpy (p, ctx->d_ovl[ctx->ovl_parity], C * ovl * 4, cudaMemcpyDeviceToHost)); p += C * ovl * 4;
-  CK (ctx, cudaMemcpy (p, ctx->d_state, C * 8 * 4, cudaMemcpyDeviceToHost)); p += C * 8 * 4;
-  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) { CK (ctx, cudaMemcpy (p, ctx->d_ring[w][k], C * R * 2, cudaMemcpyDeviceToHost)); p += C * R * 2; }
-  CK (ctx, cudaMemcpy (p, ctx->d_acc, C * hop * 4, cudaMemcpyDeviceToHost)); p += C * hop * 4;
-  CK (ctx, cudaMemcpy (p, ctx->d_proc[ctx->proc_cur], C * hop * 4, cudaMemcpyDeviceToHost)); p += C * hop * 4;
+  for (const StateSection &s : state_sections (ctx)) { CK (ctx, cudaMemcpy (p, s.d, s.bytes, cudaMemcpyDeviceToHost)); p += s.bytes; }
   if (ctx->chan) { CK (ctx, cudaDeviceSynchronize ()); if (chan64_state_save (ctx->chan, p)) return fail (ctx, SLB_ERR_CUDA, "chan64 state save failed"); p += chan64_state_bytes (ctx->chan); }
   if (ctx->q15) { CK (ctx, cudaDeviceSynchronize ()); if (rxq15_state_save (ctx->q15, p)) return fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state save failed"); p += rxq15_state_bytes (ctx->q15); }
   for (int w = 0; w < 2; w++)
@@ -1757,7 +1758,7 @@ int slb_state_load (slb_ctx *ctx, const void *buf, size_t bytes)
 {
   if (!ctx || !buf || bytes < state_bytes (ctx)) return SLB_ERR_ARG;
   CK (ctx, cudaSetDevice (ctx->cfg.device));
-  const size_t C = ctx->cfg.channels, ovl = ctx->rx.fft_len - ctx->rx.hop, hop = ctx->rx.hop, R = ctx->geo.ring_frames;
+  const size_t C = ctx->cfg.channels;
   const char *p = static_cast<const char *> (buf);
   StateHeader h; std::memcpy (&h, p, sizeof h); p += sizeof h;
   if (h.magic != kMagic || h.channels != C || h.fs != ctx->cfg.fs || h.chain != ctx->cfg.chain || h.fft_len != ctx->rx.fft_len || h.hop != ctx->rx.hop)
@@ -1768,11 +1769,7 @@ int slb_state_load (slb_ctx *ctx, const void *buf, size_t bytes)
   p += C;
   CK (ctx, cudaMemcpy (ctx->d_slot, ctx->slot_host.data (), C, cudaMemcpyHostToDevice));
   ctx->ovl_parity = 0; ctx->proc_cur = 0;
-  CK (ctx, cudaMemcpy (ctx->d_ovl[0], p, C * ovl * 4, cudaMemcpyHostToDevice)); p += C * ovl * 4;
-  CK (ctx, cudaMemcpy (ctx->d_state, p, C * 8 * 4, cudaMemcpyHostToDevice)); p += C * 8 * 4;
-  for (int w = 0; w < 2; w++) for (int k = 0; k < 2; k++) { CK (ctx, cudaMemcpy (ctx->d_ring[w][k], p, C * R * 2, cudaMemcpyHostToDevice)); p += C * R * 2; }
-  CK (ctx, cudaMemcpy (ctx->d_acc, p, C * hop * 4, cudaMemcpyHostToDevice)); p += C * hop * 4;
-  CK (ctx, cudaMemcpy (ctx->d_proc[0], p, C * hop * 4, cudaMemcpyHostToDevice)); p += C * hop * 4;
+  for (const StateSection &s : state_sections (ctx)) { CK (ctx, cudaMemcpy (s.d, p, s.bytes, cudaMemcpyHostToDevice)); p += s.bytes; }
   if (ctx->chan) { CK (ctx, cudaDeviceSynchronize ()); if (chan64_state_load (ctx->chan, p)) return fail (ctx, SLB_ERR_CUDA, "chan64 state load failed"); p += chan64_state_bytes (ctx->chan); }
   if (ctx->q15) { CK (ctx, cudaDeviceSynchronize ()); if (rxq15_state_load (ctx->q15, p)) return fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state load failed"); p += rxq15_state_bytes (ctx->q15); }
   ctx->ring_pc = false;
