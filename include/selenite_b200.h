@@ -55,6 +55,9 @@ extern "C" {
 #define SLB_CHAIN_TX_SSB_Q15  6    /* all-integer phasing SSB modulator: mic (L of L=R) -> the fir_q15 Hilbert pair of RX-SSB-q15 -> rail
                                       order by sideband -> q15 ALC -> I/Q pack (bit-exact, DESIGN.md §3.7) */
 
+#define SLB_CHAIN_RX_Q15      7    /* all-mode integer receiver: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_RX_SSB_Q15;
+                                      AM by arm_cmplx_mag_q15, FM by an integer limiter-discriminator (DESIGN.md §3.8); bit-exact */
+
 #define SLB_MAX_STAGES 4
 #define SLB_MAX_MASKS  8
 
@@ -138,6 +141,24 @@ typedef struct
   uint32_t bq_stages; int32_t bq_postshift; int16_t bq_coeffs[6 * SLB_MAX_STAGES];
 } slb_rx_q15_params;
 
+/* The AM and FM detectors of SLB_CHAIN_RX_Q15 (DESIGN.md §3.8); slb_rx_q15_params keeps the SSB pair and the AGC, which all modes share.
+ * Per channel and 48-frame block, a = arm_fir_q15 (I, taps), b = arm_fir_q15 (Q, taps) with the mode's taps on both rails, then
+ *   AM: v = arm_cmplx_mag_q15 (a, b) (2.14: about |z| / 2; the carrier's DC stays in the audio)
+ *   FM: m_n = arm_cmplx_mag_q15 (a_n, b_n), x_n = a_{n-1} b_n - b_{n-1} a_n (int64),
+ *       v_n = sat16 (trunc (x_n 2^13 / max (m_{n-1} m_n, fm_floor))): q15 sin of the phase step, the sign of Im (z[n] conj z[n-1])
+ * then the block peak [arm_abs_q15 + arm_max_q15], the gain law of slb_rx_q15_params and arm_scale_q15, written L = R. z[-1] of a call
+ * is the current mode's FIR output at the frame before it (zero at a stream start); after a mode change between calls the FIRs and the
+ * detector behave as if the channel had always been in the new mode, and the AGC's peak window carries over unchanged.
+ * SLB_CHAIN_RX_Q15 runs on the tcgen05 kernel only: a tap >= 32640 here or in slb_rx_q15_params, fm_floor < 1, bq_stages != 0 or
+ * agc_window > 17 is refused with SLB_ERR_UNSUPPORTED and the parameters stay as they were; tuning is refused too.
+ * Defaults (48 kHz): 64-tap Kaiser (beta 6) low-passes of DC gain 1, -6 dB at 3 kHz (AM) and 6 kHz (FM); fm_floor = 2^18. */
+typedef struct
+{
+  int16_t am_taps[SLB_Q15_TAPS];         /* b[0..63], q15, natural order */
+  int16_t fm_taps[SLB_Q15_TAPS];
+  int32_t fm_floor;                      /* >= 1; 2^18 = the f32 discriminator's 2^-10 soft squelch in these units */
+} slb_rx_q15_mode_params;
+
 /* ---- life cycle ---- */
 int  slb_create (const slb_config *cfg, slb_ctx **out);
 void slb_destroy (slb_ctx *ctx);
@@ -160,6 +181,10 @@ int slb_get_tx_mod_params (const slb_ctx *ctx, slb_tx_mod_params *p);
 int slb_default_rx_q15_params (uint32_t fs, slb_rx_q15_params *out);
 int slb_set_rx_q15_params (slb_ctx *ctx, const slb_rx_q15_params *p);
 int slb_get_rx_q15_params (const slb_ctx *ctx, slb_rx_q15_params *p);
+/* SLB_CHAIN_RX_Q15 contexts only (others: SLB_ERR_STATE) */
+int slb_default_rx_q15_mode_params (uint32_t fs, slb_rx_q15_mode_params *out);
+int slb_set_rx_q15_mode_params (slb_ctx *ctx, const slb_rx_q15_mode_params *p);
+int slb_get_rx_q15_mode_params (const slb_ctx *ctx, slb_rx_q15_mode_params *p);
 int slb_set_mask (slb_ctx *ctx, uint8_t mode, const float *mask);   /* host, 2*fft_len floats */
 int slb_get_mask (const slb_ctx *ctx, uint8_t mode, float *mask);
 /* which kernel serves the RX-SSB-f32 chain (DESIGN.md §4A): SLB_RX_PATH_AUTO = the tensor-core FIR kernel for every channel
@@ -237,6 +262,7 @@ int slb_rx_set_debug_taps (slb_ctx *ctx, float *d_audio, float *d_gain);
  * pointer, written by the next slb_tx_process_device call(s) for FM channels when non-NULL (other channels' rows are left alone) */
 int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase);
 /* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48].
+ * RX-Q15: the same, the pre-AGC detector output of each channel's mode (AM: the 2.14 magnitude, FM: the discriminator).
  * TX-SSB-q15: d_audio receives the pre-ALC (I, Q) int16[channels][frames][2] (after the rail order), d_gain the same gain words. */
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain);
 
@@ -388,6 +414,9 @@ int slb_design_q15_tc_block (const int16_t taps_i[64], const int16_t taps_q[64],
 /* the TX planes of the same kernel (TX-SSB-q15): window = int16[112][2] L=R mic frames from 64 before the block, out = the 48 arm_fir_q15
  * results of L with taps_i (rail fi), then with taps_q (rail fq), before the rail order; R meets zero weight */
 int slb_design_q15_tc_tx_block (const int16_t taps_i[64], const int16_t taps_q[64], const int16_t *window /* [112][2] L=R */, int32_t out96[96]);
+/* the FM planes of the same kernel (RX-Q15): window = int16[112][2] I/Q frames from 64 before the block, out = the 49 arm_fir_q15 results
+ * of rail I with taps at frames -1 .. 47 of the block, then the same of rail Q; SLB_ERR_UNSUPPORTED when a tap does not split */
+int slb_design_q15_tc_fm_block (const int16_t taps[64], const int16_t *window, int32_t out98[98]);
 int slb_design_mask (uint32_t fs, uint8_t mode, float *mask_re_im);
 /* tables of the tensor-core kernel's time-parallel biquad for blocks of 48 samples: Mp[4][16] = A^(48 k), M192[16], Cresp[48][4] */
 int slb_biquad_tc_tables (const float coef10[10], float *Mp64, float *M192, float *Cresp192);
@@ -404,7 +433,7 @@ int slb_sync (slb_ctx *ctx);
 
 /* ---- single-channel drop-in with the firmware's own names and signatures (Core/Inc/dsp_if.h:42-51).
  * They drive one process-global 1-channel context on device 0 (env SELENITE_B200_DEVICE, SELENITE_B200_FS,
- * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15|tx_ssb_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
+ * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15|tx_ssb_q15|rx_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
  * they return void; failures are reported through slb_dropin_status(). ---- */
 void DSP_Init (void);
 void DSP_Set_RX (void);

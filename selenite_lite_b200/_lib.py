@@ -35,6 +35,10 @@ class RxQ15Params(C.Structure):
                 ("bq_stages", C.c_uint32), ("bq_postshift", C.c_int32), ("bq_coeffs", C.c_int16 * 24)]
 
 
+class RxQ15ModeParams(C.Structure):
+    _fields_ = [("am_taps", C.c_int16 * 64), ("fm_taps", C.c_int16 * 64), ("fm_floor", C.c_int32)]
+
+
 class FeederIo(C.Structure):
     _fields_ = [("adc", C.c_void_p), ("usb_in", C.c_void_p), ("usb_out", C.c_void_p), ("dac", C.c_void_p)]
 

@@ -40,7 +40,7 @@ struct slb_ctx
   std::vector<uint8_t> mode_host;      // [C]
   bool tx_mode = false;
   Chan64State *chan = nullptr;         // SLB_CHAIN_CHAN64_F32 only
-  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15 and SLB_CHAIN_TX_SSB_Q15 only
+  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15, SLB_CHAIN_TX_SSB_Q15 and SLB_CHAIN_RX_Q15 only
 
   // device: chain constants + carried state
   float *d_masks = nullptr; uint8_t *d_slot = nullptr; float *d_twiddle = nullptr;
@@ -61,6 +61,9 @@ struct slb_ctx
   std::vector<int32_t> tune_inc; uint32_t n_tuned = 0;
   struct TuneList : DevList { uint32_t n = 0, n_all = 0; };
   std::map<uint64_t, TuneList> tune_lists; uint64_t tune_version = 0;
+  // RX-Q15: the channels of a range by detector kind (q15_kind_lists), cached per range like tc_lists and rebuilt on mode_version
+  struct KindList : DevList { uint32_t n[3] = {}; };
+  std::map<uint64_t, KindList> q15_lists;
   int16_t *d_ovl[2] = { nullptr, nullptr }; int ovl_parity = 0;
   float *d_state = nullptr; unsigned *d_flag = nullptr;
   unsigned flag_base = 0;
@@ -105,7 +108,7 @@ static inline bool is_f32_tx_chain (uint32_t chain) { return chain == SLB_CHAIN_
 static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || is_f32_tx_chain (chain); }
 // the direction a context was created for: slb_tx_process_* serve these chains, slb_rx_process_* the others
 static inline bool is_tx_direction (uint32_t chain) { return is_f32_tx_chain (chain) || chain == SLB_CHAIN_TX_SSB_Q15; }
-static inline bool is_q15_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15; }
+static inline bool is_q15_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15 || chain == SLB_CHAIN_RX_Q15; }
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
 
@@ -147,6 +150,28 @@ namespace sl {
 int ctx_device (const slb_ctx *ctx) { return ctx->cfg.device; }
 size_t ctx_channels (const slb_ctx *ctx) { return ctx->cfg.channels; }
 int ctx_fail (slb_ctx *ctx, int code, const char *msg) { return fail (ctx, code, msg); }
+// RX-Q15 (sl_internal.h): the channels of [ch0, ch0 + nch) by kind. A range of SSB-style channels only needs no list and gets none.
+int q15_kind_lists (slb_ctx *ctx, uint32_t ch0, uint32_t nch, Q15KindLists *out)
+{
+  auto kind = [&] (uint32_t c) { const uint8_t m = ctx->mode_host[ch0 + c]; return m == SLB_MODE_AM ? 1 : (m == SLB_MODE_FM ? 2 : 0); };
+  *out = Q15KindLists{};
+  for (uint32_t c = 0; c < nch; c++) out->n[kind (c)]++;
+  if (out->n[0] == nch) return SLB_OK;
+  slb_ctx::KindList &l = ctx->q15_lists[((uint64_t) ch0 << 32) | nch];
+  if (l.version != ctx->mode_version)
+  {
+    std::vector<uint32_t> pack;
+    pack.reserve (nch);
+    for (int k = 0; k < 3; k++)
+      for (uint32_t c = 0; c < nch; c++)
+        if (kind (c) == k) pack.push_back (c);
+    const int rc = upload_list (ctx, l, pack); if (rc) return rc;
+    for (int k = 0; k < 3; k++) l.n[k] = out->n[k];
+    l.version = ctx->mode_version;
+  }
+  out->d[0] = l.d; out->d[1] = l.d + l.n[0]; out->d[2] = l.d + l.n[0] + l.n[1];
+  return SLB_OK;
+}
 void ctx_count_launch (slb_ctx *ctx, unsigned n) { ctx->launches += n; }
 void *ctx_scratch (slb_ctx *ctx, size_t bytes)
 {
@@ -320,7 +345,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   int rc = upload_chain_constants (ctx);
   if (rc == SLB_OK) rc = reset_state (ctx);
   if (rc == SLB_OK && cfg->chain == SLB_CHAIN_CHAN64_F32) rc = chan64_create (ctx, C, cfg->fs, &ctx->chan);
-  if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, cfg->chain == SLB_CHAIN_TX_SSB_Q15, &ctx->q15);
+  if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, cfg->chain == SLB_CHAIN_TX_SSB_Q15, cfg->chain == SLB_CHAIN_RX_Q15, &ctx->q15);
   if (rc != SLB_OK) { g_create_error = ctx->err; slb_destroy (ctx); return rc; }
   *out = ctx;
   return SLB_OK;
@@ -334,7 +359,7 @@ void slb_destroy (slb_ctx *ctx)
   chan64_destroy (ctx->chan);
   rxq15_destroy (ctx->q15);
   cudaFree (ctx->d_masks); cudaFree (ctx->d_slot); cudaFree (ctx->d_twiddle); cudaFree (ctx->d_planes); cudaFree (ctx->d_tx_planes); cudaFree (ctx->d_am_planes);
-  drop_lists (ctx, ctx->tc_lists, 0); drop_lists (ctx, ctx->tune_lists, 0);
+  drop_lists (ctx, ctx->tc_lists, 0); drop_lists (ctx, ctx->tune_lists, 0); drop_lists (ctx, ctx->q15_lists, 0);
   for (int p = 0; p < 2; p++) { cudaFree (ctx->d_ovl[p]); cudaFree (ctx->d_proc[p]); }
   cudaFree (ctx->d_state); cudaFree (ctx->d_flag);
   cudaFree (ctx->d_acc_off);
@@ -447,6 +472,22 @@ int slb_get_rx_q15_params (const slb_ctx *ctx, slb_rx_q15_params *p)
 {
   if (!ctx || !p || !ctx->q15) return SLB_ERR_ARG;
   *p = *rxq15_params (ctx->q15);
+  return SLB_OK;
+}
+int slb_default_rx_q15_mode_params (uint32_t fs, slb_rx_q15_mode_params *out) { return design_default_rx_q15_modes (fs, out); }
+int slb_set_rx_q15_mode_params (slb_ctx *ctx, const slb_rx_q15_mode_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->q15 || ctx->cfg.chain != SLB_CHAIN_RX_Q15) return fail (ctx, SLB_ERR_STATE, "not an RX-Q15 context");
+  CK (ctx, cudaSetDevice (ctx->cfg.device));
+  CK (ctx, cudaStreamSynchronize (ctx->stream));
+  return rxq15_set_mode_params (ctx, ctx->q15, p);
+}
+int slb_get_rx_q15_mode_params (const slb_ctx *ctx, slb_rx_q15_mode_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->q15 || !rxq15_mode_params (ctx->q15)) return SLB_ERR_STATE;
+  *p = *rxq15_mode_params (ctx->q15);
   return SLB_OK;
 }
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain)
@@ -608,11 +649,12 @@ int SLB_DSP_Key (slb_ctx *ctx, const uint8_t *key_down)
 static int check_mode (slb_ctx *ctx, uint8_t mode)
 {
   if (mode_to_mask_slot (mode) < 0) return fail (ctx, SLB_ERR_UNSUPPORTED, "not an FT-817 mode byte (LSB, USB, CW, CW-R, AM, FM, DIG, PKT are served; rxtx_if.h:33-43)");
-  if (mode == SLB_MODE_AM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 chain (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only; "
+  const bool all_mode = ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 || ctx->cfg.chain == SLB_CHAIN_PASS || ctx->cfg.chain == SLB_CHAIN_TX_F32 || ctx->cfg.chain == SLB_CHAIN_RX_Q15;
+  if (mode == SLB_MODE_AM && !all_mode)
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 and RX-Q15 chains (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only; "
                                            "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
-  if (mode == SLB_MODE_FM && ctx->cfg.chain != SLB_CHAIN_RX_SSB_F32 && ctx->cfg.chain != SLB_CHAIN_PASS && ctx->cfg.chain != SLB_CHAIN_TX_F32)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 chain (limiter-discriminator) and the TX-f32 chain (FM modulator) only; "
+  if (mode == SLB_MODE_FM && !all_mode)
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 and RX-Q15 chains (limiter-discriminator) and the TX-f32 chain (FM modulator) only; "
                                            "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
   if (mode == SLB_MODE_FM && ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 && !ctx->tc_ok[kFmMaskSlot])
     return fail (ctx, SLB_ERR_UNSUPPORTED, "the FM slot has no tensor-core planes (fft_len must be 512 and the FM mask a 129-tap FIR)");
@@ -628,7 +670,7 @@ int SLB_DSP_Set_Mode_Channel (slb_ctx *ctx, uint32_t ch, uint8_t mode)
   if (ctx->q15)
   {
     CK (ctx, cudaStreamSynchronize (ctx->stream));
-    ctx->mode_host[ch] = mode;
+    ctx->mode_host[ch] = mode; ctx->mode_version++;                    // (RX-Q15: the kind lists follow the modes)
     return rxq15_set_sideband (ctx, ctx->q15, ch, 1, mode_to_lsb (mode));
   }
   ctx->mode_host[ch] = mode; ctx->slot_host[ch] = (uint8_t) slot; ctx->mode_version++;
@@ -654,6 +696,7 @@ int SLB_DSP_Set_Mode (slb_ctx *ctx, uint8_t mode)     // dsp_if.c:367-370 is the
   if (ctx->q15)
   {
     CK (ctx, cudaStreamSynchronize (ctx->stream));
+    ctx->mode_version++;
     return rxq15_set_sideband (ctx, ctx->q15, 0, ctx->cfg.channels, mode_to_lsb (mode));
   }
   std::fill (ctx->slot_host.begin (), ctx->slot_host.end (), (uint8_t) slot); ctx->mode_version++;
@@ -957,6 +1000,7 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
       // the integer chains demodulate (or modulate) a block in the call that delivers it (dsp_if.c:286-289): the channels that fired run through the
       // kernel (one launch per run of neighbours), the others carry their state over unchanged
       if (frames % ctx->geo.block_frames != 0) return fail (ctx, SLB_ERR_ARG, "with a q15 chain the block must be a whole number of 48-frame firmware blocks");
+      rc = drop_lists (ctx, ctx->q15_lists, 64); if (rc) return rc;        // (RX-Q15: the runs of active channels change from call to call)
       for (auto &r : channel_runs (C, is_on))
       {
         rc = rxq15_launch (ctx, ctx->q15, ctx->d_blk + (size_t) r.first * frames * 2, ctx->d_proc[0] + (size_t) r.first * frames * 2, r.first, r.second, frames, ctx->sm_count, ctx->stream, false);
@@ -1463,6 +1507,14 @@ int slb_design_q15_tc_block (const int16_t taps_i[64], const int16_t taps_q[64],
   q15_tc_apply_planes (planes.data (), window, out96);
   return SLB_OK;
 }
+int slb_design_q15_tc_fm_block (const int16_t taps[64], const int16_t *window, int32_t out98[98])
+{
+  if (!taps || !window || !out98) return SLB_ERR_ARG;
+  std::vector<uint8_t> planes (kTcQ15FmPlaneBytes);
+  if (!q15_tc_build_fm_planes (taps, planes.data ())) return SLB_ERR_UNSUPPORTED;
+  q15_tc_apply_fm_planes (planes.data (), window, out98);
+  return SLB_OK;
+}
 int slb_design_q15_tc_tx_block (const int16_t taps_i[64], const int16_t taps_q[64], const int16_t *window, int32_t out96[96])
 {
   if (!taps_i || !taps_q || !window || !out96) return SLB_ERR_ARG;
@@ -1812,7 +1864,8 @@ slb_ctx *dropin ()
     cfg.chain = (ch && std::strcmp (ch, "rx_ssb_f32") == 0) ? SLB_CHAIN_RX_SSB_F32 : (ch && std::strcmp (ch, "tx_ssb_f32") == 0) ? SLB_CHAIN_TX_SSB_F32
               : (ch && std::strcmp (ch, "tx_f32") == 0) ? SLB_CHAIN_TX_F32
               : (ch && std::strcmp (ch, "rx_ssb_q15") == 0) ? SLB_CHAIN_RX_SSB_Q15
-              : (ch && std::strcmp (ch, "tx_ssb_q15") == 0) ? SLB_CHAIN_TX_SSB_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
+              : (ch && std::strcmp (ch, "tx_ssb_q15") == 0) ? SLB_CHAIN_TX_SSB_Q15
+              : (ch && std::strcmp (ch, "rx_q15") == 0) ? SLB_CHAIN_RX_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
     g_dropin_status = slb_create (&cfg, &g_dropin);
     if (g_dropin_status != SLB_OK) std::fprintf (stderr, "selenite-b200: drop-in context failed: %s\n", slb_last_error (nullptr));
   }

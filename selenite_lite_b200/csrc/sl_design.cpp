@@ -158,6 +158,32 @@ int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p)
   return SLB_OK;
 }
 
+// RX-Q15's AM and FM detectors: 64-tap Kaiser (beta 6) windowed-sinc low-passes with the cut-off (-6 dB) at 3 kHz (AM) and 6 kHz
+// (FM), normalised to DC gain 1 in double, then llround to q15 (both rails use the same taps)
+int design_default_rx_q15_modes (uint32_t fs, slb_rx_q15_mode_params *p)
+{
+  if (!p || fs != 48000u) return p ? SLB_ERR_UNSUPPORTED : SLB_ERR_ARG;
+  std::memset (p, 0, sizeof *p);
+  const int T = SLB_Q15_TAPS;
+  const double beta = 6.0, mid = (T - 1) / 2.0;
+  auto lowpass = [&] (double fc_hz, int16_t *out)
+  {
+    const double fc = fc_hz / (double) fs;
+    double g[SLB_Q15_TAPS], dc = 0.0;
+    for (int n = 0; n < T; n++)
+    {
+      const double m = n - mid, x = 2.0 * fc * m, r = m / mid;
+      g[n] = 2.0 * fc * (std::sin (kPi * x) / (kPi * x)) * bessel_i0 (beta * std::sqrt (1.0 - r * r)) / bessel_i0 (beta);
+      dc += g[n];
+    }
+    for (int n = 0; n < T; n++) out[n] = (int16_t) std::llround (32768.0 * g[n] / dc);
+  };
+  lowpass (3000.0, p->am_taps);
+  lowpass (6000.0, p->fm_taps);
+  p->fm_floor = 1 << 18;
+  return SLB_OK;
+}
+
 // -----------------------------------------------------------------------------------------------------------
 // Time-parallel evaluation of the 2-stage df2T cascade (arm_biquad_cascade_df2T_f32.c:551-562 per sample):
 // with x = 0 the 4-vector s = {d1_0,d2_0,d1_1,d2_1} evolves linearly, s' = A s, and the cascade output is c.s.

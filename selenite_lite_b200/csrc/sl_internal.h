@@ -216,11 +216,19 @@ void chan64_advance (Chan64State *st);
 // ---- RX-SSB-q15 and TX-SSB-q15 (sl_rx_ssb_q15.cu): state object owned by the context ----
 struct RxQ15State;
 int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p);
-int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, RxQ15State **out);   // tx: TX-SSB-q15 (the same state)
+int design_default_rx_q15_modes (uint32_t fs, slb_rx_q15_mode_params *p);
+// tx: TX-SSB-q15, all_mode: RX-Q15 (the same state)
+int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, bool all_mode, RxQ15State **out);
 void rxq15_destroy (RxQ15State *st);
 int rxq15_reset (slb_ctx *ctx, RxQ15State *st);
 int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p);
 const slb_rx_q15_params *rxq15_params (const RxQ15State *st);
+int rxq15_set_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_mode_params *p);   // RX-Q15 only
+const slb_rx_q15_mode_params *rxq15_mode_params (const RxQ15State *st);                      // nullptr unless RX-Q15
+// RX-Q15: the channels of [ch0, ch0 + nch) by detector kind (Q15Kind kQ15Ssb, kQ15Am, kQ15Fm), as device lists of indices relative
+// to ch0 (sl_capi.cu: cached per range, rebuilt when a mode changes); d[k] is valid when n[k] > 0
+struct Q15KindLists { const uint32_t *d[3]; uint32_t n[3]; };
+int q15_kind_lists (slb_ctx *ctx, uint32_t ch0, uint32_t nch, Q15KindLists *out);
 void rxq15_set_debug (RxQ15State *st, int16_t *audio, uint32_t *gain);
 int rxq15_set_sideband (slb_ctx *ctx, RxQ15State *st, uint32_t ch0, uint32_t n, int lsb);
 int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_out, uint32_t ch0, uint32_t nch, uint32_t frames,
@@ -250,8 +258,14 @@ int launch_rx_am_tc (const RxAmTcLaunch &L, int sm_count, void *stream);
 
 // ---- RX-SSB-q15 on the tensor cores (sl_rx_q15_tc.cu): same chain, same state, bit-identical results; TX-SSB-q15 (tx) runs only here ----
 constexpr size_t kTcQ15PlaneBytes = 7 * 24 * 256;
+constexpr size_t kTcQ15FmPlaneBytes = 7 * 26 * 256;   // RX-Q15 FM: 208 rows, the outputs at frame -1 too
 bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes /* kTcQ15PlaneBytes */, bool tx);
+bool q15_tc_build_fm_planes (const int16_t *taps, uint8_t *planes /* kTcQ15FmPlaneBytes */);
 void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96);
+void q15_tc_apply_fm_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out98);
+// detector kind of a launch: the SSB demodulator (RX-SSB-q15, and RX-Q15's SSB-style modes), the SSB modulator (TX-SSB-q15), RX-Q15's
+// AM and FM detectors
+enum Q15Kind : int { kQ15Ssb = 0, kQ15Tx = 1, kQ15Am = 2, kQ15Fm = 3 };
 struct RxQ15TcLaunch
 {
   const int16_t *in; int16_t *out;
@@ -259,7 +273,10 @@ struct RxQ15TcLaunch
   const uint8_t *planes, *lsb; int16_t *audio_dbg; uint32_t *gain_dbg;
   const int16_t *rel;                      // host, [SLB_Q15_WIN]
   uint32_t channels, frames, window; int32_t target, floor_; uint32_t gmax;
-  bool tx;                                 // TX-SSB-q15: mic frames in, I/Q frames out, audio_dbg = pre-ALC I/Q [C][T][2]
+  int kind;                                // Q15Kind. kQ15Tx: mic frames in, I/Q frames out, audio_dbg = pre-ALC I/Q [C][T][2]
+  const uint32_t *list;                    // device, [channels] channel indices relative to in / out / tails / peaks / lsb; nullptr:
+                                           // channels 0 .. channels-1 (kQ15Ssb and kQ15Tx only)
+  int32_t fm_floor;                        // kQ15Fm
 };
 int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream);
 

@@ -17,6 +17,12 @@
 // TX-SSB-q15 (kTx, DESIGN.md §3.7) is the same kernel: the input frames are the mic (L = R), both rails' taps sit at the L byte
 // positions of the planes (R gets zero weight, so R is ignored), and the epilogue keeps (I, Q) = (fi, fq) or (fq, fi) by sideband
 // instead of mixing, takes the block peak over |I| and |Q|, scales both rails with one gain word and stores I/Q frames.
+//
+// RX-Q15 (DESIGN.md §3.8) adds two detectors. AM: the same contraction with a real low-pass on both rails, and arm_cmplx_mag_q15
+// instead of the mixer. FM: planes of N = 208 that also give each rail's FIR output at frame -1 (the sample before the block,
+// whose 64-tap window is frames 0..63 of the 112-frame window), so every block holds z[n-1] for its first sample; the epilogue
+// runs arm_cmplx_mag_q15 and the integer limiter-discriminator per sample. A launch of these kinds (and of the SSB kind in a
+// context that mixes kinds) works on a list of channels: rxq15_launch groups a channel range by kind.
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdlib>
@@ -35,7 +41,6 @@ constexpr int kChunksHist = kHist / 8;   // 8
 constexpr int kChunksNew = kSuper / 8;   // 96
 constexpr int kPlaneBytes = (kChunksHist + kChunksNew) * kChunkBytes;   // 13312
 constexpr int kKSteps = 7;               // (64 + 48) frames * 2 bytes / 32
-constexpr int kBStep = 24 * 256;         // 192 rows x 32 bytes per K-step
 constexpr int kRawRow = kSuper * 4 + 16, kHistRow = kHist * 4 + 16;
 #ifndef SL_Q15TC_SPLIT
 #define SL_Q15TC_SPLIT 0                   // A/B: both epilogue sets work on every supertile, 24 of a block's 48 samples each.
@@ -58,13 +63,21 @@ constexpr int kMmaWarp = kEpiWarps + kConvWarps, kProdWarp = kMmaWarp + 1, kThre
                                              one more live register in the epilogue, 430 vs 492 Gsamples/s */
 #endif
 constexpr unsigned kPSlots = SL_Q15TC_PSLOTS;
-constexpr int kTmemCols = 512;           // xh products in columns [0,192), xl products in [192,384)
+constexpr int kTmemCols = 512;           // xh products in columns [0,N), xl products in [N,2N) (N = 192; FM 208)
 
-struct Smem
+// detector kinds (template parameter of the kernel): the two SSB chains on contiguous channels, and the kinds of RX-Q15, which work
+// on a channel list (kKindRxList: the SSB detector of kKindRx)
+enum Kind : int { kKindRx = 0, kKindTx = 1, kKindAm = 2, kKindFm = 3, kKindRxList = 4 };
+template <int K> constexpr int kRowsN = K == kKindFm ? 208 : 192;                  // B rows = MMA N
+template <int K> constexpr int kBStepK = kRowsN<K> / 8 * 256;
+template <int K> constexpr size_t kPlaneBK = (size_t) kKSteps * kBStepK<K>;   // 43008; FM 46592 (= kTcQ15FmPlaneBytes)
+static_assert (kPlaneBK<kKindRx> == kTcQ15PlaneBytes && kPlaneBK<kKindFm> == kTcQ15FmPlaneBytes, "plane sizes");
+
+template <size_t kBBytes> struct SmemT
 {
   static constexpr size_t a = 0;
   static constexpr size_t b = a + 2 * 2 * kPlaneBytes;
-  static constexpr size_t raw = b + kTcQ15PlaneBytes;
+  static constexpr size_t raw = b + kBBytes;
   static constexpr size_t hist = raw + kRawStages * kJ * kRawRow;
   static constexpr size_t pk = hist + kRawStages * kJ * kHistRow;                // [4 tiles][16][8] int: block peaks of the last supertiles
   static constexpr size_t pkc = pk + (SL_Q15TC_SPLIT ? 2 : 1) * 4 * kQ * kJ * 4;                   // [sets][16][8] int: peaks before the stream start, by 16 - age
@@ -73,6 +86,8 @@ struct Smem
   static constexpr size_t tmem_ptr = bars + n_bars * 8;
   static constexpr size_t bytes = tmem_ptr + 16;
 };
+using Smem = SmemT<kTcQ15PlaneBytes>;
+static_assert (SmemT<kTcQ15FmPlaneBytes>::bytes <= 227 * 1024, "one CTA per SM");
 
 struct KParams
 {
@@ -84,6 +99,7 @@ struct KParams
   int16_t rel[kWin];
   uint32_t channels, frames, blocks, supers, gsz, n_groups, window;
   int32_t target, floor_; uint32_t gmax;
+  const uint32_t *list; int32_t fm_floor;      // channel list (kinds kKindAm, kKindFm, kKindRxList); FM: the discriminator's floor
 };
 
 #include "sl_tc_common.cuh"
@@ -95,10 +111,54 @@ __device__ __forceinline__ int sat16 (int v) { short r; asm ("cvt.sat.s16.s32 %0
 __device__ __forceinline__ int sat16 (int v) { return max (-32768, min (32767, v)); }
 #endif
 
-template <bool kTx>
+// arm_sqrt_q15 (FastMathFunctions/arm_sqrt_q15.c) as oracle/port/stats_cmplx.c restates it, every cast included: normalise by an even
+// shift, a float seed (a power-of-two multiply, the 0x5f3759df bit trick), three q15 Newton steps, multiply back, undo half the shift
+__device__ __forceinline__ int sqrt_q15 (int number)
+{
+  if (number <= 0) return 0;
+  const int sh = (__clz (number) - 17) & ~1;                                      // signBits1, or signBits1 - 1 when it is odd
+  number = (int) (int16_t) (number << sh);
+  const int half = number >> 1, temp1 = number;
+  const float tf = __int_as_float (0x5f3759df - (__float_as_int ((float) number * 3.051757812500000e-005f) >> 1));
+  int var1 = (int) (int16_t) (int) (tf * 16384.0f);
+#pragma unroll
+  for (int it = 0; it < 3; it++)
+  {
+    const int sq = (int) (int16_t) ((var1 * var1) >> 15);
+    const int hs = (int) (int16_t) ((sq * half) >> 15);
+    var1 = (int) (int16_t) ((int) (int16_t) ((var1 * (0x3000 - hs)) >> 15) << 2);
+  }
+  var1 = (int) (int16_t) ((int) (int16_t) ((temp1 * var1) >> 15) << 1);
+  return var1 >> (sh / 2);
+}
+// arm_cmplx_mag_q15 (arm_cmplx_mag_q15.c): sqrt_q15 ((re^2 + im^2) >> 17), 2.14 format
+__device__ __forceinline__ int cmag_q15 (int re, int im) { return sqrt_q15 ((int) (((unsigned) (re * re) + (unsigned) (im * im)) >> 17)); }
+// the limiter-discriminator (ours, DESIGN.md §3.8): sat16 (trunc ((x 2^13) / max (m_prev m, floor))), x = a_prev b - b_prev a. |quotient|
+// < 2^15 unless it saturates, so a float reciprocal estimate is within one of it and one integer correction makes it exact
+__device__ __forceinline__ int fm_disc (int pa, int pb, int pm, int a, int b, int m, int floor_)
+{
+  const long long x = (long long) pa * b - (long long) pb * a;
+  const long long den = max (pm * m, floor_);                                    // pm m <= 23170^2 < 2^31
+  const long long N = (x < 0 ? -x : x) << 13;
+  int q;
+  if (N >= (den << 15)) q = 32768;
+  else
+  {
+    q = (int) ((float) N * __frcp_rn ((float) den));
+    const long long r = N - (long long) q * den;
+    if (r < 0) q--;
+    else if (r >= den) q++;
+  }
+  return x < 0 ? -q : min (q, 32767);
+}
+
+template <int kKind>
 __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_constant__ KParams P)
 {
-  static_assert (!(kTx && SL_Q15TC_SPLIT), "the split-epilogue A/B variant serves RX only");
+  constexpr bool kTx = kKind == kKindTx, kList = kKind >= kKindAm;
+  constexpr int kN = kRowsN<kKind>;                                              // xl products from column kN on
+  using Smem = SmemT<kPlaneBK<kKind>>;
+  static_assert (!(kKind != kKindRx && SL_Q15TC_SPLIT), "the split-epilogue A/B variant serves RX only");
   extern __shared__ __align__ (1024) unsigned char smem[];
   unsigned char *sA = smem + Smem::a, *sB = smem + Smem::b, *sRaw = smem + Smem::raw, *sHist = smem + Smem::hist;
   int *sPk = reinterpret_cast<int *> (smem + Smem::pk), *sPkC = reinterpret_cast<int *> (smem + Smem::pkc);
@@ -138,14 +198,16 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
   const uint32_t supers = P.supers;
   // channels of group g: [g * gsz, g * gsz + nv); rows beyond nv repeat the last channel and are never stored
   auto group_nv = [&] (uint32_t g) { return min (P.gsz, P.channels - g * P.gsz); };
+  // channel of row jj of group g: contiguous, or the list entry (list kinds; P.channels = the list's length)
+  auto chan = [&] (uint32_t g, uint32_t jj) -> uint32_t { if constexpr (kList) return P.list[g * P.gsz + jj]; else return g * P.gsz + jj; };
 
   if (warp == kProdWarp)
   {
     if (lane == 0)
     {
       // the tap planes are the same for every channel: loaded once
-      mbar_expect_tx (b_full, (unsigned) kTcQ15PlaneBytes);
-      bulk_g2s (sB, P.planes, (unsigned) kTcQ15PlaneBytes, b_full);
+      mbar_expect_tx (b_full, (unsigned) kPlaneBK<kKind>);
+      bulk_g2s (sB, P.planes, (unsigned) kPlaneBK<kKind>, b_full);
       unsigned kk = 0;
       for (uint32_t g = blockIdx.x; g < P.n_groups; g += gridDim.x)
         for (uint32_t k = 0; k < supers; k++, kk++)
@@ -157,7 +219,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
 #pragma unroll 1
           for (int j = 0; j < kJ; j++)
           {
-            const uint32_t c = g * P.gsz + min ((uint32_t) j, nv - 1u);
+            const uint32_t c = chan (g, min ((uint32_t) j, nv - 1u));
             bulk_g2s (sRaw + (rb * kJ + j) * kRawRow, P.in + (size_t) c * P.frames + (size_t) k * kSuper, nfr * 4u, raw_full + rb);
             if (k == 0) bulk_g2s (sHist + (rb * kJ + j) * kHistRow, P.tail_in + (size_t) c * kHist, kHist * 4u, raw_full + rb);
           }
@@ -240,7 +302,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
             const int jj = i >> 4, o = i & 15;                                   // 16 uint4 = 64 frames per channel
             if ((uint32_t) jj < nv)
             {
-              const uint32_t c = g * P.gsz + jj;
+              const uint32_t c = chan (g, jj);
               const int f0 = (int) nfr - kHist + 4 * o;                            // first of the four frames, relative to the stage
               uint4 v;
               if (f0 >= 0) v = *reinterpret_cast<const uint4 *> (sRaw + (rb * kJ + jj) * kRawRow + f0 * 4);
@@ -259,7 +321,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
   else if (warp == kMmaWarp)
   {
     // ========================================== MMA issuer ==========================================
-    constexpr uint32_t id_ss = umma_idesc (192, 1, 1), id_us = umma_idesc (192, 0, 1);
+    constexpr uint32_t id_ss = umma_idesc (kN, 1, 1), id_us = umma_idesc (kN, 0, 1);
     const uint32_t aBase = smem_u32 (sA), b0 = smem_u32 (sB) >> 4;
     constexpr uint64_t kDescA = ((uint64_t) (kChunkBytes >> 4) << 16) | ((uint64_t) ((6 * kChunkBytes) >> 4) << 32) | (1ull << 46);
     constexpr uint64_t kDescB = ((uint64_t) (128 >> 4) << 16) | ((uint64_t) (256 >> 4) << 32) | (1ull << 46);
@@ -278,9 +340,9 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
 #pragma unroll kMmaUnroll
           for (int ks = 0; ks < kKSteps; ks++)
           {
-            const uint32_t ao = (uint32_t) (ks * 2 * kChunkBytes) >> 4, bo = (uint32_t) (ks * kBStep) >> 4;
-            umma_i8 (tmem, kDescA | (aHi + ao), kDescB | (b0 + bo), id_ss, ks != 0);          // xh * [hhI|hlI|hhQ|hlQ] -> [0,192)
-            umma_i8 (tmem + 192, kDescA | (aLo + ao), kDescB | (b0 + bo), id_us, ks != 0);    // xl * [...]             -> [192,384)
+            const uint32_t ao = (uint32_t) (ks * 2 * kChunkBytes) >> 4, bo = (uint32_t) (ks * kBStepK<kKind>) >> 4;
+            umma_i8 (tmem, kDescA | (aHi + ao), kDescB | (b0 + bo), id_ss, ks != 0);          // xh * [hhI|hlI|hhQ|hlQ] -> [0,N)
+            umma_i8 (tmem + kN, kDescA | (aLo + ao), kDescB | (b0 + bo), id_us, ks != 0);     // xl * [...]             -> [N,2N)
           }
           umma_commit (t_full + (kk & 1));
           umma_commit (a_empty + ab);
@@ -301,7 +363,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
     {
       const uint32_t nv = group_nv (g);
       const bool jvalid = (uint32_t) j < nv;
-      const uint32_t c = g * P.gsz + min ((uint32_t) j, nv - 1u);
+      const uint32_t c = chan (g, min ((uint32_t) j, nv - 1u));
       const bool sub = P.lsb[c] != 0;
 #if !SL_Q15TC_SPLIT && SL_Q15TC_HOIST
       const int carried_pk = (16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;   // loaded here, not between read-out and hand-over
@@ -418,22 +480,48 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         int aud[kBlk];
         int pk = 0;
         const uint32_t taddr = tmem + ((uint32_t) (32 * w) << 16);
+        // FM: z[-1] = the FIR outputs at frame -1 (rows 192 .. 195: rail I hh, hl, rail Q hh, hl) and its magnitude
+        int pa = 0, pb = 0, pm = 0;
+        if constexpr (kKind == kKindFm)
+        {
+          uint32_t h4[4], l4[4];
+          tmem_ld4 (taddr + 192, h4); tmem_ld4 (taddr + kN + 192, l4);
+          tmem_ld_wait ();
+          pa = sat16 (2 * (int) h4[0] + ((256 * ((int) h4[1] + (int) l4[0]) + (int) l4[1]) >> 15));
+          pb = sat16 (2 * (int) h4[2] + ((256 * ((int) h4[3] + (int) l4[2]) + (int) l4[3]) >> 15));
+          pm = cmag_q15 (pa, pb);
+        }
 #pragma unroll
         for (int i = 0; i < kBlk / 8; i++)
         {
           uint32_t s2[8], s1a[8], s1b[8], s0[8];
           int fi[8];
-          tmem_ld8 (taddr + 8 * i, s2); tmem_ld8 (taddr + 48 + 8 * i, s1a); tmem_ld8 (taddr + 192 + 8 * i, s1b); tmem_ld8 (taddr + 240 + 8 * i, s0);
+          tmem_ld8 (taddr + 8 * i, s2); tmem_ld8 (taddr + 48 + 8 * i, s1a); tmem_ld8 (taddr + kN + 8 * i, s1b); tmem_ld8 (taddr + kN + 48 + 8 * i, s0);
           tmem_ld_wait ();
 #pragma unroll
           for (int n = 0; n < 8; n++) fi[n] = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
-          tmem_ld8 (taddr + 96 + 8 * i, s2); tmem_ld8 (taddr + 144 + 8 * i, s1a); tmem_ld8 (taddr + 288 + 8 * i, s1b); tmem_ld8 (taddr + 336 + 8 * i, s0);
+          tmem_ld8 (taddr + 96 + 8 * i, s2); tmem_ld8 (taddr + 144 + 8 * i, s1a); tmem_ld8 (taddr + kN + 96 + 8 * i, s1b); tmem_ld8 (taddr + kN + 144 + 8 * i, s0);
           tmem_ld_wait ();
 #pragma unroll
           for (int n = 0; n < 8; n++)
           {
             const int fq = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
-            if constexpr (kTx)
+            if constexpr (kKind == kKindAm)
+            {
+              // arm_cmplx_mag_q15 (2.14, >= 0: arm_abs_q15 leaves it as it is)
+              const int v = cmag_q15 (fi[n], fq);
+              aud[8 * i + n] = v;
+              pk = max (pk, v);
+            }
+            else if constexpr (kKind == kKindFm)
+            {
+              const int m = cmag_q15 (fi[n], fq);
+              const int v = fm_disc (pa, pb, pm, fi[n], fq, m, P.fm_floor);
+              pa = fi[n]; pb = fq; pm = m;
+              aud[8 * i + n] = v;
+              pk = max (pk, min (abs (v), 32767));
+            }
+            else if constexpr (kTx)
             {
               // the rail order is the sideband: LSB / CW-R (I, Q) = (fi, fq), the others (fq, fi); the pair stays packed (I | Q << 16)
               const int vi = sub ? fi[n] : fq, vq = sub ? fq : fi[n];
@@ -569,12 +657,20 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
 // taps -> B operand: rows [rail I: hh (48) | hl (48) | rail Q: hh | hl], K byte m = 32 ks + kk = frame m / 2 of the 112-frame
 // window (64 before the block), rail m & 1; output n of the block meets tap d = 64 + n - frame. false when a tap does not
 // split into two signed bytes (|tap| >= 32640). tx: both rails filter the mic, so both place their taps at the L bytes (m = 2 frame)
-// and the R bytes get zero weight.
-bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes, bool tx)
+// and the R bytes get zero weight. fm (RX-Q15's FM planes, N = 208): the same 192 rows, then the outputs at frame n = -1 in rows
+// 192 + 2 rail + digit and 12 zero rows; so every section a thread reads starts on an 8-column boundary, as in the 192-row planes.
+static int q15_row (int rail, int digit, int n) { return n >= 0 ? rail * 96 + digit * 48 + n : 192 + 2 * rail + digit; }
+static size_t q15_plane_at (int rows, int m, int row)
 {
-  std::memset (planes, 0, kTcQ15PlaneBytes);
+  const int ks = m / 32, kk = m % 32;
+  return (size_t) ks * (rows / 8 * 256) + (row / 8) * 256 + (kk / 16) * 128 + (row % 8) * 16 + (kk % 16);
+}
+static bool build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes, bool tx, bool fm)
+{
+  const int rows = fm ? 208 : 192;
+  std::memset (planes, 0, (size_t) kKSteps * rows / 8 * 256);
   for (int rail = 0; rail < 2; rail++)
-    for (int n = 0; n < 48; n++)
+    for (int n = fm ? -1 : 0; n < 48; n++)
       for (int f = 0; f < 112; f++)
       {
         const int d = 64 + n - f;
@@ -582,36 +678,40 @@ bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t 
         const int h = rail ? taps_q[d] : taps_i[d];
         const int hl = ((h + 128) & 255) - 128, hh = (h - hl) >> 8;
         if (hh < -128 || hh > 127) return false;
-        const int m = 2 * f + (tx ? 0 : rail), ks = m / 32, kk = m % 32;
-        const int rows[2] = { rail * 96 + n, rail * 96 + 48 + n };
+        const int m = 2 * f + (tx ? 0 : rail);
         const int dg[2] = { hh, hl };
-        for (int g = 0; g < 2; g++)
-          planes[(size_t) ks * kBStep + (rows[g] / 8) * 256 + (kk / 16) * 128 + (rows[g] % 8) * 16 + (kk % 16)] = (uint8_t) (int8_t) dg[g];
+        for (int g = 0; g < 2; g++) planes[q15_plane_at (rows, m, q15_row (rail, g, n))] = (uint8_t) (int8_t) dg[g];
       }
   return true;
 }
+bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t *planes, bool tx) { return build_planes (taps_i, taps_q, planes, tx, false); }
+bool q15_tc_build_fm_planes (const int16_t *taps, uint8_t *planes) { return build_planes (taps, taps, planes, false, true); }
 
 // host-side evaluation of the planes on one raw window (design check, tests/test_tc_math.py): the integer contraction the
-// kernel runs and its reconstruction of arm_fir_q15's result; out[0..47] = rail I, out[48..95] = rail Q. The same for TX planes:
-// the contraction runs over all 224 bytes of the window as the kernel's does, and the R bytes meet zero weight there
-void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96)
+// kernel runs and its reconstruction of arm_fir_q15's result, outputs n = n0 .. 47 of rail I, then of rail Q
+static void apply_planes (const uint8_t *planes, int rows, int n0, const int16_t *window, int32_t *out)
 {
+  const int per = 48 - n0;
   for (int rail = 0; rail < 2; rail++)
-    for (int n = 0; n < 48; n++)
+    for (int n = n0; n < 48; n++)
     {
       long long s2 = 0, s1 = 0, s0 = 0;
+      const int r_hh = q15_row (rail, 0, n), r_hl = q15_row (rail, 1, n);
       for (int m = 0; m < 224; m++)
       {
-        const int ks = m / 32, kk = m % 32, x = window[m], xl = x & 255, xh = (x - xl) >> 8;
-        const int r_hh = rail * 96 + n, r_hl = rail * 96 + 48 + n;
-        const int hh = (int8_t) planes[(size_t) ks * kBStep + (r_hh / 8) * 256 + (kk / 16) * 128 + (r_hh % 8) * 16 + (kk % 16)];
-        const int hl = (int8_t) planes[(size_t) ks * kBStep + (r_hl / 8) * 256 + (kk / 16) * 128 + (r_hl % 8) * 16 + (kk % 16)];
+        const int x = window[m], xl = x & 255, xh = (x - xl) >> 8;
+        const int hh = (int8_t) planes[q15_plane_at (rows, m, r_hh)], hl = (int8_t) planes[q15_plane_at (rows, m, r_hl)];
         s2 += xh * hh; s1 += xh * hl + xl * hh; s0 += xl * hl;
       }
       const long long v = 2 * s2 + ((256 * s1 + s0) >> 15);
-      out96[rail * 48 + n] = (int32_t) (v > 32767 ? 32767 : (v < -32768 ? -32768 : v));
+      out[rail * per + n - n0] = (int32_t) (v > 32767 ? 32767 : (v < -32768 ? -32768 : v));
     }
 }
+// out[0..47] = rail I, out[48..95] = rail Q. The same for TX planes: the contraction runs over all 224 bytes of the window as the
+// kernel's does, and the R bytes meet zero weight there
+void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96) { apply_planes (planes, 192, 0, window, out96); }
+// FM planes: out[0..48] = rail I at n = -1 .. 47, out[49..97] = rail Q
+void q15_tc_apply_fm_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out98) { apply_planes (planes, 208, -1, window, out98); }
 
 int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream)
 {
@@ -624,13 +724,23 @@ int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream)
   P.gsz = (uint32_t) std::min<uint64_t> (kJ, std::max<uint64_t> (1, ((uint64_t) L.channels + (uint64_t) sm_count - 1) / (uint64_t) sm_count));
   P.n_groups = (L.channels + P.gsz - 1) / P.gsz;
   P.window = L.window; P.target = L.target; P.floor_ = L.floor_; P.gmax = L.gmax;
-  auto kernel = L.tx ? rx_q15_tc_kernel<true> : rx_q15_tc_kernel<false>;
-  cudaError_t e = cudaFuncSetAttribute (kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) Smem::bytes);
+  P.list = L.list; P.fm_floor = L.fm_floor;
+  void (*kernel) (KParams) = nullptr; size_t smem_bytes = Smem::bytes;
+  switch (L.kind)
+  {
+    case kQ15Ssb: kernel = L.list ? rx_q15_tc_kernel<kKindRxList> : rx_q15_tc_kernel<kKindRx>; break;
+    case kQ15Tx: kernel = rx_q15_tc_kernel<kKindTx>; break;
+    case kQ15Am: kernel = rx_q15_tc_kernel<kKindAm>; break;
+    case kQ15Fm: kernel = rx_q15_tc_kernel<kKindFm>; smem_bytes = SmemT<kTcQ15FmPlaneBytes>::bytes; break;
+    default: return (int) cudaErrorInvalidValue;
+  }
+  if (L.kind >= kQ15Am && !L.list) return (int) cudaErrorInvalidValue;
+  cudaError_t e = cudaFuncSetAttribute (kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem_bytes);
   if (e != cudaSuccess) return (int) e;
   uint32_t grid = (uint32_t) sm_count;
   if (grid > P.n_groups) grid = P.n_groups;
   if (const char *gs = std::getenv ("SELENITE_B200_TC_GRID")) { const long v = std::atol (gs); if (v > 0 && (uint32_t) v <= grid) grid = (uint32_t) v; }
-  kernel<<<grid, kThreads, Smem::bytes, (cudaStream_t) stream>>> (P);
+  kernel<<<grid, kThreads, smem_bytes, (cudaStream_t) stream>>> (P);
   return (int) cudaGetLastError ();
 }
 

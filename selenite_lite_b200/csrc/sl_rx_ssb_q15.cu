@@ -326,7 +326,10 @@ struct RxQ15State
 {
   uint32_t channels = 0;
   bool tx = false;                      // TX-SSB-q15: the tcgen05 kernel's kTx form, with TX planes (no mma.sync form, no biquad)
+  bool all_mode = false;                // RX-Q15: the tcgen05 kernel only (no biquad), one launch per detector kind present in a range
   slb_rx_q15_params prm{};
+  slb_rx_q15_mode_params mprm{};        // RX-Q15: AM / FM taps and the discriminator's floor
+  uint8_t *d_am_planes = nullptr, *d_fm_planes = nullptr;
   uint32_t *d_tail[2] = { nullptr, nullptr }; int16_t *d_peaks[2] = { nullptr, nullptr }; int parity = 0;
   uint32_t *d_afrag = nullptr; uint8_t *d_lsb = nullptr;
   uint8_t *d_tc_planes = nullptr; bool tc_ok = false;   // tcgen05 form of the same FIRs (sl_rx_q15_tc.cu)
@@ -408,11 +411,11 @@ static void pack_afrag (const int16_t *taps, uint32_t ntaps, uint32_t *hi /* [10
   }
 }
 
-int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, RxQ15State **out)
+int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, bool all_mode, RxQ15State **out)
 {
   if (fs != 48000u) return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "the q15 kernels are built for 48 kHz (48-frame firmware blocks)");
   RxQ15State *st = new RxQ15State ();
-  st->channels = channels; st->tx = tx;
+  st->channels = channels; st->tx = tx; st->all_mode = all_mode;
   bool ok = true;
   for (int p = 0; p < 2; p++)
   {
@@ -423,9 +426,15 @@ int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, RxQ15St
   ok = ok && cudaMalloc (&st->d_lsb, channels) == cudaSuccess;
   ok = ok && cudaMalloc (&st->d_tc_planes, kTcQ15PlaneBytes) == cudaSuccess;
   ok = ok && cudaMalloc (&st->d_bq, (size_t) channels * 16 * 2) == cudaSuccess && cudaMalloc (&st->d_pk_dummy, (size_t) channels * kWin * 2) == cudaSuccess && cudaMalloc (&st->d_rel, kWin * 2) == cudaSuccess;
+  if (all_mode) ok = ok && cudaMalloc (&st->d_am_planes, kTcQ15PlaneBytes) == cudaSuccess && cudaMalloc (&st->d_fm_planes, kTcQ15FmPlaneBytes) == cudaSuccess;
   if (!ok) { rxq15_destroy (st); return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state allocation failed"); }
   slb_rx_q15_params p; design_default_rx_q15 (fs, &p);
   int rc = rxq15_set_params (ctx, st, &p);
+  if (rc == SLB_OK && all_mode)
+  {
+    slb_rx_q15_mode_params mp; design_default_rx_q15_modes (fs, &mp);
+    rc = rxq15_set_mode_params (ctx, st, &mp);
+  }
   if (rc == SLB_OK) rc = rxq15_reset (ctx, st);
   if (rc == SLB_OK && cudaMemset (st->d_lsb, 0, channels) != cudaSuccess) rc = ctx_fail (ctx, SLB_ERR_CUDA, "memset failed");
   if (rc != SLB_OK) { rxq15_destroy (st); return rc; }
@@ -437,7 +446,7 @@ void rxq15_destroy (RxQ15State *st)
 {
   if (!st) return;
   for (int p = 0; p < 2; p++) { cudaFree (st->d_tail[p]); cudaFree (st->d_peaks[p]); }
-  cudaFree (st->d_afrag); cudaFree (st->d_lsb); cudaFree (st->d_tc_planes);
+  cudaFree (st->d_afrag); cudaFree (st->d_lsb); cudaFree (st->d_tc_planes); cudaFree (st->d_am_planes); cudaFree (st->d_fm_planes);
   cudaFree (st->d_bq); cudaFree (st->d_aud); cudaFree (st->d_blkpk); cudaFree (st->d_pk_dummy); cudaFree (st->d_rel);
   delete st;
 }
@@ -461,9 +470,11 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
   // the tcgen05 kernel serves the chain when every tap splits into two signed bytes and the AGC window fits the peaks it keeps
   std::vector<uint8_t> planes (kTcQ15PlaneBytes);
   const bool tc_ok = q15_tc_build_planes (p->taps_i, p->taps_q, planes.data (), st->tx) && p->agc_window <= 17;
-  // TX-SSB-q15 has the tcgen05 kernel only, and no audio filter: refused before anything changes
+  // TX-SSB-q15 and RX-Q15 have the tcgen05 kernel only, and no audio filter: refused before anything changes
   if (st->tx && (p->bq_stages != 0 || !tc_ok))
     return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "TX-SSB-q15 runs on the tcgen05 kernel only: bq_stages = 0, every tap < 32640, agc_window <= 17");
+  if (st->all_mode && (p->bq_stages != 0 || !tc_ok))
+    return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "RX-Q15 runs on the tcgen05 kernel only: bq_stages = 0, every tap < 32640, agc_window <= 17");
   if (p->bq_stages != st->prm.bq_stages || std::memcmp (p->bq_coeffs, st->prm.bq_coeffs, sizeof p->bq_coeffs) != 0)
     if (cudaMemset (st->d_bq, 0, (size_t) st->channels * 16 * 2) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state reset failed");   // a new filter starts from rest
   if (cudaMemcpy (st->d_rel, p->rel, kWin * 2, cudaMemcpyHostToDevice) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "release table upload failed");
@@ -477,6 +488,19 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
   return SLB_OK;
 }
 const slb_rx_q15_params *rxq15_params (const RxQ15State *st) { return &st->prm; }
+int rxq15_set_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_mode_params *p)
+{
+  if (!st->all_mode) return ctx_fail (ctx, SLB_ERR_STATE, "not an RX-Q15 context");
+  std::vector<uint8_t> am (kTcQ15PlaneBytes), fm (kTcQ15FmPlaneBytes);
+  if (!q15_tc_build_planes (p->am_taps, p->am_taps, am.data (), false) || !q15_tc_build_fm_planes (p->fm_taps, fm.data ()) || p->fm_floor < 1)
+    return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "RX-Q15 runs on the tcgen05 kernel only: every AM / FM tap < 32640, fm_floor >= 1");
+  if (cudaMemcpy (st->d_am_planes, am.data (), am.size (), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy (st->d_fm_planes, fm.data (), fm.size (), cudaMemcpyHostToDevice) != cudaSuccess)
+    return ctx_fail (ctx, SLB_ERR_CUDA, "tap upload failed");
+  st->mprm = *p;
+  return SLB_OK;
+}
+const slb_rx_q15_mode_params *rxq15_mode_params (const RxQ15State *st) { return st->all_mode ? &st->mprm : nullptr; }
 void rxq15_set_debug (RxQ15State *st, int16_t *audio, uint32_t *gain) { st->dbg_audio = audio; st->dbg_gain = gain; }
 
 int rxq15_set_sideband (slb_ctx *ctx, RxQ15State *st, uint32_t ch0, uint32_t n, int lsb)
@@ -524,7 +548,7 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
     ctx_count_launch (ctx, 2);
     return SLB_OK;
   };
-  if (st->tx || (st->tc_ok && !legacy_only))                                     // (TX: the only kernel; set_params guarantees tc_ok)
+  if (st->tx || st->all_mode || (st->tc_ok && !legacy_only))                      // (TX, RX-Q15: the only kernel; set_params guarantees tc_ok)
   {
     RxQ15TcLaunch L{};
     L.in = d_in; L.out = d_out;
@@ -534,11 +558,30 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
     L.audio_dbg = aud_tap; L.gain_dbg = gain_tap;
     L.rel = st->prm.rel; L.channels = nch; L.frames = frames; L.window = st->prm.agc_window;
     L.target = st->prm.agc_target; L.floor_ = st->prm.agc_floor; L.gmax = st->prm.agc_gmax_q15;
-    L.tx = st->tx;
-    const int e = launch_rx_q15_tc (L, sm_count, stream);
-    if (e != 0) return ctx_fail (ctx, SLB_ERR_CUDA, cudaGetErrorString ((cudaError_t) e));
-    ctx_count_launch (ctx);
-    return finish_bq ();
+    L.kind = st->tx ? kQ15Tx : kQ15Ssb; L.list = nullptr;
+    // RX-Q15: the kinds in the range (a range of SSB-style channels only runs exactly as RX-SSB-q15, with no list)
+    Q15KindLists kl{};
+    if (st->all_mode) { const int rc = q15_kind_lists (ctx, ch0, nch, &kl); if (rc) return rc; }
+    if (!st->all_mode || kl.n[0] == nch)
+    {
+      const int e = launch_rx_q15_tc (L, sm_count, stream);
+      if (e != 0) return ctx_fail (ctx, SLB_ERR_CUDA, cudaGetErrorString ((cudaError_t) e));
+      ctx_count_launch (ctx);
+      return finish_bq ();
+    }
+    // RX-Q15 with AM or FM channels in the range: one launch per kind present, each over its list
+    for (int k = 0; k < 3; k++)
+    {
+      if (kl.n[k] == 0) continue;
+      const int kind = k == 0 ? kQ15Ssb : (k == 1 ? kQ15Am : kQ15Fm);
+      L.kind = kind; L.list = kl.d[k]; L.channels = kl.n[k];
+      L.planes = kind == kQ15Am ? st->d_am_planes : (kind == kQ15Fm ? st->d_fm_planes : st->d_tc_planes);
+      L.fm_floor = st->mprm.fm_floor;
+      const int e = launch_rx_q15_tc (L, sm_count, stream);
+      if (e != 0) return ctx_fail (ctx, SLB_ERR_CUDA, cudaGetErrorString ((cudaError_t) e));
+      ctx_count_launch (ctx);
+    }
+    return SLB_OK;
   }
   KParams P{};
   P.in = reinterpret_cast<const uint32_t *> (d_in); P.out = reinterpret_cast<uint32_t *> (d_out);

@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _lib
 
-CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15 = 0, 1, 2, 3, 4, 5, 6
+CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15, CHAIN_RX_Q15 = 0, 1, 2, 3, 4, 5, 6, 7
 MODE_LSB, MODE_USB, MODE_CW, MODE_CWR, MODE_AM, MODE_FM, MODE_DIG, MODE_PKT = 0x00, 0x01, 0x02, 0x03, 0x04, 0x08, 0x0A, 0x0C
 RX_PATH_AUTO, RX_PATH_FFT = 0, 1
 
@@ -82,6 +82,23 @@ def q15_params_to_dict(p, lsb=0):
                 taps_i=np.array(p.taps_i[:], np.int16), taps_q=np.array(p.taps_q[:], np.int16), rel=np.array(p.rel[:], np.int16),
                 agc_target=p.agc_target, agc_floor=p.agc_floor, agc_gmax_q15=p.agc_gmax_q15,
                 bq_stages=p.bq_stages, bq_postshift=p.bq_postshift, bq_coeffs=np.array(p.bq_coeffs[:], np.int16))
+
+
+def default_rx_q15_mode_params(fs=48000):
+    p = _lib.RxQ15ModeParams()
+    rc = _lib.load().slb_default_rx_q15_mode_params(fs, C.byref(p))
+    if rc:
+        raise SeleniteError("slb_default_rx_q15_mode_params -> %d" % rc)
+    return p
+
+
+def q15_mode_params_to_dict(p, mp, mode=MODE_USB):
+    """RX-Q15 oracle parameters of one channel in `mode`: the RX-SSB-q15 dict plus the detector kind (0 SSB, 1 AM, 2 FM) and the AM / FM
+    constants (slb_rx_q15_mode_params)."""
+    d = q15_params_to_dict(p, lsb=mode in (MODE_LSB, MODE_CWR))
+    d.update(kind={MODE_AM: 1, MODE_FM: 2}.get(mode, 0), am_taps=np.array(mp.am_taps[:], np.int16), fm_taps=np.array(mp.fm_taps[:], np.int16),
+             fm_floor=int(mp.fm_floor))
+    return d
 
 
 def default_mask(fs=48000, fft_len=512, mode=MODE_USB):
@@ -361,6 +378,13 @@ class DspIf:
 
     def set_rx_q15_params(self, p): self._ck(self.lib.slb_set_rx_q15_params(self.h, C.byref(p)), "set_rx_q15_params")
 
+    def rx_q15_mode_params(self):
+        p = _lib.RxQ15ModeParams()
+        self._ck(self.lib.slb_get_rx_q15_mode_params(self.h, C.byref(p)), "get_rx_q15_mode_params")
+        return p
+
+    def set_rx_q15_mode_params(self, p): self._ck(self.lib.slb_set_rx_q15_mode_params(self.h, C.byref(p)), "set_rx_q15_mode_params")
+
     def set_q15_debug_taps(self, audio=None, gain=None):
         """audio: torch CUDA int16 [channels][frames] (RX-SSB-q15: pre-AGC audio) or [channels][frames][2] (TX-SSB-q15: pre-ALC I/Q);
         gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block)."""
@@ -369,6 +393,8 @@ class DspIf:
                                                     gain.data_ptr() if gain is not None else None), "rx_q15_set_debug_taps")
 
     def oracle_params(self, mode=MODE_USB):
+        if self.chain == CHAIN_RX_Q15:
+            return q15_mode_params_to_dict(self.rx_q15_params(), self.rx_q15_mode_params(), mode)
         if self.chain in (CHAIN_RX_SSB_Q15, CHAIN_TX_SSB_Q15):
             return q15_params_to_dict(self.rx_q15_params(), lsb=mode in (MODE_LSB, MODE_CWR))
         if self.chain == CHAIN_CHAN64_F32:
