@@ -58,6 +58,9 @@ extern "C" {
 #define SLB_CHAIN_RX_Q15      7    /* all-mode integer receiver: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_RX_SSB_Q15;
                                       AM by arm_cmplx_mag_q15, FM by an integer limiter-discriminator (DESIGN.md §3.8); bit-exact */
 
+#define SLB_CHAIN_TX_Q15      8    /* all-mode integer transmitter: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_TX_SSB_Q15;
+                                      AM (carrier + scaled audio) and FM (integer phase, table NCO) (DESIGN.md §3.9); bit-exact */
+
 #define SLB_MAX_STAGES 4
 #define SLB_MAX_MASKS  8
 
@@ -159,6 +162,31 @@ typedef struct
   int32_t fm_floor;                      /* >= 1; 2^18 = the f32 discriminator's 2^-10 soft squelch in these units */
 } slb_rx_q15_mode_params;
 
+/* The AM and FM modulators of SLB_CHAIN_TX_Q15 (DESIGN.md §3.9); slb_rx_q15_params keeps the SSB pair and the ALC constants, which all
+ * modes share (agc_target is the SSB modes' target). Per channel and 48-frame block, mic = L of the L = R frames,
+ *   a = arm_fir_q15 (mic, taps) -> block peak [arm_abs_q15 + arm_max_q15] -> the gain law of slb_rx_q15_params with the mode's target
+ *   -> y = arm_scale_q15 (a, q >> s, s), then
+ *   AM (target am_depth): I = arm_add_q15 (arm_scale_q15 (y, am_carrier, 0), am_carrier) (saturating), Q = 0
+ *   FM (target fm_target): phi[n] = phi[n-1] + y[n] fm_inc mod 2^32 (a uint32 per channel, carried), (I, Q) = fm_level (cos, sin) of
+ *       phi by the table NCO of SLB_CHAIN_TX_F32 (arm_cos_f32 / arm_sin_f32 -> arm_float_to_q15); a positive y moves the carrier up
+ * written interleaved I, Q. The phase advances in FM blocks only; a direction switch and SLB_DSP_Init zero it, the checkpoint keeps it.
+ * After a mode change between calls the FIR behaves as if the channel had always been in the new mode; the ALC's peak window carries over.
+ * SLB_CHAIN_TX_Q15 runs on the tcgen05 kernel only: a tap >= 32640 here or in slb_rx_q15_params, bq_stages != 0, agc_window > 17,
+ * am_carrier < 0, am_depth < 1, fm_target < 1 or |fm_inc| > 65535 is refused with SLB_ERR_UNSUPPORTED and the parameters stay as they
+ * were; tuning is refused too.
+ * Defaults (48 kHz): RX-Q15's AM low-pass (64-tap Kaiser, beta 6, DC gain 1, -6 dB at 3 kHz) for both modes, am_carrier 0.5,
+ * am_depth 0.8, fm_target 0.25, fm_inc = llround (2500 2^32 / 48000 / 8192) (2.5 kHz peak deviation), fm_level 0.5. */
+typedef struct
+{
+  int16_t am_taps[SLB_Q15_TAPS];         /* b[0..63], q15, natural order */
+  int16_t fm_taps[SLB_Q15_TAPS];
+  int16_t am_carrier;                    /* q15, >= 0 */
+  int16_t am_depth;                      /* q15, >= 1: the AM ALC target */
+  int16_t fm_target;                     /* q15, >= 1: the FM ALC target */
+  int32_t fm_inc;                        /* 2^-32 turn per sample per LSB of y, |fm_inc| <= 65535 */
+  float fm_level;                        /* NCO amplitude (full scale 1) */
+} slb_tx_q15_mode_params;
+
 /* ---- life cycle ---- */
 int  slb_create (const slb_config *cfg, slb_ctx **out);
 void slb_destroy (slb_ctx *ctx);
@@ -185,6 +213,10 @@ int slb_get_rx_q15_params (const slb_ctx *ctx, slb_rx_q15_params *p);
 int slb_default_rx_q15_mode_params (uint32_t fs, slb_rx_q15_mode_params *out);
 int slb_set_rx_q15_mode_params (slb_ctx *ctx, const slb_rx_q15_mode_params *p);
 int slb_get_rx_q15_mode_params (const slb_ctx *ctx, slb_rx_q15_mode_params *p);
+/* SLB_CHAIN_TX_Q15 contexts only (others: SLB_ERR_STATE) */
+int slb_default_tx_q15_mode_params (uint32_t fs, slb_tx_q15_mode_params *out);
+int slb_set_tx_q15_mode_params (slb_ctx *ctx, const slb_tx_q15_mode_params *p);
+int slb_get_tx_q15_mode_params (const slb_ctx *ctx, slb_tx_q15_mode_params *p);
 int slb_set_mask (slb_ctx *ctx, uint8_t mode, const float *mask);   /* host, 2*fft_len floats */
 int slb_get_mask (const slb_ctx *ctx, uint8_t mode, float *mask);
 /* which kernel serves the RX-SSB-f32 chain (DESIGN.md §4A): SLB_RX_PATH_AUTO = the tensor-core FIR kernel for every channel
@@ -263,7 +295,8 @@ int slb_rx_set_debug_taps (slb_ctx *ctx, float *d_audio, float *d_gain);
 int slb_tx_set_phase_tap (slb_ctx *ctx, uint32_t *d_phase);
 /* RX-SSB-q15: pre-AGC q15 audio int16[channels][frames] and the per-block gain q (Q15) uint32[channels][frames/48].
  * RX-Q15: the same, the pre-AGC detector output of each channel's mode (AM: the 2.14 magnitude, FM: the discriminator).
- * TX-SSB-q15: d_audio receives the pre-ALC (I, Q) int16[channels][frames][2] (after the rail order), d_gain the same gain words. */
+ * TX-SSB-q15: d_audio receives the pre-ALC (I, Q) int16[channels][frames][2] (after the rail order), d_gain the same gain words.
+ * TX-Q15: the same; AM and FM channels give (a, 0), the pre-ALC low-passed mic. */
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain);
 
 /* ---- per-channel tuning within the I/Q band (DESIGN.md §3.5): SLB_CHAIN_RX_SSB_F32, SLB_CHAIN_TX_SSB_F32, SLB_CHAIN_TX_F32 ----
@@ -433,7 +466,7 @@ int slb_sync (slb_ctx *ctx);
 
 /* ---- single-channel drop-in with the firmware's own names and signatures (Core/Inc/dsp_if.h:42-51).
  * They drive one process-global 1-channel context on device 0 (env SELENITE_B200_DEVICE, SELENITE_B200_FS,
- * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15|tx_ssb_q15|rx_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
+ * SELENITE_B200_CHAIN=pass|rx_ssb_f32|tx_ssb_f32|tx_f32|rx_ssb_q15|tx_ssb_q15|rx_q15|tx_q15; default pass at 48000 = the firmware's behaviour). Like the firmware
  * they return void; failures are reported through slb_dropin_status(). ---- */
 void DSP_Init (void);
 void DSP_Set_RX (void);

@@ -39,6 +39,11 @@ class RxQ15ModeParams(C.Structure):
     _fields_ = [("am_taps", C.c_int16 * 64), ("fm_taps", C.c_int16 * 64), ("fm_floor", C.c_int32)]
 
 
+class TxQ15ModeParams(C.Structure):
+    _fields_ = [("am_taps", C.c_int16 * 64), ("fm_taps", C.c_int16 * 64), ("am_carrier", C.c_int16), ("am_depth", C.c_int16),
+                ("fm_target", C.c_int16), ("fm_inc", C.c_int32), ("fm_level", C.c_float)]
+
+
 class FeederIo(C.Structure):
     _fields_ = [("adc", C.c_void_p), ("usb_in", C.c_void_p), ("usb_out", C.c_void_p), ("dac", C.c_void_p)]
 

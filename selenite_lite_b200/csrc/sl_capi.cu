@@ -40,7 +40,7 @@ struct slb_ctx
   std::vector<uint8_t> mode_host;      // [C]
   bool tx_mode = false;
   Chan64State *chan = nullptr;         // SLB_CHAIN_CHAN64_F32 only
-  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15, SLB_CHAIN_TX_SSB_Q15 and SLB_CHAIN_RX_Q15 only
+  RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15, SLB_CHAIN_TX_SSB_Q15, SLB_CHAIN_RX_Q15 and SLB_CHAIN_TX_Q15 only
 
   // device: chain constants + carried state
   float *d_masks = nullptr; uint8_t *d_slot = nullptr; float *d_twiddle = nullptr;
@@ -107,8 +107,11 @@ struct slb_ctx
 static inline bool is_f32_tx_chain (uint32_t chain) { return chain == SLB_CHAIN_TX_SSB_F32 || chain == SLB_CHAIN_TX_F32; }
 static inline bool is_ssb_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_F32 || is_f32_tx_chain (chain); }
 // the direction a context was created for: slb_tx_process_* serve these chains, slb_rx_process_* the others
-static inline bool is_tx_direction (uint32_t chain) { return is_f32_tx_chain (chain) || chain == SLB_CHAIN_TX_SSB_Q15; }
-static inline bool is_q15_chain (uint32_t chain) { return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15 || chain == SLB_CHAIN_RX_Q15; }
+static inline bool is_tx_direction (uint32_t chain) { return is_f32_tx_chain (chain) || chain == SLB_CHAIN_TX_SSB_Q15 || chain == SLB_CHAIN_TX_Q15; }
+static inline bool is_q15_chain (uint32_t chain)
+{
+  return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15 || chain == SLB_CHAIN_RX_Q15 || chain == SLB_CHAIN_TX_Q15;
+}
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
 
@@ -345,7 +348,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   int rc = upload_chain_constants (ctx);
   if (rc == SLB_OK) rc = reset_state (ctx);
   if (rc == SLB_OK && cfg->chain == SLB_CHAIN_CHAN64_F32) rc = chan64_create (ctx, C, cfg->fs, &ctx->chan);
-  if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, cfg->chain == SLB_CHAIN_TX_SSB_Q15, cfg->chain == SLB_CHAIN_RX_Q15, &ctx->q15);
+  if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, is_tx_direction (cfg->chain), cfg->chain == SLB_CHAIN_RX_Q15 || cfg->chain == SLB_CHAIN_TX_Q15, &ctx->q15);
   if (rc != SLB_OK) { g_create_error = ctx->err; slb_destroy (ctx); return rc; }
   *out = ctx;
   return SLB_OK;
@@ -488,6 +491,22 @@ int slb_get_rx_q15_mode_params (const slb_ctx *ctx, slb_rx_q15_mode_params *p)
   if (!ctx || !p) return SLB_ERR_ARG;
   if (!ctx->q15 || !rxq15_mode_params (ctx->q15)) return SLB_ERR_STATE;
   *p = *rxq15_mode_params (ctx->q15);
+  return SLB_OK;
+}
+int slb_default_tx_q15_mode_params (uint32_t fs, slb_tx_q15_mode_params *out) { return design_default_tx_q15_modes (fs, out); }
+int slb_set_tx_q15_mode_params (slb_ctx *ctx, const slb_tx_q15_mode_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->q15 || ctx->cfg.chain != SLB_CHAIN_TX_Q15) return fail (ctx, SLB_ERR_STATE, "not a TX-Q15 context");
+  CK (ctx, cudaSetDevice (ctx->cfg.device));
+  CK (ctx, cudaStreamSynchronize (ctx->stream));
+  return rxq15_set_tx_mode_params (ctx, ctx->q15, p);
+}
+int slb_get_tx_q15_mode_params (const slb_ctx *ctx, slb_tx_q15_mode_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->q15 || !rxq15_tx_mode_params (ctx->q15)) return SLB_ERR_STATE;
+  *p = *rxq15_tx_mode_params (ctx->q15);
   return SLB_OK;
 }
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain)
@@ -649,12 +668,13 @@ int SLB_DSP_Key (slb_ctx *ctx, const uint8_t *key_down)
 static int check_mode (slb_ctx *ctx, uint8_t mode)
 {
   if (mode_to_mask_slot (mode) < 0) return fail (ctx, SLB_ERR_UNSUPPORTED, "not an FT-817 mode byte (LSB, USB, CW, CW-R, AM, FM, DIG, PKT are served; rxtx_if.h:33-43)");
-  const bool all_mode = ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 || ctx->cfg.chain == SLB_CHAIN_PASS || ctx->cfg.chain == SLB_CHAIN_TX_F32 || ctx->cfg.chain == SLB_CHAIN_RX_Q15;
+  const bool all_mode = ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 || ctx->cfg.chain == SLB_CHAIN_PASS || ctx->cfg.chain == SLB_CHAIN_TX_F32 || ctx->cfg.chain == SLB_CHAIN_RX_Q15 ||
+                        ctx->cfg.chain == SLB_CHAIN_TX_Q15;
   if (mode == SLB_MODE_AM && !all_mode)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 and RX-Q15 chains (envelope detector), the channelizer and the TX-f32 chain (AM modulator) only; "
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "AM is served by the RX-SSB-f32 and RX-Q15 chains (envelope detector), the channelizer and the TX-f32 and TX-Q15 chains (AM modulator) only; "
                                            "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
   if (mode == SLB_MODE_FM && !all_mode)
-    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 and RX-Q15 chains (limiter-discriminator) and the TX-f32 chain (FM modulator) only; "
+    return fail (ctx, SLB_ERR_UNSUPPORTED, "FM is served by the RX-SSB-f32 and RX-Q15 chains (limiter-discriminator) and the TX-f32 and TX-Q15 chains (FM modulator) only; "
                                            "TX-SSB-f32, RX-SSB-q15 and TX-SSB-q15 are SSB-only");
   if (mode == SLB_MODE_FM && ctx->cfg.chain == SLB_CHAIN_RX_SSB_F32 && !ctx->tc_ok[kFmMaskSlot])
     return fail (ctx, SLB_ERR_UNSUPPORTED, "the FM slot has no tensor-core planes (fft_len must be 512 and the FM mask a 129-tap FIR)");
@@ -1865,7 +1885,8 @@ slb_ctx *dropin ()
               : (ch && std::strcmp (ch, "tx_f32") == 0) ? SLB_CHAIN_TX_F32
               : (ch && std::strcmp (ch, "rx_ssb_q15") == 0) ? SLB_CHAIN_RX_SSB_Q15
               : (ch && std::strcmp (ch, "tx_ssb_q15") == 0) ? SLB_CHAIN_TX_SSB_Q15
-              : (ch && std::strcmp (ch, "rx_q15") == 0) ? SLB_CHAIN_RX_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
+              : (ch && std::strcmp (ch, "rx_q15") == 0) ? SLB_CHAIN_RX_Q15
+              : (ch && std::strcmp (ch, "tx_q15") == 0) ? SLB_CHAIN_TX_Q15 : SLB_CHAIN_PASS;   // (the channelizer has no single-channel drop-in)
     g_dropin_status = slb_create (&cfg, &g_dropin);
     if (g_dropin_status != SLB_OK) std::fprintf (stderr, "selenite-b200: drop-in context failed: %s\n", slb_last_error (nullptr));
   }

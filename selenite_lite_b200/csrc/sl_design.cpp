@@ -184,6 +184,22 @@ int design_default_rx_q15_modes (uint32_t fs, slb_rx_q15_mode_params *p)
   return SLB_OK;
 }
 
+// TX-Q15's AM and FM modulators: RX-Q15's AM low-pass (3 kHz) for both; carrier 0.5, AM depth 0.8, FM ALC target 0.25 and an increment
+// that puts y = fm_target at 2.5 kHz: llround (2500 2^32 / 48000 / 8192) = 27307; NCO level 0.5
+int design_default_tx_q15_modes (uint32_t fs, slb_tx_q15_mode_params *p)
+{
+  if (!p || fs != 48000u) return p ? SLB_ERR_UNSUPPORTED : SLB_ERR_ARG;
+  slb_rx_q15_mode_params rx;
+  const int rc = design_default_rx_q15_modes (fs, &rx); if (rc) return rc;
+  std::memset (p, 0, sizeof *p);
+  std::memcpy (p->am_taps, rx.am_taps, sizeof p->am_taps);
+  std::memcpy (p->fm_taps, rx.am_taps, sizeof p->fm_taps);
+  p->am_carrier = 16384; p->am_depth = 26214; p->fm_target = 8192;
+  p->fm_inc = (int32_t) std::llround (2500.0 * 4294967296.0 / (double) fs / 8192.0);
+  p->fm_level = 0.5f;
+  return SLB_OK;
+}
+
 // -----------------------------------------------------------------------------------------------------------
 // Time-parallel evaluation of the 2-stage df2T cascade (arm_biquad_cascade_df2T_f32.c:551-562 per sample):
 // with x = 0 the 4-vector s = {d1_0,d2_0,d1_1,d2_1} evolves linearly, s' = A s, and the cascade output is c.s.

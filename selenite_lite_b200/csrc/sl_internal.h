@@ -217,7 +217,7 @@ void chan64_advance (Chan64State *st);
 struct RxQ15State;
 int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p);
 int design_default_rx_q15_modes (uint32_t fs, slb_rx_q15_mode_params *p);
-// tx: TX-SSB-q15, all_mode: RX-Q15 (the same state)
+// tx: TX-SSB-q15, all_mode: RX-Q15, both: TX-Q15 (the same state; TX-Q15 adds a phase word per channel)
 int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, bool all_mode, RxQ15State **out);
 void rxq15_destroy (RxQ15State *st);
 int rxq15_reset (slb_ctx *ctx, RxQ15State *st);
@@ -225,7 +225,10 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p);
 const slb_rx_q15_params *rxq15_params (const RxQ15State *st);
 int rxq15_set_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_mode_params *p);   // RX-Q15 only
 const slb_rx_q15_mode_params *rxq15_mode_params (const RxQ15State *st);                      // nullptr unless RX-Q15
-// RX-Q15: the channels of [ch0, ch0 + nch) by detector kind (Q15Kind kQ15Ssb, kQ15Am, kQ15Fm), as device lists of indices relative
+int design_default_tx_q15_modes (uint32_t fs, slb_tx_q15_mode_params *p);
+int rxq15_set_tx_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_tx_q15_mode_params *p);   // TX-Q15 only
+const slb_tx_q15_mode_params *rxq15_tx_mode_params (const RxQ15State *st);                   // nullptr unless TX-Q15
+// RX-Q15 and TX-Q15: the channels of [ch0, ch0 + nch) by detector kind (Q15Kind kQ15Ssb, kQ15Am, kQ15Fm), as device lists of indices relative
 // to ch0 (sl_capi.cu: cached per range, rebuilt when a mode changes); d[k] is valid when n[k] > 0
 struct Q15KindLists { const uint32_t *d[3]; uint32_t n[3]; };
 int q15_kind_lists (slb_ctx *ctx, uint32_t ch0, uint32_t nch, Q15KindLists *out);
@@ -263,9 +266,9 @@ bool q15_tc_build_planes (const int16_t *taps_i, const int16_t *taps_q, uint8_t 
 bool q15_tc_build_fm_planes (const int16_t *taps, uint8_t *planes /* kTcQ15FmPlaneBytes */);
 void q15_tc_apply_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out96);
 void q15_tc_apply_fm_planes (const uint8_t *planes, const int16_t *window /* [112][2] */, int32_t *out98);
-// detector kind of a launch: the SSB demodulator (RX-SSB-q15, and RX-Q15's SSB-style modes), the SSB modulator (TX-SSB-q15), RX-Q15's
-// AM and FM detectors
-enum Q15Kind : int { kQ15Ssb = 0, kQ15Tx = 1, kQ15Am = 2, kQ15Fm = 3 };
+// detector kind of a launch: the SSB demodulator (RX-SSB-q15, and RX-Q15's SSB-style modes), the SSB modulator (TX-SSB-q15, and
+// TX-Q15's SSB-style modes), RX-Q15's AM and FM detectors, TX-Q15's AM and FM modulators
+enum Q15Kind : int { kQ15Ssb = 0, kQ15Tx = 1, kQ15Am = 2, kQ15Fm = 3, kQ15TxAm = 4, kQ15TxFm = 5 };
 struct RxQ15TcLaunch
 {
   const int16_t *in; int16_t *out;
@@ -277,6 +280,9 @@ struct RxQ15TcLaunch
   const uint32_t *list;                    // device, [channels] channel indices relative to in / out / tails / peaks / lsb; nullptr:
                                            // channels 0 .. channels-1 (kQ15Ssb and kQ15Tx only)
   int32_t fm_floor;                        // kQ15Fm
+  // kQ15TxAm / kQ15TxFm (target = am_depth / fm_target; audio_dbg = pre-ALC (a, 0) [C][T][2]): the AM carrier (q15), FM: 2^-32 turn
+  // per LSB of y, the NCO level, [channels] phase words (device, relative like tails), arm_sin_f32's 513-entry table (device)
+  int32_t am_carrier, fm_inc; float fm_level; uint32_t *phase; const float *sin513;
 };
 int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream);
 

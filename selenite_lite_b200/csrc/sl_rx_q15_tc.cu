@@ -23,6 +23,10 @@
 // whose 64-tap window is frames 0..63 of the 112-frame window), so every block holds z[n-1] for its first sample; the epilogue
 // runs arm_cmplx_mag_q15 and the integer limiter-discriminator per sample. A launch of these kinds (and of the SSB kind in a
 // context that mixes kinds) works on a list of channels: rxq15_launch groups a channel range by kind.
+//
+// TX-Q15 (DESIGN.md §3.9) adds two modulators on the TX planes (both rails filter the mic with the mode's low-pass; the epilogue reads
+// rail I only): AM adds the scaled audio to the carrier, FM integrates y fm_inc into a per-channel uint32 phase and evaluates the table
+// NCO of the f32 chains. The SSB modulator (kTx) takes a channel list too, for the SSB-style channels of a context that mixes kinds.
 #include <cuda_runtime.h>
 #include <cstdint>
 #include <cstdlib>
@@ -66,14 +70,14 @@ constexpr unsigned kPSlots = SL_Q15TC_PSLOTS;
 constexpr int kTmemCols = 512;           // xh products in columns [0,N), xl products in [N,2N) (N = 192; FM 208)
 
 // detector kinds (template parameter of the kernel): the two SSB chains on contiguous channels, and the kinds of RX-Q15, which work
-// on a channel list (kKindRxList: the SSB detector of kKindRx)
-enum Kind : int { kKindRx = 0, kKindTx = 1, kKindAm = 2, kKindFm = 3, kKindRxList = 4 };
+// on a channel list (kKindRxList: the SSB detector of kKindRx); TX-Q15's kinds work on a list too (kKindTxList: the modulator of kKindTx)
+enum Kind : int { kKindRx = 0, kKindTx = 1, kKindAm = 2, kKindFm = 3, kKindRxList = 4, kKindTxList = 5, kKindTxAm = 6, kKindTxFm = 7 };
 template <int K> constexpr int kRowsN = K == kKindFm ? 208 : 192;                  // B rows = MMA N
 template <int K> constexpr int kBStepK = kRowsN<K> / 8 * 256;
 template <int K> constexpr size_t kPlaneBK = (size_t) kKSteps * kBStepK<K>;   // 43008; FM 46592 (= kTcQ15FmPlaneBytes)
 static_assert (kPlaneBK<kKindRx> == kTcQ15PlaneBytes && kPlaneBK<kKindFm> == kTcQ15FmPlaneBytes, "plane sizes");
 
-template <size_t kBBytes> struct SmemT
+template <size_t kBBytes, size_t kExtra = 0> struct SmemT
 {
   static constexpr size_t a = 0;
   static constexpr size_t b = a + 2 * 2 * kPlaneBytes;
@@ -84,10 +88,15 @@ template <size_t kBBytes> struct SmemT
   static constexpr size_t bars = pkc + kSets * kQ * kJ * 4;
   static constexpr int n_bars = 24;
   static constexpr size_t tmem_ptr = bars + n_bars * 8;
-  static constexpr size_t bytes = tmem_ptr + 16;
+  static constexpr size_t extra = tmem_ptr + 16;                                  // kind-specific (TX FM: kTxFmExtra)
+  static constexpr size_t bytes = extra + kExtra;
 };
+// TX FM: arm_sin_f32's table (513 floats), the per-channel phase advance of the last four supertiles ([4][8] uint32, slots as the
+// peak tiles) and the scan's per-warp totals ([sets][4 warps][8] uint32)
+constexpr size_t kSinBytes = 2064, kTotBytes = 4 * kJ * 4, kTxFmExtra = kSinBytes + kTotBytes + kSets * 4 * kJ * 4;
+template <int K> using SmemK = SmemT<kPlaneBK<K>, K == kKindTxFm ? kTxFmExtra : 0>;
 using Smem = SmemT<kTcQ15PlaneBytes>;
-static_assert (SmemT<kTcQ15FmPlaneBytes>::bytes <= 227 * 1024, "one CTA per SM");
+static_assert (SmemT<kTcQ15FmPlaneBytes>::bytes <= 227 * 1024 && SmemK<kKindTxFm>::bytes <= 227 * 1024, "one CTA per SM");
 
 struct KParams
 {
@@ -100,9 +109,12 @@ struct KParams
   uint32_t channels, frames, blocks, supers, gsz, n_groups, window;
   int32_t target, floor_; uint32_t gmax;
   const uint32_t *list; int32_t fm_floor;      // channel list (kinds kKindAm, kKindFm, kKindRxList); FM: the discriminator's floor
+  uint32_t *phase; const float *sin513;        // TX FM: [C] phase words (read at the stream start, written at its end); the NCO table
+  int32_t am_carrier, fm_inc; float fm_level15; // TX AM: the carrier (q15); TX FM: 2^-32 turn per LSB of y, NCO level x 32768
 };
 
 #include "sl_tc_common.cuh"
+#include "sl_nco.cuh"
 
 // (A/B: cvt.sat.s16.s32 is one instruction but runs on the conversion pipe: 403 vs 467 Gsamples/s. Raw stages with the MMA issue loop rolled: 2 -> 475, 3 -> 486, 4 -> 489 Gsamples/s; with it unrolled 468 .. 470 whatever the stages)
 #ifdef SL_Q15TC_CVTSAT
@@ -155,9 +167,10 @@ __device__ __forceinline__ int fm_disc (int pa, int pb, int pm, int a, int b, in
 template <int kKind>
 __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_constant__ KParams P)
 {
-  constexpr bool kTx = kKind == kKindTx, kList = kKind >= kKindAm;
+  constexpr bool kTx = kKind == kKindTx || kKind == kKindTxList, kList = kKind >= kKindAm;
+  constexpr bool kMono = kKind == kKindTxAm || kKind == kKindTxFm;               // TX AM / FM: one rail, a = the mic's low-pass
   constexpr int kN = kRowsN<kKind>;                                              // xl products from column kN on
-  using Smem = SmemT<kPlaneBK<kKind>>;
+  using Smem = SmemK<kKind>;
   static_assert (!(kKind != kKindRx && SL_Q15TC_SPLIT), "the split-epilogue A/B variant serves RX only");
   extern __shared__ __align__ (1024) unsigned char smem[];
   unsigned char *sA = smem + Smem::a, *sB = smem + Smem::b, *sRaw = smem + Smem::raw, *sHist = smem + Smem::hist;
@@ -172,8 +185,12 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
   // barrier and the late wait never returns; on four the next arrival on kk - 1's slot is kk + 3, which needs this set's read-out
   // of kk + 2.
   uint32_t *tmem_ptr = reinterpret_cast<uint32_t *> (smem + Smem::tmem_ptr);
+  float *sSin = reinterpret_cast<float *> (smem + Smem::extra);
+  uint32_t *sTot = reinterpret_cast<uint32_t *> (smem + Smem::extra + kSinBytes), *sScan = sTot + 4 * kJ;
 
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if constexpr (kKind == kKindTxFm)
+    for (int i = tid; i < 513; i += kThreads) sSin[i] = P.sin513[i];
   if (tid == 0)
   {
     for (int i = 0; i < kRawStages; i++) { mbar_init (raw_full + i, 1); mbar_init (raw_empty + i, kConvWarps); }
@@ -365,6 +382,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
       const bool jvalid = (uint32_t) j < nv;
       const uint32_t c = chan (g, min ((uint32_t) j, nv - 1u));
       const bool sub = P.lsb[c] != 0;
+      uint32_t fm_end = 0;                        // TX FM: the phase after this set's last supertile of the group
 #if !SL_Q15TC_SPLIT && SL_Q15TC_HOIST
       const int carried_pk = (16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;   // loaded here, not between read-out and hand-over
 #endif
@@ -500,6 +518,13 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
           tmem_ld_wait ();
 #pragma unroll
           for (int n = 0; n < 8; n++) fi[n] = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
+          if constexpr (kMono)
+          {
+            // TX AM / FM: a = rail I (rail Q holds the same FIR), |.| for the block peak (arm_abs_q15 + arm_max_q15)
+#pragma unroll
+            for (int n = 0; n < 8; n++) { aud[8 * i + n] = fi[n]; pk = max (pk, min (abs (fi[n]), 32767)); }
+            continue;
+          }
           tmem_ld8 (taddr + 96 + 8 * i, s2); tmem_ld8 (taddr + 144 + 8 * i, s1a); tmem_ld8 (taddr + kN + 96 + 8 * i, s1b); tmem_ld8 (taddr + kN + 144 + 8 * i, s0);
           tmem_ld_wait ();
 #pragma unroll
@@ -548,7 +573,8 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         if (k == 0) myC[q * kJ + j] = (16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;
 #endif
         __syncwarp ();
-        if (lane == 0) mbar_arrive (p_bar + (kk % kPSlots));
+        // (TX FM arrives after its phase advance is published, below)
+        if constexpr (kKind != kKindTxFm) { if (lane == 0) mbar_arrive (p_bar + (kk % kPSlots)); }
         // (every supertile but the CTA's first waits for its predecessor's peaks, also across groups where they are not used)
         if (kk != 0) mbar_wait (p_bar + ((kk - 1) % kPSlots), ((kk - 1) / kPSlots) & 1);
         named_bar (1 + es, 128);
@@ -565,11 +591,77 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         // it fit a q15; arm_scale_q15.c: __SSAT ((in * scaleFract) >> (15 - s), 16)
         const unsigned gq = min ((unsigned) (P.target << 15) / (unsigned) max (max (e, pk), P.floor_), P.gmax);
         const int sh = max (0, 17 - __clz (gq)), m = (int) (gq >> sh);
+        uint32_t ph = 0;                                                          // TX FM: the phase before this thread's block
+        if constexpr (kMono)
+        {
+          if (q < nblk && jvalid && P.audio_dbg)
+          {
+            // pre-ALC (a, 0) frames, int16 [C][T][2]
+            uint4 *ad = reinterpret_cast<uint4 *> (P.audio_dbg + 2 * ((size_t) c * P.frames + ((size_t) k * kQ + q) * kBlk));
+#pragma unroll
+            for (int n = 0; n < kBlk; n += 4)
+              ad[n / 4] = make_uint4 ((uint32_t) (uint16_t) aud[n], (uint32_t) (uint16_t) aud[n + 1], (uint32_t) (uint16_t) aud[n + 2], (uint32_t) (uint16_t) aud[n + 3]);
+          }
+          // y = arm_scale_q15 (a, q >> s, s)
+#pragma unroll
+          for (int n = 0; n < kBlk; n++) aud[n] = sat16 ((aud[n] * m) >> (15 - sh));
+        }
+        if constexpr (kKind == kKindTxFm)
+        {
+          // ---- the phase (ours, DESIGN.md §3.9): inc[n] = y[n] fm_inc (|.| < 2^31), phi[n] = phi[n-1] + inc[n] mod 2^32. A block's advance,
+          //      an inclusive scan over the channel's 16 blocks (lanes j + 8 a of the set's four warps hold blocks 4 w + a), and the phase at
+          //      the supertile's start: the state word at the group's first two supertiles, else this set's own end two supertiles back;
+          //      plus the other set's advance over the supertile in between (published before its p_bar arrival, which this set has waited
+          //      for). Blocks past the end of the stream advance nothing. The advance needs this supertile's gains, i.e. kk - 1's peaks, so
+          //      this kind arrives for kk only after its wait for kk - 1: the p_bar sequence becomes a strict chain, and no slot can complete
+          //      its next phase before every waiter has seen the current one (DESIGN.md §5A).
+          uint32_t adv = 0;
+          if (q < nblk)
+#pragma unroll
+            for (int n = 0; n < kBlk; n++) adv += (uint32_t) (aud[n] * P.fm_inc);
+          uint32_t x = adv, t = __shfl_up_sync (0xffffffffu, x, 8);
+          if (a >= 1) x += t;
+          t = __shfl_up_sync (0xffffffffu, x, 16);
+          if (a >= 2) x += t;
+          if (a == 3) sScan[(es * 4 + w) * kJ + j] = x;
+          named_bar (1 + es, 128);
+          uint32_t tot = 0, before = x - adv;
+#pragma unroll
+          for (int w2 = 0; w2 < 4; w2++) { const uint32_t v = sScan[(es * 4 + w2) * kJ + j]; tot += v; if (w2 < w) before += v; }
+          const uint32_t start = (k < 2 ? P.phase[c] : fm_end) + (k == 0 ? 0u : sTot[((kk - 1) & 3) * kJ + j]);
+          fm_end = start + tot; ph = start + before;
+          if (q == 0) sTot[(kk & 3) * kJ + j] = tot;
+          __syncwarp ();
+          if (lane == 0) mbar_arrive (p_bar + (kk % kPSlots));
+        }
         if (q < nblk && jvalid)
         {
           const size_t blk = (size_t) k * kQ + q, t0 = blk * kBlk;
           if (P.gain_dbg) P.gain_dbg[(size_t) c * P.blocks + blk] = gq;
-          if constexpr (kTx)
+          if constexpr (kMono)
+          {
+            uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0);
+#pragma unroll
+            for (int n = 0; n < kBlk; n += 8)
+            {
+              uint32_t o[8];
+#pragma unroll
+              for (int u = 0; u < 8; u++)
+              {
+                if constexpr (kKind == kKindTxAm)
+                  // I = arm_add_q15 (arm_scale_q15 (y, am_carrier, 0), am_carrier), Q = 0
+                  o[u] = (uint32_t) (uint16_t) sat16 (sat16 ((aud[n + u] * P.am_carrier) >> 15) + P.am_carrier);
+                else
+                {
+                  ph += (uint32_t) (aud[n + u] * P.fm_inc);
+                  o[u] = fm_nco (ph, sSin, P.fm_level15);
+                }
+              }
+              asm volatile ("st.global.L1::no_allocate.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst + n / 4),
+                            "r"(o[0]), "r"(o[1]), "r"(o[2]), "r"(o[3]), "r"(o[4]), "r"(o[5]), "r"(o[6]), "r"(o[7]) : "memory");
+            }
+          }
+          else if constexpr (kTx)
           {
             if (P.audio_dbg)
             {
@@ -638,6 +730,11 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         // — a warp that is through here could be there before a slower one has read it (inside a group only tiles kk and kk - 1
         // are read, and kk + 2 cannot touch those). Found under compute-sanitizer's timing; one barrier per group closes it.
         if (k + 1 == supers) named_bar (1 + es, 128);
+        // TX FM: the phase after the group goes back to the state word only here, after the barrier above. Its readers are the group's
+        // first two supertiles: this set's warps read it before they reached that barrier, and the other set's warps read it before
+        // their p_bar arrival for that supertile, which the strict p_bar chain puts before this set's last wait (DESIGN.md §5A).
+        if constexpr (kKind == kKindTxFm)
+          if (k + 1 == supers && jvalid && q == 0) P.phase[c] = fm_end;
       }
 #endif
     }
@@ -725,11 +822,14 @@ int launch_rx_q15_tc (const RxQ15TcLaunch &L, int sm_count, void *stream)
   P.n_groups = (L.channels + P.gsz - 1) / P.gsz;
   P.window = L.window; P.target = L.target; P.floor_ = L.floor_; P.gmax = L.gmax;
   P.list = L.list; P.fm_floor = L.fm_floor;
+  P.phase = L.phase; P.sin513 = L.sin513; P.am_carrier = L.am_carrier; P.fm_inc = L.fm_inc; P.fm_level15 = L.fm_level * 32768.0f;
   void (*kernel) (KParams) = nullptr; size_t smem_bytes = Smem::bytes;
   switch (L.kind)
   {
     case kQ15Ssb: kernel = L.list ? rx_q15_tc_kernel<kKindRxList> : rx_q15_tc_kernel<kKindRx>; break;
-    case kQ15Tx: kernel = rx_q15_tc_kernel<kKindTx>; break;
+    case kQ15Tx: kernel = L.list ? rx_q15_tc_kernel<kKindTxList> : rx_q15_tc_kernel<kKindTx>; break;
+    case kQ15TxAm: kernel = rx_q15_tc_kernel<kKindTxAm>; break;
+    case kQ15TxFm: kernel = rx_q15_tc_kernel<kKindTxFm>; smem_bytes = SmemK<kKindTxFm>::bytes; break;
     case kQ15Am: kernel = rx_q15_tc_kernel<kKindAm>; break;
     case kQ15Fm: kernel = rx_q15_tc_kernel<kKindFm>; smem_bytes = SmemT<kTcQ15FmPlaneBytes>::bytes; break;
     default: return (int) cudaErrorInvalidValue;

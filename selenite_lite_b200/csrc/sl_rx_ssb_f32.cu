@@ -188,13 +188,6 @@ __device__ __forceinline__ int32_t f2q31 (float x)
   asm ("cvt.rzi.sat.s32.f32 %0, %1;" : "=r"(v) : "f"(x * 2147483648.0f));
   return v;
 }
-// FM NCO of one sample (oracle tx_fm_nco): arm_q31_to_float ((int32) phi) -> arm_scale_f32 (pi) -> arm_cos_f32 / arm_sin_f32 ->
-// arm_scale_f32 (level) -> arm_float_to_q15. The 1/2^31 of arm_q31_to_float and the x32768 are powers of two, folded into the constants.
-__device__ __forceinline__ uint32_t fm_nco (uint32_t phi, const float *tab, float level15)
-{
-  const float x = nco_arg (phi);
-  return pack_iq (__fmul_rn (arm_sincos (x, tab, true), level15), __fmul_rn (arm_sincos (x, tab, false), level15));
-}
 
 // ---- bulk asynchronous copy (TMA engine, SASS UBLKCP) + mbarrier: raw tiles are staged global -> shared without
 // passing through registers, two tiles ahead of the FFTs ----

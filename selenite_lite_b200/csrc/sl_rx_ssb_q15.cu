@@ -326,10 +326,12 @@ struct RxQ15State
 {
   uint32_t channels = 0;
   bool tx = false;                      // TX-SSB-q15: the tcgen05 kernel's kTx form, with TX planes (no mma.sync form, no biquad)
-  bool all_mode = false;                // RX-Q15: the tcgen05 kernel only (no biquad), one launch per detector kind present in a range
+  bool all_mode = false;                // RX-Q15 (TX-Q15 with tx): the tcgen05 kernel only (no biquad), one launch per kind present in a range
   slb_rx_q15_params prm{};
   slb_rx_q15_mode_params mprm{};        // RX-Q15: AM / FM taps and the discriminator's floor
-  uint8_t *d_am_planes = nullptr, *d_fm_planes = nullptr;
+  slb_tx_q15_mode_params tmprm{};       // TX-Q15: AM / FM taps and the modulators' constants
+  uint8_t *d_am_planes = nullptr, *d_fm_planes = nullptr;   // RX-Q15: the AM and FM planes; TX-Q15: TX planes of the AM and FM taps
+  uint32_t *d_phase = nullptr; float *d_sin513 = nullptr;   // TX-Q15: the FM phase word per channel (in place), arm_sin_f32's table
   uint32_t *d_tail[2] = { nullptr, nullptr }; int16_t *d_peaks[2] = { nullptr, nullptr }; int parity = 0;
   uint32_t *d_afrag = nullptr; uint8_t *d_lsb = nullptr;
   uint8_t *d_tc_planes = nullptr; bool tc_ok = false;   // tcgen05 form of the same FIRs (sl_rx_q15_tc.cu)
@@ -426,14 +428,22 @@ int rxq15_create (slb_ctx *ctx, uint32_t channels, uint32_t fs, bool tx, bool al
   ok = ok && cudaMalloc (&st->d_lsb, channels) == cudaSuccess;
   ok = ok && cudaMalloc (&st->d_tc_planes, kTcQ15PlaneBytes) == cudaSuccess;
   ok = ok && cudaMalloc (&st->d_bq, (size_t) channels * 16 * 2) == cudaSuccess && cudaMalloc (&st->d_pk_dummy, (size_t) channels * kWin * 2) == cudaSuccess && cudaMalloc (&st->d_rel, kWin * 2) == cudaSuccess;
-  if (all_mode) ok = ok && cudaMalloc (&st->d_am_planes, kTcQ15PlaneBytes) == cudaSuccess && cudaMalloc (&st->d_fm_planes, kTcQ15FmPlaneBytes) == cudaSuccess;
+  if (all_mode) ok = ok && cudaMalloc (&st->d_am_planes, kTcQ15PlaneBytes) == cudaSuccess && cudaMalloc (&st->d_fm_planes, tx ? kTcQ15PlaneBytes : kTcQ15FmPlaneBytes) == cudaSuccess;
+  if (all_mode && tx)
+    ok = ok && cudaMalloc (&st->d_phase, (size_t) channels * 4) == cudaSuccess && cudaMalloc (&st->d_sin513, 513 * sizeof (float)) == cudaSuccess &&
+         cudaMemcpy (st->d_sin513, host_sin_table (), 513 * sizeof (float), cudaMemcpyHostToDevice) == cudaSuccess;
   if (!ok) { rxq15_destroy (st); return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state allocation failed"); }
   slb_rx_q15_params p; design_default_rx_q15 (fs, &p);
   int rc = rxq15_set_params (ctx, st, &p);
-  if (rc == SLB_OK && all_mode)
+  if (rc == SLB_OK && all_mode && !tx)
   {
     slb_rx_q15_mode_params mp; design_default_rx_q15_modes (fs, &mp);
     rc = rxq15_set_mode_params (ctx, st, &mp);
+  }
+  if (rc == SLB_OK && all_mode && tx)
+  {
+    slb_tx_q15_mode_params mp; design_default_tx_q15_modes (fs, &mp);
+    rc = rxq15_set_tx_mode_params (ctx, st, &mp);
   }
   if (rc == SLB_OK) rc = rxq15_reset (ctx, st);
   if (rc == SLB_OK && cudaMemset (st->d_lsb, 0, channels) != cudaSuccess) rc = ctx_fail (ctx, SLB_ERR_CUDA, "memset failed");
@@ -447,6 +457,7 @@ void rxq15_destroy (RxQ15State *st)
   if (!st) return;
   for (int p = 0; p < 2; p++) { cudaFree (st->d_tail[p]); cudaFree (st->d_peaks[p]); }
   cudaFree (st->d_afrag); cudaFree (st->d_lsb); cudaFree (st->d_tc_planes); cudaFree (st->d_am_planes); cudaFree (st->d_fm_planes);
+  cudaFree (st->d_phase); cudaFree (st->d_sin513);
   cudaFree (st->d_bq); cudaFree (st->d_aud); cudaFree (st->d_blkpk); cudaFree (st->d_pk_dummy); cudaFree (st->d_rel);
   delete st;
 }
@@ -457,6 +468,7 @@ int rxq15_reset (slb_ctx *ctx, RxQ15State *st)
     if (cudaMemset (st->d_tail[p], 0, (size_t) st->channels * kTaps * 4) != cudaSuccess || cudaMemset (st->d_peaks[p], 0, (size_t) st->channels * kWin * 2) != cudaSuccess)
       return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state reset failed");
   if (cudaMemset (st->d_bq, 0, (size_t) st->channels * 16 * 2) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state reset failed");
+  if (st->d_phase && cudaMemset (st->d_phase, 0, (size_t) st->channels * 4) != cudaSuccess) return ctx_fail (ctx, SLB_ERR_CUDA, "TX-Q15 state reset failed");
   st->parity = 0;
   return SLB_OK;
 }
@@ -471,6 +483,8 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
   std::vector<uint8_t> planes (kTcQ15PlaneBytes);
   const bool tc_ok = q15_tc_build_planes (p->taps_i, p->taps_q, planes.data (), st->tx) && p->agc_window <= 17;
   // TX-SSB-q15 and RX-Q15 have the tcgen05 kernel only, and no audio filter: refused before anything changes
+  if (st->tx && st->all_mode && (p->bq_stages != 0 || !tc_ok))
+    return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "TX-Q15 runs on the tcgen05 kernel only: bq_stages = 0, every tap < 32640, agc_window <= 17");
   if (st->tx && (p->bq_stages != 0 || !tc_ok))
     return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "TX-SSB-q15 runs on the tcgen05 kernel only: bq_stages = 0, every tap < 32640, agc_window <= 17");
   if (st->all_mode && (p->bq_stages != 0 || !tc_ok))
@@ -490,7 +504,7 @@ int rxq15_set_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_params *p)
 const slb_rx_q15_params *rxq15_params (const RxQ15State *st) { return &st->prm; }
 int rxq15_set_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_mode_params *p)
 {
-  if (!st->all_mode) return ctx_fail (ctx, SLB_ERR_STATE, "not an RX-Q15 context");
+  if (!st->all_mode || st->tx) return ctx_fail (ctx, SLB_ERR_STATE, "not an RX-Q15 context");
   std::vector<uint8_t> am (kTcQ15PlaneBytes), fm (kTcQ15FmPlaneBytes);
   if (!q15_tc_build_planes (p->am_taps, p->am_taps, am.data (), false) || !q15_tc_build_fm_planes (p->fm_taps, fm.data ()) || p->fm_floor < 1)
     return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "RX-Q15 runs on the tcgen05 kernel only: every AM / FM tap < 32640, fm_floor >= 1");
@@ -500,7 +514,22 @@ int rxq15_set_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_rx_q15_mode_p
   st->mprm = *p;
   return SLB_OK;
 }
-const slb_rx_q15_mode_params *rxq15_mode_params (const RxQ15State *st) { return st->all_mode ? &st->mprm : nullptr; }
+const slb_rx_q15_mode_params *rxq15_mode_params (const RxQ15State *st) { return st->all_mode && !st->tx ? &st->mprm : nullptr; }
+int rxq15_set_tx_mode_params (slb_ctx *ctx, RxQ15State *st, const slb_tx_q15_mode_params *p)
+{
+  if (!st->all_mode || !st->tx) return ctx_fail (ctx, SLB_ERR_STATE, "not a TX-Q15 context");
+  std::vector<uint8_t> am (kTcQ15PlaneBytes), fm (kTcQ15PlaneBytes);
+  if (!q15_tc_build_planes (p->am_taps, p->am_taps, am.data (), true) || !q15_tc_build_planes (p->fm_taps, p->fm_taps, fm.data (), true) ||
+      p->am_carrier < 0 || p->am_depth < 1 || p->fm_target < 1 || p->fm_inc > 65535 || p->fm_inc < -65535)
+    return ctx_fail (ctx, SLB_ERR_UNSUPPORTED, "TX-Q15 runs on the tcgen05 kernel only: every AM / FM tap < 32640, am_carrier >= 0, am_depth >= 1, "
+                                               "fm_target >= 1, |fm_inc| <= 65535 (y fm_inc stays in int32)");
+  if (cudaMemcpy (st->d_am_planes, am.data (), am.size (), cudaMemcpyHostToDevice) != cudaSuccess ||
+      cudaMemcpy (st->d_fm_planes, fm.data (), fm.size (), cudaMemcpyHostToDevice) != cudaSuccess)
+    return ctx_fail (ctx, SLB_ERR_CUDA, "tap upload failed");
+  st->tmprm = *p;
+  return SLB_OK;
+}
+const slb_tx_q15_mode_params *rxq15_tx_mode_params (const RxQ15State *st) { return st->all_mode && st->tx ? &st->tmprm : nullptr; }
 void rxq15_set_debug (RxQ15State *st, int16_t *audio, uint32_t *gain) { st->dbg_audio = audio; st->dbg_gain = gain; }
 
 int rxq15_set_sideband (slb_ctx *ctx, RxQ15State *st, uint32_t ch0, uint32_t n, int lsb)
@@ -559,7 +588,7 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
     L.rel = st->prm.rel; L.channels = nch; L.frames = frames; L.window = st->prm.agc_window;
     L.target = st->prm.agc_target; L.floor_ = st->prm.agc_floor; L.gmax = st->prm.agc_gmax_q15;
     L.kind = st->tx ? kQ15Tx : kQ15Ssb; L.list = nullptr;
-    // RX-Q15: the kinds in the range (a range of SSB-style channels only runs exactly as RX-SSB-q15, with no list)
+    // RX-Q15 / TX-Q15: the kinds in the range (a range of SSB-style channels only runs exactly as RX-SSB-q15 / TX-SSB-q15, with no list)
     Q15KindLists kl{};
     if (st->all_mode) { const int rc = q15_kind_lists (ctx, ch0, nch, &kl); if (rc) return rc; }
     if (!st->all_mode || kl.n[0] == nch)
@@ -569,14 +598,21 @@ int rxq15_launch (slb_ctx *ctx, RxQ15State *st, const int16_t *d_in, int16_t *d_
       ctx_count_launch (ctx);
       return finish_bq ();
     }
-    // RX-Q15 with AM or FM channels in the range: one launch per kind present, each over its list
+    // RX-Q15 / TX-Q15 with AM or FM channels in the range: one launch per kind present, each over its list
+    static const int kKinds[2][3] = { { kQ15Ssb, kQ15Am, kQ15Fm }, { kQ15Tx, kQ15TxAm, kQ15TxFm } };
     for (int k = 0; k < 3; k++)
     {
       if (kl.n[k] == 0) continue;
-      const int kind = k == 0 ? kQ15Ssb : (k == 1 ? kQ15Am : kQ15Fm);
-      L.kind = kind; L.list = kl.d[k]; L.channels = kl.n[k];
-      L.planes = kind == kQ15Am ? st->d_am_planes : (kind == kQ15Fm ? st->d_fm_planes : st->d_tc_planes);
+      L.kind = kKinds[st->tx][k]; L.list = kl.d[k]; L.channels = kl.n[k];
+      L.planes = k == 1 ? st->d_am_planes : (k == 2 ? st->d_fm_planes : st->d_tc_planes);
       L.fm_floor = st->mprm.fm_floor;
+      if (st->tx)
+      {
+        // TX-Q15: the modulator's own ALC target; the phase words are carried in place
+        L.target = k == 1 ? st->tmprm.am_depth : (k == 2 ? st->tmprm.fm_target : st->prm.agc_target);
+        L.am_carrier = st->tmprm.am_carrier; L.fm_inc = st->tmprm.fm_inc; L.fm_level = st->tmprm.fm_level;
+        L.phase = st->d_phase + ch0; L.sin513 = st->d_sin513;
+      }
       const int e = launch_rx_q15_tc (L, sm_count, stream);
       if (e != 0) return ctx_fail (ctx, SLB_ERR_CUDA, cudaGetErrorString ((cudaError_t) e));
       ctx_count_launch (ctx);
@@ -628,7 +664,8 @@ int rxq15_carry_idle (RxQ15State *st, uint32_t ch0, uint32_t nch, void *stream)
   return (int) e;
 }
 
-size_t rxq15_state_bytes (const RxQ15State *st) { return (size_t) st->channels * (kTaps * 4 + kWin * 2 + 1 + 16 * 2); }
+// TX-Q15: the same sections, then the phase words
+size_t rxq15_state_bytes (const RxQ15State *st) { return (size_t) st->channels * (kTaps * 4 + kWin * 2 + 1 + 16 * 2 + (st->d_phase ? 4 : 0)); }
 int rxq15_state_save (RxQ15State *st, char *dst)
 {
   const size_t C = st->channels;
@@ -636,6 +673,7 @@ int rxq15_state_save (RxQ15State *st, char *dst)
   if (cudaMemcpy (dst + C * kTaps * 4, st->d_peaks[st->parity], C * kWin * 2, cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
   if (cudaMemcpy (dst + C * (kTaps * 4 + kWin * 2), st->d_lsb, C, cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
   if (cudaMemcpy (dst + C * (kTaps * 4 + kWin * 2 + 1), st->d_bq, C * 16 * 2, cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
+  if (st->d_phase && cudaMemcpy (dst + C * (kTaps * 4 + kWin * 2 + 1 + 16 * 2), st->d_phase, C * 4, cudaMemcpyDeviceToHost) != cudaSuccess) return 1;
   return 0;
 }
 int rxq15_state_load (RxQ15State *st, const char *src)
@@ -645,6 +683,7 @@ int rxq15_state_load (RxQ15State *st, const char *src)
   if (cudaMemcpy (st->d_peaks[st->parity], src + C * kTaps * 4, C * kWin * 2, cudaMemcpyHostToDevice) != cudaSuccess) return 1;
   if (cudaMemcpy (st->d_lsb, src + C * (kTaps * 4 + kWin * 2), C, cudaMemcpyHostToDevice) != cudaSuccess) return 1;
   if (cudaMemcpy (st->d_bq, src + C * (kTaps * 4 + kWin * 2 + 1), C * 16 * 2, cudaMemcpyHostToDevice) != cudaSuccess) return 1;
+  if (st->d_phase && cudaMemcpy (st->d_phase, src + C * (kTaps * 4 + kWin * 2 + 1 + 16 * 2), C * 4, cudaMemcpyHostToDevice) != cudaSuccess) return 1;
   return 0;
 }
 

@@ -10,7 +10,7 @@ import numpy as np
 
 from . import _lib
 
-CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15, CHAIN_RX_Q15 = 0, 1, 2, 3, 4, 5, 6, 7
+CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15, CHAIN_RX_Q15, CHAIN_TX_Q15 = 0, 1, 2, 3, 4, 5, 6, 7, 8
 MODE_LSB, MODE_USB, MODE_CW, MODE_CWR, MODE_AM, MODE_FM, MODE_DIG, MODE_PKT = 0x00, 0x01, 0x02, 0x03, 0x04, 0x08, 0x0A, 0x0C
 RX_PATH_AUTO, RX_PATH_FFT = 0, 1
 
@@ -98,6 +98,24 @@ def q15_mode_params_to_dict(p, mp, mode=MODE_USB):
     d = q15_params_to_dict(p, lsb=mode in (MODE_LSB, MODE_CWR))
     d.update(kind={MODE_AM: 1, MODE_FM: 2}.get(mode, 0), am_taps=np.array(mp.am_taps[:], np.int16), fm_taps=np.array(mp.fm_taps[:], np.int16),
              fm_floor=int(mp.fm_floor))
+    return d
+
+
+def default_tx_q15_mode_params(fs=48000):
+    p = _lib.TxQ15ModeParams()
+    rc = _lib.load().slb_default_tx_q15_mode_params(fs, C.byref(p))
+    if rc:
+        raise SeleniteError("slb_default_tx_q15_mode_params -> %d" % rc)
+    return p
+
+
+def tx_q15_mode_params_to_dict(p, mp, mode=MODE_USB):
+    """TX-Q15 oracle parameters of one channel in `mode`: the RX-SSB-q15 dict plus the modulator kind (0 SSB, 1 AM, 2 FM) and the AM / FM
+    constants (slb_tx_q15_mode_params)."""
+    d = q15_params_to_dict(p, lsb=mode in (MODE_LSB, MODE_CWR))
+    d.update(kind={MODE_AM: 1, MODE_FM: 2}.get(mode, 0), am_taps=np.array(mp.am_taps[:], np.int16), fm_taps=np.array(mp.fm_taps[:], np.int16),
+             am_carrier=int(mp.am_carrier), am_depth=int(mp.am_depth), fm_target=int(mp.fm_target), fm_inc=int(mp.fm_inc),
+             fm_level=float(mp.fm_level))
     return d
 
 
@@ -385,8 +403,15 @@ class DspIf:
 
     def set_rx_q15_mode_params(self, p): self._ck(self.lib.slb_set_rx_q15_mode_params(self.h, C.byref(p)), "set_rx_q15_mode_params")
 
+    def tx_q15_mode_params(self):
+        p = _lib.TxQ15ModeParams()
+        self._ck(self.lib.slb_get_tx_q15_mode_params(self.h, C.byref(p)), "get_tx_q15_mode_params")
+        return p
+
+    def set_tx_q15_mode_params(self, p): self._ck(self.lib.slb_set_tx_q15_mode_params(self.h, C.byref(p)), "set_tx_q15_mode_params")
+
     def set_q15_debug_taps(self, audio=None, gain=None):
-        """audio: torch CUDA int16 [channels][frames] (RX-SSB-q15: pre-AGC audio) or [channels][frames][2] (TX-SSB-q15: pre-ALC I/Q);
+        """audio: torch CUDA int16 [channels][frames] (RX-SSB-q15: pre-AGC audio) or [channels][frames][2] (TX-SSB-q15, TX-Q15: pre-ALC I/Q);
         gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block)."""
         self._keep_taps = (audio, gain)
         self._ck(self.lib.slb_rx_q15_set_debug_taps(self.h, audio.data_ptr() if audio is not None else None,
@@ -395,6 +420,8 @@ class DspIf:
     def oracle_params(self, mode=MODE_USB):
         if self.chain == CHAIN_RX_Q15:
             return q15_mode_params_to_dict(self.rx_q15_params(), self.rx_q15_mode_params(), mode)
+        if self.chain == CHAIN_TX_Q15:
+            return tx_q15_mode_params_to_dict(self.rx_q15_params(), self.tx_q15_mode_params(), mode)
         if self.chain in (CHAIN_RX_SSB_Q15, CHAIN_TX_SSB_Q15):
             return q15_params_to_dict(self.rx_q15_params(), lsb=mode in (MODE_LSB, MODE_CWR))
         if self.chain == CHAIN_CHAN64_F32:
@@ -426,7 +453,7 @@ class DspIf:
         return out
 
     def tx_process(self, x, out=None, stream=None):
-        """TX direction (context created with CHAIN_TX_SSB_F32, CHAIN_TX_F32 or CHAIN_TX_SSB_Q15): mic frames (L = R) in, modulated I/Q
+        """TX direction (context created with CHAIN_TX_SSB_F32, CHAIN_TX_F32, CHAIN_TX_SSB_Q15 or CHAIN_TX_Q15): mic frames (L = R) in, modulated I/Q
         frames out."""
         return self.rx_process(x, out, stream, _dir="tx")
 

@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """Device-resident throughput of the chains that are not the headline bench line (TX-SSB-f32 = config 3,
-CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, TX-SSB-q15, RX-Q15 AM / FM, tuned channels). Prints one JSON line per chain after a line naming the card, its power
-limit and the HBM copy rate measured in the same run (hbm_frac_measured divides by that). Profiling aid, not the bench contract."""
+CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, TX-SSB-q15, RX-Q15 AM / FM, TX-Q15 AM / FM, tuned channels).
+Prints one JSON line per chain after a line naming the card, its power limit and the HBM copy rate measured in the same run
+(hbm_frac_measured divides by that). Profiling aid, not the bench contract."""
 import argparse
 import json
 import os
@@ -91,6 +92,13 @@ def main():
             m = torch.randint(-8000, 8000, (C, T, 1), dtype=torch.int16, device=dev, generator=g).expand(C, T, 2).contiguous()
             d = slb.DspIf(C, chain=slb.CHAIN_TX_SSB_Q15); y = torch.empty_like(m)
             ms = timeit(lambda: d.tx_process(m, y), args.steps); n = C * T; name = "tx_ssb_q15 (%d mic channels x %d s)" % (C, args.seconds)
+        elif which in ("tx_q15_am", "tx_q15_fm", "tx_q15_ssb"):
+            # TX-Q15 (DESIGN.md §3.9) with every mic channel in AM, FM or USB (the USB form is the TX-SSB-q15 kernel on the same context)
+            C, T = args.rx_channels, 48000 * args.seconds
+            m = torch.randint(-8000, 8000, (C, T, 1), dtype=torch.int16, device=dev, generator=g).expand(C, T, 2).contiguous()
+            d = slb.DspIf(C, chain=slb.CHAIN_TX_Q15); y = torch.empty_like(m)
+            d.DSP_Set_Mode({"tx_q15_am": slb.MODE_AM, "tx_q15_fm": slb.MODE_FM, "tx_q15_ssb": slb.MODE_USB}[which])
+            ms = timeit(lambda: d.tx_process(m, y), args.steps); n = C * T; name = "%s (%d mic channels x %d s)" % (which, C, args.seconds)
         elif which in ("rx_q15_am", "rx_q15_fm", "rx_q15_ssb"):
             # RX-Q15 (DESIGN.md §3.8) with every channel in AM, FM or USB (the USB form is the RX-SSB-q15 kernel on the same context)
             C, T = args.rx_channels, 48000 * args.seconds
