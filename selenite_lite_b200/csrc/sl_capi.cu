@@ -52,7 +52,7 @@ struct slb_ctx
   struct DevList { uint32_t *d = nullptr; size_t cap = 0; uint64_t version = ~0ull; };
   // channel lists of the tensor-core launches, cached per channel range (the bulk paths cut the batch the same way every
   // call) and rebuilt when a mode or a mask changes (mode_version)
-  struct TcLists : DevList { uint32_t groups = 0, groups_ssb = 0, n_chan = 0, n_pairs = 0; std::vector<uint8_t> on_tc; };
+  struct TcLists : DevList { uint32_t groups = 0, groups_ssb = 0; std::vector<uint8_t> on_tc; };
   std::map<uint64_t, TcLists> tc_lists; uint64_t mode_version = 0;
   bool force_fft = false;              // slb_set_rx_path (SLB_RX_PATH_FFT)
   // per-channel tuning (slb_set_tune, DESIGN.md §3.5): NCO increments (2^-32 turn per sample), empty until a non-zero offset is set;
@@ -850,22 +850,11 @@ static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint
     const uint32_t G = (uint32_t) gstart.size ();
     tl.groups_ssb = G;
     for (uint32_t gi = 0; gi < G; gi++) if ((ginfo[gi] & 0xFFu) >= (uint32_t) kAmMaskSlot) { tl.groups_ssb = gi; break; }   // slot-major: AM and FM groups (complex detector) are last
-    // the RX-SSB kernel runs on CTA pairs (tcgen05.mma.cta_group::2 shares the map operand between two SMs): consecutive groups
-    // of one mask slot pair up, a slot's odd group gets a partner that only runs along (0xFFFFFFFF)
-    std::vector<uint32_t> pairs;
-    for (uint32_t gi = 0; gi < tl.groups_ssb;)
-    {
-      const bool two = gi + 1 < tl.groups_ssb && (ginfo[gi + 1] & 0xFFu) == (ginfo[gi] & 0xFFu);
-      pairs.push_back (gi); pairs.push_back (two ? gi + 1 : 0xFFFFFFFFu);
-      gi += two ? 2 : 1;
-    }
-    tl.n_chan = (uint32_t) chan.size (); tl.n_pairs = (uint32_t) (pairs.size () / 2);
     if (G != 0)
     {
-      std::vector<uint32_t> pack (2 * (size_t) G + chan.size () + pairs.size ());
+      std::vector<uint32_t> pack (2 * (size_t) G + chan.size ());
       std::memcpy (pack.data (), gstart.data (), G * 4); std::memcpy (pack.data () + G, ginfo.data (), G * 4);
       std::memcpy (pack.data () + 2 * (size_t) G, chan.data (), chan.size () * 4);
-      if (!pairs.empty ()) std::memcpy (pack.data () + 2 * (size_t) G + chan.size (), pairs.data (), pairs.size () * 4);
       const int rc = upload_list (ctx, tl, pack); if (rc) return rc;
     }
     tl.groups = G; tl.version = ctx->mode_version;
@@ -895,7 +884,6 @@ static int run_rx_chain (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint
       L.in = d_in; L.out = d_out; L.audio_dbg = dbg_audio; L.gain_dbg = dbg_gain;
       set_carry (L, ctx, ch0);
       L.gstart = tl.d; L.ginfo = tl.d + G; L.chan = tl.d + 2 * (size_t) G;
-      L.pairs = tl.d + 2 * (size_t) G + tl.n_chan; L.n_pairs = tl.n_pairs;
       L.planes = ctx->d_planes; L.s0 = ctx->tc_s0; L.sz = ctx->tc_sz;
       L.flag_final = flag_final;
       L.n_groups = Gs; L.frames = frames;
@@ -1588,7 +1576,7 @@ static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, ui
 int slb_rx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream) { return process_device (ctx, d_in, d_out, frames, stream, false); }
 int slb_tx_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream) { return process_device (ctx, d_in, d_out, frames, stream, true); }
 
-// Staging of the host bulk paths: kBulkSlots device buffer pairs of at least `bytes` each, and one stream per slot
+// Staging of the host bulk paths: kBulkSlots slots of two device buffers of at least `bytes` each, and one stream per slot
 static int ensure_bulk (slb_ctx *ctx, size_t bytes)
 {
   if (bytes <= ctx->bulk_bytes && ctx->bulk_stream[0]) return SLB_OK;

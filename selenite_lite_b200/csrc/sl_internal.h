@@ -168,7 +168,6 @@ struct RxTcLaunch
   const uint32_t *chan;                    // channels served by this launch, grouped by mask slot
   const uint32_t *gstart;                  // [n_groups] index of the group's first channel in chan[]
   const uint32_t *ginfo;                   // [n_groups] mask slot | channels in the group (1..8) << 8
-  const uint32_t *pairs; uint32_t n_pairs; // [n_pairs][2]: the two groups (same mask slot) served by a CTA pair; second = 0xFFFFFFFF when the slot has an odd group
   const uint8_t *planes;                   // [SLB_MAX_MASKS][kTcPlaneBytes]
   const float *s0, *sz;                    // host, [SLB_MAX_MASKS]: units of the audio / state outputs
   unsigned flag_final;

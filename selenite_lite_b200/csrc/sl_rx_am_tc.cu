@@ -32,13 +32,7 @@ constexpr int kKSteps = 11;              // (128 + 48) frames * 2 bytes / 32
 constexpr int kBStep = 18 * 256;         // B bytes per K-step and rail: 18 row groups (3 digits x 48) x 2 chunks x 128 B
 constexpr int kRawRow = kSuper * 4 + 16;
 constexpr int kHistRow = kHist * 4 + 16;
-#ifndef SL_AMTC_IEEE
-#define SL_AMTC_IEEE 0
-#endif
-#ifndef SL_AMTC_MMA_UNROLL
-#define SL_AMTC_MMA_UNROLL 1                     /* 1: rolled MMA issue loops (instruction fetch, as in the TX / q15 kernels); 10: unrolled */
-#endif
-constexpr int kMmaUnroll = SL_AMTC_MMA_UNROLL, kRailUnroll = SL_AMTC_MMA_UNROLL > 1 ? 2 : 1;
+constexpr int kMmaUnroll = 1, kRailUnroll = 1;   // rolled MMA issue loops (instruction fetch, as in the TX / q15 kernels)
 constexpr int kSets = 2, kEpiWarps = 4 * kSets, kConvWarps = 2, kRawStages = 2;
 constexpr int kMmaWarp = kEpiWarps + kConvWarps, kProdWarp = kMmaWarp + 1;
 constexpr int kThreads = 32 * (kProdWarp + 1);
@@ -101,17 +95,12 @@ __device__ __forceinline__ float fm_discriminator (float a, float b, float pr, f
 {
   const float c = pr, d = -pi;
   const float re = __fsub_rn (__fmul_rn (a, c), __fmul_rn (b, d)), im = __fadd_rn (__fmul_rn (a, d), __fmul_rn (b, c));
-#if SL_AMTC_IEEE
-  const float m = __fsqrt_rn (__fadd_rn (__fmul_rn (re, re), __fmul_rn (im, im)));
-  return __fdiv_rn (im, fmaxf (m, kFmFloor));
-#else
   // Im w / max (|w|, floor) = Im w * rsqrt (max (|w|^2, floor^2)): one MUFU.RSQ and a multiply instead of an IEEE square root and an
   // IEEE division (a quarter of this kernel's instructions, which are what bounds it). rsqrt.approx is good to 2^-22: the detector
-  // output moves by <= 2e-7 of its value, against the chain's bar of 1e-5 (tests/test_gpu_rx_fm_f32.py, golden fixture included);
-  // -DSL_AMTC_IEEE=1 restores the oracle's two roundings.
+  // output moves by <= 2e-7 of its value, against the chain's bar of 1e-5 (tests/test_gpu_rx_fm_f32.py, golden fixture included).
+  // The oracle's two roundings (an IEEE square root and division) are recorded in DESIGN.md.
   const float s = fmaf (re, re, im * im);
   return im * rsqrtf (fmaxf (s, kFmFloor * kFmFloor));
-#endif
 }
 
 __global__ void __launch_bounds__ (kThreads, 1) rx_am_tc_kernel (const __grid_constant__ KParams P)

@@ -46,27 +46,12 @@ constexpr int kChunksNew = kSuper / 8;   // 96
 constexpr int kPlaneBytes = (kChunksHist + kChunksNew) * kChunkBytes;   // 13312
 constexpr int kKSteps = 7;               // (64 + 48) frames * 2 bytes / 32
 constexpr int kRawRow = kSuper * 4 + 16, kHistRow = kHist * 4 + 16;
-#ifndef SL_Q15TC_SPLIT
-#define SL_Q15TC_SPLIT 0                   // A/B: both epilogue sets work on every supertile, 24 of a block's 48 samples each.
-                                           // Bit-identical, but slower than alternating supertiles: 392 vs 467 Gsamples/s (one barrier of
-                                           // all eight warps per supertile puts the sets in lockstep)
-#endif
-#ifndef SL_Q15TC_RAWSTAGES
-#define SL_Q15TC_RAWSTAGES 4
-#endif
-#ifndef SL_Q15TC_MMA_UNROLL
-#define SL_Q15TC_MMA_UNROLL 1                   /* rolled: 489 vs 470 Gsamples/s (the unrolled issue loop costs instruction fetch: gcc requests at 78 % of peak) */
-#endif
-constexpr int kSets = 2, kEpiWarps = 4 * kSets, kConvWarps = 2, kRawStages = SL_Q15TC_RAWSTAGES, kMmaUnroll = SL_Q15TC_MMA_UNROLL;
+// The two epilogue sets alternate supertiles. Splitting every supertile between them, 24 of a block's 48 samples each, is
+// bit-identical but slower: 392 vs 467 Gsamples/s (one barrier of all eight warps per supertile puts the sets in lockstep).
+constexpr int kSets = 2, kEpiWarps = 4 * kSets, kConvWarps = 2, kRawStages = 4;
+constexpr int kMmaUnroll = 1;            // rolled: 489 vs 470 Gsamples/s (the unrolled issue loop costs instruction fetch: gcc requests at 78 % of peak)
 constexpr int kMmaWarp = kEpiWarps + kConvWarps, kProdWarp = kMmaWarp + 1, kThreads = 32 * (kProdWarp + 1);
-#ifndef SL_Q15TC_PSLOTS
-#define SL_Q15TC_PSLOTS 4
-#endif
-#ifndef SL_Q15TC_HOIST
-#define SL_Q15TC_HOIST 0                    /* 1: the carried peak of a group's first supertile is loaded at the group's start instead of between read-out and hand-over:
-                                             one more live register in the epilogue, 430 vs 492 Gsamples/s */
-#endif
-constexpr unsigned kPSlots = SL_Q15TC_PSLOTS;
+constexpr unsigned kPSlots = 4;
 constexpr int kTmemCols = 512;           // xh products in columns [0,N), xl products in [N,2N) (N = 192; FM 208)
 
 // detector kinds (template parameter of the kernel): the two SSB chains on contiguous channels, and the kinds of RX-Q15, which work
@@ -84,7 +69,7 @@ template <size_t kBBytes, size_t kExtra = 0> struct SmemT
   static constexpr size_t raw = b + kBBytes;
   static constexpr size_t hist = raw + kRawStages * kJ * kRawRow;
   static constexpr size_t pk = hist + kRawStages * kJ * kHistRow;                // [4 tiles][16][8] int: block peaks of the last supertiles
-  static constexpr size_t pkc = pk + (SL_Q15TC_SPLIT ? 2 : 1) * 4 * kQ * kJ * 4;                   // [sets][16][8] int: peaks before the stream start, by 16 - age
+  static constexpr size_t pkc = pk + 4 * kQ * kJ * 4;                            // [sets][16][8] int: peaks before the stream start, by 16 - age
   static constexpr size_t bars = pkc + kSets * kQ * kJ * 4;
   static constexpr int n_bars = 24;
   static constexpr size_t tmem_ptr = bars + n_bars * 8;
@@ -116,12 +101,8 @@ struct KParams
 #include "sl_tc_common.cuh"
 #include "sl_nco.cuh"
 
-// (A/B: cvt.sat.s16.s32 is one instruction but runs on the conversion pipe: 403 vs 467 Gsamples/s. Raw stages with the MMA issue loop rolled: 2 -> 475, 3 -> 486, 4 -> 489 Gsamples/s; with it unrolled 468 .. 470 whatever the stages)
-#ifdef SL_Q15TC_CVTSAT
-__device__ __forceinline__ int sat16 (int v) { short r; asm ("cvt.sat.s16.s32 %0, %1;" : "=h"(r) : "r"(v)); return (int) r; }
-#else
+// (cvt.sat.s16.s32 is one instruction but runs on the conversion pipe: 403 vs 467 Gsamples/s. Raw stages with the MMA issue loop rolled: 2 -> 475, 3 -> 486, 4 -> 489 Gsamples/s; with it unrolled 468 .. 470 whatever the stages)
 __device__ __forceinline__ int sat16 (int v) { return max (-32768, min (32767, v)); }
-#endif
 
 // arm_sqrt_q15 (FastMathFunctions/arm_sqrt_q15.c) as oracle/port/stats_cmplx.c restates it, every cast included: normalise by an even
 // shift, a float seed (a power-of-two multiply, the 0x5f3759df bit trick), three q15 Newton steps, multiply back, undo half the shift
@@ -171,7 +152,6 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
   constexpr bool kMono = kKind == kKindTxAm || kKind == kKindTxFm;               // TX AM / FM: one rail, a = the mic's low-pass
   constexpr int kN = kRowsN<kKind>;                                              // xl products from column kN on
   using Smem = SmemK<kKind>;
-  static_assert (!(kKind != kKindRx && SL_Q15TC_SPLIT), "the split-epilogue A/B variant serves RX only");
   extern __shared__ __align__ (1024) unsigned char smem[];
   unsigned char *sA = smem + Smem::a, *sB = smem + Smem::b, *sRaw = smem + Smem::raw, *sHist = smem + Smem::hist;
   int *sPk = reinterpret_cast<int *> (smem + Smem::pk), *sPkC = reinterpret_cast<int *> (smem + Smem::pkc);
@@ -200,7 +180,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
       mbar_init (t_full + i, 1);
     }
     for (int i = 0; i < kPSlots; i++) mbar_init (p_bar + i, 4);
-    mbar_init (t_empty, SL_Q15TC_SPLIT ? 4 * kSets : 4); mbar_init (b_full, 1);
+    mbar_init (t_empty, 4); mbar_init (b_full, 1);
     asm volatile ("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   if (warp == kMmaWarp)
@@ -371,9 +351,7 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
   {
     // ========================================== epilogue (all integer) ==========================================
     const int es = warp >> 2, w = warp & 3, a = lane >> 3, j = lane & 7, q = 4 * w + a;
-#if !SL_Q15TC_SPLIT
     int *myC = sPkC + es * (kQ * kJ);
-#endif
     const int window = (int) P.window;
     unsigned kk = 0;
     for (uint32_t g = blockIdx.x; g < P.n_groups; g += gridDim.x)
@@ -383,109 +361,6 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
       const uint32_t c = chan (g, min ((uint32_t) j, nv - 1u));
       const bool sub = P.lsb[c] != 0;
       uint32_t fm_end = 0;                        // TX FM: the phase after this set's last supertile of the group
-#if !SL_Q15TC_SPLIT && SL_Q15TC_HOIST
-      const int carried_pk = (16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;   // loaded here, not between read-out and hand-over
-#endif
-#if SL_Q15TC_SPLIT
-      // Both sets work on EVERY supertile: set es takes samples [24 es, 24 es + 24) of each block. The accumulators are read
-      // out in half the time — with one accumulator buffer the next supertile's MMAs wait for exactly that — and a block's
-      // peak is the larger of the two halves' (tiles keep both halves; one barrier of all eight warps per supertile).
-      for (uint32_t k = 0; k < supers; k++, kk++)
-      {
-        constexpr int kH = kBlk / 2;
-        const uint32_t nfr = min ((uint32_t) kSuper, P.frames - k * kSuper);
-        const int nblk = (int) (nfr / kBlk);
-        mbar_wait (t_full + (kk & 1), (kk >> 1) & 1);
-        tc_fence_after ();
-        int aud[kH];
-        int pk = 0;
-        const uint32_t taddr = tmem + ((uint32_t) (32 * w) << 16) + (uint32_t) (kH * es);
-#pragma unroll
-        for (int i = 0; i < kH / 8; i++)
-        {
-          uint32_t s2[8], s1a[8], s1b[8], s0[8];
-          int fi[8];
-          tmem_ld8 (taddr + 8 * i, s2); tmem_ld8 (taddr + 48 + 8 * i, s1a); tmem_ld8 (taddr + 192 + 8 * i, s1b); tmem_ld8 (taddr + 240 + 8 * i, s0);
-          tmem_ld_wait ();
-#pragma unroll
-          for (int n = 0; n < 8; n++) fi[n] = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
-          tmem_ld8 (taddr + 96 + 8 * i, s2); tmem_ld8 (taddr + 144 + 8 * i, s1a); tmem_ld8 (taddr + 288 + 8 * i, s1b); tmem_ld8 (taddr + 336 + 8 * i, s0);
-          tmem_ld_wait ();
-#pragma unroll
-          for (int n = 0; n < 8; n++)
-          {
-            const int fq = sat16 (2 * (int) s2[n] + ((256 * ((int) s1a[n] + (int) s1b[n]) + (int) s0[n]) >> 15));
-            const int v = sat16 (sub ? fi[n] - fq : fi[n] + fq);
-            aud[8 * i + n] = v;
-            pk = max (pk, min (abs (v), 32767));
-          }
-        }
-        tc_fence_before ();
-        __syncwarp ();
-        if (lane == 0) mbar_arrive (t_empty);
-        // ---- block peaks by half into tile kk & 3; at a stream start the peaks before it (carried by age) into the carry tile,
-        //      laid out like a previous supertile (block 16 - age): set 0 writes the values, set 1 zeros (max-neutral)
-        int *tile = sPk + (kk & 3) * (2 * kQ * kJ);
-        tile[(es * kQ + q) * kJ + j] = pk;
-        if (k == 0) sPkC[(es * kQ + q) * kJ + j] = (es == 0 && 16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;
-        named_bar (1, 32 * kEpiWarps);
-        const int *own = tile, *prev = (k == 0) ? sPkC : sPk + ((kk - 1) & 3) * (2 * kQ * kJ);
-        pk = max (own[q * kJ + j], own[(kQ + q) * kJ + j]);
-        int e = 0;
-        for (int age = 1; age < window; age++)
-        {
-          const int bq = q - age;
-          const int *t = (bq >= 0) ? own + bq * kJ + j : prev + (16 + bq) * kJ + j;
-          e = max (e, (max (t[0], t[kQ * kJ]) * (int) P.rel[age]) >> 15);
-        }
-        const unsigned gq = min ((unsigned) (P.target << 15) / (unsigned) max (max (e, pk), P.floor_), P.gmax);
-        const int sh = max (0, 17 - __clz (gq)), m = (int) (gq >> sh);
-        if (q < nblk && jvalid)
-        {
-          const size_t blk = (size_t) k * kQ + q, t0 = blk * kBlk + (size_t) (kH * es);
-          if (P.gain_dbg && es == 0) P.gain_dbg[(size_t) c * P.blocks + blk] = gq;
-          if (P.audio_dbg)
-          {
-            uint4 *ad = reinterpret_cast<uint4 *> (P.audio_dbg + (size_t) c * P.frames + t0);
-#pragma unroll
-            for (int n = 0; n < kH; n += 8)
-              ad[n / 8] = make_uint4 ((uint32_t) (uint16_t) aud[n] | ((uint32_t) (uint16_t) aud[n + 1] << 16), (uint32_t) (uint16_t) aud[n + 2] | ((uint32_t) (uint16_t) aud[n + 3] << 16),
-                                      (uint32_t) (uint16_t) aud[n + 4] | ((uint32_t) (uint16_t) aud[n + 5] << 16), (uint32_t) (uint16_t) aud[n + 6] | ((uint32_t) (uint16_t) aud[n + 7] << 16));
-          }
-          uint4 *dst = reinterpret_cast<uint4 *> (P.out + (size_t) c * P.frames + t0);
-#define SL_Q15_OUT(n) __byte_perm ((uint32_t) sat16 ((aud[n] * m) >> (15 - sh)), 0u, 0x1010)
-#pragma unroll
-          for (int n = 0; n < kH; n += 8)
-            asm volatile ("st.global.L1::no_allocate.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(dst + n / 4),
-                          "r"(SL_Q15_OUT (n)), "r"(SL_Q15_OUT (n + 1)), "r"(SL_Q15_OUT (n + 2)), "r"(SL_Q15_OUT (n + 3)),
-                          "r"(SL_Q15_OUT (n + 4)), "r"(SL_Q15_OUT (n + 5)), "r"(SL_Q15_OUT (n + 6)), "r"(SL_Q15_OUT (n + 7)) : "memory");
-#undef SL_Q15_OUT
-        }
-        if (k + 1 == supers && jvalid && es == 0)
-        {
-          // ---- the end of the call: the peak window by age; this thread takes ages q + 1 and q + 17
-          const int blocks = (int) P.blocks;
-#pragma unroll
-          for (int h = 0; h < 2; h++)
-          {
-            const int age = q + 1 + 16 * h;
-            if (age <= kWin - 1)
-            {
-              const int bi = blocks - age;
-              int v;
-              if (bi >= 0)
-              {
-                const unsigned tk = kk - (k - (unsigned) (bi / 16));                // running index of the supertile that holds block bi
-                const int *t = sPk + (tk & 3) * (2 * kQ * kJ) + (bi & 15) * kJ + j;
-                v = max (t[0], t[kQ * kJ]);
-              }
-              else v = (age - blocks <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (age - blocks) - 1] : 0;
-              P.peaks_out[(size_t) c * kWin + age - 1] = (int16_t) v;
-            }
-          }
-        }
-      }
-#else
       for (uint32_t k = 0; k < supers; k++, kk++)
       {
         if ((int) (kk % kSets) != es) continue;
@@ -567,11 +442,8 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         // ---- block peaks: this supertile's into tile kk & 3; at a stream start the peaks before it (carried by age) into
         //      this set's carry tile, laid out like a previous supertile (block 16 - age)
         sPk[((kk & 3) * kQ + q) * kJ + j] = pk;
-#if SL_Q15TC_HOIST
-        if (k == 0) myC[q * kJ + j] = carried_pk;
-#else
+        // (loading it at the group's start instead costs one more live register in the epilogue: 430 vs 492 Gsamples/s)
         if (k == 0) myC[q * kJ + j] = (16 - q <= kWin - 1) ? (int) P.peaks_in[(size_t) c * kWin + (16 - q) - 1] : 0;
-#endif
         __syncwarp ();
         // (TX FM arrives after its phase advance is published, below)
         if constexpr (kKind != kKindTxFm) { if (lane == 0) mbar_arrive (p_bar + (kk % kPSlots)); }
@@ -736,7 +608,6 @@ __global__ void __launch_bounds__ (kThreads, 1) rx_q15_tc_kernel (const __grid_c
         if constexpr (kKind == kKindTxFm)
           if (k + 1 == supers && jvalid && q == 0) P.phase[c] = fm_end;
       }
-#endif
     }
   }
 

@@ -26,7 +26,6 @@
 #include <cuda_runtime.h>
 #include <cmath>
 #include <cstdint>
-#include <cstdlib>
 #include "sl_internal.h"
 
 namespace sl {
@@ -38,10 +37,7 @@ namespace {
 constexpr int kN = 512;                          // FFT length
 constexpr int kHop = 384;                        // new frames per FFT frame
 constexpr int kOvl = kN - kHop;                  // 128 carried frames
-#ifndef SL_RX_FFTWARPS
-#define SL_RX_FFTWARPS 4
-#endif
-constexpr int kFftWarps = SL_RX_FFTWARPS;        // = frames per tile
+constexpr int kFftWarps = 4;                     // = frames per tile
 constexpr int kTile = kHop * kFftWarps;          // 1536 frames
 constexpr int kThreads = 32 * (kFftWarps + 1);   // + the recurrence warp
 constexpr int kBlocksPerTile = kTile / kAgcBlock; // 32 AGC blocks of 48 samples = one per recurrence lane
@@ -52,22 +48,14 @@ constexpr int kTxBlkStride = 100;                // TX tile: 48 complex per bloc
 constexpr int kTilesPerItem = 16;                // tiles a CTA processes with the recurrence state in registers
 constexpr int kPlane = kN;                       // floats per re / im scratch plane (XOR swizzle: no padding)
 constexpr int kRawWords = kTile + kOvl;          // raw frames (one u32 each) a tile needs: its 1536 + the 128 before it
-#ifndef SL_RX_RAWBUFS
-#define SL_RX_RAWBUFS 2
-#endif
-#ifndef SL_RX_AUDIOBUFS
-#define SL_RX_AUDIOBUFS 3
-#endif
-#ifndef SL_RX_CTAS
-#define SL_RX_CTAS 4
-#endif
-constexpr int kRawBufs = SL_RX_RAWBUFS;          // raw staging: filled by bulk asynchronous copies kRawBufs tiles ahead
+constexpr int kCtas = 4;                         // CTAs per SM the launch bounds ask for
+constexpr int kRawBufs = 2;                      // raw staging: filled by bulk asynchronous copies kRawBufs tiles ahead
 
 // dynamic shared memory layout (bytes). RX keeps three audio tiles in flight so that the FFT warps and the recurrence
 // warp only meet when one side is a whole tile late; the TX tile is twice as large (complex) and stays double-buffered.
 template <bool kTx, bool kMod = false> struct Smem
 {
-  static constexpr int kAudioBufs = kTx ? 2 : SL_RX_AUDIOBUFS;
+  static constexpr int kAudioBufs = kTx ? 2 : 3;
   static constexpr int kAudioWords = kBlocksPerTile * (kTx ? kTxBlkStride : kBlkStride);
   static constexpr size_t scratch = 0;
   static constexpr size_t audio = scratch + (size_t) kFftWarps * 2 * kPlane * 4;
@@ -208,15 +196,8 @@ __device__ __forceinline__ void mbar_arrive (uint64_t *bar)
 __device__ __forceinline__ void mbar_wait (uint64_t *bar, unsigned parity)
 {
   sl_jitter ();
-  asm volatile (
-#ifdef SL_RX_WAIT_HINT
-      // the time hint lets the hardware park the warp until the phase flips instead of spinning through issue slots
-      "{\n .reg .pred p;\n WAIT_%=:\n mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1, %2;\n @p bra DONE_%=;\n bra WAIT_%=;\n DONE_%=:\n}\n"
-      ::"r"(smem_u32 (bar)), "r"(parity), "r"(SL_RX_WAIT_HINT) : "memory");
-#else
-      "{\n .reg .pred p;\n WAIT_%=:\n mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n @p bra DONE_%=;\n bra WAIT_%=;\n DONE_%=:\n}\n"
-      ::"r"(smem_u32 (bar)), "r"(parity) : "memory");
-#endif
+  asm volatile ("{\n .reg .pred p;\n WAIT_%=:\n mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n @p bra DONE_%=;\n bra WAIT_%=;\n DONE_%=:\n}\n"
+                ::"r"(smem_u32 (bar)), "r"(parity) : "memory");
 }
 __device__ __forceinline__ void bulk_g2s (void *dst, const void *src, unsigned bytes, uint64_t *bar)
 {
@@ -380,11 +361,7 @@ __device__ __forceinline__ void fft512x2 (u64 *xr, u64 *xi, float *sre, const fl
 // kMod (TX only, SLB_CHAIN_TX_F32): channels on the AM and FM slots are modulated as DESIGN.md §3.4 describes; the other slots run the
 //              TX-SSB code unchanged.
 template <bool kTx, bool kMod = false>
-#ifdef SL_RX_MAXNREG
-__global__ void __maxnreg__ (SL_RX_MAXNREG) ssb_f32_kernel
-#else
-__global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
-#endif
+__global__ void __launch_bounds__ (kThreads, kCtas) ssb_f32_kernel
  (const __grid_constant__ KParams P)
 {
   typedef Smem<kTx, kMod> S;
@@ -443,8 +420,8 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
     }
     for (; it.valid (); tile_seq++)
     {
-      const int rbuf = (kRawBufs == 1) ? 0 : (int) (tile_seq & 1);
-      const unsigned rpar = (kRawBufs == 1) ? (tile_seq & 1) : ((tile_seq >> 1) & 1);
+      const int rbuf = (int) (tile_seq & 1);
+      const unsigned rpar = (tile_seq >> 1) & 1;
       const bool mine = warp < it.hops (P);
       const uint32_t c = it.c, t0 = it.t0 ();
       u64 xr[8], xi[8];
@@ -490,9 +467,7 @@ __global__ void __launch_bounds__ (kThreads, SL_RX_CTAS) ssb_f32_kernel
       {
         if (mine)
         {
-#ifndef SL_RX_ABLATE_FFT                                                            // (profiling aid: time the recurrence side alone)
           fft512x2 (xr, xi, sre, sTw, lane);
-#endif
         }
         if (dir == 0)
         {
@@ -924,7 +899,6 @@ int launch_rx_ssb_f32 (const RxF32Launch &L, int sm_count, void *stream_)
   // (Measured, profiles/r01_summary.md: throughput is proportional to the number of resident CTAs — 592: 155, 512: 132,
   // 448: 117 Gsamples/s — i.e. every CTA is an internally latency-bound pipeline; shrinking the grid to make the segment
   // hand-over trivially satisfied costs more than the polling it removes.)
-  if (const char *g = std::getenv ("SELENITE_B200_RX_GRID")) { const long v = std::atol (g); if (v > 0 && (uint64_t) v <= (uint64_t) sm_count * per_sm) grid = (uint64_t) v; }   // profiling aid
   // Cooperative launch: consecutive segments of a channel hand over through a flag the successor polls, so every CTA of the
   // grid must be resident at once. The cooperative attribute makes the driver schedule the grid as a gang — next to other
   // work on the device (a second stream of this library, another context, MPS) the launch waits for room or fails with

@@ -38,10 +38,7 @@ namespace {
 constexpr int kTaps = SLB_Q15_TAPS;              // 64
 constexpr int kWin = SLB_Q15_WIN;                // peak ring length (>= agc_window)
 constexpr int kBlk = 48;                         // AGC block = firmware block at 48 kHz = 3 MMA blocks of 16 frames
-#ifndef SL_Q15_CHUNK
-#define SL_Q15_CHUNK 2
-#endif
-constexpr int kChunkBlocks = SL_Q15_CHUNK;       // AGC blocks per staged chunk
+constexpr int kChunkBlocks = 2;                  // AGC blocks per staged chunk
 constexpr int kChunk = kChunkBlocks * kBlk;      // 96 frames
 constexpr int kRowWords = kTaps + kChunk + 16;   // words per channel row of a raw stage: 64 history + 96 new + 16 pad;
                                                  // 704 B = 64 mod 128, so the 16-byte loads of lanes (ch, tig), (ch+1, tig)

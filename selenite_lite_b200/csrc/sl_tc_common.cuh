@@ -16,6 +16,10 @@ __device__ __forceinline__ void mbar_arrive (uint64_t *bar)
   sl_jitter ();
   asm volatile ("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32 (bar)) : "memory");
 }
+// A plain try_wait loop polls every ~20 clocks, and every poll is a shared-memory wavefront on the L1 data pipe the tensor core
+// fetches its operands through (ncu, round 2: 411 polls per supertile). Still, a suspend-time hint or a nanosleep back-off
+// measured slower (profiles/r02_summary.md): plain polling 416 Gsamples/s, hint 2000 ns 412, sleep 64 ns 410, both 409 — the
+// polls do not cost what their count suggests and the wake-up latency does.
 __device__ __forceinline__ void mbar_wait (uint64_t *bar, unsigned parity)
 {
   sl_jitter ();
@@ -41,47 +45,10 @@ __device__ __forceinline__ void mbar_wait_guarded (uint64_t *bar, unsigned parit
   mbar_wait (bar, parity);
 #endif
 }
-// The same for the roles that wait long (producer, converters, MMA issuer, an epilogue set waiting for its accumulators): a
-// plain try_wait loop polls every ~20 clocks, and every poll is a shared-memory wavefront on the L1 data pipe the tensor core
-// fetches its operands through (ncu, round 2: 411 polls per supertile). A/B option: the try_wait carries a suspend-time hint
-// and / or a failed poll backs off with nanosleep. Measured (profiles/r02_summary.md): plain polling 416 Gsamples/s, hint 2000 ns
-// 412, sleep 64 ns 410, both 409 — the polls do not cost what their count suggests and the wake-up latency does; default off.
-#ifndef SL_TC_WAIT_HINT_NS
-#define SL_TC_WAIT_HINT_NS 0
-#endif
-#ifndef SL_TC_WAIT_SLEEP_NS
-#define SL_TC_WAIT_SLEEP_NS 0
-#endif
-__device__ __forceinline__ void mbar_wait_long (uint64_t *bar, unsigned parity)
-{
-#if SL_TC_WAIT_SLEEP_NS == 0 && SL_TC_WAIT_HINT_NS == 0
-  mbar_wait (bar, parity);
-#else
-  uint32_t done;
-  do
-  {
-    asm volatile ("{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n selp.u32 %0, 1, 0, p;\n}\n"
-                  : "=r"(done) : "r"(smem_u32 (bar)), "r"(parity), "r"((unsigned) SL_TC_WAIT_HINT_NS) : "memory");
-#if SL_TC_WAIT_SLEEP_NS > 0
-    if (!done) __nanosleep (SL_TC_WAIT_SLEEP_NS);
-#endif
-  } while (!done);
-#endif
-}
 __device__ __forceinline__ void bulk_g2s (void *dst, const void *src, unsigned bytes, uint64_t *bar)
 {
   asm volatile ("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                 ::"r"(smem_u32 (dst)), "l"(src), "r"(bytes), "r"(smem_u32 (bar)) : "memory");
-}
-// the same with an L2 eviction-priority hint: the raw stream is read exactly once
-__device__ __forceinline__ void bulk_g2s_stream (void *dst, const void *src, unsigned bytes, uint64_t *bar, uint64_t policy)
-{
-  asm volatile ("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-                ::"r"(smem_u32 (dst)), "l"(src), "r"(bytes), "r"(smem_u32 (bar)), "l"(policy) : "memory");
-}
-__device__ __forceinline__ void bulk_s2g (void *dst, const void *src, unsigned bytes)
-{
-  asm volatile ("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32 (src)), "r"(bytes) : "memory");
 }
 __device__ __forceinline__ void named_bar (int id, int threads) { sl_jitter (); asm volatile ("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory"); }
 
@@ -145,42 +112,3 @@ template <int cols> __device__ __forceinline__ void tmem_zero (uint32_t addr)
 }
 __device__ __forceinline__ void tmem_ld_wait () { asm volatile ("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-
-// ---- CTA pairs (cta_group::2): the leader CTA's elected lane issues M = 256 MMAs over both SMs; each CTA supplies its own 128 rows
-// of A and HALF of the B rows (its tensor core receives the other half from the peer), accumulators land in each CTA's own TMEM ----
-__device__ __forceinline__ uint32_t cluster_ctarank () { uint32_t r; asm volatile ("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_id_x () { uint32_t r; asm volatile ("mov.u32 %0, %%clusterid.x;" : "=r"(r)); return r; }
-__device__ __forceinline__ uint32_t cluster_n_x () { uint32_t r; asm volatile ("mov.u32 %0, %%nclusterid.x;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all ()
-{
-  asm volatile ("barrier.cluster.arrive.release.aligned;\n barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// address of the same shared-memory object in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32 (uint32_t addr, uint32_t rank)
-{
-  uint32_t r; asm volatile ("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank)); return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster (uint32_t cluster_addr)
-{
-  asm volatile ("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// wait on a barrier of THIS CTA whose arrivals come from both CTAs of the pair (acquire at cluster scope)
-__device__ __forceinline__ void mbar_wait_cluster (uint64_t *bar, unsigned parity)
-{
-  asm volatile ("{\n .reg .pred p;\n WAIT_%=:\n mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n @p bra DONE_%=;\n bra WAIT_%=;\n DONE_%=:\n}\n"
-                ::"r"(smem_u32 (bar)), "r"(parity) : "memory");
-}
-__host__ __device__ constexpr uint32_t umma_idesc_pair (int N, int a_signed, int b_signed)   // M = 256 over the pair
-{
-  return (2u << 4) | ((uint32_t) a_signed << 7) | ((uint32_t) b_signed << 10) | ((uint32_t) (N >> 3) << 17) | ((uint32_t) (256 >> 4) << 24);
-}
-__device__ __forceinline__ void umma_i8_pair (uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate)
-{
-  asm volatile ("{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n}\n"
-                ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
-}
-// completion of all MMAs issued so far -> the barrier at this shared-memory offset in BOTH CTAs of the pair
-__device__ __forceinline__ void umma_commit_pair (uint64_t *bar)
-{
-  asm volatile ("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32 (bar)), "h"((uint16_t) 3) : "memory");
-}

@@ -39,17 +39,8 @@ constexpr int kKSteps = 6;               // ceil ((128 + 48) / 32)
 constexpr int kBStep = 18 * 256;         // B bytes per K-step and rail: 18 row groups (3 digits x 48) x 2 chunks x 128 B
 constexpr int kRawRow = kSuper * 4 + 16;
 constexpr int kHistRow = kHist * 4 + 16;
-#ifndef SL_TXTC_RAIL_UNROLL
-#define SL_TXTC_RAIL_UNROLL 1
-#endif
-#ifndef SL_TXTC_MMA_UNROLL
-#define SL_TXTC_MMA_UNROLL 1                 /* rolled MMA loops: the kernel's instruction fetch sat at 88 % of the GPC cache's request rate (icc hit 84.6 %) */
-#endif
-constexpr int kMmaUnroll = SL_TXTC_MMA_UNROLL, kRailUnroll = SL_TXTC_RAIL_UNROLL;
-#ifndef SL_TXTC_RAWSTAGES
-#define SL_TXTC_RAWSTAGES 4
-#endif
-constexpr int kSets = 2, kEpiWarps = 4 * kSets, kConvWarps = 2, kRawStages = SL_TXTC_RAWSTAGES;   // raw stages: a bulk copy lands ~4000 clocks after it is issued
+constexpr int kMmaUnroll = 1, kRailUnroll = 1;  // rolled MMA loops: the kernel's instruction fetch sat at 88 % of the GPC cache's request rate (icc hit 84.6 %)
+constexpr int kSets = 2, kEpiWarps = 4 * kSets, kConvWarps = 2, kRawStages = 4;   // raw stages: a bulk copy lands ~4000 clocks after it is issued
 constexpr int kGroups = kChunksNew / 4;  // groups of 4 chunks (64 samples) of a supertile: 12; converter warp cw takes the groups t = cw (mod kConvWarps)
 constexpr int kMmaWarp = kEpiWarps + kConvWarps, kProdWarp = kMmaWarp + 1;
 constexpr int kThreads = 32 * (kProdWarp + 1);
