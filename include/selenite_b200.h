@@ -61,6 +61,9 @@ extern "C" {
 #define SLB_CHAIN_TX_Q15      8    /* all-mode integer transmitter: LSB, USB, CW, CW-R, DIG, PKT exactly as SLB_CHAIN_TX_SSB_Q15;
                                       AM (carrier + scaled audio) and FM (integer phase, table NCO) (DESIGN.md §3.9); bit-exact */
 
+#define SLB_CHAIN_CHAN64_Q15  9    /* all-integer channelizer, 192 kHz only: 64-branch arm_fir_q15 polyphase bank -> arm_cfft_q15 (64) -> per-bin
+                                      product or envelope detector -> q15 AGC -> pack (DESIGN.md §3.10); bit-exact */
+
 #define SLB_MAX_STAGES 4
 #define SLB_MAX_MASKS  8
 
@@ -187,6 +190,28 @@ typedef struct
   float fm_level;                        /* NCO amplitude (full scale 1) */
 } slb_tx_q15_mode_params;
 
+/* CHAN-64-q15 chain parameters (DESIGN.md §3.10), the integer sibling of slb_chan_params. Per wideband stream and hop of 64 frames:
+ *   branch r, rail I and rail Q separately: arm_fir_q15 with the 8 taps e_r[p] = proto[64 p + 63 - r] on the stride-64 commutated input
+ *   -> arm_cfft_q15 (64, forward, the Cortex-M4 branch, natural order) of the 64 branch outputs: bin k in 7.9 format (X / 64)
+ *   -> per bin: Re (product detector) or arm_cmplx_mag_q15 (envelope, 2.14) by SLB_DSP_Set_Mode (AM: envelope; FM is refused)
+ *   -> per block of agc_block narrowband samples: peak [arm_abs_q15 + arm_max_q15], the finite-window gain law of slb_rx_q15_params,
+ *      arm_scale_q15 -> int16 L = R in [stream][bin][hop][2], the layout of CHAN-64-f32.
+ * Geometry other than 64 / 8 / 3 or agc_window > 17 is refused with SLB_ERR_UNSUPPORTED and the parameters stay as they were.
+ * Defaults: CHAN-64-f32's Kaiser (beta 8) prototype scaled to DC gain 32 (llround to q15: no branch can saturate, an in-bin tone of
+ * amplitude A leaves the FFT at A / 2), and the AGC of RX-SSB-q15 (window 16, rel[j] = e^(-j/6), target 8192, floor 16, gmax 64). */
+typedef struct
+{
+  uint32_t bins;                         /* branches = FFT length = decimation [arm_cfft_q15]; this build: 64 */
+  uint32_t taps_per_branch;              /* [arm_fir_q15 numTaps per branch]; this build: 8 */
+  uint32_t agc_block;                    /* narrowband samples per AGC block (1 ms); this build: 3 */
+  uint32_t envelope;                     /* 0 = product detector (real part), 1 = envelope [arm_cmplx_mag_q15] */
+  int16_t  proto[SLB_CHAN_BINS * SLB_CHAN_TAPS];   /* prototype low-pass h[n], q15 */
+  uint32_t agc_window;                   /* blocks of peak history the envelope sees (finite release), 1..17 */
+  int16_t  rel[SLB_Q15_WIN];             /* q15 release weight of a block peak by age in blocks; rel[0] unused */
+  int16_t  agc_target, agc_floor;        /* q15 */
+  uint32_t agc_gmax_q15;                 /* gain limit in Q15 (1.0 = 32768) [arm_scale_q15 scaleFract << shift] */
+} slb_chan_q15_params;
+
 /* ---- life cycle ---- */
 int  slb_create (const slb_config *cfg, slb_ctx **out);
 void slb_destroy (slb_ctx *ctx);
@@ -286,6 +311,12 @@ int slb_set_chan_params (slb_ctx *ctx, const slb_chan_params *p);
 int slb_get_chan_params (const slb_ctx *ctx, slb_chan_params *p);
 int slb_chan_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream);
 int slb_chan_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames);
+/* CHAN-64-q15 (context created with SLB_CHAIN_CHAN64_Q15, fs 192000 only): slb_chan_process_* with the same shapes and rules; the debug
+ * taps are slb_rx_q15_set_debug_taps: d_audio int16 [streams][64][frames/64] (the pre-AGC detector output), d_gain uint32
+ * [streams][64][frames/192] (the Q15 gain word per block). Parameter calls on other contexts: SLB_ERR_STATE. */
+int slb_default_chan_q15_params (uint32_t fs, slb_chan_q15_params *out);
+int slb_set_chan_q15_params (slb_ctx *ctx, const slb_chan_q15_params *p);
+int slb_get_chan_q15_params (const slb_ctx *ctx, slb_chan_q15_params *p);
 /* optional float tap: post-biquad, pre-AGC audio [channels][frames] f32 and per-block gains [channels][frames/agc_block]
  * are written by the next slb_rx_process_device call(s) when non-NULL (device pointers). TX chain: d_audio receives
  * the pre-ALC complex baseband [channels][frames][2] f32. */

@@ -54,6 +54,12 @@ class ChanParams(C.Structure):
                 ("proto", C.c_float * 512)]
 
 
+class ChanQ15Params(C.Structure):
+    _fields_ = [("bins", C.c_uint32), ("taps_per_branch", C.c_uint32), ("agc_block", C.c_uint32), ("envelope", C.c_uint32),
+                ("proto", C.c_int16 * 512), ("agc_window", C.c_uint32), ("rel", C.c_int16 * 32),
+                ("agc_target", C.c_int16), ("agc_floor", C.c_int16), ("agc_gmax_q15", C.c_uint32)]
+
+
 # every symbol include/selenite_b200.h declares: name -> (restype, argtypes), derived from the header text so the
 # binding cannot drift from the ABI
 _P = C.c_void_p

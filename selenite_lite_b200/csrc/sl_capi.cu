@@ -40,6 +40,7 @@ struct slb_ctx
   std::vector<uint8_t> mode_host;      // [C]
   bool tx_mode = false;
   Chan64State *chan = nullptr;         // SLB_CHAIN_CHAN64_F32 only
+  ChanQ15State *chanq = nullptr;       // SLB_CHAIN_CHAN64_Q15 only
   RxQ15State *q15 = nullptr;           // SLB_CHAIN_RX_SSB_Q15, SLB_CHAIN_TX_SSB_Q15, SLB_CHAIN_RX_Q15 and SLB_CHAIN_TX_Q15 only
 
   // device: chain constants + carried state
@@ -112,6 +113,9 @@ static inline bool is_q15_chain (uint32_t chain)
 {
   return chain == SLB_CHAIN_RX_SSB_Q15 || chain == SLB_CHAIN_TX_SSB_Q15 || chain == SLB_CHAIN_RX_Q15 || chain == SLB_CHAIN_TX_Q15;
 }
+
+// the two channelizers: wideband streams in, bulk calls only (no firmware ring, no single-channel path)
+static inline bool is_chan (const slb_ctx *ctx) { return ctx->chan || ctx->chanq; }
 
 static int fail (slb_ctx *ctx, int code, const char *msg) { if (ctx) ctx->err = msg; else g_create_error = msg; return code; }
 
@@ -276,6 +280,7 @@ static int reset_state (slb_ctx *ctx)
   ctx->ring_pc = false;
   if (ctx->d_key) { CK (ctx, cudaMemset (ctx->d_key, 0, C)); CK (ctx, cudaMemset (ctx->d_tone_cnt, 0, (size_t) C * 4)); ctx->any_key = false; }
   if (ctx->chan) return chan64_reset (ctx, ctx->chan);
+  if (ctx->chanq) return chanq15_reset (ctx, ctx->chanq);
   if (ctx->q15) return rxq15_reset (ctx, ctx->q15);
   return SLB_OK;
 }
@@ -297,7 +302,9 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   *out = nullptr;
   if (cfg->channels == 0) return fail (nullptr, SLB_ERR_ARG, "channels must be > 0");
   if (cfg->fs != 48000u && cfg->fs != 96000u && cfg->fs != 192000u) return fail (nullptr, SLB_ERR_ARG, "fs must be 48000, 96000 or 192000");
-  if (cfg->chain != SLB_CHAIN_PASS && !is_ssb_chain (cfg->chain) && cfg->chain != SLB_CHAIN_CHAN64_F32 && !is_q15_chain (cfg->chain)) return fail (nullptr, SLB_ERR_ARG, "unknown chain");
+  if (cfg->chain != SLB_CHAIN_PASS && !is_ssb_chain (cfg->chain) && cfg->chain != SLB_CHAIN_CHAN64_F32 && cfg->chain != SLB_CHAIN_CHAN64_Q15 && !is_q15_chain (cfg->chain))
+    return fail (nullptr, SLB_ERR_ARG, "unknown chain");
+  if (cfg->chain == SLB_CHAIN_CHAN64_Q15 && cfg->fs != 192000u) return fail (nullptr, SLB_ERR_ARG, "the integer channelizer takes 192 kHz wideband streams only");
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount (&ndev);
   if (e != cudaSuccess || ndev == 0)
@@ -348,6 +355,7 @@ int slb_create (const slb_config *cfg, slb_ctx **out)
   int rc = upload_chain_constants (ctx);
   if (rc == SLB_OK) rc = reset_state (ctx);
   if (rc == SLB_OK && cfg->chain == SLB_CHAIN_CHAN64_F32) rc = chan64_create (ctx, C, cfg->fs, &ctx->chan);
+  if (rc == SLB_OK && cfg->chain == SLB_CHAIN_CHAN64_Q15) rc = chanq15_create (ctx, C, cfg->fs, &ctx->chanq);
   if (rc == SLB_OK && is_q15_chain (cfg->chain)) rc = rxq15_create (ctx, C, cfg->fs, is_tx_direction (cfg->chain), cfg->chain == SLB_CHAIN_RX_Q15 || cfg->chain == SLB_CHAIN_TX_Q15, &ctx->q15);
   if (rc != SLB_OK) { g_create_error = ctx->err; slb_destroy (ctx); return rc; }
   *out = ctx;
@@ -360,6 +368,7 @@ void slb_destroy (slb_ctx *ctx)
   cudaSetDevice (ctx->cfg.device);
   cudaDeviceSynchronize ();
   chan64_destroy (ctx->chan);
+  chanq15_destroy (ctx->chanq);
   rxq15_destroy (ctx->q15);
   cudaFree (ctx->d_masks); cudaFree (ctx->d_slot); cudaFree (ctx->d_twiddle); cudaFree (ctx->d_planes); cudaFree (ctx->d_tx_planes); cudaFree (ctx->d_am_planes);
   drop_lists (ctx, ctx->tc_lists, 0); drop_lists (ctx, ctx->tune_lists, 0); drop_lists (ctx, ctx->q15_lists, 0);
@@ -511,6 +520,7 @@ int slb_get_tx_q15_mode_params (const slb_ctx *ctx, slb_tx_q15_mode_params *p)
 }
 int slb_rx_q15_set_debug_taps (slb_ctx *ctx, int16_t *d_audio, uint32_t *d_gain)
 {
+  if (ctx && ctx->chanq) { chanq15_set_debug (ctx->chanq, d_audio, d_gain); return SLB_OK; }
   if (!ctx || !ctx->q15) return SLB_ERR_ARG;
   rxq15_set_debug (ctx->q15, d_audio, d_gain);
   return SLB_OK;
@@ -619,7 +629,7 @@ static int switch_direction (slb_ctx *ctx, bool tx)
 {
   if (ctx->tx_mode == tx) return SLB_OK;                                                   // ptt_set_tx / ptt_set_rx act on a change only
   ctx->tx_mode = tx;
-  if (ctx->chan) return SLB_OK;                                                            // the channelizer has no firmware rings
+  if (is_chan (ctx)) return SLB_OK;                                                        // the channelizers have no firmware rings
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   { const int rc = clear_chain_state (ctx); if (rc) return rc; }
   if (ctx->q15) return rxq15_reset (ctx, ctx->q15);
@@ -633,7 +643,7 @@ int slb_get_direction (const slb_ctx *ctx) { return ctx ? (ctx->tx_mode ? 1 : 0)
 int SLB_DSP_Set_Sidetone (slb_ctx *ctx, uint32_t freq_hz, float level)
 {
   if (!ctx) return SLB_ERR_ARG;
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chains have no firmware ring (bulk calls only)");
   if (freq_hz >= ctx->cfg.fs / 2 || !(level >= 0.f) || !(level < 1.0f)) return fail (ctx, SLB_ERR_ARG, "side-tone: 0 <= freq < fs / 2, 0 <= level < 1");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   const uint32_t C = ctx->cfg.channels, fs = ctx->cfg.fs;
@@ -708,6 +718,15 @@ int SLB_DSP_Set_Mode (slb_ctx *ctx, uint8_t mode)     // dsp_if.c:367-370 is the
     p.envelope = (mode == SLB_MODE_AM) ? 1u : 0u;
     CK (ctx, cudaSetDevice (ctx->cfg.device));
     return chan64_set_params (ctx, ctx->chan, &p);
+  }
+  if (ctx->chanq)
+  {
+    if (mode == SLB_MODE_FM) return fail (ctx, SLB_ERR_UNSUPPORTED, "no FM discriminator in the channelizer chain");
+    slb_chan_q15_params p = *chanq15_params (ctx->chanq);
+    p.envelope = (mode == SLB_MODE_AM) ? 1u : 0u;
+    CK (ctx, cudaSetDevice (ctx->cfg.device));
+    CK (ctx, cudaDeviceSynchronize ());
+    return chanq15_set_params (ctx, ctx->chanq, &p);
   }
   const int slot = mode_to_mask_slot (mode);
   { const int rc = check_mode (ctx, mode); if (rc) return rc; }
@@ -984,7 +1003,7 @@ static int ring_pc_mask (slb_ctx *ctx, const uint8_t *active, const uint8_t **d_
 
 static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_t frames, const uint8_t *active = nullptr, bool per_channel = false)
 {
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chains have no firmware ring (bulk calls only)");
   const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames;
   if (!pbuf || frames == 0 || frames + 1 > R) return fail (ctx, SLB_ERR_ARG, "block must hold 1..DSP_BUFF_SIZE-1 frames");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
@@ -1115,7 +1134,7 @@ static int ring_write_common (slb_ctx *ctx, int which, const void *pbuf, uint32_
 
 static int ring_read_common (slb_ctx *ctx, int which, void *pbuf, uint32_t frames, const uint8_t *active = nullptr, bool per_channel = false)
 {
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chains have no firmware ring (bulk calls only)");
   const uint32_t C = ctx->cfg.channels, R = ctx->geo.ring_frames;
   if (!pbuf || frames == 0) return fail (ctx, SLB_ERR_ARG, "empty read");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
@@ -1204,7 +1223,7 @@ int SLB_AUDIO_AudioCmd (slb_ctx *ctx, uint8_t *pbuf, uint32_t size, uint8_t cmd)
 // takes whole super-blocks
 static int check_feeder (slb_ctx *ctx, bool with_rx, uint32_t ticks)
 {
-  if (ctx->chan) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chain has no firmware ring (bulk calls only)");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_UNSUPPORTED, "the channelizer chains have no firmware ring (bulk calls only)");
   if (ctx->ring_pc) return fail (ctx, SLB_ERR_STATE, "the feeder replays one shared cadence; per-channel cadence is on");
   if (with_rx && is_ssb_chain (ctx->cfg.chain) && (ticks % (ctx->rx.hop / ctx->geo.block_frames) != 0 || ctx->acc_fill != 0))
     return fail (ctx, SLB_ERR_ARG, "with an FFT chain the feeder moves whole 384-frame super-blocks (ticks % 8 == 0)");
@@ -1550,7 +1569,7 @@ int slb_biquad_tc_tables (const float coef10[10], float *Mp64, float *M192, floa
 static int process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream, bool want_tx)
 {
   if (!ctx || !d_in || !d_out || frames == 0) return SLB_ERR_ARG;
-  if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
   if (want_tx != is_tx_direction (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   if (ctx->cfg.chain == SLB_CHAIN_PASS)
@@ -1690,7 +1709,7 @@ static int process_host_sliced (slb_ctx *ctx, const int16_t *h_in, int16_t *h_ou
 static int process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames, bool want_tx)
 {
   if (!ctx || !h_in || !h_out || frames == 0) return SLB_ERR_ARG;
-  if (ctx->chan) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
+  if (is_chan (ctx)) return fail (ctx, SLB_ERR_STATE, "channelizer context: use slb_chan_process_*");
   if (want_tx != is_tx_direction (ctx->cfg.chain)) return fail (ctx, SLB_ERR_STATE, "context was created for the other direction (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   const bool chain = is_ssb_chain (ctx->cfg.chain);
@@ -1708,7 +1727,7 @@ int slb_rx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint
 int slb_tx_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames) { return process_host (ctx, h_in, h_out, frames, true); }
 
 // ------------------------------------------------------------------------------------------------------------------
-// Channelizer bulk path (SLB_CHAIN_CHAN64_F32)
+// Channelizer bulk path (SLB_CHAIN_CHAN64_F32, SLB_CHAIN_CHAN64_Q15)
 // ------------------------------------------------------------------------------------------------------------------
 int slb_default_chan_params (uint32_t fs, slb_chan_params *out) { return design_default_chan (fs, out); }
 int slb_set_chan_params (slb_ctx *ctx, const slb_chan_params *p)
@@ -1725,11 +1744,34 @@ int slb_get_chan_params (const slb_ctx *ctx, slb_chan_params *p)
   *p = *chan64_params (ctx->chan);
   return SLB_OK;
 }
+int slb_default_chan_q15_params (uint32_t fs, slb_chan_q15_params *out) { return design_default_chan_q15 (fs, out); }
+int slb_set_chan_q15_params (slb_ctx *ctx, const slb_chan_q15_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->chanq) return fail (ctx, SLB_ERR_STATE, "not a CHAN-64-q15 context");
+  CK (ctx, cudaSetDevice (ctx->cfg.device));
+  CK (ctx, cudaDeviceSynchronize ());
+  return chanq15_set_params (ctx, ctx->chanq, p);
+}
+int slb_get_chan_q15_params (const slb_ctx *ctx, slb_chan_q15_params *p)
+{
+  if (!ctx || !p) return SLB_ERR_ARG;
+  if (!ctx->chanq) return SLB_ERR_STATE;
+  *p = *chanq15_params (ctx->chanq);
+  return SLB_OK;
+}
 int slb_chan_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, uint32_t frames, void *stream)
 {
   if (!ctx || !d_in || !d_out || frames == 0) return SLB_ERR_ARG;
-  if (!ctx->chan) return fail (ctx, SLB_ERR_STATE, "not a channelizer context (cfg.chain)");
+  if (!is_chan (ctx)) return fail (ctx, SLB_ERR_STATE, "not a channelizer context (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
+  if (ctx->chanq)
+  {
+    const int rc = chanq15_launch (ctx, ctx->chanq, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->sm_count, stream, true);
+    if (rc) return rc;
+    chanq15_advance (ctx->chanq);
+    return SLB_OK;
+  }
   int rc = chan64_launch (ctx, ctx->chan, d_in, d_out, 0, ctx->cfg.channels, frames, ctx->sm_count, stream, true);
   if (rc) return rc;
   chan64_advance (ctx->chan);
@@ -1738,14 +1780,15 @@ int slb_chan_process_device (slb_ctx *ctx, const int16_t *d_in, int16_t *d_out, 
 int slb_chan_process_host (slb_ctx *ctx, const int16_t *h_in, int16_t *h_out, uint32_t frames)
 {
   if (!ctx || !h_in || !h_out || frames == 0) return SLB_ERR_ARG;
-  if (!ctx->chan) return fail (ctx, SLB_ERR_STATE, "not a channelizer context (cfg.chain)");
+  if (!is_chan (ctx)) return fail (ctx, SLB_ERR_STATE, "not a channelizer context (cfg.chain)");
   CK (ctx, cudaSetDevice (ctx->cfg.device));
   // (a stream takes as many bytes out as in: 64 bins x frames/64 x 4 B)
   const int rc = process_host_groups (ctx, h_in, h_out, frames, [&] (const int16_t *d_in, int16_t *d_out, uint32_t s0, uint32_t n, cudaStream_t st) {
-    return chan64_launch (ctx, ctx->chan, d_in, d_out, s0, n, frames, ctx->sm_count, st, false);
+    return ctx->chanq ? chanq15_launch (ctx, ctx->chanq, d_in, d_out, s0, n, frames, ctx->sm_count, st, false)
+                      : chan64_launch (ctx, ctx->chan, d_in, d_out, s0, n, frames, ctx->sm_count, st, false);
   });
   if (rc) return rc;
-  chan64_advance (ctx->chan);
+  if (ctx->chanq) chanq15_advance (ctx->chanq); else chan64_advance (ctx->chan);
   return SLB_OK;
 }
 
@@ -1780,7 +1823,7 @@ static size_t state_bytes (const slb_ctx *ctx)
   const size_t C = ctx->cfg.channels;
   size_t n = sizeof (StateHeader) + C /*modes*/;
   for (const StateSection &s : state_sections (ctx)) n += s.bytes;
-  return n + (ctx->chan ? chan64_state_bytes (ctx->chan) : 0) + (ctx->q15 ? rxq15_state_bytes (ctx->q15) : 0) + 2 * C * 4 * sizeof (uint32_t) /* per-channel ring pointers */;
+  return n + (ctx->chan ? chan64_state_bytes (ctx->chan) : 0) + (ctx->chanq ? chanq15_state_bytes (ctx->chanq) : 0) + (ctx->q15 ? rxq15_state_bytes (ctx->q15) : 0) + 2 * C * 4 * sizeof (uint32_t) /* per-channel ring pointers */;
 }
 int slb_state_size (const slb_ctx *ctx, size_t *bytes) { if (!ctx || !bytes) return SLB_ERR_ARG; *bytes = state_bytes (ctx); return SLB_OK; }
 
@@ -1801,6 +1844,7 @@ int slb_state_save (slb_ctx *ctx, void *buf, size_t bytes)
   std::memcpy (p, ctx->mode_host.data (), C); p += C;
   for (const StateSection &s : state_sections (ctx)) { CK (ctx, cudaMemcpy (p, s.d, s.bytes, cudaMemcpyDeviceToHost)); p += s.bytes; }
   if (ctx->chan) { CK (ctx, cudaDeviceSynchronize ()); if (chan64_state_save (ctx->chan, p)) return fail (ctx, SLB_ERR_CUDA, "chan64 state save failed"); p += chan64_state_bytes (ctx->chan); }
+  if (ctx->chanq) { CK (ctx, cudaDeviceSynchronize ()); if (chanq15_state_save (ctx->chanq, p)) return fail (ctx, SLB_ERR_CUDA, "chan64-q15 state save failed"); p += chanq15_state_bytes (ctx->chanq); }
   if (ctx->q15) { CK (ctx, cudaDeviceSynchronize ()); if (rxq15_state_save (ctx->q15, p)) return fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state save failed"); p += rxq15_state_bytes (ctx->q15); }
   for (int w = 0; w < 2; w++)
   {
@@ -1831,6 +1875,7 @@ int slb_state_load (slb_ctx *ctx, const void *buf, size_t bytes)
   ctx->ovl_parity = 0; ctx->proc_cur = 0;
   for (const StateSection &s : state_sections (ctx)) { CK (ctx, cudaMemcpy (s.d, p, s.bytes, cudaMemcpyHostToDevice)); p += s.bytes; }
   if (ctx->chan) { CK (ctx, cudaDeviceSynchronize ()); if (chan64_state_load (ctx->chan, p)) return fail (ctx, SLB_ERR_CUDA, "chan64 state load failed"); p += chan64_state_bytes (ctx->chan); }
+  if (ctx->chanq) { CK (ctx, cudaDeviceSynchronize ()); if (chanq15_state_load (ctx->chanq, p)) return fail (ctx, SLB_ERR_CUDA, "chan64-q15 state load failed"); p += chanq15_state_bytes (ctx->chanq); }
   if (ctx->q15) { CK (ctx, cudaDeviceSynchronize ()); if (rxq15_state_load (ctx->q15, p)) return fail (ctx, SLB_ERR_CUDA, "RX-SSB-q15 state load failed"); p += rxq15_state_bytes (ctx->q15); }
   ctx->ring_pc = false;
   if (h.ring_pc)

@@ -158,6 +158,25 @@ int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p)
   return SLB_OK;
 }
 
+// CHAN-64-q15 (DESIGN.md §3.10): CHAN-64-f32's prototype at DC gain 32, llround to q15. Every branch then sums to about 0.5 (at most
+// 0.75 in absolute value), so no branch FIR saturates and an in-bin tone of amplitude A leaves the FFT (which divides by 64) at A / 2;
+// at DC gain 1 the branch outputs would lose 6 bits. The AGC is RX-SSB-q15's.
+int design_default_chan_q15 (uint32_t fs, slb_chan_q15_params *p)
+{
+  if (!p) return SLB_ERR_ARG;
+  if (fs != 192000u) return SLB_ERR_UNSUPPORTED;
+  std::memset (p, 0, sizeof *p);
+  p->bins = SLB_CHAN_BINS; p->taps_per_branch = SLB_CHAN_TAPS; p->agc_block = 3; p->envelope = 0;
+  double h[SLB_CHAN_BINS * SLB_CHAN_TAPS];
+  chan_prototype (h);
+  for (int i = 0; i < SLB_CHAN_BINS * SLB_CHAN_TAPS; i++) p->proto[i] = (int16_t) std::llround (32.0 * 32768.0 * h[i]);
+  slb_rx_q15_params q;
+  design_default_rx_q15 (48000u, &q);
+  p->agc_window = q.agc_window; std::memcpy (p->rel, q.rel, sizeof p->rel);
+  p->agc_target = q.agc_target; p->agc_floor = q.agc_floor; p->agc_gmax_q15 = q.agc_gmax_q15;
+  return SLB_OK;
+}
+
 // RX-Q15's AM and FM detectors: 64-tap Kaiser (beta 6) windowed-sinc low-passes with the cut-off (-6 dB) at 3 kHz (AM) and 6 kHz
 // (FM), normalised to DC gain 1 in double, then llround to q15 (both rails use the same taps)
 int design_default_rx_q15_modes (uint32_t fs, slb_rx_q15_mode_params *p)

@@ -28,29 +28,7 @@ namespace sl {
 
 namespace {
 
-// ------------------------------------------------------------------ q15 lane arithmetic ------------------------------------------------------------------
-struct C16 { int x, y; };                                                   // one complex q15 sample, lanes sign-extended
-__device__ __forceinline__ int sat16 (int v) { return max (-32768, min (32767, v)); }
-__device__ __forceinline__ C16 unpack16 (uint32_t w) { return C16{ (int) (int16_t) (w & 0xFFFFu), (int) (int16_t) (w >> 16) }; }
-__device__ __forceinline__ uint32_t pack16 (C16 v) { return ((uint32_t) v.x & 0xFFFFu) | ((uint32_t) v.y << 16); }
-__device__ __forceinline__ C16 shr (C16 a, int s) { return C16{ a.x >> s, a.y >> s }; }
-__device__ __forceinline__ C16 qadd (C16 a, C16 b) { return C16{ sat16 (a.x + b.x), sat16 (a.y + b.y) }; }            // __QADD16
-__device__ __forceinline__ C16 qsub (C16 a, C16 b) { return C16{ sat16 (a.x - b.x), sat16 (a.y - b.y) }; }            // __QSUB16
-__device__ __forceinline__ C16 hadd (C16 a, C16 b) { return C16{ (a.x + b.x) >> 1, (a.y + b.y) >> 1 }; }              // __SHADD16
-__device__ __forceinline__ C16 hsub (C16 a, C16 b) { return C16{ (a.x - b.x) >> 1, (a.y - b.y) >> 1 }; }              // __SHSUB16
-// a - j b and a + j b on the lanes: __QASX (re - im', im + re'), __QSAX (re + im', im - re'), and their halving forms
-__device__ __forceinline__ C16 qasx (C16 a, C16 b) { return C16{ sat16 (a.x - b.y), sat16 (a.y + b.x) }; }
-__device__ __forceinline__ C16 qsax (C16 a, C16 b) { return C16{ sat16 (a.x + b.y), sat16 (a.y - b.x) }; }
-__device__ __forceinline__ C16 hasx (C16 a, C16 b) { return C16{ (a.x - b.y) >> 1, (a.y + b.x) >> 1 }; }
-__device__ __forceinline__ C16 hsax (C16 a, C16 b) { return C16{ (a.x + b.y) >> 1, (a.y - b.x) >> 1 }; }
-// twiddle product, truncated to the high half-word of the wrapping 32-bit sums: forward v * (co - j si) = __SMUAD >> 16 | __SMUSDX,
-// inverse v * (co + j si) = __SMUSD >> 16 | __SMUADX
-template <bool INV> __device__ __forceinline__ C16 twid (C16 c, C16 v)
-{
-  const uint32_t xx = (uint32_t) (c.x * v.x), yy = (uint32_t) (c.y * v.y), xy = (uint32_t) (c.x * v.y), yx = (uint32_t) (c.y * v.x);
-  const int re = (int) (INV ? xx - yy : xx + yy), im = (int) (INV ? xy + yx : xy - yx);
-  return C16{ re >> 16, im >> 16 };
-}
+#include "sl_q15.cuh"
 
 // one radix-4 transform of length L at s[0..L), twiddle index step m0 (1: own table, 2: half of a radix-4-by-2 transform)
 template <bool INV> __device__ void radix4_q15 (uint32_t *s, int L, int m0, const uint32_t *__restrict__ tw, int b0, int nb, int tid, int nthreads)

@@ -212,6 +212,23 @@ int chan64_launch (slb_ctx *ctx, Chan64State *st, const int16_t *d_in, int16_t *
                    int sm_count, void *stream, bool with_debug);
 void chan64_advance (Chan64State *st);
 
+// ---- CHAN-64-q15 (sl_chan64_q15.cu): state object owned by the context ----
+void chan_prototype (double *h /* [SLB_CHAN_BINS * SLB_CHAN_TAPS] */);   // CHAN-64-f32's default low-pass, DC gain 1 (sl_chan64.cu)
+struct ChanQ15State;
+int design_default_chan_q15 (uint32_t fs, slb_chan_q15_params *p);
+int chanq15_create (slb_ctx *ctx, uint32_t streams, uint32_t fs, ChanQ15State **out);
+void chanq15_destroy (ChanQ15State *st);
+int chanq15_reset (slb_ctx *ctx, ChanQ15State *st);
+int chanq15_set_params (slb_ctx *ctx, ChanQ15State *st, const slb_chan_q15_params *p);
+const slb_chan_q15_params *chanq15_params (const ChanQ15State *st);
+void chanq15_set_debug (ChanQ15State *st, int16_t *audio, uint32_t *gain);
+size_t chanq15_state_bytes (const ChanQ15State *st);
+int chanq15_state_save (ChanQ15State *st, char *dst);
+int chanq15_state_load (ChanQ15State *st, const char *src);
+int chanq15_launch (slb_ctx *ctx, ChanQ15State *st, const int16_t *d_in, int16_t *d_out, uint32_t s0, uint32_t ns, uint32_t frames,
+                    int sm_count, void *stream, bool with_debug);
+void chanq15_advance (ChanQ15State *st);
+
 // ---- RX-SSB-q15 and TX-SSB-q15 (sl_rx_ssb_q15.cu): state object owned by the context ----
 struct RxQ15State;
 int design_default_rx_q15 (uint32_t fs, slb_rx_q15_params *p);

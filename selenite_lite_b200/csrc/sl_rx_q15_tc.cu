@@ -102,30 +102,7 @@ struct KParams
 #include "sl_nco.cuh"
 
 // (cvt.sat.s16.s32 is one instruction but runs on the conversion pipe: 403 vs 467 Gsamples/s. Raw stages with the MMA issue loop rolled: 2 -> 475, 3 -> 486, 4 -> 489 Gsamples/s; with it unrolled 468 .. 470 whatever the stages)
-__device__ __forceinline__ int sat16 (int v) { return max (-32768, min (32767, v)); }
-
-// arm_sqrt_q15 (FastMathFunctions/arm_sqrt_q15.c) as oracle/port/stats_cmplx.c restates it, every cast included: normalise by an even
-// shift, a float seed (a power-of-two multiply, the 0x5f3759df bit trick), three q15 Newton steps, multiply back, undo half the shift
-__device__ __forceinline__ int sqrt_q15 (int number)
-{
-  if (number <= 0) return 0;
-  const int sh = (__clz (number) - 17) & ~1;                                      // signBits1, or signBits1 - 1 when it is odd
-  number = (int) (int16_t) (number << sh);
-  const int half = number >> 1, temp1 = number;
-  const float tf = __int_as_float (0x5f3759df - (__float_as_int ((float) number * 3.051757812500000e-005f) >> 1));
-  int var1 = (int) (int16_t) (int) (tf * 16384.0f);
-#pragma unroll
-  for (int it = 0; it < 3; it++)
-  {
-    const int sq = (int) (int16_t) ((var1 * var1) >> 15);
-    const int hs = (int) (int16_t) ((sq * half) >> 15);
-    var1 = (int) (int16_t) ((int) (int16_t) ((var1 * (0x3000 - hs)) >> 15) << 2);
-  }
-  var1 = (int) (int16_t) ((int) (int16_t) ((temp1 * var1) >> 15) << 1);
-  return var1 >> (sh / 2);
-}
-// arm_cmplx_mag_q15 (arm_cmplx_mag_q15.c): sqrt_q15 ((re^2 + im^2) >> 17), 2.14 format
-__device__ __forceinline__ int cmag_q15 (int re, int im) { return sqrt_q15 ((int) (((unsigned) (re * re) + (unsigned) (im * im)) >> 17)); }
+#include "sl_q15.cuh"
 // the limiter-discriminator (ours, DESIGN.md §3.8): sat16 (trunc ((x 2^13) / max (m_prev m, floor))), x = a_prev b - b_prev a. |quotient|
 // < 2^15 unless it saturates, so a float reciprocal estimate is within one of it and one integer correction makes it exact
 __device__ __forceinline__ int fm_disc (int pa, int pb, int pm, int a, int b, int m, int floor_)

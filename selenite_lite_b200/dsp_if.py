@@ -11,6 +11,7 @@ import numpy as np
 from . import _lib
 
 CHAIN_PASS, CHAIN_RX_SSB_F32, CHAIN_TX_SSB_F32, CHAIN_CHAN64_F32, CHAIN_RX_SSB_Q15, CHAIN_TX_F32, CHAIN_TX_SSB_Q15, CHAIN_RX_Q15, CHAIN_TX_Q15 = 0, 1, 2, 3, 4, 5, 6, 7, 8
+CHAIN_CHAN64_Q15 = 9
 MODE_LSB, MODE_USB, MODE_CW, MODE_CWR, MODE_AM, MODE_FM, MODE_DIG, MODE_PKT = 0x00, 0x01, 0x02, 0x03, 0x04, 0x08, 0x0A, 0x0C
 RX_PATH_AUTO, RX_PATH_FFT = 0, 1
 
@@ -67,6 +68,21 @@ def chan_params_to_dict(p):
     return dict(bins=p.bins, taps_per_branch=p.taps_per_branch, agc_block=p.agc_block, envelope=p.envelope,
                 agc_target=p.agc_target, agc_decay=p.agc_decay, agc_floor=p.agc_floor, agc_gmax=p.agc_gmax,
                 proto=np.array(p.proto[:p.bins * p.taps_per_branch], np.float32))
+
+
+def default_chan_q15_params(fs=192000):
+    p = _lib.ChanQ15Params()
+    rc = _lib.load().slb_default_chan_q15_params(fs, C.byref(p))
+    if rc:
+        raise SeleniteError("slb_default_chan_q15_params -> %d" % rc)
+    return p
+
+
+def chan_q15_params_to_dict(p):
+    """CHAN-64-q15 parameters as plain data (the oracle's chan_q15 parameters)."""
+    return dict(bins=p.bins, taps_per_branch=p.taps_per_branch, agc_block=p.agc_block, envelope=p.envelope,
+                proto=np.array(p.proto[:], np.int16), agc_window=p.agc_window, rel=np.array(p.rel[:], np.int16),
+                agc_target=p.agc_target, agc_floor=p.agc_floor, agc_gmax_q15=p.agc_gmax_q15)
 
 
 def default_rx_q15_params(fs=48000):
@@ -389,6 +405,13 @@ class DspIf:
 
     def set_chan_params(self, p): self._ck(self.lib.slb_set_chan_params(self.h, C.byref(p)), "set_chan_params")
 
+    def chan_q15_params(self):
+        p = _lib.ChanQ15Params()
+        self._ck(self.lib.slb_get_chan_q15_params(self.h, C.byref(p)), "get_chan_q15_params")
+        return p
+
+    def set_chan_q15_params(self, p): self._ck(self.lib.slb_set_chan_q15_params(self.h, C.byref(p)), "set_chan_q15_params")
+
     def rx_q15_params(self):
         p = _lib.RxQ15Params()
         self._ck(self.lib.slb_get_rx_q15_params(self.h, C.byref(p)), "get_rx_q15_params")
@@ -412,7 +435,8 @@ class DspIf:
 
     def set_q15_debug_taps(self, audio=None, gain=None):
         """audio: torch CUDA int16 [channels][frames] (RX-SSB-q15: pre-AGC audio) or [channels][frames][2] (TX-SSB-q15, TX-Q15: pre-ALC I/Q);
-        gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block)."""
+        gain: torch CUDA int32 [channels][frames/48] (Q15 gain per block). CHAN-64-q15: audio int16 [streams][64][frames/64] (pre-AGC detector
+        output), gain int32 [streams][64][frames/192]."""
         self._keep_taps = (audio, gain)
         self._ck(self.lib.slb_rx_q15_set_debug_taps(self.h, audio.data_ptr() if audio is not None else None,
                                                     gain.data_ptr() if gain is not None else None), "rx_q15_set_debug_taps")
@@ -426,6 +450,8 @@ class DspIf:
             return q15_params_to_dict(self.rx_q15_params(), lsb=mode in (MODE_LSB, MODE_CWR))
         if self.chain == CHAIN_CHAN64_F32:
             return chan_params_to_dict(self.chan_params())
+        if self.chain == CHAIN_CHAN64_Q15:
+            return chan_q15_params_to_dict(self.chan_q15_params())
         if self.chain == CHAIN_TX_F32 and mode in (MODE_AM, MODE_FM):
             return tx_mod_params_to_dict(self.tx_params(), self.tx_mod_params(), self.mask(mode), self.fs, mode)
         if self.chain in (CHAIN_TX_SSB_F32, CHAIN_TX_F32):
@@ -458,7 +484,7 @@ class DspIf:
         return self.rx_process(x, out, stream, _dir="tx")
 
     def chan_process(self, x, out=None, stream=None):
-        """Channelizer (context created with CHAIN_CHAN64_F32): x int16 [streams][frames][2] wideband I/Q ->
+        """Channelizer (context created with CHAIN_CHAN64_F32 or CHAIN_CHAN64_Q15): x int16 [streams][frames][2] wideband I/Q ->
         int16 [streams][64][frames/64][2] demodulated narrowband audio (L = R), channel-major."""
         if isinstance(x, np.ndarray):
             x = np.ascontiguousarray(x, np.int16)

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Device-resident throughput of the chains that are not the headline bench line (TX-SSB-f32 = config 3,
-CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, TX-SSB-q15, RX-Q15 AM / FM, TX-Q15 AM / FM, tuned channels).
+CHAN-64-f32 = config 4, RX at other widths, TX AM / FM, TX-SSB-q15, RX-Q15 AM / FM, TX-Q15 AM / FM, tuned channels, CHAN-64-q15).
 Prints one JSON line per chain after a line naming the card, its power limit and the HBM copy rate measured in the same run
 (hbm_frac_measured divides by that). Profiling aid, not the bench contract."""
 import argparse
@@ -82,6 +82,16 @@ def main():
             x = torch.randint(-3000, 3000, (S, T, 2), dtype=torch.int16, device=dev, generator=g)
             d = slb.DspIf(S, fs=192000, chain=slb.CHAIN_CHAN64_F32); y = torch.empty((S, 64, T // 64, 2), dtype=torch.int16, device=dev)
             ms = timeit(lambda: d.chan_process(x, y), args.steps); n = S * T; name = "chan64_f32 (config 4: 64 x 192 kHz streams -> 4096 channels, %d s)" % args.seconds
+        elif which in ("chan64_q15", "chan64_q15_1024", "chan_1024"):
+            # CHAN-64-q15 (DESIGN.md §3.10) at config 4's width and at 1024 streams; chan_1024 = CHAN-64-f32 at 1024 streams beside it
+            S, T = (1024 if which.endswith("1024") else 64), 192000 * args.seconds // 768 * 768
+            x = torch.randint(-3000, 3000, (S, T, 2), dtype=torch.int16, device=dev, generator=g)
+            q15 = which.startswith("chan64_q15")
+            d = slb.DspIf(S, fs=192000, chain=slb.CHAIN_CHAN64_Q15 if q15 else slb.CHAIN_CHAN64_F32)
+            y = torch.empty((S, 64, T // 64, 2), dtype=torch.int16, device=dev)
+            ms = timeit(lambda: d.chan_process(x, y), args.steps); n = S * T
+            name = "%s (%d x 192 kHz streams -> %d channels, %d s)" % ("chan64_q15" if q15 else "chan64_f32", S, 64 * S, args.seconds)
+            del x, y
         elif which == "q15":
             C, T = args.rx_channels, 48000 * args.seconds
             x = torch.randint(-8000, 8000, (C, T, 2), dtype=torch.int16, device=dev, generator=g)
