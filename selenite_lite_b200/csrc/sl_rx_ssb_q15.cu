@@ -141,8 +141,10 @@ __global__ void __launch_bounds__ (kThreads, 4) rx_ssb_q15_kernel (const __grid_
     const bool ok0 = ch_o0 < P.channels, ok1 = ch_o1 < P.channels;
     const uint32_t b_emit = seg * P.seg_blocks;                                  // first block this item writes
     const uint32_t b_end = min (P.blocks, b_emit + P.seg_blocks);
-    // blocks re-derived (not stored) so that the peak window of block b_emit is complete; whole chunks only
-    uint32_t b_first = (b_emit >= (uint32_t) (window - 1)) ? b_emit - (uint32_t) (window - 1) : 0u;
+    // blocks re-derived (not stored) so that the peak window of block b_emit is complete; whole chunks only. The segment that ends
+    // the call reaches back kWin - 1 blocks whatever the window: it carries every age to the next call, whose window may be longer
+    const uint32_t reach = (b_end == P.blocks) ? (uint32_t) (kWin - 1) : (uint32_t) (window - 1);
+    uint32_t b_first = (b_emit >= reach) ? b_emit - reach : 0u;
     b_first -= b_first % kChunkBlocks;
     const bool sub0 = ok0 && P.lsb[ch_o0], sub1 = ok1 && P.lsb[ch_o1];
 
